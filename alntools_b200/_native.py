@@ -37,15 +37,6 @@ class EcbResult(ctypes.Structure):
     ]
 
 
-class EcbExport(ctypes.Structure):
-    _fields_ = [
-        ("n_ec", ctypes.c_int64), ("n_rows", ctypes.c_int64),
-        ("meta", ctypes.POINTER(ctypes.c_int64)), ("rows", _i32p),
-        ("part_ec_counts", ctypes.POINTER(ctypes.c_int64)), ("part_row_counts", ctypes.POINTER(ctypes.c_int64)),
-        ("min_base", ctypes.c_int64), ("max_end", ctypes.c_int64),
-    ]
-
-
 class EcbStats(ctypes.Structure):
     _fields_ = [
         ("group_ms", ctypes.c_double), ("harvest_ms", ctypes.c_double),
@@ -90,17 +81,6 @@ SIGNATURES = {
     "ecb_get_stats": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbStats)]),
     "ecb_destroy": (ctypes.c_int, [ctypes.c_void_p]),
     "ecb_last_error": (ctypes.c_char_p, [ctypes.c_void_p]),
-    "ecb_export_partition": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(EcbExport)]),
-    "ecb_import_entries": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
-                                          ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64),
-                                          ctypes.c_int]),
-    "ecb_global_mark": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64]),
-    "ecb_global_count": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
-                                        ctypes.POINTER(ctypes.c_int64)]),
-    "ecb_global_lens": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
-    "ecb_global_indptr": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
-                                         ctypes.POINTER(ctypes.c_int64)]),
-    "ecb_global_rows": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
 }
 
 _lib = None
@@ -249,29 +229,7 @@ class EcBuilder(object):
     def reset(self):
         self._check(self._lib.ecb_reset(self._ctx))
 
-    # ---- multi-GPU exchange primitives (see alntools_b200/multi_gpu.py) -------------------------
-    def export_partition(self, world):
-        """-> (meta int64[n_ec, 5], rows int32[n_rows, 2]) torch device tensors (copies), per-owner
-        EC / row counts (lists) and the pushed order-key range."""
-        import torch
-        exp = EcbExport()
-        self._check(self._lib.ecb_export_partition(self._ctx, int(world), ctypes.byref(exp)))
-        dev = torch.device("cuda", torch.cuda.current_device())
-        # copies into torch-owned memory: the collectives then only ever see torch allocations, and the
-        # library is free to reuse its export buffers
-        meta = _device_view(ctypes.cast(exp.meta, ctypes.c_void_p).value, (exp.n_ec, 5), "<i8", torch.int64, dev).clone()
-        rows = _device_view(ctypes.cast(exp.rows, ctypes.c_void_p).value, (exp.n_rows, 2), "<i4", torch.int32, dev).clone()
-        ec_counts = [int(exp.part_ec_counts[i]) for i in range(world)]
-        row_counts = [int(exp.part_row_counts[i]) for i in range(world)]
-        return meta, rows, ec_counts, row_counts, int(exp.min_base), int(exp.max_end)
-
-    def import_entries(self, meta, rows, ec_counts, row_counts):
-        n = len(ec_counts)
-        a = (ctypes.c_int64 * n)(*ec_counts)
-        b = (ctypes.c_int64 * n)(*row_counts)
-        self._check(self._lib.ecb_import_entries(self._ctx, meta.data_ptr(), rows.data_ptr(), a, b, n))
-
-    # ---- exchange over peer memory (CUDA IPC arenas, see include/ecb200.h) -------------------------
+    # ---- multi-GPU exchange: CUDA IPC arenas (see include/ecb200.h and multi_gpu.py) ---------------
     def arena_create(self, cap_records):
         """-> (64-byte IPC handle, base address) of this OWNER context's arena (cap_records records of 32 bytes)."""
         handle = ctypes.create_string_buffer(64)
@@ -322,25 +280,6 @@ class EcBuilder(object):
         return {"n_ec": int(sl.n_ec), "nnz": int(sl.nnz), "a_indptr": view(sl.a_indptr, sl.n_ec + 1),
                 "a_indices": view(sl.a_indices, max(sl.nnz, 1))[:sl.nnz], "a_data": view(sl.a_data, max(sl.nnz, 1))[:sl.nnz],
                 "n_data": view(sl.n_data, max(sl.n_ec, 1))[:sl.n_ec]}
-
-    def global_mark(self, min_base, bitmap):
-        self._check(self._lib.ecb_global_mark(self._ctx, int(min_base), bitmap.data_ptr(), bitmap.numel()))
-
-    def global_count(self, bitmap):
-        total = ctypes.c_int64()
-        self._check(self._lib.ecb_global_count(self._ctx, bitmap.data_ptr(), bitmap.numel(), ctypes.byref(total)))
-        return int(total.value)
-
-    def global_lens(self, lens, counts):
-        self._check(self._lib.ecb_global_lens(self._ctx, lens.data_ptr(), counts.data_ptr()))
-
-    def global_indptr(self, lens):
-        nnz = ctypes.c_int64()
-        self._check(self._lib.ecb_global_indptr(self._ctx, lens.data_ptr(), lens.numel(), ctypes.byref(nnz)))
-        return int(nnz.value)
-
-    def global_rows(self, indptr, indices, data):
-        self._check(self._lib.ecb_global_rows(self._ctx, indptr.data_ptr(), indices.data_ptr(), data.data_ptr()))
 
     def stats(self):
         st = EcbStats()

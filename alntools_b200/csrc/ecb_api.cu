@@ -82,16 +82,10 @@ struct ecb_ctx {
   ecb_stats stats{};
   cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   bool long_attr_set = false;
-  // multi-GPU exchange
-  DevBuf x_meta, x_rows, x_counts, x_base;
-  // arena of the peer-memory exchange (plain cudaMalloc: must be exportable through CUDA IPC)
+  // arena of the multi-GPU exchange (plain cudaMalloc: must be exportable through CUDA IPC)
   void* xa_base = nullptr;
   int64_t xa_cap_ec = 0;
   std::vector<void*> xa_opened;
-  int64_t x_part_ec[ECB_MAX_WORLD], x_part_rows[ECB_MAX_WORLD];
-  u64 g_min_base = 0;
-  u64 g_n_ec_total = 0;
-  u32 g_n_wide = 0;
   std::string err;
 };
 
@@ -538,7 +532,7 @@ void cells_release(ecb_ctx* c) {
 
 extern "C" {
 
-int ecb_version(void) { return 1000; }
+int ecb_version(void) { return 2000; }
 
 const char* ecb_last_error(const ecb_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
@@ -1030,114 +1024,6 @@ int ecb_rebase(ecb_ctx* c, int64_t delta) {
   return ECB_OK;
 }
 
-int ecb_export_partition(ecb_ctx* c, int world, ecb_export* out) {
-  if (!c || !out) return ECB_ERR_INVALID;
-  if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
-  if (c->with_cells) return fail(c, ECB_ERR_INVALID, "the multi-GPU exchange covers the single-sample path only");
-  memset(out, 0, sizeof *out);
-  CK(cudaSetDevice(c->device));
-  if (!c->table_slots) CKR(init_table(c));
-  const u32 n_ec = c->n_ec;
-  CKR(ensure(c, c->x_counts, (size_t)2 * world * 4));
-  CKR(ensure(c, c->x_base, (size_t)2 * world * 8));
-  CK(cudaMemsetAsync(c->x_counts.p, 0, (size_t)2 * world * 4, c->stream));
-  ExportParams P{};
-  P.table = (const EcbEntry*)c->table.p;
-  P.ec_slot = (const u32*)c->ec_slot.p;
-  P.row_len = (const u32*)c->row_len.p;
-  P.row_off = (const u32*)c->row_off.p;
-  P.arena = (const uint2*)c->arena.p;
-  P.n_ec = n_ec;
-  P.world = (u32)world;
-  P.counts = (u32*)c->x_counts.p;
-  P.base = (const u64*)c->x_base.p;
-  std::vector<u32> h_counts(2 * world, 0);
-  const int g = grid_for(std::max<u32>(n_ec, 1), 256, c->sm_count * 8);
-  if (n_ec) {
-    ecb_export_count_kernel<<<g, 256, 0, c->stream>>>(P);
-    LAUNCH_CHECK("export_count");
-    CK(cudaMemcpyAsync(h_counts.data(), c->x_counts.p, (size_t)2 * world * 4, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-  }
-  std::vector<u64> h_base(2 * world, 0);
-  u64 ec_run = 0, row_run = 0;
-  for (int w = 0; w < world; ++w) {
-    h_base[w] = ec_run;
-    h_base[world + w] = row_run;
-    c->x_part_ec[w] = h_counts[w];
-    c->x_part_rows[w] = h_counts[world + w];
-    ec_run += h_counts[w];
-    row_run += h_counts[world + w];
-  }
-  CKR(ensure(c, c->x_meta, std::max<u64>(ec_run, 1) * ECB_META_WORDS * 8));
-  CKR(ensure(c, c->x_rows, std::max<u64>(row_run, 1) * 8));
-  if (n_ec) {
-    CK(cudaMemcpyAsync(c->x_base.p, h_base.data(), (size_t)2 * world * 8, cudaMemcpyHostToDevice, c->stream));
-    CK(cudaMemsetAsync(c->x_counts.p, 0, (size_t)2 * world * 4, c->stream));
-    P.meta = (long long*)c->x_meta.p;
-    P.rows = (int2*)c->x_rows.p;
-    ecb_export_fill_kernel<<<g, 256, 0, c->stream>>>(P);
-    LAUNCH_CHECK("export_fill");
-    CK(cudaStreamSynchronize(c->stream));
-  }
-  out->n_ec = (int64_t)ec_run;
-  out->n_rows = (int64_t)row_run;
-  out->meta = (const int64_t*)c->x_meta.p;
-  out->rows = (const int32_t*)c->x_rows.p;
-  out->part_ec_counts = c->x_part_ec;
-  out->part_row_counts = c->x_part_rows;
-  out->min_base = n_ec ? (int64_t)c->min_base : 0;
-  out->max_end = n_ec ? (int64_t)c->max_end : 0;
-  return ECB_OK;
-}
-
-int ecb_import_entries(ecb_ctx* c, const int64_t* meta_device, const int32_t* rows_device,
-                       const int64_t* part_ec_counts, const int64_t* part_row_counts, int n_parts) {
-  if (!c) return ECB_ERR_INVALID;
-  if (n_parts < 1 || n_parts > ECB_MAX_WORLD || !part_ec_counts || !part_row_counts)
-    return fail(c, ECB_ERR_INVALID, "bad partition description");
-  CK(cudaSetDevice(c->device));
-  if (!c->table_slots) CKR(init_table(c));
-  PartTable parts{};
-  parts.n = (u32)n_parts;
-  u64 n_rec = 0, n_rows = 0;
-  for (int p = 0; p < n_parts; ++p) {
-    if (part_ec_counts[p] < 0 || part_row_counts[p] < 0) return fail(c, ECB_ERR_INVALID, "negative partition size");
-    parts.row_base[p] = (long long)n_rows;
-    n_rec += (u64)part_ec_counts[p];
-    n_rows += (u64)part_row_counts[p];
-    parts.ec_end[p] = (long long)n_rec;
-  }
-  if (n_rec == 0) return ECB_OK;
-  if (!meta_device || (n_rows && !rows_device)) return fail(c, ECB_ERR_INVALID, "NULL exchange buffer");
-  if (n_rec > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "too many records in one import");
-  // the owner table must be able to take every incoming record as a new EC without filling up
-  const u64 need = ((u64)c->n_ec + n_rec) * 2;
-  if (need > c->table_slots) CKR(grow_table(c, pow2_ceil(need)));
-  // room for every received row (each new EC brings one): the kernel reserves what it needs on the device
-  if (c->arena_used + n_rows > 0xFFFFFFFFull) return fail(c, ECB_ERR_LIMIT, "row arena exceeds 2^32 entries");
-  CKR(ensure(c, c->arena, std::max<u64>(c->arena_used + n_rows, 1) * sizeof(uint2), true));
-  ImportParams P{};
-  P.meta = (const long long*)meta_device;
-  P.rows = (const int2*)rows_device;
-  P.parts = parts;
-  P.n_rec = (u32)n_rec;
-  P.table = (EcbEntry*)c->table.p;
-  P.mask = c->table_slots - 1;
-  P.ec_slot = (u32*)c->ec_slot.p;
-  P.ec_rep = (u32*)c->ec_rep.p;
-  P.row_len = (u32*)c->row_len.p;
-  P.row_off = (u32*)c->row_off.p;
-  P.arena = (uint2*)c->arena.p;
-  P.ctr = c->d_ctr;
-  ecb_import_insert_kernel<<<grid_for(n_rec, 256, c->sm_count * 8), 256, 0, c->stream>>>(P);
-  LAUNCH_CHECK("import_insert");
-  CKR(sync_counters(c));   // the one round trip of the merge: ECs and arena fill are known to the host again
-  CKR(check_device_error(c));
-  c->n_ec = c->h_ctr->n_ec;
-  return ECB_OK;
-}
-
 int ecb_arena_create(ecb_ctx* c, int64_t cap_records, void* ipc_handle_out, void** base_out) {
   if (!c || cap_records < 1 || !base_out) return ECB_ERR_INVALID;
   if (c->xa_base) return fail(c, ECB_ERR_STATE, "this context already has an arena");
@@ -1347,100 +1233,6 @@ int ecb_order_build(ecb_ctx* c, const ecb_ctx* local, int64_t shard_lo, int64_t 
   return ECB_OK;
 }
 
-static FinalizeParams global_params(ecb_ctx* c) {
-  FinalizeParams F{};
-  F.table = (const EcbEntry*)c->table.p;
-  F.ec_slot = (const u32*)c->ec_slot.p;
-  F.row_len = (const u32*)c->row_len.p;
-  F.row_off = (const u32*)c->row_off.p;
-  F.arena = (const uint2*)c->arena.p;
-  F.n_ec = c->n_ec;
-  F.min_base = c->g_min_base;
-  F.first_rel = (u64*)c->first_rel.p;
-  F.ecid_of = (u32*)c->ecid_of.p;
-  F.count_of = (u32*)c->count_of.p;
-  return F;
-}
-
-int ecb_global_mark(ecb_ctx* c, int64_t min_base, uint32_t* bitmap_device, int64_t n_words) {
-  if (!c || !bitmap_device || n_words <= 0 || min_base < 0) return ECB_ERR_INVALID;
-  CK(cudaSetDevice(c->device));
-  c->g_min_base = (u64)min_base;
-  if (c->n_ec == 0) return ECB_OK;
-  CKR(ensure(c, c->first_rel, (size_t)c->n_ec * 8));
-  CKR(ensure(c, c->ecid_of, (size_t)c->n_ec * 4));
-  CKR(ensure(c, c->count_of, (size_t)c->n_ec * 4));
-  FinalizeParams F = global_params(c);
-  F.bitmap = bitmap_device;
-  ecb_fin_mark_kernel<<<grid_for(c->n_ec, 256, c->sm_count * 8), 256, 0, c->stream>>>(F);
-  LAUNCH_CHECK("fin_mark");
-  CK(cudaStreamSynchronize(c->stream));
-  return ECB_OK;
-}
-
-int ecb_global_count(ecb_ctx* c, const uint32_t* bitmap_device, int64_t n_words, int64_t* n_ec_total) {
-  if (!c || !bitmap_device || n_words <= 0 || !n_ec_total) return ECB_ERR_INVALID;
-  CK(cudaSetDevice(c->device));
-  CKR(ensure(c, c->word_rank, (size_t)n_words * 4));
-  CKR(ensure(c, c->bitmap, (size_t)n_words * 4));
-  CK(cudaMemcpyAsync(c->bitmap.p, bitmap_device, (size_t)n_words * 4, cudaMemcpyDeviceToDevice, c->stream));
-  u64 total = 0;
-  CKR(device_scan<true>(c, (const u32*)c->bitmap.p, (u32*)c->word_rank.p, (u64)n_words, 0, &total));
-  c->g_n_ec_total = total;
-  *n_ec_total = (int64_t)total;
-  return ECB_OK;
-}
-
-int ecb_global_lens(ecb_ctx* c, int32_t* lens_device, int32_t* counts_device) {
-  if (!c || !lens_device || !counts_device) return ECB_ERR_INVALID;
-  CK(cudaSetDevice(c->device));
-  if (c->n_ec == 0) return ECB_OK;
-  FinalizeParams F = global_params(c);
-  F.bitmap = (u32*)c->bitmap.p;
-  F.word_rank = (const u32*)c->word_rank.p;
-  F.a_indptr = lens_device;
-  F.n_data = counts_device;
-  CKR(ensure(c, c->r_n_indices, (size_t)c->g_n_ec_total * 4));
-  F.n_indices = (int32_t*)c->r_n_indices.p;
-  F.wide_count = &c->d_ctr->scratch[2];        // rows with more than 8 entries are listed for ecb_global_rows
-  F.wide_list = (u32*)c->long_list.p;
-  CK(cudaMemsetAsync(&c->d_ctr->scratch[2], 0, sizeof(u32), c->stream));
-  ecb_fin_rank_kernel<true><<<grid_for(c->n_ec, 256, c->sm_count * 8), 256, 0, c->stream>>>(F);
-  LAUNCH_CHECK("fin_rank");
-  CKR(sync_counters(c));
-  c->g_n_wide = c->h_ctr->scratch[2];
-  return ECB_OK;
-}
-
-int ecb_global_indptr(ecb_ctx* c, int32_t* lens_device, int64_t n, int64_t* nnz) {
-  if (!c || !lens_device || n < 1 || !nnz) return ECB_ERR_INVALID;
-  CK(cudaSetDevice(c->device));
-  u64 total = 0;
-  CKR(device_scan<false>(c, (const u32*)lens_device, (u32*)lens_device, (u64)n, 0, &total));
-  if (total > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "A matrix has more than 2^31-1 non-zeros");
-  *nnz = (int64_t)total;
-  return ECB_OK;
-}
-
-int ecb_global_rows(ecb_ctx* c, const int32_t* indptr_device, int32_t* indices_device, int32_t* data_device) {
-  if (!c || !indptr_device || !indices_device || !data_device) return ECB_ERR_INVALID;
-  CK(cudaSetDevice(c->device));
-  if (c->n_ec == 0) return ECB_OK;
-  FinalizeParams F = global_params(c);
-  F.a_indptr = const_cast<int32_t*>(indptr_device);
-  F.a_indices = indices_device;
-  F.a_data = data_device;
-  ecb_fin_rows_kernel<<<grid_for(c->n_ec, 256, c->sm_count * 16), 256, 0, c->stream>>>(F);
-  LAUNCH_CHECK("fin_rows");
-  if (c->g_n_wide) {
-    ecb_fin_rows_long_kernel<<<grid_for((u64)c->g_n_wide * 32, 256, c->sm_count * 8), 256, 0, c->stream>>>(
-        F, (const u32*)c->long_list.p, c->g_n_wide);
-    LAUNCH_CHECK("fin_rows_long");
-  }
-  CK(cudaStreamSynchronize(c->stream));
-  return ECB_OK;
-}
-
 int ecb_destroy(ecb_ctx* c) {
   if (!c) return ECB_OK;
   cudaSetDevice(c->device);
@@ -1450,7 +1242,7 @@ int ecb_destroy(ecb_ctx* c) {
                     &c->overflow_bits,
                     &c->scan_partials, &c->bitmap, &c->word_rank, &c->first_rel, &c->ecid_of, &c->ec_keep,
                     &c->r_a_indptr, &c->r_a_indices, &c->r_a_data, &c->r_n_indptr, &c->r_n_indices,
-                    &c->r_n_data, &c->r_cell_order, &c->x_meta, &c->x_rows, &c->x_counts, &c->x_base};
+                    &c->r_n_data, &c->r_cell_order};
   for (DevBuf* b : bufs) release(c, *b);
   cells_release(c);
   if (c->stream) cudaStreamSynchronize(c->stream);

@@ -3,94 +3,16 @@
 // Reads shard across GPUs by contiguous chunk (the reference's utils.partition + ordered imap,
 // alntools/bam_utils.py:647-680); every GPU builds a local EC table.  Global dedup = the chunk merge
 // of alntools/bam_utils.py:680-698 (sum the counts of equal keys, EC id = rank of the GLOBAL first
-// occurrence).  Two forms:
-//   * any transport (NCCL all-to-all, gloo in the CPU tests): ecb_export_* pack the local ECs WITH their rows
-//     into partitions by owner rank, the owner merges them (ecb_import_insert_kernel), global ids come from
-//     a first-occurrence bitmap OR-ed across ranks, the matrices are assembled on every rank.  Record layout
-//     of an exported EC ("meta", 5 x int64): key_lo, key_hi, first, count << 32 | row_len, row offset inside
-//     the partition (in (target, mask) pairs);
-//   * peer memory (the multi-GPU product path): two dispatches of fixed-size records through IPC-mapped
-//     arenas, rows never travel, nothing global is built - see "the exchange over peer memory" below.
+// occurrence).  It runs over peer memory: two dispatches of fixed-size records through IPC-mapped arenas,
+// rows never travel, nothing global is built - see "the exchange over peer memory" below.
 #pragma once
 #include "ecb_common.cuh"
 #include "ecb_group.cuh"
 
-#define ECB_META_WORDS 5
 #define ECB_MAX_WORLD 64
 
 __device__ __forceinline__ u32 ecb_owner_of(const Key128& k, u32 world) {
   return fmix32((u32)(k.hi >> 32) ^ 0x5bd1e995u) % world;
-}
-
-struct ExportParams {
-  const EcbEntry* table;
-  const u32* ec_slot;
-  const u32* row_len;
-  const u32* row_off;
-  const uint2* arena;
-  u32 n_ec;
-  u32 world;
-  u32* counts;       // [2*world] ECs, rows per owner (count pass) / running cursors (fill pass)
-  const u64* base;   // [2*world] partition bases (fill pass)
-  long long* meta;
-  int2* rows;
-};
-
-// Both export kernels aggregate per CTA in shared memory: a plain atomicAdd per EC on the `world`
-// owner counters would serialise millions of operations on a handful of addresses.
-__global__ void __launch_bounds__(256) ecb_export_count_kernel(const ExportParams P) {
-  __shared__ u32 s_cnt[2 * ECB_MAX_WORLD];
-  for (u32 i = threadIdx.x; i < 2 * P.world; i += blockDim.x) s_cnt[i] = 0u;
-  __syncthreads();
-  for (u32 e = blockIdx.x * blockDim.x + threadIdx.x; e < P.n_ec; e += gridDim.x * blockDim.x) {
-    const EcbEntry* en = P.table + P.ec_slot[e];
-    const u32 owner = ecb_owner_of(Key128{en->key_lo, en->key_hi}, P.world);
-    atomicAdd(&s_cnt[owner], 1u);
-    atomicAdd(&s_cnt[P.world + owner], P.row_len[e]);
-  }
-  __syncthreads();
-  for (u32 i = threadIdx.x; i < 2 * P.world; i += blockDim.x)
-    if (s_cnt[i]) atomicAdd(&P.counts[i], s_cnt[i]);
-}
-
-__global__ void __launch_bounds__(256) ecb_export_fill_kernel(const ExportParams P) {
-  __shared__ u32 s_cnt[2 * ECB_MAX_WORLD];   // per tile: ECs / rows per owner, then their global bases
-  const u32 tiles = (P.n_ec + blockDim.x - 1) / blockDim.x;
-  for (u32 tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-    for (u32 i = threadIdx.x; i < 2 * P.world; i += blockDim.x) s_cnt[i] = 0u;
-    __syncthreads();
-    const u32 e = tile * blockDim.x + threadIdx.x;
-    const bool live = e < P.n_ec;
-    EcbEntry en{};
-    u32 owner = 0, len = 0, idx = 0, roff = 0;
-    if (live) {
-      en = P.table[P.ec_slot[e]];
-      owner = ecb_owner_of(Key128{en.key_lo, en.key_hi}, P.world);
-      len = P.row_len[e];
-      idx = atomicAdd(&s_cnt[owner], 1u);
-      roff = atomicAdd(&s_cnt[P.world + owner], len);
-    }
-    __syncthreads();
-    for (u32 i = threadIdx.x; i < 2 * P.world; i += blockDim.x) {
-      const u32 c = s_cnt[i];
-      s_cnt[i] = c ? atomicAdd(&P.counts[i], c) : 0u;
-    }
-    __syncthreads();
-    if (live) {
-      idx += s_cnt[owner];
-      roff += s_cnt[P.world + owner];
-      long long* m = P.meta + (P.base[owner] + idx) * ECB_META_WORDS;
-      m[0] = (long long)en.key_lo;
-      m[1] = (long long)en.key_hi;
-      m[2] = (long long)en.first;
-      m[3] = (long long)(((u64)(en.countm1 + 1u) << 32) | len);
-      m[4] = (long long)roff;
-      const uint2* src = P.arena + P.row_off[e];
-      int2* dst = P.rows + P.base[P.world + owner] + roff;
-      for (u32 j = 0; j < len; ++j) dst[j] = make_int2((int)src[j].x, (int)src[j].y);
-    }
-    __syncthreads();
-  }
 }
 
 // ---- the exchange over peer memory: two dispatches of fixed-size records, no rows ----------------------
@@ -321,82 +243,6 @@ __global__ void __launch_bounds__(256) ecb_order_rows_kernel(const u32* __restri
     for (u32 j = 0; j < len; ++j) {
       indices[dst + j] = (int32_t)src[j].x;
       data[dst + j] = (int32_t)src[j].y;
-    }
-  }
-}
-
-struct PartTable {
-  long long row_base[ECB_MAX_WORLD];  // first row of each source partition in the receive buffer
-  long long ec_end[ECB_MAX_WORLD];    // cumulative record count after each source partition
-  u32 n;
-};
-
-struct ImportParams {
-  const long long* meta;
-  const int2* rows;      // received rows
-  PartTable parts;
-  u32 n_rec;
-  EcbEntry* table;
-  u32 mask;
-  u32* ec_slot;
-  u32* ec_rep;     // provisional id -> record index of the import that created it
-  u32* row_len;
-  u32* row_off;
-  uint2* arena;
-  EcbCounters* ctr;
-};
-
-// Merge received records into the owner table: sum counts, min first (bam_utils.py:693-698); the records that
-// bring a NEW key also get their provisional id and their row's place in the arena here - ids and arena space
-// are reserved once per CTA tile (a reservation per warp would put a hundred thousand atomics on one address)
-// - and their row is copied on the spot: one kernel, no scan, no host round trip in between.
-__global__ void __launch_bounds__(256) ecb_import_insert_kernel(const ImportParams P) {
-  __shared__ u32 s_scan[10];
-  const u32 tiles = (P.n_rec + blockDim.x - 1) / blockDim.x;
-  for (u32 tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-    const u32 i = tile * blockDim.x + threadIdx.x;
-    const bool live = i < P.n_rec;
-    bool claimed = false;
-    u32 slot = ECB_NONE, len = 0;
-    const long long* m = P.meta + (size_t)(live ? i : 0u) * ECB_META_WORDS;
-    if (live) {
-      const Key128 key{(u64)m[0], (u64)m[1]};
-      const u64 first = (u64)m[2];
-      const u32 count = (u32)((u64)m[3] >> 32);
-      u64 seen;
-      slot = table_find_or_claim<true>(P.table, P.mask, key, claimed, seen);
-      if (slot == ECB_NONE) {
-        atomicOr(&P.ctr->error, ECB_DEVERR_EC_CAPACITY);
-        claimed = false;
-      } else {
-        EcbEntry* e = P.table + slot;
-        atomicAdd(&e->countm1, count);
-        if (first < seen) atomicMin(&e->first, first);
-      }
-      if (claimed) len = (u32)((u64)m[3] & 0xFFFFFFFFull);
-    }
-    // provisional ids and arena space of the tile's new ECs
-    u32 n_new, n_rows;
-    const u32 id_excl = block_excl_scan_u32(claimed ? 1u : 0u, s_scan, n_new);
-    const u32 row_excl = block_excl_scan_u32(len, s_scan, n_rows);
-    if (threadIdx.x == 0) {
-      s_scan[8] = n_new ? atomicAdd(&P.ctr->n_ec, n_new) : 0u;
-      s_scan[9] = n_rows ? (u32)atomicAdd((unsigned long long*)&P.ctr->arena_used, (unsigned long long)n_rows) : 0u;
-    }
-    __syncthreads();
-    const u32 id = s_scan[8] + id_excl, off = s_scan[9] + row_excl;
-    __syncthreads();
-    if (claimed) {
-      P.table[slot].aux = id;
-      P.ec_slot[id] = slot;
-      P.ec_rep[id] = i;
-      P.row_len[id] = len;
-      P.row_off[id] = off;
-      u32 part = 0;
-      while (part + 1 < P.parts.n && (long long)i >= P.parts.ec_end[part]) ++part;
-      const int2* src = P.rows + P.parts.row_base[part] + m[4];
-      uint2* dst = P.arena + off;
-      for (u32 j = 0; j < len; ++j) dst[j] = make_uint2((u32)src[j].x, (u32)src[j].y);
     }
   }
 }

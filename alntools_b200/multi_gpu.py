@@ -11,15 +11,12 @@ its shard (order_base = global offset of the shard) and the merge becomes:
                occurrence; there a bitmap over the rank's own positions orders them (ids are ranks of
                first occurrences and the shards partition the positions) and the rows come from the
                rank's LOCAL context - it has met the EC in its own reads.  Rows never travel; every
-               rank ends up with one contiguous id range of the final matrices
-               (result_on="slices")                                                      [NVLink]
+               rank ends up with one contiguous id range of the final matrices          [NVLink]
   The barriers between these steps are tiny collectives on the stream the kernels run on: nothing in
-  between waits for the host.  (result_on="all" / "rank0" and the NCCL / gloo path keep the first form:
-  all-to-all, first-occurrence bitmap OR-ed by an all-reduce, rows scattered at their global ids.)
+  between waits for the host.
 
 torch.distributed is the plumbing (process group, collectives on device tensors); every compute
-step is a libecb200 kernel behind the C ABI.  The same orchestration runs on gloo/CPU in the tests
-with a stand-in for the kernels.
+step is a libecb200 kernel behind the C ABI.
 """
 import os
 import time
@@ -61,166 +58,94 @@ def _stream_barrier(device, group):
     dist.all_reduce(_BARRIER_WORD[key], group=group)
 
 
-def _all_to_all_counts(counts, device, group):
-    """counts: world * k values, k per destination rank -> the world * k values the peers sent here."""
-    send = torch.tensor(counts, dtype=torch.int64, device=device)
-    recv = torch.empty_like(send)
-    dist.all_to_all_single(recv, send, group=group)
-    return recv.tolist()
-
-
-def _combine(t, group, result_on):
-    """SUM of arrays with disjoint supports: everywhere, or only where the result is needed."""
-    if result_on == "rank0":
-        dist.reduce(t, dst=dist.get_global_rank(group, 0) if group is not None else 0, op=dist.ReduceOp.SUM,
-                    group=group)
-    else:
-        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
-
-
-def distributed_finalize(local, make_owner, device, group=None, result_on="all"):
-    """local: builder holding this rank's shard; make_owner(): fresh builder for the owner role.
-    Returns dict(a_indptr, a_indices, a_data, n_data, n_ec, nnz_a) of int32 tensors on `device`,
-    identical on every rank (result_on="all") or complete on rank 0 only (result_on="rank0": the rank
-    that writes the EC file; the other ranks then hold partial a_indices / a_data / n_data).
-    result_on="slices" (peer-memory exchange only): the final matrices stay partitioned by EC-id range,
-    rank j holding ids [id_base, id_base + n_ec_local) with a_indptr local to its slice; the dict then
-    also carries id_base, n_ec_local, nnz_local.  Nothing is padded to the global size on any rank."""
+def distributed_finalize(local, make_owner, device, group=None, result_on="slices"):
+    """local: builder holding this rank's shard; make_owner(): builder for the owner role (the same one on every
+    step of a job keeps its arena).  The final matrices stay partitioned by EC-id range: rank j holds ids
+    [id_base, id_base + n_ec_local).  Returns dict(a_indptr, a_indices, a_data, n_data) of int32 tensors on
+    `device` for that slice, with a_indptr local to it, and n_ec (all ranks), id_base, n_ec_local, nnz_local;
+    nnz_a is None.  Nothing is padded to the global size on any rank.  result_on="slices" is the only layout."""
+    if result_on != "slices":
+        raise ValueError('result_on must be "slices", got %r' % (result_on,))
+    if device.type != "cuda":
+        raise ValueError("device must be a CUDA device (the exchange maps the ranks' GPU memory), got %s" % device)
     world = dist.get_world_size(group)
     # library kernels and torch's collectives must be ordered against each other: both builders work
     # on torch's current stream from here on (NCCL orders itself against that stream)
-    cur = torch.cuda.current_stream(device).cuda_stream if device.type == "cuda" else None
-    if cur is not None:
-        local.set_stream(cur)
+    cur = torch.cuda.current_stream(device).cuda_stream
+    local.set_stream(cur)
     ph = _Phases(device)
     me = dist.get_rank(group)
-    p2p = result_on == "slices"
-    if p2p and not (device.type == "cuda" and hasattr(local, "export_to_arenas")):
-        raise RuntimeError('result_on="slices" needs the peer-memory exchange (CUDA devices that can map each other)')
-    if p2p:
-        # ---- fused partition + dispatch: every local EC is stored straight into its owner's arena
-        # over NVLink by ONE kernel (peer memory mapped through CUDA IPC); no staging, no all-to-all
-        owner = make_owner()
-        owner.set_stream(cur)
-        arena = getattr(owner, "_exchange_arena", None)
-        if arena is not None:
-            # the arenas exist (a later step of the same job): clear the header and put ONE small collective on
-            # the stream as the barrier between "every arena is clear" and "peers store" - no host round trip;
-            # whether everything fits is decided by the overflow flag in the arena header
-            owner.arena_reset()
-            _stream_barrier(device, group)
-        else:
-            # first call of a job: size the arenas (an owner receives about one rank's worth of ECs; twice the
-            # largest local table leaves room for a skewed partition), create them, map the peers'
-            info = torch.tensor([local.stats()["table_used"]], dtype=torch.int64, device=device)
-            gathered = [torch.empty_like(info) for _ in range(world)]
-            dist.all_gather(gathered, info, group=group)
-            need_ec = 2 * max(int(t.item()) for t in gathered) + 1024
-            handle, base = owner.arena_create(need_ec)
-            hs = [torch.empty(64, dtype=torch.uint8, device=device) for _ in range(world)]
-            dist.all_gather(hs, torch.frombuffer(bytearray(handle), dtype=torch.uint8).to(device), group=group)
-            bases = [base if r == me else owner.arena_open_peer(bytes(hs[r].cpu().tolist())) for r in range(world)]
-            arena = {"bases": bases, "cap_ec": need_ec}
-            owner._exchange_arena = arena
-            dist.barrier(group=group)                     # every arena exists and is zeroed
-        ph.mark("setup")
-        min_base, max_end = local.export_to_arenas(arena["bases"], arena["cap_ec"])
-        ph.mark("dispatch 1")
-        # every rank's shard of the read order; the all-gather is the barrier between "store" and "merge"
-        mine = torch.tensor([min_base, max_end], dtype=torch.int64, device=device)
-        spans = torch.empty(2 * world, dtype=torch.int64, device=device)
-        dist.all_gather_into_tensor(spans, mine, group=group)
-        # a rank that fails from here on (an arena that turned out too small) must not leave its peers waiting in
-        # a collective: it carries on with what it has, the failure travels with the all-gather of the slice
-        # sizes below, and every rank raises
-        failure = None
-        try:
-            owner.import_arena()
-        except Exception as exc:         # noqa: BLE001 - re-raised on every rank below
-            failure = exc
-        owner.arena_reset()              # reused by the second dispatch ...
-        _stream_barrier(device, group)   # ... once every rank has merged what it received
-        ph.mark("merge")
-        spans = spans.tolist()
-        lo, hi = spans[0::2], spans[1::2]
-        if not any(h > l for l, h in zip(lo, hi)):
-            raise RuntimeError("The shape must be a tuple of three positive integers.")  # zero ECs everywhere
-        owner.order_dispatch(arena["bases"], arena["cap_ec"], lo, hi)
-        _stream_barrier(device, group)   # every rank's ECs have landed
-        ph.mark("dispatch 2")
-        sl = None
-        try:
-            sl = owner.order_build(local, lo[me], hi[me])
-        except Exception as exc:         # noqa: BLE001
-            failure = failure or exc
-        ph.mark("order build")
-        # the id range of a rank starts behind the ECs of the shards in front of it
-        sizes = torch.empty(2 * world, dtype=torch.int64, device=device)
-        dist.all_gather_into_tensor(sizes, torch.tensor([sl["n_ec"] if sl else 0, 1 if failure else 0],
-                                                        dtype=torch.int64, device=device), group=group)
-        sizes = sizes.tolist()
-        if failure is not None:
-            raise failure
-        if any(sizes[1::2]):
-            raise RuntimeError("the multi-GPU exchange failed on rank(s) %s" % [r for r in range(world) if sizes[2 * r + 1]])
-        sizes = sizes[0::2]
-        id_base = sum(n for r, n in enumerate(sizes) if hi[r] > lo[r] and (lo[r], r) < (lo[me], me))
-        ph.report()
-        return {"a_indptr": sl["a_indptr"], "a_indices": sl["a_indices"], "a_data": sl["a_data"],
-                "n_data": sl["n_data"], "n_ec": sum(sizes), "id_base": id_base, "n_ec_local": sl["n_ec"],
-                "nnz_local": sl["nnz"], "nnz_a": None}
+    # ---- fused partition + dispatch: every local EC is stored straight into its owner's arena
+    # over NVLink by ONE kernel (peer memory mapped through CUDA IPC); no staging
+    owner = make_owner()
+    owner.set_stream(cur)
+    arena = getattr(owner, "_exchange_arena", None)
+    if arena is not None:
+        # the arenas exist (a later step of the same job): clear the header and put ONE small collective on
+        # the stream as the barrier between "every arena is clear" and "peers store" - no host round trip;
+        # whether everything fits is decided by the overflow flag in the arena header
+        owner.arena_reset()
+        _stream_barrier(device, group)
     else:
-        meta, rows, ec_counts, row_counts, min_base, max_end = local.export_partition(world)
-        ph.mark("export")
-
-        # ---- all-to-all of the hash-partitioned local ECs -------------------------------------------
-        # one all-gather carries every rank's partition sizes and its pushed position range
-        info = torch.tensor(list(ec_counts) + list(row_counts) + [min_base if max_end > min_base else (1 << 62), max_end],
-                            dtype=torch.int64, device=device)
+        # first call of a job: size the arenas (an owner receives about one rank's worth of ECs; twice the
+        # largest local table leaves room for a skewed partition), create them, map the peers'
+        info = torch.tensor([local.stats()["table_used"]], dtype=torch.int64, device=device)
         gathered = [torch.empty_like(info) for _ in range(world)]
         dist.all_gather(gathered, info, group=group)
-        g = torch.stack(gathered).tolist()
-        recv_ec = [g[src][me] for src in range(world)]
-        recv_rows = [g[src][world + me] for src in range(world)]
-        g_min = min(row[2 * world] for row in g)
-        g_max = max(row[2 * world + 1] for row in g)
-        meta_in = torch.empty((sum(recv_ec), 5), dtype=torch.int64, device=device)
-        rows_in = torch.empty((sum(recv_rows), 2), dtype=torch.int32, device=device)
-        dist.all_to_all_single(meta_in, meta, output_split_sizes=recv_ec, input_split_sizes=ec_counts, group=group)
-        dist.all_to_all_single(rows_in, rows, output_split_sizes=recv_rows, input_split_sizes=row_counts, group=group)
-        ph.mark("all_to_all")
-        owner = make_owner()
-        if cur is not None:
-            owner.set_stream(cur)
-        owner.import_entries(meta_in, rows_in, recv_ec, recv_rows)
-        ph.mark("import")
-
-    # ---- global EC ids from the OR-ed first-occurrence bitmap ------------------------------------
-    if g_max <= g_min:
+        need_ec = 2 * max(int(t.item()) for t in gathered) + 1024
+        handle, base = owner.arena_create(need_ec)
+        hs = [torch.empty(64, dtype=torch.uint8, device=device) for _ in range(world)]
+        dist.all_gather(hs, torch.frombuffer(bytearray(handle), dtype=torch.uint8).to(device), group=group)
+        bases = [base if r == me else owner.arena_open_peer(bytes(hs[r].cpu().tolist())) for r in range(world)]
+        arena = {"bases": bases, "cap_ec": need_ec}
+        owner._exchange_arena = arena
+        dist.barrier(group=group)                     # every arena exists and is zeroed
+    ph.mark("setup")
+    min_base, max_end = local.export_to_arenas(arena["bases"], arena["cap_ec"])
+    ph.mark("dispatch 1")
+    # every rank's shard of the read order; the all-gather is the barrier between "store" and "merge"
+    mine = torch.tensor([min_base, max_end], dtype=torch.int64, device=device)
+    spans = torch.empty(2 * world, dtype=torch.int64, device=device)
+    dist.all_gather_into_tensor(spans, mine, group=group)
+    # a rank that fails from here on (an arena that turned out too small) must not leave its peers waiting in
+    # a collective: it carries on with what it has, the failure travels with the all-gather of the slice
+    # sizes below, and every rank raises
+    failure = None
+    try:
+        owner.import_arena()
+    except Exception as exc:         # noqa: BLE001 - re-raised on every rank below
+        failure = exc
+    owner.arena_reset()              # reused by the second dispatch ...
+    _stream_barrier(device, group)   # ... once every rank has merged what it received
+    ph.mark("merge")
+    spans = spans.tolist()
+    lo, hi = spans[0::2], spans[1::2]
+    if not any(h > l for l, h in zip(lo, hi)):
         raise RuntimeError("The shape must be a tuple of three positive integers.")  # zero ECs everywhere
-    n_words = (g_max - g_min + 31) // 32 + 1
-    bitmap = torch.zeros(n_words, dtype=torch.int32, device=device)
-    owner.global_mark(g_min, bitmap)
-    dist.all_reduce(bitmap, op=dist.ReduceOp.SUM, group=group)   # disjoint bits: SUM == OR
-    ph.mark("bitmap")
-    n_ec = owner.global_count(bitmap)
-    ph.mark("count")
-    lens = torch.zeros(n_ec + 1, dtype=torch.int32, device=device)
-    counts = torch.zeros(n_ec, dtype=torch.int32, device=device)
-    owner.global_lens(lens, counts)
-    dist.all_reduce(lens, op=dist.ReduceOp.SUM, group=group)     # every owner needs the global indptr
-    _combine(counts, group, result_on)
-    ph.mark("lens")
-    nnz = owner.global_indptr(lens)                              # lens becomes indptr in place
-    indices = torch.zeros(max(nnz, 1), dtype=torch.int32, device=device)
-    data = torch.zeros(max(nnz, 1), dtype=torch.int32, device=device)
-    owner.global_rows(lens, indices, data)
-    _combine(indices, group, result_on)
-    _combine(data, group, result_on)
-    ph.mark("rows")
+    owner.order_dispatch(arena["bases"], arena["cap_ec"], lo, hi)
+    _stream_barrier(device, group)   # every rank's ECs have landed
+    ph.mark("dispatch 2")
+    sl = None
+    try:
+        sl = owner.order_build(local, lo[me], hi[me])
+    except Exception as exc:         # noqa: BLE001
+        failure = failure or exc
+    ph.mark("order build")
+    # the id range of a rank starts behind the ECs of the shards in front of it
+    sizes = torch.empty(2 * world, dtype=torch.int64, device=device)
+    dist.all_gather_into_tensor(sizes, torch.tensor([sl["n_ec"] if sl else 0, 1 if failure else 0],
+                                                    dtype=torch.int64, device=device), group=group)
+    sizes = sizes.tolist()
+    if failure is not None:
+        raise failure
+    if any(sizes[1::2]):
+        raise RuntimeError("the multi-GPU exchange failed on rank(s) %s" % [r for r in range(world) if sizes[2 * r + 1]])
+    sizes = sizes[0::2]
+    id_base = sum(n for r, n in enumerate(sizes) if hi[r] > lo[r] and (lo[r], r) < (lo[me], me))
     ph.report()
-    return {"a_indptr": lens, "a_indices": indices[:nnz], "a_data": data[:nnz], "n_data": counts,
-            "n_ec": n_ec, "nnz_a": nnz}
+    return {"a_indptr": sl["a_indptr"], "a_indices": sl["a_indices"], "a_data": sl["a_data"],
+            "n_data": sl["n_data"], "n_ec": sum(sizes), "id_base": id_base, "n_ec_local": sl["n_ec"],
+            "nnz_local": sl["nnz"], "nnz_a": None}
 
 
 def shard_bounds(read_group, world):

@@ -152,48 +152,17 @@ const char* ecb_last_error(const ecb_ctx* ctx);
 /* ---- multi-GPU exchange -------------------------------------------------------------------------
  * Reads shard across GPUs by contiguous chunk (alntools/utils.py:67-87 + bam_utils.py:647-680: each
  * worker gets a contiguous run of chunks and results are merged in chunk order).  Each rank pushes its
- * shard into a LOCAL context with order_base = global offset of the shard.  The merge of
- * alntools/bam_utils.py:680-698 then becomes:
- *   1. ecb_export_partition on the local context: local ECs packed into `world` partitions by owner
- *      rank (hash of the 128-bit key);
- *   2. the host exchanges the partitions (NCCL all-to-all through torch.distributed);
- *   3. ecb_import_entries on a fresh OWNER context: equal keys are merged (counts summed, smallest
- *      first-occurrence kept), rows adopted;
- *   4. ecb_global_mark / all-reduce(bitmap) / ecb_global_count: EC ids = rank of the first-occurrence
- *      bit in the bitmap OR-ed over all ranks;
- *   5. ecb_global_lens / all-reduce / ecb_global_indptr / ecb_global_rows / all-reduce: every rank
- *      scatters its owned rows and counts into zero-initialised global arrays; supports are disjoint,
- *      so a SUM all-reduce assembles the final CSR A matrix and the counts on every rank.
- * That is the form for any transport (NCCL, gloo in the CPU tests); it leaves the whole matrix on every rank
- * (or on rank 0).  Where the ranks can map each other's memory the exchange further down replaces all five
- * steps and leaves the final matrices partitioned, one contiguous EC-id range per rank.
- * All pointers marked "device" are device memory of the context's GPU owned by the caller.
+ * shard into a LOCAL context with order_base = global offset of the shard, or counted from its own first
+ * alignment and moved there with ecb_rebase.  The merge of alntools/bam_utils.py:680-698 (counts of equal
+ * keys summed, EC id = rank of the first occurrence over all shards) is the exchange over peer memory
+ * further down; it leaves the final matrices partitioned, one contiguous EC-id range per rank.
  */
 /* Add `delta` (>= 0) to the order key of everything pushed so far: a rank that decodes one shard of a file
  * pushes with order_base counted from its own first alignment and is moved to its global position once every
  * rank knows how many alignments the shards in front of it hold.  Single-sample contexts, before the exchange. */
 int ecb_rebase(ecb_ctx* ctx, int64_t delta);
 
-#define ECB_EXPORT_META_WORDS 5
-typedef struct ecb_export {
-  int64_t n_ec;                    /* local ECs exported                                           */
-  int64_t n_rows;                  /* (target, mask) pairs exported                                */
-  const int64_t* meta;             /* device [n_ec * 5]: key_lo, key_hi, first, count<<32|row_len,
-                                      row offset inside its partition                              */
-  const int32_t* rows;             /* device [n_rows * 2]: (target_idx, hap_mask), partition-major */
-  const int64_t* part_ec_counts;   /* host [world]                                                 */
-  const int64_t* part_row_counts;  /* host [world]                                                 */
-  int64_t min_base, max_end;       /* order-key range this rank has pushed                         */
-} ecb_export;
-
-int ecb_export_partition(ecb_ctx* ctx, int world, ecb_export* out);
-
-/* Merge n_parts received partitions (concatenated, in source-rank order) into this OWNER context. */
-int ecb_import_entries(ecb_ctx* ctx, const int64_t* meta_device, const int32_t* rows_device,
-                       const int64_t* part_ec_counts, const int64_t* part_row_counts, int n_parts);
-
-/* ---- the exchange over peer memory (one process per GPU on an NVLink / NVSwitch box; the default of the
- * multi-GPU path) ---------------------------------------------------------------------------------------
+/* ---- the exchange over peer memory (one process per GPU on an NVLink / NVSwitch box) --------------------
  * Each rank creates an ARENA on its OWNER context (device memory from cudaMalloc, exportable through CUDA IPC),
  * hands the 64-byte IPC handle to its peers and maps theirs.  Two dispatches of fixed-size records go through
  * it, each one kernel that stores straight into the destination ranks' arenas over NVLink (one remote
@@ -210,10 +179,10 @@ int ecb_import_entries(ecb_ctx* ctx, const int64_t* meta_device, const int32_t* 
  *                                          it is ordered with a bitmap over this rank's OWN positions and the
  *                                          rows are taken from the LOCAL context - the rank that holds an EC's
  *                                          first occurrence has met the EC in its own reads.  Rows never travel;
- *                                          nothing global is built (no bitmap over all positions, no all-reduce,
- *                                          no ecb_global_* call).  id_base of the result is left 0: the slice
- *                                          starts after the ECs of the shards in front, which the caller learns
- *                                          from one all-gather of the slice sizes.
+ *                                          nothing global is built (no bitmap over all positions, no
+ *                                          all-reduce).  id_base of the result is left 0: the slice starts after
+ *                                          the ECs of the shards in front, which the caller learns from one
+ *                                          all-gather of the slice sizes.
  * The caller brackets the stores with barriers:
  *     ecb_arena_reset (every rank) - barrier - ecb_export_to_arenas - barrier - ecb_import_arena -
  *     ecb_arena_reset - barrier - ecb_order_dispatch - barrier - ecb_order_build.
@@ -237,24 +206,6 @@ typedef struct ecb_slice {
 int ecb_order_dispatch(ecb_ctx* owner_ctx, int world, void* const* arena_bases, int64_t cap_records,
                        const int64_t* shard_lo, const int64_t* shard_hi);
 int ecb_order_build(ecb_ctx* owner_ctx, const ecb_ctx* local_ctx, int64_t shard_lo, int64_t shard_hi, ecb_slice* out);
-
-/* Set the first-occurrence bits of the ECs this context owns in bitmap[n_words] (bit i = order key
- * min_base + i).  The caller zero-fills the bitmap and all-reduces it afterwards. */
-int ecb_global_mark(ecb_ctx* ctx, int64_t min_base, uint32_t* bitmap_device, int64_t n_words);
-
-/* Rank the bits of the (all-reduced) bitmap: *n_ec_total = number of set bits = global EC count. */
-int ecb_global_count(ecb_ctx* ctx, const uint32_t* bitmap_device, int64_t n_words, int64_t* n_ec_total);
-
-/* Scatter row lengths and read counts of the owned ECs into zero-filled lens[n_ec_total+1] and
- * counts[n_ec_total] at their global ids. */
-int ecb_global_lens(ecb_ctx* ctx, int32_t* lens_device, int32_t* counts_device);
-
-/* In-place exclusive scan lens -> indptr (n = n_ec_total + 1); *nnz = indptr[n_ec_total]. */
-int ecb_global_indptr(ecb_ctx* ctx, int32_t* lens_device, int64_t n, int64_t* nnz);
-
-/* Scatter the owned rows into zero-filled indices[nnz] / data[nnz] at indptr[global id]. */
-int ecb_global_rows(ecb_ctx* ctx, const int32_t* indptr_device, int32_t* indices_device,
-                    int32_t* data_device);
 
 #ifdef __cplusplus
 }

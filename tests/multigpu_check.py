@@ -4,8 +4,9 @@
         --master-port 29533 tests/multigpu_check.py [n_reads]
 
 Every rank builds its contiguous shard of a seeded synthetic workload on its own B200, the ranks
-exchange hash-partitioned ECs over NCCL (alntools_b200/multi_gpu.py) and every rank must end up with
-exactly the matrices the C oracle computes for the whole, unsharded input."""
+exchange their ECs over peer memory (alntools_b200/multi_gpu.py) and every rank must end up with its
+EC-id range of exactly the matrices the C oracle computes for the whole, unsharded input.  N = 1 runs
+the whole orchestration with a single rank."""
 import os
 import sys
 
@@ -15,6 +16,25 @@ import torch.distributed as dist
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+
+
+def check_slice(label, sl, oracle, dev):
+    """This rank's slice must be rows [id_base, id_base + n_ec_local) of the oracle's matrices; one line per case."""
+    indptr, indices, data, counts = oracle[:4]
+    a, b = sl["id_base"], sl["id_base"] + sl["n_ec_local"]
+    ok = (sl["n_ec"] == len(counts)
+          and np.array_equal(sl["a_indptr"].cpu().numpy(), indptr[a:b + 1] - indptr[a])
+          and np.array_equal(sl["a_indices"].cpu().numpy(), indices[indptr[a]:indptr[b]])
+          and np.array_equal(sl["a_data"].cpu().numpy(), data[indptr[a]:indptr[b]])
+          and np.array_equal(sl["n_data"].cpu().numpy(), counts[a:b]))
+    flag = torch.tensor([1 if ok else 0], device=dev)
+    dist.all_reduce(flag, op=dist.ReduceOp.MIN)
+    if dist.get_rank() == 0:
+        print("multigpu_check world=%d %s ECs=%d: %s" % (dist.get_world_size(), label, len(counts),
+                                                           "OK" if flag.item() else "MISMATCH"), flush=True)
+    if not flag.item():
+        dist.destroy_process_group()
+        sys.exit(1)
 
 
 def main():
@@ -44,20 +64,9 @@ def main():
             owner_b.reset()
             local_b.push(np.ascontiguousarray(rg[a:b]), np.ascontiguousarray(tg[a:b]),
                          np.ascontiguousarray(hp[a:b]), order_base=a)
-            res = multi_gpu.distributed_finalize(local_b, lambda: owner_b, dev)
-        indptr, indices, data, counts, n_reads_o = c_oracle.ec_from_columns(rg, tg, hp)
-        ok = (np.array_equal(res["a_indptr"].cpu().numpy(), indptr)
-              and np.array_equal(res["a_indices"].cpu().numpy(), indices)
-              and np.array_equal(res["a_data"].cpu().numpy(), data)
-              and np.array_equal(res["n_data"].cpu().numpy(), counts))
-        flag = torch.tensor([1 if ok else 0], device=dev)
-        dist.all_reduce(flag, op=dist.ReduceOp.MIN)
-        if rank == 0:
-            print("multigpu_check world=%d mode=%s reads=%d alignments=%d ECs=%d: %s"
-                  % (world, mode, reads, len(rg), len(counts), "OK" if flag.item() else "MISMATCH"), flush=True)
-        if not flag.item():
-            dist.destroy_process_group()
-            sys.exit(1)
+            sl = multi_gpu.distributed_finalize(local_b, lambda: owner_b, dev, result_on="slices")
+        check_slice("mode=%s reads=%d alignments=%d" % (mode, reads, len(rg)), sl,
+                    c_oracle.ec_from_columns(rg, tg, hp), dev)
         local_b.close()
         owner_b.close()
 
@@ -73,41 +82,14 @@ def main():
         local_b.reset()
         owner_b.reset()
         local_b.push(mine["read_group"], mine["target_idx"], mine["hap_idx"], order_base=base)
-        res = multi_gpu.distributed_finalize(local_b, lambda: owner_b, dev)
+        sl = multi_gpu.distributed_finalize(local_b, lambda: owner_b, dev, result_on="slices")
     rg = np.concatenate([s["read_group"] + 10 ** 8 * r for r, s in enumerate(shards)])   # reads stay distinct
     tg = np.concatenate([s["target_idx"] for s in shards])
     hp = np.concatenate([s["hap_idx"] for s in shards])
-    indptr, indices, data, counts, _ = c_oracle.ec_from_columns(rg.astype(np.int32), tg, hp)
-    ok = (np.array_equal(res["a_indptr"].cpu().numpy(), indptr) and np.array_equal(res["a_indices"].cpu().numpy(), indices)
-          and np.array_equal(res["a_data"].cpu().numpy(), data) and np.array_equal(res["n_data"].cpu().numpy(), counts))
-    flag = torch.tensor([1 if ok else 0], device=dev)
-    dist.all_reduce(flag, op=dist.ReduceOp.MIN)
-    if rank == 0:
-        print("multigpu_check world=%d own-shards device-resident reuse: alignments=%d ECs=%d: %s"
-              % (world, len(rg), len(counts), "OK" if flag.item() else "MISMATCH"), flush=True)
-    # the same job with the result left partitioned by EC-id range (peer-memory exchange only)
-    if os.environ.get("ECB_EXCHANGE", "p2p") != "nccl":
-        for _ in range(2):
-            local_b.reset()
-            owner_b.reset()
-            local_b.push(mine["read_group"], mine["target_idx"], mine["hap_idx"], order_base=base)
-            sl = multi_gpu.distributed_finalize(local_b, lambda: owner_b, dev, result_on="slices")
-        a, b = sl["id_base"], sl["id_base"] + sl["n_ec_local"]
-        ok = (sl["n_ec"] == len(counts)
-              and np.array_equal(sl["a_indptr"].cpu().numpy(), indptr[a:b + 1] - indptr[a])
-              and np.array_equal(sl["a_indices"].cpu().numpy(), indices[indptr[a]:indptr[b]])
-              and np.array_equal(sl["a_data"].cpu().numpy(), data[indptr[a]:indptr[b]])
-              and np.array_equal(sl["n_data"].cpu().numpy(), counts[a:b]))
-        flag2 = torch.tensor([1 if ok else 0], device=dev)
-        dist.all_reduce(flag2, op=dist.ReduceOp.MIN)
-        if rank == 0:
-            print("multigpu_check world=%d slices: %s" % (world, "OK" if flag2.item() else "MISMATCH"), flush=True)
-        flag = torch.minimum(flag, flag2)
+    check_slice("own-shards device-resident reuse: alignments=%d" % len(rg), sl,
+                c_oracle.ec_from_columns(rg.astype(np.int32), tg, hp), dev)
     local_b.close()
     owner_b.close()
-    if not flag.item():
-        dist.destroy_process_group()
-        sys.exit(1)
     dist.destroy_process_group()
 
 

@@ -366,22 +366,22 @@ def test_full_size_cfg4_cells_50k(native):
         assert np.array_equal(got[k], want[k]), k
 
 
-# ---------------------------------------------------------------- multi-GPU exchange (needs >= 2 GPUs)
+# ---------------------------------------------------------------- multi-GPU exchange
 def test_multigpu_exchange_matches_oracle(native):
+    """The NCCL job of tests/multigpu_check.py: at world 2 or 4 where the GPUs are there, else at world 1, which
+    still runs the whole orchestration (arena, stream barriers, both dispatches, id_base)."""
     import subprocess
     import sys
     import torch
     from conftest import ROOT
     n = torch.cuda.device_count()
-    if n < 2:
-        pytest.skip("needs at least 2 GPUs")
-    world = 2 if n < 4 else 4
+    world = 1 if n < 2 else 2 if n < 4 else 4
     out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(world),
                           "--master-addr", "127.0.0.1", "--master-port", "29533",
                           os.path.join(ROOT, "tests", "multigpu_check.py"), "300000"],
                          capture_output=True, text=True, timeout=400)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
-    assert out.stdout.count("OK") == 4
+    assert out.stdout.count("OK") == 3 and "MISMATCH" not in out.stdout, out.stdout[-2000:]
 
 
 def test_multigpu_convert_writes_the_golden_files(native):
@@ -410,71 +410,6 @@ def test_rebase_moves_the_order_keys(native):
         b.push(cols["read_group"], cols["target_idx"], cols["hap_idx"], order_base=0)
         b.rebase(123456789)
         _assert_same(b.finalize(), want)
-
-
-def test_exchange_primitives_single_gpu(native):
-    """The export -> import -> global id path (the form for any transport) with world = 1..3 emulated on ONE GPU:
-    all partitions are imported into owner contexts on the same device and the bitmap 'all-reduce' is a local sum."""
-    import torch
-    from alntools_b200 import synth
-    cols = synth.make_columns(120000, 4000, 2, seed=41, mode="diploid", dup_rate=0.02)
-    rg, tg, hp = cols["read_group"], cols["target_idx"], cols["hap_idx"]
-    want = _oracle(cols)
-    dev = torch.device("cuda", 0)
-    from alntools_b200 import multi_gpu
-    for world in (1, 2, 3):
-        cuts = multi_gpu.shard_bounds(rg, world)
-        exports = []
-        locals_ = []
-        for r in range(world):
-            a, b = cuts[r], cuts[r + 1]
-            lb = native.EcBuilder(4000, 2, alignments_hint=b - a)
-            lb.push(np.ascontiguousarray(rg[a:b]), np.ascontiguousarray(tg[a:b]), np.ascontiguousarray(hp[a:b]), order_base=a)
-            locals_.append(lb)
-            exports.append(lb.export_partition(world))
-        owners = []
-        for o in range(world):   # what all_to_all would deliver to owner o
-            metas, rows, ecn, rown = [], [], [], []
-            for src in range(world):
-                meta, row, ec_counts, row_counts, _, _ = exports[src]
-                e0, r0 = sum(ec_counts[:o]), sum(row_counts[:o])
-                metas.append(meta[e0:e0 + ec_counts[o]])
-                rows.append(row[r0:r0 + row_counts[o]])
-                ecn.append(ec_counts[o])
-                rown.append(row_counts[o])
-            ob = native.EcBuilder(4000, 2, alignments_hint=len(rg))
-            ob.import_entries(torch.cat(metas).contiguous(), torch.cat(rows).contiguous(), ecn, rown)
-            owners.append(ob)
-        n_words = (len(rg) + 31) // 32 + 1
-        bitmap = torch.zeros(n_words, dtype=torch.int32, device=dev)
-        for ob in owners:
-            part = torch.zeros_like(bitmap)
-            ob.global_mark(0, part)
-            bitmap += part
-        totals = [ob.global_count(bitmap) for ob in owners]
-        assert len(set(totals)) == 1 and totals[0] == len(want[3])
-        n_ec = totals[0]
-        lens = torch.zeros(n_ec + 1, dtype=torch.int32, device=dev)
-        counts = torch.zeros(n_ec, dtype=torch.int32, device=dev)
-        for ob in owners:
-            l, c = torch.zeros_like(lens), torch.zeros_like(counts)
-            ob.global_lens(l, c)
-            lens += l
-            counts += c
-        nnz = owners[0].global_indptr(lens)
-        indices = torch.zeros(nnz, dtype=torch.int32, device=dev)
-        data = torch.zeros(nnz, dtype=torch.int32, device=dev)
-        for ob in owners:
-            i, d = torch.zeros_like(indices), torch.zeros_like(data)
-            ob.global_rows(lens, i, d)
-            indices += i
-            data += d
-        assert np.array_equal(lens.cpu().numpy(), want[0])
-        assert np.array_equal(indices.cpu().numpy(), want[1])
-        assert np.array_equal(data.cpu().numpy(), want[2])
-        assert np.array_equal(counts.cpu().numpy(), want[3])
-        for b in locals_ + owners:
-            b.close()
 
 
 @pytest.mark.parametrize("world,mode", [(1, "diploid"), (2, "diploid"), (3, "diploid"), (4, "heavy"), (3, "empty-rank")])

@@ -97,6 +97,17 @@ def test_partition_matches_reference_semantics():
     assert utils.partition(list(range(2)), 4) == [[0], [1]]
 
 
+def test_shard_bounds_never_split_a_read():
+    from alntools_b200 import multi_gpu
+    rg = np.repeat(np.arange(50), np.random.default_rng(0).integers(1, 9, 50)).astype(np.int32)
+    for world in (1, 2, 3, 8, 64):
+        cuts = multi_gpu.shard_bounds(rg, world)
+        assert cuts[0] == 0 and cuts[-1] == len(rg) and len(cuts) == world + 1
+        assert all(b >= a for a, b in zip(cuts[:-1], cuts[1:]))
+        for c in cuts[1:-1]:
+            assert c == len(rg) or c == 0 or rg[c] != rg[c - 1]
+
+
 class _StubBuilder(object):
     """Stands in for the GPU builder: accepts every push and returns fixed, well-formed result arrays, so that
     the host side of convert() (decode, tables, file writing) can run on a machine without a GPU."""
