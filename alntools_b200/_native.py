@@ -57,6 +57,14 @@ class EcbSlice(ctypes.Structure):
                 ("a_indptr", _i32p), ("a_indices", _i32p), ("a_data", _i32p), ("n_data", _i32p)]
 
 
+class EcbCellsSlice(ctypes.Structure):
+    _i32p = ctypes.POINTER(ctypes.c_int32)
+    _fields_ = [("n_ec", ctypes.c_int64), ("nnz", ctypes.c_int64),
+                ("a_indptr", _i32p), ("a_indices", _i32p), ("a_data", _i32p),
+                ("n_samples", ctypes.c_int64), ("nnz_n", ctypes.c_int64),
+                ("n_col_counts", _i32p), ("n_indices", _i32p), ("n_data", _i32p)]
+
+
 # every symbol include/ecb200.h declares, with its ctypes signature
 SIGNATURES = {
     "ecb_version": (ctypes.c_int, []),
@@ -74,6 +82,22 @@ SIGNATURES = {
     "ecb_export_to_arenas": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_void_p), ctypes.c_int64,
                                             ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]),
     "ecb_import_arena": (ctypes.c_int, [ctypes.c_void_p]),
+    "ecb_cells_summary": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p,
+                                         ctypes.c_void_p]),
+    "ecb_cells_order": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
+                                       ctypes.c_int64, ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64),
+                                       ctypes.POINTER(ctypes.c_void_p)]),
+    "ecb_cells_dispatch_counts": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_int64),
+                                                 ctypes.POINTER(ctypes.c_int64), ctypes.c_void_p]),
+    "ecb_cells_arena_create": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_char_p,
+                                              ctypes.POINTER(ctypes.c_void_p)]),
+    "ecb_cells_export_to_arenas": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_void_p), ctypes.c_int64,
+                                                  ctypes.c_int64, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]),
+    "ecb_cells_import_arena": (ctypes.c_int, [ctypes.c_void_p]),
+    "ecb_cells_order_dispatch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_void_p), ctypes.c_int64,
+                                                ctypes.c_int64, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]),
+    "ecb_cells_order_build": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64,
+                                             ctypes.POINTER(EcbCellsSlice)]),
     "ecb_push": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                 ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int, ctypes.c_int]),
     "ecb_finalize": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.POINTER(EcbResult)]),
@@ -280,6 +304,81 @@ class EcBuilder(object):
         return {"n_ec": int(sl.n_ec), "nnz": int(sl.nnz), "a_indptr": view(sl.a_indptr, sl.n_ec + 1),
                 "a_indices": view(sl.a_indices, max(sl.nnz, 1))[:sl.nnz], "a_data": view(sl.a_data, max(sl.nnz, 1))[:sl.nnz],
                 "n_data": view(sl.n_data, max(sl.n_ec, 1))[:sl.n_ec]}
+
+    # ---- per-cell exchange (see include/ecb200.h and multi_gpu.distributed_finalize_cells) ------------------
+    def cells_summary(self, cell_map, n_cells):
+        """-> (cell_key, cell_total): int64 device tensors [n_cells] (uint64 bit patterns) indexed by GLOBAL cell id:
+        this LOCAL context's sort key of every cell (-1 = ~0 when absent) and its reads here.  cell_map: int32
+        device tensor local id -> global id, or None (identity)."""
+        import torch
+        dev = torch.device("cuda", torch.cuda.current_device())
+        key = torch.empty(int(n_cells), dtype=torch.int64, device=dev)
+        total = torch.empty(int(n_cells), dtype=torch.int64, device=dev)
+        self._check(self._lib.ecb_cells_summary(self._ctx, _ptr(cell_map), 0 if cell_map is None else int(cell_map.numel()),
+                                                int(n_cells), key.data_ptr(), total.data_ptr()))
+        return key, total
+
+    def cells_order(self, cell_keys, cell_totals, min_cell_count, cell_map, world):
+        """The cell decision from the gathered keys [world * n_cells] and summed totals [n_cells] (int64 device
+        tensors).  -> (n_samples, cell_order: int32 device view [n_samples] of global cell ids)."""
+        import torch
+        n_samples, order = ctypes.c_int64(), ctypes.c_void_p()
+        self._check(self._lib.ecb_cells_order(self._ctx, int(world), cell_keys.data_ptr(), cell_totals.data_ptr(),
+                                              int(cell_totals.numel()), int(min_cell_count), _ptr(cell_map),
+                                              ctypes.byref(n_samples), ctypes.byref(order)))
+        dev = torch.device("cuda", torch.cuda.current_device())
+        return int(n_samples.value), _device_view(order.value, (int(n_samples.value),), "<i4", torch.int32, dev)
+
+    def cells_dispatch_counts(self, world, shard_lo=None, shard_hi=None):
+        """-> int64 device tensor [2 * world]: records of the next dispatch per destination rank (ECs, then pairs).
+        Without shards: dispatch 1 of this LOCAL context; with them: dispatch 2 of this OWNER context."""
+        import torch
+        counts = torch.empty(2 * int(world), dtype=torch.int64, device=torch.device("cuda", torch.cuda.current_device()))
+        lo = hi = None
+        if shard_lo is not None:
+            lo = (ctypes.c_int64 * world)(*[int(x) for x in shard_lo])
+            hi = (ctypes.c_int64 * world)(*[int(x) for x in shard_hi])
+        self._check(self._lib.ecb_cells_dispatch_counts(self._ctx, int(world), lo, hi, counts.data_ptr()))
+        return counts
+
+    def cells_arena_create(self, cap_ec, cap_pairs):
+        """-> (64-byte IPC handle, base address) of this OWNER context's per-cell arena; replaces an earlier one."""
+        handle = ctypes.create_string_buffer(64)
+        base = ctypes.c_void_p()
+        self._check(self._lib.ecb_cells_arena_create(self._ctx, int(cap_ec), int(cap_pairs), handle, ctypes.byref(base)))
+        return handle.raw, int(base.value)
+
+    def cells_export_to_arenas(self, bases, cap_ec, cap_pairs):
+        """Dispatch 1 of the per-cell exchange.  -> (min_base, max_end) of the positions pushed here."""
+        arr = (ctypes.c_void_p * len(bases))(*bases)
+        lo, hi = ctypes.c_int64(), ctypes.c_int64()
+        self._check(self._lib.ecb_cells_export_to_arenas(self._ctx, len(bases), arr, int(cap_ec), int(cap_pairs),
+                                                         ctypes.byref(lo), ctypes.byref(hi)))
+        return int(lo.value), int(hi.value)
+
+    def cells_import_arena(self):
+        self._check(self._lib.ecb_cells_import_arena(self._ctx))
+
+    def cells_order_dispatch(self, bases, cap_ec, cap_pairs, shard_lo, shard_hi):
+        arr = (ctypes.c_void_p * len(bases))(*bases)
+        lo = (ctypes.c_int64 * len(bases))(*[int(x) for x in shard_lo])
+        hi = (ctypes.c_int64 * len(bases))(*[int(x) for x in shard_hi])
+        self._check(self._lib.ecb_cells_order_dispatch(self._ctx, len(bases), arr, int(cap_ec), int(cap_pairs), lo, hi))
+
+    def cells_order_build(self, local, shard_lo, shard_hi, n_samples):
+        """-> dict(n_ec, nnz, a_indptr, a_indices, a_data, nnz_n, n_col_counts, n_indices, n_data): this rank's slice
+        as torch views of library memory (valid until the next call on this context); n_indices are local to
+        the slice."""
+        import torch
+        sl = EcbCellsSlice()
+        self._check(self._lib.ecb_cells_order_build(self._ctx, local._ctx, int(shard_lo), int(shard_hi), int(n_samples),
+                                                    ctypes.byref(sl)))
+        dev = torch.device("cuda", torch.cuda.current_device())
+        view = lambda p, n: _device_view(ctypes.cast(p, ctypes.c_void_p).value, (max(n, 1),), "<i4", torch.int32, dev)[:n]
+        return {"n_ec": int(sl.n_ec), "nnz": int(sl.nnz), "a_indptr": view(sl.a_indptr, sl.n_ec + 1),
+                "a_indices": view(sl.a_indices, sl.nnz), "a_data": view(sl.a_data, sl.nnz), "nnz_n": int(sl.nnz_n),
+                "n_col_counts": view(sl.n_col_counts, sl.n_samples), "n_indices": view(sl.n_indices, sl.nnz_n),
+                "n_data": view(sl.n_data, sl.nnz_n)}
 
     def stats(self):
         st = EcbStats()

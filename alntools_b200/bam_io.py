@@ -70,12 +70,18 @@ def write_bam(filename, references, alignments, block_payload=60000, level=6):
         fh.write(BGZF_EOF)
 
 
+_CID_FIELDS = b"|||CR|||x|||CY|||x|||UR|||x|||UY|||x|||BC|||x|||QT|||x|||CID|||cell"
+_CID_DIGITS = 7
+
+
 def write_bam_columns(filename, references, qname_ids, flags, tids, name_fmt="read%09d",
-                      block_payload=60000, level=1):
+                      block_payload=60000, level=1, cell_ids=None):
     """Vectorised writer for large synthetic BAMs: record i is (name_fmt % qname_ids[i], flags[i],
-    tids[i]); all names must have the same byte length."""
+    tids[i]); all names must have the same byte length.  cell_ids: per-record cell ids (< 10^7) put in field 14
+    of a 10x-style '|||'-separated name as 'cell%07d' (what the per-cell path reads)."""
     n = len(tids)
-    name_len = len(name_fmt % 0) + 1
+    tail = 0 if cell_ids is None else len(_CID_FIELDS) + _CID_DIGITS
+    name_len = len(name_fmt % 0) + tail + 1
     rec_len = 4 + 32 + name_len
     raw = np.zeros((n, rec_len), dtype=np.uint8)
     raw[:, 0:4] = np.frombuffer(struct.pack("<i", 32 + name_len), dtype=np.uint8)
@@ -93,12 +99,19 @@ def write_bam_columns(filename, references, qname_ids, flags, tids, name_fmt="re
     raw[:, 4:36] = core.view(np.uint8).reshape(n, 32)
     ids = np.asarray(qname_ids, dtype=np.int64)
     prefix = name_fmt.split("%")[0].encode()
-    ndig = name_len - 1 - len(prefix)
+    ndig = name_len - 1 - tail - len(prefix)
     raw[:, 36:36 + len(prefix)] = np.frombuffer(prefix, dtype=np.uint8)
     rem = ids.copy()
     for d in range(ndig - 1, -1, -1):
         raw[:, 36 + len(prefix) + d] = (rem % 10 + 48).astype(np.uint8)
         rem //= 10
+    if cell_ids is not None:
+        at = 36 + len(prefix) + ndig
+        raw[:, at:at + len(_CID_FIELDS)] = np.frombuffer(_CID_FIELDS, dtype=np.uint8)
+        rem = np.asarray(cell_ids, dtype=np.int64).copy()
+        for d in range(_CID_DIGITS - 1, -1, -1):
+            raw[:, at + len(_CID_FIELDS) + d] = (rem % 10 + 48).astype(np.uint8)
+            rem //= 10
     flat = raw.reshape(-1)
     per_block = max(1, block_payload // rec_len) * rec_len
     with open(filename, "wb") as fh:

@@ -171,69 +171,6 @@ def _convert_python_emitter(bam_filename, target_filename, device, start_time):
     return res, tables, cols.valid_alignments
 
 
-def _requested_gpus(devices):
-    """How many GPUs the caller asked for: the `devices` keyword, else the environment variable ALNTOOLS_GPUS
-    (the CLI keeps the reference's options, so the environment is its only way to say it), else one."""
-    if devices is not None:
-        return max(1, int(devices))
-    try:
-        return max(1, int(os.environ.get("ALNTOOLS_GPUS", "1") or 1))
-    except ValueError:
-        raise ValueError("ALNTOOLS_GPUS must be a number of GPUs, found %r" % os.environ.get("ALNTOOLS_GPUS"))
-
-
-def _under_launcher():
-    """True inside a one-process-per-GPU job (torchrun sets RANK / WORLD_SIZE / LOCAL_RANK)."""
-    return int(os.environ.get("WORLD_SIZE", "1") or 1) > 1 and "RANK" in os.environ
-
-
-def _spawn_ranks(n_gpus, kwargs):
-    """convert() on `n_gpus` GPUs from an ordinary call: one worker process per GPU (the contract of the
-    multi-GPU path), each running convert_rank on its shard of the file; rank 0 reports the totals."""
-    import json
-    import socket
-    import subprocess
-    import sys
-    import tempfile
-    with socket.socket() as sock:
-        sock.bind(("127.0.0.1", 0))
-        port = sock.getsockname()[1]
-    with tempfile.TemporaryDirectory(prefix="alntools_b200_") as tmp:
-        job = os.path.join(tmp, "job.json")
-        with open(job, "w") as fh:
-            json.dump(kwargs, fh)
-        procs = []
-        for rank in range(n_gpus):
-            env = dict(os.environ, RANK=str(rank), LOCAL_RANK=str(rank), WORLD_SIZE=str(n_gpus),
-                       MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), ALNTOOLS_B200_SUMMARY=os.path.join(tmp, "summary.json"),
-                       ALNTOOLS_B200_VERBOSE="1" if LOG.isEnabledFor(20) else "0")
-            procs.append(subprocess.Popen([sys.executable, "-m", "alntools_b200._rank_worker", job], env=env))
-        # one worker that fails would leave the others waiting in a collective: when the first non-zero exit code
-        # shows up the remaining workers (exactly the processes started above) are terminated
-        codes = [None] * n_gpus
-        while any(c is None for c in codes):
-            for i, p in enumerate(procs):
-                if codes[i] is None:
-                    codes[i] = p.poll()
-            if any(c not in (None, 0) for c in codes):
-                for i, p in enumerate(procs):
-                    if codes[i] is None:
-                        p.terminate()
-                for i, p in enumerate(procs):
-                    if codes[i] is None:
-                        try:
-                            codes[i] = p.wait(timeout=20)
-                        except subprocess.TimeoutExpired:
-                            p.kill()
-                            codes[i] = p.wait()
-                break
-            time.sleep(0.02)
-        if any(codes):
-            raise RuntimeError("multi-GPU bam2ec failed: worker exit codes %s" % codes)
-        with open(os.path.join(tmp, "summary.json")) as fh:
-            return json.load(fh)
-
-
 def convert_rank(bam_filename, ec_filename, emase_filename, num_chunks=0, number_processes=-1, temp_dir=None,
                  range_filename=None, sample=None, target_filename=None):
     """One rank of the multi-GPU convert (one process per GPU; RANK / WORLD_SIZE / LOCAL_RANK / MASTER_* in
@@ -363,14 +300,14 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
     job = dict(bam_filename=bam_filename, ec_filename=ec_filename, emase_filename=emase_filename, num_chunks=num_chunks,
                number_processes=number_processes, temp_dir=temp_dir, range_filename=range_filename, sample=sample,
                target_filename=target_filename)
-    if _under_launcher():
+    if utils.under_launcher():
         if emitter.use_python_emitter():
             raise NotImplementedError("the multi-GPU path needs the native emitter (unset ALNTOOLS_B200_EMITTER)")
         return convert_rank(**job)
-    if _requested_gpus(devices) > 1:
+    if utils.requested_gpus(devices) > 1:
         if emitter.use_python_emitter():
             raise NotImplementedError("the multi-GPU path needs the native emitter (unset ALNTOOLS_B200_EMITTER)")
-        return _spawn_ranks(_requested_gpus(devices), job)
+        return utils.spawn_ranks(utils.requested_gpus(devices), job)
     if range_filename is not None and emitter.use_python_emitter():
         raise NotImplementedError("--rangefile needs the native emitter (unset ALNTOOLS_B200_EMITTER)")
     num_chunks, num_processes = _job_plan(num_chunks, number_processes)

@@ -108,6 +108,35 @@ def ec_header_bytes(haplotypes, target_names, lengths, sample_names, target_sect
     return b"".join(parts)
 
 
+def _a_layout(header_bytes, n_ec_total, nnz_total):
+    """Byte offsets of the A (CSR) section behind the header: len(indptr), nnz, indptr[E + 1], indices[Z],
+    data[Z].  -> (a_at, a_indptr_at, a_indices_at, a_data_at, end)."""
+    E, Z = int(n_ec_total), int(nnz_total)
+    a_at = header_bytes
+    a_indptr_at = a_at + 8
+    a_indices_at = a_indptr_at + 4 * (E + 1)
+    a_data_at = a_indices_at + 4 * Z
+    return a_at, a_indptr_at, a_indices_at, a_data_at, a_data_at + 4 * Z
+
+
+def _create_a(fh, header, n_ec_total, nnz_total):
+    """Header sections, the A sizes and indptr[0] (the part of the file only its creator writes)."""
+    fh.write(header)
+    fh.write(struct.pack("<ii", int(n_ec_total) + 1, int(nnz_total)))
+    fh.write(struct.pack("<i", 0))
+
+
+def _write_a_slice(fd, layout, id_base, nnz_base, a_indptr_local, a_indices, a_data):
+    """A slice's byte ranges of the A section: indptr[id_base + 1 ..], indices and data at nnz_base."""
+    _, a_indptr_at, a_indices_at, a_data_at, _ = layout
+    if len(a_indptr_local) > 1:
+        indptr = (np.asarray(a_indptr_local[1:], dtype=np.int64) + int(nnz_base)).astype("<i4")
+        os.pwrite(fd, _i32(indptr), a_indptr_at + 4 * (int(id_base) + 1))
+    if len(a_indices):
+        os.pwrite(fd, _i32(a_indices), a_indices_at + 4 * int(nnz_base))
+        os.pwrite(fd, _i32(a_data), a_data_at + 4 * int(nnz_base))
+
+
 def ecsave2_slice(ec_filename, header, n_ec_total, nnz_total, id_base, nnz_base, a_indptr_local, a_indices, a_data,
                   counts, create):
     """Single-sample EC file written by several processes, each holding the ECs [id_base, id_base + n) of the
@@ -116,37 +145,69 @@ def ecsave2_slice(ec_filename, header, n_ec_total, nnz_total, id_base, nnz_base,
     file out (header sections, the four size fields, indptr[0], N's indptr) and must run first.
     a_indptr_local: [n + 1] offsets local to the slice (a_indptr_local[0] == 0); nnz_base = non-zeros of the
     slices in front.  Same bytes as ecsave2_arrays on the assembled matrices (alntools/bin_utils.py:105-277)."""
-    E, Z = int(n_ec_total), int(nnz_total)
+    E = int(n_ec_total)
     n = len(counts)
-    hdr = len(header)
-    a_at = hdr                                   # A: len(indptr), nnz, indptr[E + 1], indices[Z], data[Z]
-    a_indptr_at = a_at + 8
-    a_indices_at = a_indptr_at + 4 * (E + 1)
-    a_data_at = a_indices_at + 4 * Z
-    n_at = a_data_at + 4 * Z                     # N: 2, E, [0, E], indices[E] = 0..E-1, data[E] = counts
+    layout = _a_layout(len(header), n_ec_total, nnz_total)
+    n_at = layout[4]                             # N: 2, E, [0, E], indices[E] = 0..E-1, data[E] = counts
     n_indices_at = n_at + 16
     n_data_at = n_indices_at + 4 * E
     total = n_data_at + 4 * E
     if create:
         with open(ec_filename, "wb") as fh:
-            fh.write(header)
-            fh.write(struct.pack("<ii", E + 1, Z))
-            fh.write(struct.pack("<i", 0))
+            _create_a(fh, header, n_ec_total, nnz_total)
             fh.truncate(total)
             fh.seek(n_at)
             fh.write(struct.pack("<iiii", 2, E, 0, E))
     fd = os.open(ec_filename, os.O_WRONLY)
     try:
+        _write_a_slice(fd, layout, id_base, nnz_base, a_indptr_local, a_indices, a_data)
         if n:
-            indptr = (np.asarray(a_indptr_local[1:], dtype=np.int64) + int(nnz_base)).astype("<i4")
-            os.pwrite(fd, _i32(indptr), a_indptr_at + 4 * (int(id_base) + 1))
             os.pwrite(fd, _i32(np.arange(int(id_base), int(id_base) + n, dtype=np.int32)), n_indices_at + 4 * int(id_base))
             os.pwrite(fd, _i32(counts), n_data_at + 4 * int(id_base))
-        if len(a_indices):
-            os.pwrite(fd, _i32(a_indices), a_indices_at + 4 * int(nnz_base))
-            os.pwrite(fd, _i32(a_data), a_data_at + 4 * int(nnz_base))
     finally:
         os.close(fd)
+
+
+def ecsave2_cells_slice(ec_filename, header, n_ec_total, nnz_total, id_base, nnz_base, a_indptr_local, a_indices, a_data,
+                        n_indptr, n_col_counts, n_col_offset, n_indices_local, n_data, create):
+    """Per-cell EC file written by several processes, each holding the ECs [id_base, id_base + n) (as
+    ecsave2_slice; `header` names the cells in column order).  The A part is written as by ecsave2_slice.  N
+    (CSC, E x S): this process holds, for every column c, n_col_counts[c] entries (n_indices_local: EC ids local
+    to the slice, ascending inside a column; n_data: counts; both in column-major order); they go to
+    n_indptr[c] + n_col_offset[c] on, where n_col_offset[c] = entries of column c held by the slices in front in
+    id order, in one vectorised scatter.  The process with create=True lays the file out (header, sizes, the
+    global n_indptr [S + 1]) and must run first.  Same bytes as ecsave2_arrays on the assembled matrices."""
+    n_indptr = np.asarray(n_indptr, dtype=np.int64)
+    S, nnz_n = len(n_indptr) - 1, int(n_indptr[-1])
+    layout = _a_layout(len(header), n_ec_total, nnz_total)
+    n_at = layout[4]                             # N: S + 1, nnz, indptr[S + 1], indices[nnz], data[nnz]
+    n_indices_at = n_at + 8 + 4 * (S + 1)
+    n_data_at = n_indices_at + 4 * nnz_n
+    if create:
+        with open(ec_filename, "wb") as fh:
+            _create_a(fh, header, n_ec_total, nnz_total)
+            fh.truncate(n_data_at + 4 * nnz_n)
+            fh.seek(n_at)
+            fh.write(struct.pack("<ii", S + 1, nnz_n))
+            fh.write(_i32(n_indptr.astype("<i4")))
+    fd = os.open(ec_filename, os.O_WRONLY)
+    try:
+        _write_a_slice(fd, layout, id_base, nnz_base, a_indptr_local, a_indices, a_data)
+    finally:
+        os.close(fd)
+    counts = np.asarray(n_col_counts, dtype=np.int64)
+    m = int(counts.sum())
+    if m:
+        if len(n_indices_local) != m or len(n_data) != m:
+            raise ValueError("%d N entries given, the column counts say %d" % (len(n_indices_local), m))
+        starts = np.cumsum(counts) - counts
+        col = np.repeat(np.arange(S), counts)
+        dest = n_indptr[col] + np.asarray(n_col_offset, dtype=np.int64)[col] + (np.arange(m) - starts[col])
+        section = np.memmap(ec_filename, dtype="<i4", mode="r+", offset=n_indices_at, shape=(2, nnz_n))
+        section[0, dest] = np.asarray(n_indices_local, dtype=np.int64) + int(id_base)
+        section[1, dest] = n_data
+        section.flush()
+        del section
 
 
 def ecload_arrays(ec_filename):

@@ -16,6 +16,7 @@
 #include "ecb_sort.cuh"
 #include "ecb_cells.cuh"
 #include "ecb_exchange.cuh"
+#include "ecb_cells_exchange.cuh"
 
 namespace {
 
@@ -85,7 +86,11 @@ struct ecb_ctx {
   // arena of the multi-GPU exchange (plain cudaMalloc: must be exportable through CUDA IPC)
   void* xa_base = nullptr;
   int64_t xa_cap_ec = 0;
+  int64_t xa_cap_pairs = 0;                  // > 0: a per-cell arena (ecb_cells_arena_create)
   std::vector<void*> xa_opened;
+  // per-cell exchange: kept reads per local EC, column of every global cell, entries per column of the slice
+  DevBuf cx_kept, cx_col_of_cell, cx_col_counts;
+  u32 cx_n_local_cells = 0;
   std::string err;
 };
 
@@ -424,13 +429,12 @@ CellParams make_cell_params(ecb_ctx* c, const CellResult* cr) {
   return P;
 }
 
-// Cell order, minimum-count filter and the ec_keep flags (bam_utils_multisample.py:503-636).
-int cells_prepare(ecb_ctx* c, int64_t min_cell_count, CellResult* cr) {
+// The local passes over the (file, EC, cell) table: every cell's sort key and total, the (EC, cell) counts
+// summed over files (cr->n_cells = largest cell id + 1).  Needs at least one triple.
+int cells_local(ecb_ctx* c, CellResult* cr) {
   CellScratch& S = c->cells;
   if (c->max_end - c->min_base > 0xFFFFFFFFull)
     return fail(c, ECB_ERR_LIMIT, "per-cell mode needs the pushed order range to span less than 2^32 positions");
-  if (c->n_triples == 0) return fail(c, ECB_ERR_EMPTY, "no (EC, cell) counts were recorded");
-  const u64 min_count = min_cell_count <= 0 ? 1ull : (u64)min_cell_count;  // :596-597
   S.fe_slots = std::max<u32>(1024u, pow2_ceil((u64)c->n_triples * 2));
   S.pair_slots = S.fe_slots;
   CKR(ensure(c, S.fe_table, (size_t)S.fe_slots * sizeof(EcbEntry)));
@@ -461,6 +465,19 @@ int cells_prepare(ecb_ctx* c, int64_t min_cell_count, CellResult* cr) {
   LAUNCH_CHECK("cells_pass2");
   cells_total_reduce_kernel<<<grid_for(n_cells, 256, c->sm_count * 8), 256, 0, c->stream>>>((u64*)S.cell_total.p, n_cells);
   LAUNCH_CHECK("cells_total_reduce");
+  return ECB_OK;
+}
+
+// Cell order, minimum-count filter and the ec_keep flags (bam_utils_multisample.py:503-636).
+int cells_prepare(ecb_ctx* c, int64_t min_cell_count, CellResult* cr) {
+  CellScratch& S = c->cells;
+  if (c->max_end - c->min_base > 0xFFFFFFFFull)
+    return fail(c, ECB_ERR_LIMIT, "per-cell mode needs the pushed order range to span less than 2^32 positions");
+  if (c->n_triples == 0) return fail(c, ECB_ERR_EMPTY, "no (EC, cell) counts were recorded");
+  const u64 min_count = min_cell_count <= 0 ? 1ull : (u64)min_cell_count;  // :596-597
+  CKR(cells_local(c, cr));
+  const u32 n_cells = (u32)cr->n_cells;
+  CellParams P = make_cell_params(c, cr);
 
   // order the cells by their nested first-occurrence key
   CKR(ensure(c, S.sort_k[0], (size_t)n_cells * 8));
@@ -532,7 +549,7 @@ void cells_release(ecb_ctx* c) {
 
 extern "C" {
 
-int ecb_version(void) { return 2000; }
+int ecb_version(void) { return 2001; }
 
 const char* ecb_last_error(const ecb_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
@@ -1058,6 +1075,9 @@ int ecb_arena_reset(ecb_ctx* c) {
   if (!c || !c->xa_base) return ECB_ERR_INVALID;
   CK(cudaSetDevice(c->device));
   CK(cudaMemsetAsync(c->xa_base, 0, ECB_ARENA_HEADER_BYTES, c->stream));
+  if (c->xa_cap_pairs)   // the pair area's header
+    CK(cudaMemsetAsync((char*)c->xa_base + ECB_ARENA_HEADER_BYTES + (size_t)c->xa_cap_ec * ECB_KEYREC_WORDS * 8, 0,
+                       ECB_ARENA_HEADER_BYTES, c->stream));
   // on a caller-provided stream (ecb_set_stream) the call is stream-ordered - a collective on that stream is the
   // barrier in front of the peers' stores; a context on its own stream synchronises
   if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));
@@ -1101,6 +1121,8 @@ int ecb_export_to_arenas(ecb_ctx* c, int world, void* const* arena_bases, int64_
   return ECB_OK;
 }
 
+static int import_keys(ecb_ctx* c, const unsigned long long* rec, u64 n_rec);
+
 int ecb_import_arena(ecb_ctx* c) {
   if (!c || !c->xa_base) return ECB_ERR_INVALID;
   CK(cudaSetDevice(c->device));
@@ -1109,7 +1131,11 @@ int ecb_import_arena(ecb_ctx* c) {
   CK(cudaStreamSynchronize(c->stream));
   if (hdr[2] || hdr[0] > (unsigned long long)c->xa_cap_ec)
     return fail(c, ECB_ERR_LIMIT, "exchange arena too small: %llu records arrived, capacity %lld", hdr[0], (long long)c->xa_cap_ec);
-  const u64 n_rec = hdr[0];
+  return import_keys(c, (const unsigned long long*)((const char*)c->xa_base + ECB_ARENA_HEADER_BYTES), hdr[0]);
+}
+
+// Owner merge of n_rec dispatch-1 EC records (ecb_import_arena, ecb_cells_import_arena).
+static int import_keys(ecb_ctx* c, const unsigned long long* rec, u64 n_rec) {
   if (n_rec == 0) return ECB_OK;
   if (n_rec > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "too many records in one import");
   if (!c->table_slots) CKR(init_table(c));
@@ -1117,7 +1143,7 @@ int ecb_import_arena(ecb_ctx* c) {
   const u64 need = ((u64)c->n_ec + n_rec) * 2;
   if (need > c->table_slots) CKR(grow_table(c, pow2_ceil(need)));
   KeyImportParams P{};
-  P.rec = (const unsigned long long*)((const char*)c->xa_base + ECB_ARENA_HEADER_BYTES);
+  P.rec = rec;
   P.n_rec = (u32)n_rec;
   P.table = (EcbEntry*)c->table.p;
   P.mask = c->table_slots - 1;
@@ -1128,6 +1154,27 @@ int ecb_import_arena(ecb_ctx* c) {
   CKR(sync_counters(c));   // the one round trip of the merge: the number of merged ECs is known to the host again
   CKR(check_device_error(c));
   c->n_ec = c->h_ctr->n_ec;
+  return ECB_OK;
+}
+
+// Shards with alignments, by position, and the rank that holds each (dispatch 2); they must not overlap (one
+// read order over all ranks).
+static int shard_routes(ecb_ctx* c, int world, const int64_t* shard_lo, const int64_t* shard_hi, u64* lo, u32* dest,
+                        u32* n_shards) {
+  std::vector<int> order;
+  for (int r = 0; r < world; ++r)
+    if (shard_hi[r] > shard_lo[r]) order.push_back(r);
+  std::sort(order.begin(), order.end(), [&](int a, int b) { return shard_lo[a] < shard_lo[b]; });
+  if (order.empty()) return fail(c, ECB_ERR_STATE, "no rank has pushed alignments");
+  for (size_t k = 0; k < order.size(); ++k) {
+    if (k && shard_lo[order[k]] < shard_hi[order[k - 1]])
+      return fail(c, ECB_ERR_INVALID, "the ranks' order_base ranges overlap");
+    if (shard_hi[order[k]] - shard_lo[order[k]] > 0xFFFFFFFEll)
+      return fail(c, ECB_ERR_LIMIT, "a rank's alignments span more than 2^32 positions");
+    lo[k] = (u64)shard_lo[order[k]];
+    dest[k] = (u32)order[k];
+  }
+  *n_shards = (u32)order.size();
   return ECB_OK;
 }
 
@@ -1142,21 +1189,7 @@ int ecb_order_dispatch(ecb_ctx* c, int world, void* const* arena_bases, int64_t 
   P.ec_slot = (const u32*)c->ec_slot.p;
   P.n_ec = c->n_ec;
   P.world = (u32)world;
-  // shards with alignments, by position; they must not overlap (one read order over all ranks)
-  std::vector<int> order;
-  for (int r = 0; r < world; ++r)
-    if (shard_hi[r] > shard_lo[r]) order.push_back(r);
-  std::sort(order.begin(), order.end(), [&](int a, int b) { return shard_lo[a] < shard_lo[b]; });
-  if (order.empty()) return fail(c, ECB_ERR_STATE, "no rank has pushed alignments");
-  for (size_t k = 0; k < order.size(); ++k) {
-    if (k && shard_lo[order[k]] < shard_hi[order[k - 1]])
-      return fail(c, ECB_ERR_INVALID, "the ranks' order_base ranges overlap");
-    if (shard_hi[order[k]] - shard_lo[order[k]] > 0xFFFFFFFEll)
-      return fail(c, ECB_ERR_LIMIT, "a rank's alignments span more than 2^32 positions");
-    P.lo[k] = (u64)shard_lo[order[k]];
-    P.dest[k] = (u32)order[k];
-  }
-  P.n_shards = (u32)order.size();
+  CKR(shard_routes(c, world, shard_lo, shard_hi, P.lo, P.dest, &P.n_shards));
   ArenaTargets A{};
   CKR(arena_targets(c, &A, world, arena_bases, cap_records));
   ecb_key_dispatch_kernel<true><<<grid_for(c->n_ec, 256, c->sm_count * 8), 256, 0, c->stream>>>(P, A);
@@ -1233,6 +1266,370 @@ int ecb_order_build(ecb_ctx* c, const ecb_ctx* local, int64_t shard_lo, int64_t 
   return ECB_OK;
 }
 
+// ---- the per-cell exchange (see include/ecb200.h and ecb_cells_exchange.cuh) ------------------------------
+
+int ecb_cells_summary(ecb_ctx* c, const int32_t* cell_map, int64_t map_len, int64_t n_cells, uint64_t* cell_key,
+                      uint64_t* cell_total) {
+  if (!c || !cell_key || !cell_total || n_cells < 1 || n_cells > 0x7FFFFFFFll || (cell_map && map_len < 0))
+    return ECB_ERR_INVALID;
+  if (!c->with_cells) return fail(c, ECB_ERR_INVALID, "the per-cell exchange needs a context created with cells");
+  CK(cudaSetDevice(c->device));
+  CK(cudaMemsetAsync(cell_key, 0xFF, (size_t)n_cells * 8, c->stream));
+  CK(cudaMemsetAsync(cell_total, 0, (size_t)n_cells * 8, c->stream));
+  c->cx_n_local_cells = 0;
+  if (!c->table_slots || c->n_triples == 0) return ECB_OK;   // a rank without reads takes part with an empty summary
+  CellResult cr{};
+  CKR(cells_local(c, &cr));
+  const u32 n_local = (u32)cr.n_cells;
+  if (cell_map && (int64_t)n_local > map_len)
+    return fail(c, ECB_ERR_INVALID, "local cell id %u outside the cell map of %lld entries", n_local - 1, (long long)map_len);
+  c->cx_n_local_cells = n_local;
+  CK(cudaMemsetAsync(&c->d_ctr->scratch[5], 0, sizeof(u32), c->stream));
+  cells_summary_kernel<<<grid_for(n_local, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+      (const u64*)c->cells.cell_key.p, (const u64*)c->cells.cell_total.p, n_local, cell_map, (u32)n_cells, (u64*)cell_key,
+      (u64*)cell_total, &c->d_ctr->scratch[5]);
+  LAUNCH_CHECK("cells_summary");
+  CKR(sync_counters(c));
+  if (c->h_ctr->scratch[5]) return fail(c, ECB_ERR_INVALID, "a cell id lies outside the %lld global cells", (long long)n_cells);
+  return ECB_OK;
+}
+
+int ecb_cells_order(ecb_ctx* c, int world, const uint64_t* cell_keys, const uint64_t* cell_totals, int64_t n_cells,
+                    int64_t min_cell_count, const int32_t* cell_map, int64_t* n_samples, const int32_t** cell_order) {
+  if (!c || !cell_keys || !cell_totals || !n_samples || !cell_order || n_cells < 1 || n_cells > 0x7FFFFFFFll)
+    return ECB_ERR_INVALID;
+  if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
+  if (!c->with_cells) return fail(c, ECB_ERR_INVALID, "the per-cell exchange needs a context created with cells");
+  CK(cudaSetDevice(c->device));
+  *n_samples = 0;
+  *cell_order = nullptr;
+  CellScratch& S = c->cells;
+  const u32 C = (u32)n_cells;
+  const u64 min_count = min_cell_count <= 0 ? 1ull : (u64)min_cell_count;  // bam_utils_multisample.py:596-597
+  // sort by (first rank that holds the cell, its key there): on the key, then stably on the rank
+  CKR(ensure(c, S.sort_k[0], (size_t)C * 8));
+  CKR(ensure(c, S.sort_v[0], (size_t)C * 4));
+  const int g_c = grid_for(C, 256, c->sm_count * 8);
+  cells_first_key_kernel<<<g_c, 256, 0, c->stream>>>((const u64*)cell_keys, (u32)world, C, (u64*)S.sort_k[0].p, (u32*)S.sort_v[0].p);
+  LAUNCH_CHECK("cells_first_key");
+  int rb = 0;
+  CKR(radix_sort(c, C, 64, &rb));
+  cells_first_rank_kernel<<<g_c, 256, 0, c->stream>>>((const u64*)cell_keys, (u32)world, C, (const u32*)S.sort_v[rb].p,
+                                                      (u64*)S.sort_k[0].p, (u32*)S.sort_v[0].p);
+  LAUNCH_CHECK("cells_first_rank");
+  CKR(radix_sort(c, C, 8, &rb));
+  CKR(ensure(c, S.flags, (size_t)C * 4));
+  CKR(ensure(c, S.offsets, (size_t)C * 4));
+  cells_keep_flags_kernel<<<g_c, 256, 0, c->stream>>>((const u64*)S.sort_k[rb].p, (const u32*)S.sort_v[rb].p, C,
+                                                      (const u64*)cell_totals, min_count, (u32*)S.flags.p);
+  LAUNCH_CHECK("cells_keep_flags");
+  u64 n_kept = 0;
+  CKR(device_scan<false>(c, (const u32*)S.flags.p, (u32*)S.offsets.p, C, 0, &n_kept));
+  if (n_kept == 0) return fail(c, ECB_ERR_EMPTY, "no cell reaches the minimum count %llu", (unsigned long long)min_count);
+  CKR(ensure(c, c->cx_col_of_cell, (size_t)C * 4));
+  CKR(ensure(c, c->r_cell_order, (size_t)C * 4));
+  cells_assign_kernel<<<g_c, 256, 0, c->stream>>>((const u64*)S.sort_k[rb].p, (const u32*)S.sort_v[rb].p, C,
+                                                  (const u64*)cell_totals, min_count, (const u32*)S.offsets.p,
+                                                  (int32_t*)c->cx_col_of_cell.p, (int32_t*)c->r_cell_order.p);
+  LAUNCH_CHECK("cells_assign");
+  // this rank's side: the column of every local cell, and the reads of every local EC in kept cells
+  CKR(ensure(c, c->cx_kept, (size_t)std::max<u32>(c->n_ec, 1) * 4));
+  CK(cudaMemsetAsync(c->cx_kept.p, 0, (size_t)std::max<u32>(c->n_ec, 1) * 4, c->stream));
+  if (c->cx_n_local_cells) {
+    cells_local_columns_kernel<<<grid_for(c->cx_n_local_cells, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+        cell_map, c->cx_n_local_cells, (const int32_t*)c->cx_col_of_cell.p, C, (int32_t*)S.cell_new.p);
+    LAUNCH_CHECK("cells_local_columns");
+    cells_kept_reads_kernel<<<grid_for(S.pair_slots, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+        (const EcbEntry*)S.pair_table.p, S.pair_slots - 1, (const EcbEntry*)c->table.p, (const int32_t*)S.cell_new.p,
+        (u32*)c->cx_kept.p);
+    LAUNCH_CHECK("cells_kept_reads");
+  }
+  if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));
+  *n_samples = (int64_t)n_kept;
+  *cell_order = (const int32_t*)c->r_cell_order.p;
+  return ECB_OK;
+}
+
+// Both record areas of every rank's per-cell arena (the same capacities on every rank).  The device-side overflow
+// flag is set by the record width of the dispatch (`order`: dispatch 2), so that it fires at the capacity in
+// records the host checks.
+static int cells_arena_targets(ecb_ctx* c, ArenaTargets* E, ArenaTargets* P, int world, void* const* bases, int64_t cap_ec,
+                               int64_t cap_pairs, bool order) {
+  CKR(arena_targets(c, E, world, bases, cap_ec));
+  E->cap_words = (unsigned long long)cap_ec * (order ? ECB_ORDREC_WORDS : ECB_KEYREC_WORDS);
+  for (int r = 0; r < world; ++r) {
+    char* b = (char*)bases[r] + ECB_ARENA_HEADER_BYTES + (size_t)cap_ec * ECB_KEYREC_WORDS * 8;
+    P->hdr[r] = (unsigned long long*)b;
+    P->rec[r] = (unsigned long long*)(b + ECB_ARENA_HEADER_BYTES);
+  }
+  P->cap_words = (unsigned long long)cap_pairs * (order ? ECB_CPAIR2_WORDS : ECB_CPAIR1_WORDS);
+  return ECB_OK;
+}
+
+static void key_dispatch_params(ecb_ctx* c, int world, KeyDispatchParams* K) {
+  K->table = (const EcbEntry*)c->table.p;
+  K->ec_slot = (const u32*)c->ec_slot.p;
+  K->n_ec = c->table_slots ? c->n_ec : 0;
+  K->world = (u32)world;
+}
+
+int ecb_cells_dispatch_counts(ecb_ctx* c, int world, const int64_t* shard_lo, const int64_t* shard_hi, int64_t* counts) {
+  if (!c || !counts || (!shard_lo) != (!shard_hi)) return ECB_ERR_INVALID;
+  if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
+  CK(cudaSetDevice(c->device));
+  CK(cudaMemsetAsync(counts, 0, (size_t)world * 2 * 8, c->stream));
+  KeyDispatchParams K{};
+  key_dispatch_params(c, world, &K);
+  CellPairDispatchParams P{};
+  P.ec_table = K.table;
+  P.ec_slot = K.ec_slot;
+  P.world = (u32)world;
+  if (shard_lo) {   // dispatch 2, an owner context
+    if (K.n_ec == 0) return ECB_OK;
+    CKR(shard_routes(c, world, shard_lo, shard_hi, K.lo, K.dest, &K.n_shards));
+    memcpy(P.lo, K.lo, sizeof P.lo);
+    memcpy(P.dest, K.dest, sizeof P.dest);
+    P.n_shards = K.n_shards;
+    P.pair_table = (const EcbEntry*)c->cells.pair_table.p;
+    P.pair_slots = c->xa_cap_pairs ? c->cells.pair_slots : 0;
+    cells_dispatch_count_kernel<true><<<c->sm_count * 4, 256, 0, c->stream>>>(K, P, (unsigned long long*)counts);
+  } else {          // dispatch 1, a local context after ecb_cells_order
+    if (K.n_ec && !c->cx_kept.p) return fail(c, ECB_ERR_STATE, "ecb_cells_order has not run on this context");
+    P.pair_table = (const EcbEntry*)c->cells.pair_table.p;
+    P.pair_slots = c->cx_n_local_cells ? c->cells.pair_slots : 0;
+    P.cell_new = (const int32_t*)c->cells.cell_new.p;
+    if (K.n_ec == 0 && P.pair_slots == 0) return ECB_OK;
+    cells_dispatch_count_kernel<false><<<c->sm_count * 4, 256, 0, c->stream>>>(K, P, (unsigned long long*)counts);
+  }
+  LAUNCH_CHECK("cells_dispatch_count");
+  if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));   // counts are read on another stream
+  return ECB_OK;
+}
+
+int ecb_cells_arena_create(ecb_ctx* c, int64_t cap_ec, int64_t cap_pairs, void* ipc_handle_out, void** base_out) {
+  if (!c || cap_ec < 1 || cap_pairs < 1 || !base_out) return ECB_ERR_INVALID;
+  CK(cudaSetDevice(c->device));
+  // a smaller arena of an earlier call is replaced: nothing in flight may still use it or the peers' old ones
+  CK(cudaStreamSynchronize(c->stream));
+  for (void* p : c->xa_opened) CK(cudaIpcCloseMemHandle(p));
+  c->xa_opened.clear();
+  if (c->xa_base) CK(cudaFree(c->xa_base));
+  c->xa_base = nullptr;
+  c->xa_cap_ec = c->xa_cap_pairs = 0;
+  const size_t pair_hdr = ECB_ARENA_HEADER_BYTES + (size_t)cap_ec * ECB_KEYREC_WORDS * 8;
+  const size_t bytes = pair_hdr + ECB_ARENA_HEADER_BYTES + (size_t)cap_pairs * ECB_CPAIR1_WORDS * 8;
+  CK(cudaMalloc(&c->xa_base, bytes));
+  CK(cudaMemset(c->xa_base, 0, ECB_ARENA_HEADER_BYTES));
+  CK(cudaMemset((char*)c->xa_base + pair_hdr, 0, ECB_ARENA_HEADER_BYTES));
+  c->xa_cap_ec = cap_ec;
+  c->xa_cap_pairs = cap_pairs;
+  if (ipc_handle_out) {
+    cudaIpcMemHandle_t h;
+    CK(cudaIpcGetMemHandle(&h, c->xa_base));
+    memcpy(ipc_handle_out, &h, sizeof h);
+  }
+  *base_out = c->xa_base;
+  return ECB_OK;
+}
+
+int ecb_cells_export_to_arenas(ecb_ctx* c, int world, void* const* arena_bases, int64_t cap_ec, int64_t cap_pairs,
+                               int64_t* min_base, int64_t* max_end) {
+  if (!c || !arena_bases || cap_ec < 1 || cap_pairs < 1) return ECB_ERR_INVALID;
+  if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
+  if (!c->with_cells) return fail(c, ECB_ERR_INVALID, "the per-cell exchange needs a context created with cells");
+  CK(cudaSetDevice(c->device));
+  const u32 n_ec = c->table_slots ? c->n_ec : 0;
+  if (min_base) *min_base = n_ec ? (int64_t)c->min_base : 0;
+  if (max_end) *max_end = n_ec ? (int64_t)c->max_end : 0;
+  if (n_ec == 0) return ECB_OK;
+  if (!c->cx_kept.p) return fail(c, ECB_ERR_STATE, "ecb_cells_order has not run on this context");
+  ArenaTargets E{}, A{};
+  CKR(cells_arena_targets(c, &E, &A, world, arena_bases, cap_ec, cap_pairs, false));
+  // EVERY local EC goes, with the reads it has in kept cells (0 too: this rank may hold its first occurrence)
+  KeyDispatchParams K{};
+  key_dispatch_params(c, world, &K);
+  K.count_of = (const u32*)c->cx_kept.p;
+  ecb_key_dispatch_kernel<false><<<grid_for(n_ec, 256, c->sm_count * 8), 256, 0, c->stream>>>(K, E);
+  LAUNCH_CHECK("cells_export_ecs");
+  if (c->cx_n_local_cells) {
+    CellPairDispatchParams P{};
+    P.pair_table = (const EcbEntry*)c->cells.pair_table.p;
+    P.pair_slots = c->cells.pair_slots;
+    P.ec_table = K.table;
+    P.cell_new = (const int32_t*)c->cells.cell_new.p;
+    P.world = (u32)world;
+    cells_pair_dispatch_kernel<false><<<grid_for(P.pair_slots, 256, c->sm_count * 8), 256, 0, c->stream>>>(P, A);
+    LAUNCH_CHECK("cells_export_pairs");
+  }
+  if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));   // (as ecb_export_to_arenas)
+  return ECB_OK;
+}
+
+// Both headers {records, unused, overflow} of this context's per-cell arena (one host round trip).
+static int cells_arena_headers(ecb_ctx* c, unsigned long long* h_ec, unsigned long long* h_pair) {
+  CK(cudaMemcpyAsync(h_ec, c->xa_base, 3 * 8, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(h_pair, (const char*)c->xa_base + ECB_ARENA_HEADER_BYTES + (size_t)c->xa_cap_ec * ECB_KEYREC_WORDS * 8,
+                     3 * 8, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  if (h_ec[2] || h_ec[0] > (unsigned long long)c->xa_cap_ec || h_pair[2] || h_pair[0] > (unsigned long long)c->xa_cap_pairs)
+    return fail(c, ECB_ERR_LIMIT, "exchange arena too small: %llu ECs and %llu pairs arrived, capacity %lld and %lld", h_ec[0],
+                h_pair[0], (long long)c->xa_cap_ec, (long long)c->xa_cap_pairs);
+  return ECB_OK;
+}
+
+static const unsigned long long* cells_pair_records(const ecb_ctx* c) {
+  return (const unsigned long long*)((const char*)c->xa_base + 2 * ECB_ARENA_HEADER_BYTES +
+                                     (size_t)c->xa_cap_ec * ECB_KEYREC_WORDS * 8);
+}
+
+int ecb_cells_import_arena(ecb_ctx* c) {
+  if (!c || !c->xa_base || !c->xa_cap_pairs) return ECB_ERR_INVALID;
+  CK(cudaSetDevice(c->device));
+  unsigned long long h_ec[3], h_pair[3];
+  CKR(cells_arena_headers(c, h_ec, h_pair));
+  CKR(import_keys(c, (const unsigned long long*)((const char*)c->xa_base + ECB_ARENA_HEADER_BYTES), h_ec[0]));
+  const u64 n_pair = h_pair[0];
+  if (n_pair > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "too many records in one import");
+  if (n_pair && !c->table_slots) return fail(c, ECB_ERR_INVALID, "pairs arrived without their ECs");
+  CellScratch& S = c->cells;
+  S.pair_slots = std::max<u32>(1024u, pow2_ceil(n_pair * 2));
+  CKR(ensure(c, S.pair_table, (size_t)S.pair_slots * sizeof(EcbEntry)));
+  CK(cudaMemsetAsync(S.pair_table.p, 0xFF, (size_t)S.pair_slots * sizeof(EcbEntry), c->stream));
+  if (n_pair) {
+    cells_pair_import_kernel<<<grid_for(n_pair, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+        cells_pair_records(c), (u32)n_pair, (const EcbEntry*)c->table.p, c->table_slots - 1, (EcbEntry*)S.pair_table.p,
+        S.pair_slots - 1, c->d_ctr);
+    LAUNCH_CHECK("cells_import_pairs");
+    CKR(sync_counters(c));
+    CKR(check_device_error(c));
+  }
+  return ECB_OK;
+}
+
+int ecb_cells_order_dispatch(ecb_ctx* c, int world, void* const* arena_bases, int64_t cap_ec, int64_t cap_pairs,
+                             const int64_t* shard_lo, const int64_t* shard_hi) {
+  if (!c || !arena_bases || !shard_lo || !shard_hi || cap_ec < 1 || cap_pairs < 1 || !c->xa_cap_pairs) return ECB_ERR_INVALID;
+  if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
+  CK(cudaSetDevice(c->device));
+  KeyDispatchParams K{};
+  key_dispatch_params(c, world, &K);
+  if (K.n_ec == 0) return ECB_OK;
+  CKR(shard_routes(c, world, shard_lo, shard_hi, K.lo, K.dest, &K.n_shards));
+  ArenaTargets E{}, A{};
+  CKR(cells_arena_targets(c, &E, &A, world, arena_bases, cap_ec, cap_pairs, true));
+  ecb_key_dispatch_kernel<true, true><<<grid_for(K.n_ec, 256, c->sm_count * 8), 256, 0, c->stream>>>(K, E);
+  LAUNCH_CHECK("cells_order_dispatch_ecs");
+  CellPairDispatchParams P{};
+  P.pair_table = (const EcbEntry*)c->cells.pair_table.p;
+  P.pair_slots = c->cells.pair_slots;
+  P.ec_table = K.table;
+  P.ec_slot = K.ec_slot;
+  P.world = (u32)world;
+  memcpy(P.lo, K.lo, sizeof P.lo);
+  memcpy(P.dest, K.dest, sizeof P.dest);
+  P.n_shards = K.n_shards;
+  cells_pair_dispatch_kernel<true><<<grid_for(P.pair_slots, 256, c->sm_count * 8), 256, 0, c->stream>>>(P, A);
+  LAUNCH_CHECK("cells_order_dispatch_pairs");
+  if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));
+  return ECB_OK;
+}
+
+int ecb_cells_order_build(ecb_ctx* c, const ecb_ctx* local, int64_t shard_lo, int64_t shard_hi, int64_t n_samples,
+                          ecb_cells_slice* out) {
+  if (!c || !local || !out || !c->xa_base || !c->xa_cap_pairs || shard_hi < shard_lo || n_samples < 1 ||
+      n_samples > 0x7FFFFFFFll)
+    return ECB_ERR_INVALID;
+  if (local->device != c->device) return fail(c, ECB_ERR_INVALID, "the local context lives on another device");
+  memset(out, 0, sizeof *out);
+  CK(cudaSetDevice(c->device));
+  unsigned long long h_ec[3], h_pair[3];
+  CKR(cells_arena_headers(c, h_ec, h_pair));
+  const u64 n_local = h_ec[0], n_pair = h_pair[0];
+  const u64 span = (u64)(shard_hi - shard_lo);
+  const u32 local_n_ec = local->table_slots ? local->n_ec : 0;
+  if (span > 0xFFFFFFFEull) return fail(c, ECB_ERR_LIMIT, "a rank's alignments span more than 2^32 positions");
+  if (n_local > span) return fail(c, ECB_ERR_INVALID, "%llu ECs arrived for a shard of %llu positions", n_local, (unsigned long long)span);
+  if (n_local > local_n_ec) return fail(c, ECB_ERR_INVALID, "%llu ECs arrived but the local context holds %u", n_local, local_n_ec);
+  if (n_local + 1 > 0x7FFFFFFFull || n_pair > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "slice exceeds the int32 fields of the EC file");
+  const unsigned long long* rec = (const unsigned long long*)((const char*)c->xa_base + ECB_ARENA_HEADER_BYTES);
+  const size_t words = (size_t)(span / 32) + 1;
+  CKR(ensure(c, c->bitmap, words * 4));
+  CKR(ensure(c, c->word_rank, words * 4));
+  CKR(ensure(c, c->r_a_indptr, (n_local + 1) * 4));
+  CKR(ensure(c, c->count_of, std::max<u64>(n_local, 1) * 4));     // the merged counts (not part of the slice)
+  CKR(ensure(c, c->first_rel, std::max<u64>(n_local, 1) * 8));   // scratch: local id per record, then per slice id
+  const u64 z_bound = std::max<u64>(local->arena_used, 1);
+  CKR(ensure(c, c->r_a_indices, z_bound * 4));
+  CKR(ensure(c, c->r_a_data, z_bound * 4));
+  CKR(ensure(c, c->cx_col_counts, (size_t)n_samples * 4));
+  u32* lid_of_rec = (u32*)c->first_rel.p;
+  u32* lid_of_id = lid_of_rec + n_local;
+  CK(cudaMemsetAsync(c->bitmap.p, 0, words * 4, c->stream));
+  CK(cudaMemsetAsync(c->r_a_indptr.p, 0, (n_local + 1) * 4, c->stream));
+  CK(cudaMemsetAsync(c->cx_col_counts.p, 0, (size_t)n_samples * 4, c->stream));
+  CK(cudaMemsetAsync(&c->d_ctr->scratch[5], 0, sizeof(u32), c->stream));
+  auto check_bad = [&]() -> int {
+    CKR(sync_counters(c));
+    const u32 bad = c->h_ctr->scratch[5];
+    if (bad)
+      return fail(c, ECB_ERR_INVALID, "second dispatch: %s",
+                  (bad & 4u) ? "an EC arrived that the local context has never seen" : (bad & 2u) ? "two ECs share a first read"
+                  : (bad & 1u) ? "a record outside the shard's positions arrived" : (bad & 8u) ? "a pair arrived without its EC"
+                               : "a pair's column is out of range");
+    return ECB_OK;
+  };
+  u64 nnz = 0;
+  if (n_local) {
+    const int g = grid_for(n_local, 256, c->sm_count * 8);
+    ecb_order_mark_kernel<<<g, 256, 0, c->stream>>>(rec, (u32)n_local, (u32)span, (const EcbEntry*)local->table.p,
+                                                    local->table_slots - 1, (u32*)c->bitmap.p, lid_of_rec, &c->d_ctr->scratch[5]);
+    LAUNCH_CHECK("order_mark");
+    CKR(check_bad());   // nothing below indexes with what the mark pass produced before it is known to be sound
+    CKR(device_scan<true>(c, (const u32*)c->bitmap.p, (u32*)c->word_rank.p, words, 0, nullptr));
+    ecb_order_lens_kernel<<<g, 256, 0, c->stream>>>(rec, (u32)n_local, (u32)span, (const u32*)c->bitmap.p,
+                                                    (const u32*)c->word_rank.p, lid_of_rec, (const u32*)local->row_len.p,
+                                                    (int32_t*)c->r_a_indptr.p, (int32_t*)c->count_of.p, lid_of_id);
+    LAUNCH_CHECK("order_lens");
+    CKR(device_scan<false>(c, (const u32*)c->r_a_indptr.p, (u32*)c->r_a_indptr.p, n_local + 1, 0, &nnz));
+    if (nnz > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "slice exceeds the int32 fields of the EC file");
+    ecb_order_rows_kernel<<<grid_for(n_local, 256, c->sm_count * 16), 256, 0, c->stream>>>(
+        lid_of_id, (const u32*)local->row_len.p, (const u32*)local->row_off.p, (const uint2*)local->arena.p,
+        (const int32_t*)c->r_a_indptr.p, (u32)n_local, (int32_t*)c->r_a_indices.p, (int32_t*)c->r_a_data.p);
+    LAUNCH_CHECK("order_rows");
+  }
+  CKR(ensure(c, c->r_n_indices, std::max<u64>(n_pair, 1) * 4));
+  CKR(ensure(c, c->r_n_data, std::max<u64>(n_pair, 1) * 4));
+  if (n_pair) {
+    CellScratch& S = c->cells;
+    CKR(ensure(c, S.sort_k[0], (size_t)n_pair * 8));
+    CKR(ensure(c, S.sort_v[0], (size_t)n_pair * 4));
+    cells_pair_slice_kernel<<<grid_for(n_pair, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+        cells_pair_records(c), (u32)n_pair, (u32)span, (u32)n_samples, (const u32*)c->bitmap.p, (const u32*)c->word_rank.p,
+        (u64*)S.sort_k[0].p, (u32*)S.sort_v[0].p, &c->d_ctr->scratch[5]);
+    LAUNCH_CHECK("cells_pair_slice");
+    CKR(check_bad());
+    int rb = 0;
+    CKR(radix_sort(c, (u32)n_pair, 32 + bits_for((u64)n_samples), &rb));
+    cells_slice_csc_kernel<<<grid_for(n_pair, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+        (const u64*)S.sort_k[rb].p, (const u32*)S.sort_v[rb].p, (u32)n_pair, (int32_t*)c->cx_col_counts.p,
+        (int32_t*)c->r_n_indices.p, (int32_t*)c->r_n_data.p);
+    LAUNCH_CHECK("cells_slice_csc");
+  }
+  CKR(sync_counters(c));
+  CKR(check_device_error(c));
+  out->n_ec = (int64_t)n_local;
+  out->nnz = (int64_t)nnz;
+  out->a_indptr = (const int32_t*)c->r_a_indptr.p;
+  out->a_indices = (const int32_t*)c->r_a_indices.p;
+  out->a_data = (const int32_t*)c->r_a_data.p;
+  out->n_samples = n_samples;
+  out->nnz_n = (int64_t)n_pair;
+  out->n_col_counts = (const int32_t*)c->cx_col_counts.p;
+  out->n_indices = (const int32_t*)c->r_n_indices.p;
+  out->n_data = (const int32_t*)c->r_n_data.p;
+  return ECB_OK;
+}
+
 int ecb_destroy(ecb_ctx* c) {
   if (!c) return ECB_OK;
   cudaSetDevice(c->device);
@@ -1242,7 +1639,7 @@ int ecb_destroy(ecb_ctx* c) {
                     &c->overflow_bits,
                     &c->scan_partials, &c->bitmap, &c->word_rank, &c->first_rel, &c->ecid_of, &c->ec_keep,
                     &c->r_a_indptr, &c->r_a_indices, &c->r_a_data, &c->r_n_indptr, &c->r_n_indices,
-                    &c->r_n_data, &c->r_cell_order};
+                    &c->r_n_data, &c->r_cell_order, &c->cx_kept, &c->cx_col_of_cell, &c->cx_col_counts};
   for (DevBuf* b : bufs) release(c, *b);
   cells_release(c);
   if (c->stream) cudaStreamSynchronize(c->stream);

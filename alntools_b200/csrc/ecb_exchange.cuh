@@ -47,6 +47,7 @@ struct KeyDispatchParams {
   const u32* ec_slot;
   u32 n_ec;
   u32 world;
+  const u32* count_of;   // dispatch 1: the count sent for provisional id e (NULL: the EC's own count)
   // dispatch 2 only: shards with alignments, ascending by first position, and the rank that holds each
   u64 lo[ECB_MAX_WORLD];
   u32 dest[ECB_MAX_WORLD];
@@ -54,8 +55,9 @@ struct KeyDispatchParams {
 };
 
 // ORDER = false: dispatch 1 (destination = owner of the key); true: dispatch 2 (destination = rank of the shard
-// that holds the first occurrence).
-template <bool ORDER>
+// that holds the first occurrence).  KEPT_ONLY (dispatch 2 of the per-cell exchange): ECs whose merged count is 0
+// - no read in a kept cell on any rank - stay behind.
+template <bool ORDER, bool KEPT_ONLY = false>
 __global__ void __launch_bounds__(256) ecb_key_dispatch_kernel(const KeyDispatchParams P, const ArenaTargets A) {
   constexpr u32 WORDS = ORDER ? ECB_ORDREC_WORDS : ECB_KEYREC_WORDS;
   __shared__ u32 s_cnt[ECB_MAX_WORLD];                  // per tile: records per destination
@@ -69,12 +71,13 @@ __global__ void __launch_bounds__(256) ecb_key_dispatch_kernel(const KeyDispatch
     for (u32 i = threadIdx.x; i < W; i += blockDim.x) s_cnt[i] = 0u;
     __syncthreads();
     const u32 e = tile * blockDim.x + threadIdx.x;
-    const bool live = e < P.n_ec;
+    bool live = e < P.n_ec;
     EcbEntry en{};
     u32 dest = 0, idx = 0;
     u64 rel = 0;
+    if (live) en = P.table[P.ec_slot[e]];
+    if (KEPT_ONLY && en.countm1 == 0xFFFFFFFFu) live = false;
     if (live) {
-      en = P.table[P.ec_slot[e]];
       if (ORDER) {
         u32 k = 0;   // the last shard that starts at or before the position
         while (k + 1 < P.n_shards && P.lo[k + 1] <= en.first) ++k;
@@ -115,7 +118,7 @@ __global__ void __launch_bounds__(256) ecb_key_dispatch_kernel(const KeyDispatch
         r[2] = (rel > 0xFFFFFFFEull ? 0xFFFFFFFFull : rel) | ((unsigned long long)(en.countm1 + 1u) << 32);
       } else {
         r[2] = en.first;
-        r[3] = (unsigned long long)(en.countm1 + 1u);
+        r[3] = (unsigned long long)(P.count_of ? P.count_of[e] : en.countm1 + 1u);
       }
     }
     __syncthreads();

@@ -15,6 +15,10 @@ its shard (order_base = global offset of the shard) and the merge becomes:
   The barriers between these steps are tiny collectives on the stream the kernels run on: nothing in
   between waits for the host.
 
+The per-cell path (distributed_finalize_cells) runs the same two dispatches with (EC, cell) pairs beside the ECs,
+after every rank has taken the same cell decision from the all-gathered cell summaries; see the per-cell section
+of include/ecb200.h.
+
 torch.distributed is the plumbing (process group, collectives on device tensors); every compute
 step is a libecb200 kernel behind the C ABI.
 """
@@ -25,13 +29,15 @@ import torch
 import torch.distributed as dist
 
 _TIMING = bool(os.environ.get("ECB_MGPU_TIMING"))
+LAST_PHASES = {}   # with ECB_MGPU_TIMING: the (phase, ms) rows of the last call of each exchange, for tools
 
 
 class _Phases(object):
-    """Per-phase wall clock of distributed_finalize (ECB_MGPU_TIMING=1; synchronises after every phase)."""
+    """Per-phase wall clock of an exchange (ECB_MGPU_TIMING=1; synchronises after every phase).  rows keeps
+    (phase, ms) for callers that report them themselves."""
 
-    def __init__(self, device):
-        self.device, self.t, self.rows = device, time.perf_counter(), []
+    def __init__(self, device, name="distributed_finalize"):
+        self.device, self.name, self.t, self.rows = device, name, time.perf_counter(), []
 
     def mark(self, name):
         if _TIMING:
@@ -41,8 +47,10 @@ class _Phases(object):
             self.t = now
 
     def report(self):
+        if _TIMING:
+            LAST_PHASES[self.name] = list(self.rows)
         if _TIMING and dist.get_rank() == 0:
-            print("distributed_finalize: " + ", ".join("%s %.2f ms" % r for r in self.rows), flush=True)
+            print(self.name + ": " + ", ".join("%s %.2f ms" % r for r in self.rows), flush=True)
 
 
 _BARRIER_WORD = {}
@@ -56,6 +64,45 @@ def _stream_barrier(device, group):
     if key not in _BARRIER_WORD:
         _BARRIER_WORD[key] = torch.zeros(1, dtype=torch.int32, device=device)
     dist.all_reduce(_BARRIER_WORD[key], group=group)
+
+
+class _Failure(object):
+    """A rank that fails inside the exchange must not leave its peers waiting in a collective: it carries on with
+    what it has, the failure travels with the final all-gather (_gather_rows) and every rank raises."""
+
+    def __init__(self):
+        self.exc = None
+
+    def attempt(self, fn):
+        try:
+            return fn()
+        except Exception as exc:     # noqa: BLE001 - re-raised on every rank by _gather_rows
+            self.exc = self.exc or exc
+            return None
+
+
+def _gather_rows(values, failure, device, group):
+    """All-gather one int64 row per rank (`values` plus this rank's failure flag) and raise on every rank when any
+    rank failed.  -> [world] lists of the values."""
+    world = dist.get_world_size(group)
+    row = torch.cat([torch.as_tensor(values, dtype=torch.int64).to(device).reshape(-1),
+                     torch.tensor([1 if failure.exc else 0], dtype=torch.int64, device=device)])
+    out = torch.empty(world * row.numel(), dtype=torch.int64, device=device)
+    dist.all_gather_into_tensor(out, row, group=group)
+    rows = out.view(world, -1).tolist()
+    if failure.exc is not None:
+        raise failure.exc
+    if any(r[-1] for r in rows):
+        raise RuntimeError("the multi-GPU exchange failed on rank(s) %s" % [r for r in range(world) if rows[r][-1]])
+    return [r[:-1] for r in rows]
+
+
+def _open_arenas(owner, handle, base, device, group):
+    """Every rank's arena base as seen from this process: the IPC handles are all-gathered and the peers' mapped."""
+    world, me = dist.get_world_size(group), dist.get_rank(group)
+    hs = [torch.empty(64, dtype=torch.uint8, device=device) for _ in range(world)]
+    dist.all_gather(hs, torch.frombuffer(bytearray(handle), dtype=torch.uint8).to(device), group=group)
+    return [base if r == me else owner.arena_open_peer(bytes(hs[r].cpu().tolist())) for r in range(world)]
 
 
 def distributed_finalize(local, make_owner, device, group=None, result_on="slices"):
@@ -94,9 +141,7 @@ def distributed_finalize(local, make_owner, device, group=None, result_on="slice
         dist.all_gather(gathered, info, group=group)
         need_ec = 2 * max(int(t.item()) for t in gathered) + 1024
         handle, base = owner.arena_create(need_ec)
-        hs = [torch.empty(64, dtype=torch.uint8, device=device) for _ in range(world)]
-        dist.all_gather(hs, torch.frombuffer(bytearray(handle), dtype=torch.uint8).to(device), group=group)
-        bases = [base if r == me else owner.arena_open_peer(bytes(hs[r].cpu().tolist())) for r in range(world)]
+        bases = _open_arenas(owner, handle, base, device, group)
         arena = {"bases": bases, "cap_ec": need_ec}
         owner._exchange_arena = arena
         dist.barrier(group=group)                     # every arena exists and is zeroed
@@ -107,14 +152,9 @@ def distributed_finalize(local, make_owner, device, group=None, result_on="slice
     mine = torch.tensor([min_base, max_end], dtype=torch.int64, device=device)
     spans = torch.empty(2 * world, dtype=torch.int64, device=device)
     dist.all_gather_into_tensor(spans, mine, group=group)
-    # a rank that fails from here on (an arena that turned out too small) must not leave its peers waiting in
-    # a collective: it carries on with what it has, the failure travels with the all-gather of the slice
-    # sizes below, and every rank raises
-    failure = None
-    try:
-        owner.import_arena()
-    except Exception as exc:         # noqa: BLE001 - re-raised on every rank below
-        failure = exc
+    # a rank that fails from here on (an arena that turned out too small) carries on; see _Failure
+    failure = _Failure()
+    failure.attempt(owner.import_arena)
     owner.arena_reset()              # reused by the second dispatch ...
     _stream_barrier(device, group)   # ... once every rank has merged what it received
     ph.mark("merge")
@@ -125,27 +165,133 @@ def distributed_finalize(local, make_owner, device, group=None, result_on="slice
     owner.order_dispatch(arena["bases"], arena["cap_ec"], lo, hi)
     _stream_barrier(device, group)   # every rank's ECs have landed
     ph.mark("dispatch 2")
-    sl = None
-    try:
-        sl = owner.order_build(local, lo[me], hi[me])
-    except Exception as exc:         # noqa: BLE001
-        failure = failure or exc
+    sl = failure.attempt(lambda: owner.order_build(local, lo[me], hi[me]))
     ph.mark("order build")
     # the id range of a rank starts behind the ECs of the shards in front of it
-    sizes = torch.empty(2 * world, dtype=torch.int64, device=device)
-    dist.all_gather_into_tensor(sizes, torch.tensor([sl["n_ec"] if sl else 0, 1 if failure else 0],
-                                                    dtype=torch.int64, device=device), group=group)
-    sizes = sizes.tolist()
-    if failure is not None:
-        raise failure
-    if any(sizes[1::2]):
-        raise RuntimeError("the multi-GPU exchange failed on rank(s) %s" % [r for r in range(world) if sizes[2 * r + 1]])
-    sizes = sizes[0::2]
-    id_base = sum(n for r, n in enumerate(sizes) if hi[r] > lo[r] and (lo[r], r) < (lo[me], me))
+    sizes = [r[0] for r in _gather_rows([sl["n_ec"] if sl else 0], failure, device, group)]
+    id_base = sum(n for r, n in enumerate(sizes) if _in_front(lo, hi, r, me))
     ph.report()
     return {"a_indptr": sl["a_indptr"], "a_indices": sl["a_indices"], "a_data": sl["a_data"],
             "n_data": sl["n_data"], "n_ec": sum(sizes), "id_base": id_base, "n_ec_local": sl["n_ec"],
             "nnz_local": sl["nnz"], "nnz_a": None}
+
+
+def _in_front(lo, hi, r, me):
+    """Whether rank r's slice precedes rank me's in EC-id order: ids are ranks of first occurrences, so slices
+    follow the order of the ranks' shards of the read order (ranks without alignments hold nothing)."""
+    return hi[r] > lo[r] and (lo[r], r) < (lo[me], me)
+
+
+def _cells_arena(owner, counts, device, group):
+    """The per-cell arenas for the next dispatch, sized from its exact per-destination record counts (all-reduced:
+    every rank takes the same decision).  Arenas that are large enough are cleared behind a stream barrier;
+    otherwise every rank re-creates its own and the new IPC handles are exchanged before anyone stores."""
+    world = dist.get_world_size(group)
+    c = counts.tolist()
+    need_ec, need_pairs = max(c[:world]), max(c[world:])
+    arena = getattr(owner, "_cells_arena", None)
+    if arena is not None and need_ec <= arena["cap_ec"] and need_pairs <= arena["cap_pairs"]:
+        owner.arena_reset()
+        _stream_barrier(device, group)
+        return arena
+    # a little headroom, so that the steps of a job with similar inputs keep their arenas
+    cap_ec = max(need_ec + need_ec // 8, 1024, arena["cap_ec"] if arena else 0)
+    cap_pairs = max(need_pairs + need_pairs // 8, 1024, arena["cap_pairs"] if arena else 0)
+    dist.barrier(group=group)          # no rank still works on the arenas about to be replaced
+    handle, base = owner.cells_arena_create(cap_ec, cap_pairs)
+    arena = {"bases": _open_arenas(owner, handle, base, device, group), "cap_ec": cap_ec, "cap_pairs": cap_pairs,
+             "created": (arena or {}).get("created", 0) + 1}
+    owner._cells_arena = arena
+    dist.barrier(group=group)          # every arena exists and its headers are zeroed
+    return arena
+
+
+def distributed_finalize_cells(local, make_owner, device, min_count, cell_map, n_cells, group=None):
+    """The per-cell (multisample) exchange.  local: builder (with cells) holding this rank's files, pushed at
+    rank-major order keys (order_base = rank * 2^40 + alignments of this rank's earlier files; see the per-cell
+    section of include/ecb200.h); make_owner(): builder for the owner role, kept from step to step of a job with
+    its arena.  cell_map: int32 device tensor, this rank's cell ids -> global ids (first appearance over the
+    ranks' name lists in rank order), or None for identity; n_cells: number of global cell ids.
+
+    The final matrices stay partitioned by EC-id range, as with distributed_finalize.  Returns, for this rank,
+    int32 device tensors a_indptr (local to the slice), a_indices, a_data, the N pieces n_col_counts [S] (entries
+    of every column held here), n_indices (EC ids local to the slice, ascending inside a column), n_data, and
+    n_col_offset [S] (entries of each column held by the slices in front), n_indptr [S + 1] (global), cell_order
+    [S] (global cell id of every column); scalars n_ec (all ranks), id_base, n_ec_local, nnz_local, nnz_a, nnz_n,
+    n_samples.  Every rank gets the same cell_order, n_indptr and sizes."""
+    if device.type != "cuda":
+        raise ValueError("device must be a CUDA device (the exchange maps the ranks' GPU memory), got %s" % device)
+    world, me = dist.get_world_size(group), dist.get_rank(group)
+    cur = torch.cuda.current_stream(device).cuda_stream
+    local.set_stream(cur)
+    owner = make_owner()
+    owner.set_stream(cur)
+    ph = _Phases(device, "distributed_finalize_cells")
+    # a rank that fails carries on with empty results (see _Failure): a failure before dispatch 1 travels with the
+    # all-reduce of its counts and every rank raises there; one after it travels with the final all-gather
+    failure = _Failure()
+    # ---- cell summary by global id; keys all-gathered, totals summed
+    summary = failure.attempt(lambda: local.cells_summary(cell_map, n_cells))
+    if summary is None:
+        summary = (torch.full((int(n_cells),), -1, dtype=torch.int64, device=device),
+                   torch.zeros(int(n_cells), dtype=torch.int64, device=device))
+    keys, totals = summary
+    keys_all = torch.empty(world * int(n_cells), dtype=torch.int64, device=device)
+    dist.all_gather_into_tensor(keys_all, keys, group=group)
+    dist.all_reduce(totals, group=group)
+    ph.mark("cell summary")
+    # ---- the same cell decision on every rank (no kept cell: every rank raises the same ECB_ERR_EMPTY)
+    decided = None if failure.exc else failure.attempt(lambda: local.cells_order(keys_all, totals, min_count, cell_map, world))
+    ph.mark("cell order")
+    # ---- dispatch 1: ECs and kept pairs to the owner of the EC's key; the last word counts failed ranks
+    counts = None if failure.exc else failure.attempt(lambda: local.cells_dispatch_counts(world))
+    if counts is None:
+        counts = torch.zeros(2 * world, dtype=torch.int64, device=device)
+    counts = torch.cat([counts, torch.tensor([1 if failure.exc else 0], dtype=torch.int64, device=device)])
+    dist.all_reduce(counts, group=group)
+    if int(counts[-1]):
+        _gather_rows([0], failure, device, group)   # raises on every rank
+    n_samples, cell_order = decided
+    arena = _cells_arena(owner, counts[:-1], device, group)
+    ph.mark("setup 1")
+    span = failure.attempt(lambda: local.cells_export_to_arenas(arena["bases"], arena["cap_ec"], arena["cap_pairs"]))
+    min_base, max_end = span if span is not None else (0, 0)
+    spans = torch.empty(2 * world, dtype=torch.int64, device=device)
+    dist.all_gather_into_tensor(spans, torch.tensor([min_base, max_end], dtype=torch.int64, device=device), group=group)
+    ph.mark("dispatch 1")
+    spans = spans.tolist()
+    lo, hi = spans[0::2], spans[1::2]
+    failure.attempt(owner.cells_import_arena)
+    ph.mark("merge")
+    # ---- dispatch 2: merged ECs with kept reads, and merged pairs, to the rank that holds the first occurrence
+    counts = failure.attempt(lambda: owner.cells_dispatch_counts(world, lo, hi))
+    if counts is None:
+        counts = torch.zeros(2 * world, dtype=torch.int64, device=device)
+    dist.all_reduce(counts, group=group)
+    arena = _cells_arena(owner, counts, device, group)
+    ph.mark("setup 2")
+    failure.attempt(lambda: owner.cells_order_dispatch(arena["bases"], arena["cap_ec"], arena["cap_pairs"], lo, hi))
+    _stream_barrier(device, group)   # every rank's records have landed
+    ph.mark("dispatch 2")
+    sl = failure.attempt(lambda: owner.cells_order_build(local, lo[me], hi[me], n_samples))
+    ph.mark("order build")
+    col = sl["n_col_counts"].to(torch.int64) if sl else torch.zeros(n_samples, dtype=torch.int64, device=device)
+    rows = _gather_rows(torch.cat([torch.tensor([sl["n_ec"] if sl else 0, sl["nnz"] if sl else 0], dtype=torch.int64,
+                                                device=device), col]), failure, device, group)
+    front = [r for r in range(world) if _in_front(lo, hi, r, me)]
+    col_all = torch.tensor([r[2:] for r in rows], dtype=torch.int64)
+    n_indptr = torch.zeros(n_samples + 1, dtype=torch.int64)
+    torch.cumsum(col_all.sum(0), 0, out=n_indptr[1:])
+    if int(n_indptr[-1]) > 0x7FFFFFFF:
+        raise RuntimeError("the N matrix has more than 2^31-1 entries")
+    col_offset = col_all[front].sum(0) if front else torch.zeros(n_samples, dtype=torch.int64)
+    ph.report()
+    return {"a_indptr": sl["a_indptr"], "a_indices": sl["a_indices"], "a_data": sl["a_data"],
+            "n_col_counts": sl["n_col_counts"], "n_indices": sl["n_indices"], "n_data": sl["n_data"],
+            "n_col_offset": col_offset.to(torch.int32).to(device), "n_indptr": n_indptr.to(torch.int32).to(device),
+            "cell_order": cell_order, "n_ec": sum(r[0] for r in rows), "id_base": sum(rows[r][0] for r in front),
+            "n_ec_local": sl["n_ec"], "nnz_local": sl["nnz"], "nnz_a": sum(r[1] for r in rows),
+            "nnz_n": int(n_indptr[-1]), "n_samples": n_samples}
 
 
 def shard_bounds(read_group, world):

@@ -91,6 +91,15 @@ def reference_names(n_targets, n_haps, hap_letters="ABCDEFGH"):
             for t in range(n_targets) for h in range(n_haps)]
 
 
+def columns_to_bam_cells(filename, cols, n_targets, n_haps, level=1):
+    """Materialise per-cell columns as one name-grouped BAM file of the per-cell path: the cell of every read is
+    field 14 of its '|||'-separated name ('cell%07d' % cell_idx)."""
+    from . import bam_io
+    tids = cols["target_idx"].astype(np.int64) * n_haps + cols["hap_idx"]
+    bam_io.write_bam_columns(filename, reference_names(n_targets, n_haps), cols["read_group"],
+                             np.zeros(len(tids), dtype=np.uint16), tids, level=level, cell_ids=cols["cell_idx"])
+
+
 def columns_to_bam(filename, cols, n_targets, n_haps, level=1):
     """Materialise single-sample columns as a name-grouped BAM (read names 'read%09d')."""
     from . import bam_io

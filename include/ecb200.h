@@ -207,6 +207,65 @@ int ecb_order_dispatch(ecb_ctx* owner_ctx, int world, void* const* arena_bases, 
                        const int64_t* shard_lo, const int64_t* shard_hi);
 int ecb_order_build(ecb_ctx* owner_ctx, const ecb_ctx* local_ctx, int64_t shard_lo, int64_t shard_hi, ecb_slice* out);
 
+/* ---- the per-cell exchange (contexts created with cells; since version 2001) ----------------------------
+ * The same two dispatches, with (EC, cell) pairs travelling beside the ECs.  Every rank pushes its own files,
+ * one push per file with drop_last_group = 1, at RANK-MAJOR order keys: order_base = rank * 2^40 + (alignments
+ * of this rank's earlier files).  So every position of a rank lies behind those of all ranks in front of it, no
+ * count is exchanged before the pushes, no rebase is needed, and a rank's positions still span less than 2^32.
+ * Cells carry GLOBAL ids: the first appearance over the ranks' cell-name lists taken in rank order (the id the
+ * one-GPU build gives); cell_map[local id] = global id (device int32, NULL = identity).  Sequence, per rank:
+ *   ecb_cells_summary        (LOCAL)  cell_key[g] = this rank's sort key of global cell g (~0 if absent),
+ *                                     cell_total[g] = its reads here (device uint64 arrays of n_cells);
+ *   caller: all-gather the keys as [world x n_cells], all-reduce the totals with SUM;
+ *   ecb_cells_order          (LOCAL)  every rank takes the same decision: a cell's key is (first rank that
+ *                                     holds it, that rank's key); cells below min_cell_count (<= 0: 1) are
+ *                                     dropped.  -> n_samples (kept cells, ECB_ERR_EMPTY when none, the same on
+ *                                     every rank) and cell_order (device, global cell id of every column, valid
+ *                                     until the next call on the context);
+ *   ecb_cells_dispatch_counts         exact records per destination rank of the next dispatch: counts[r] ECs,
+ *                                     counts[world + r] pairs (device int64 [2 * world], written on the
+ *                                     context's stream).  shard_lo / shard_hi NULL: dispatch 1 (LOCAL context,
+ *                                     after ecb_cells_order); given: dispatch 2 (OWNER, after the import).  The
+ *                                     caller all-reduces them and sizes the arenas from the largest;
+ *   ecb_cells_arena_create   (OWNER)  one IPC allocation with two record areas (cap_ec EC records, cap_pairs
+ *                                     pair records), each with its own header; replaces a smaller arena of an
+ *                                     earlier call, closing the peer arenas opened through ecb_arena_open_peer
+ *                                     (the caller exchanges the new handles).  ecb_arena_reset clears both
+ *                                     headers;
+ *   ecb_cells_export_to_arenas (LOCAL) every local EC as {key, first, reads in kept cells} - ECs without such
+ *                                     reads too: this rank may hold the EC's first occurrence - and every local
+ *                                     (EC, cell) pair with a kept column as {EC key, column, count} to the owner;
+ *   ecb_cells_import_arena   (OWNER)  ECs merged as by ecb_import_arena, pairs merged by (EC, column);
+ *   ecb_cells_order_dispatch (OWNER)  merged ECs with reads in kept cells, and every merged pair, to the rank
+ *                                     whose shard holds the EC's first occurrence;
+ *   ecb_cells_order_build    (OWNER + LOCAL) the A slice as ecb_order_build, and the slice's N entries.
+ * Barriers as in the single-sample exchange.  cap_ec / cap_pairs are the same on every rank.  An arena that
+ * turns out too small sets its overflow flag; import and build then fail with ECB_ERR_LIMIT. */
+int ecb_cells_summary(ecb_ctx* local_ctx, const int32_t* cell_map, int64_t map_len, int64_t n_cells, uint64_t* cell_key,
+                      uint64_t* cell_total);
+int ecb_cells_order(ecb_ctx* local_ctx, int world, const uint64_t* cell_keys, const uint64_t* cell_totals, int64_t n_cells,
+                    int64_t min_cell_count, const int32_t* cell_map, int64_t* n_samples, const int32_t** cell_order);
+int ecb_cells_dispatch_counts(ecb_ctx* ctx, int world, const int64_t* shard_lo, const int64_t* shard_hi, int64_t* counts);
+int ecb_cells_arena_create(ecb_ctx* owner_ctx, int64_t cap_ec, int64_t cap_pairs, void* ipc_handle_out /* 64 bytes */,
+                           void** base_out);
+int ecb_cells_export_to_arenas(ecb_ctx* local_ctx, int world, void* const* arena_bases, int64_t cap_ec, int64_t cap_pairs,
+                               int64_t* min_base, int64_t* max_end);
+int ecb_cells_import_arena(ecb_ctx* owner_ctx);
+int ecb_cells_order_dispatch(ecb_ctx* owner_ctx, int world, void* const* arena_bases, int64_t cap_ec, int64_t cap_pairs,
+                             const int64_t* shard_lo, const int64_t* shard_hi);
+
+/* This rank's slice of the per-cell matrices: the A part as ecb_slice; N as the slice's entries in column-major
+ * order - n_col_counts[n_samples] entries per column, n_indices (EC ids local to the slice, ascending inside a
+ * column), n_data (counts).  Device memory of the owner context, valid until the next call on it. */
+typedef struct ecb_cells_slice {
+  int64_t n_ec, nnz;
+  const int32_t *a_indptr, *a_indices, *a_data;
+  int64_t n_samples, nnz_n;
+  const int32_t *n_col_counts, *n_indices, *n_data;
+} ecb_cells_slice;
+int ecb_cells_order_build(ecb_ctx* owner_ctx, const ecb_ctx* local_ctx, int64_t shard_lo, int64_t shard_hi, int64_t n_samples,
+                          ecb_cells_slice* out);
+
 #ifdef __cplusplus
 }
 #endif
