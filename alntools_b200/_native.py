@@ -20,8 +20,10 @@ ECB_OPT_HOT_CACHE = 5
 ECB_OPT_VERIFY_KEYS = 6
 ECB_OPT_CHUNK_LEN = 7
 ECB_OPT_PAGEABLE_RESULTS = 8
+ECB_OPT_BAM_WINDOW = 9
 
 ECB_ERR_EMPTY = -5
+ECB_ERR_FORMAT = -7
 
 _i32p = ctypes.POINTER(ctypes.c_int32)
 
@@ -65,6 +67,18 @@ class EcbCellsSlice(ctypes.Structure):
                 ("n_col_counts", _i32p), ("n_indices", _i32p), ("n_data", _i32p)]
 
 
+class EcbBamStats(ctypes.Structure):
+    _fields_ = [
+        ("h2d_bytes", ctypes.c_int64), ("inflated_bytes", ctypes.c_int64), ("blocks", ctypes.c_int64),
+        ("windows", ctypes.c_int64), ("hop_rounds", ctypes.c_int64), ("records", ctypes.c_int64),
+        ("h2d_ms", ctypes.c_double), ("inflate_ms", ctypes.c_double), ("hop_ms", ctypes.c_double),
+        ("rules_ms", ctypes.c_double),
+    ]
+
+    def as_dict(self):
+        return {name: getattr(self, name) for name, _ in self._fields_}
+
+
 # every symbol include/ecb200.h declares, with its ctypes signature
 SIGNATURES = {
     "ecb_version": (ctypes.c_int, []),
@@ -105,6 +119,16 @@ SIGNATURES = {
     "ecb_get_stats": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbStats)]),
     "ecb_destroy": (ctypes.c_int, [ctypes.c_void_p]),
     "ecb_last_error": (ctypes.c_char_p, [ctypes.c_void_p]),
+    "ecb_bam_create": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int,
+                                      ctypes.POINTER(ctypes.c_void_p)]),
+    "ecb_bam_decode": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
+                                      ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int,
+                                      ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p),
+                                      ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_int64)]),
+    "ecb_bam_counters": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]),
+    "ecb_bam_ranges": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "ecb_bam_get_stats": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbBamStats)]),
+    "ecb_bam_destroy": (ctypes.c_int, [ctypes.c_void_p]),
 }
 
 _lib = None
@@ -182,6 +206,7 @@ class EcBuilder(object):
         if rc != 0:
             raise EcbError(rc, self._lib.ecb_last_error(None).decode())
         self.with_cells = bool(with_cells)
+        self.device = int(device)               # the CUDA device of this context (not necessarily torch's current one)
         self._result_on_device = False
         for key, value in options.items():
             self.set_option(key, value)
@@ -189,7 +214,8 @@ class EcBuilder(object):
     _OPTIONS = {"result_on_device": ECB_OPT_RESULT_ON_DEVICE, "table_slots": ECB_OPT_TABLE_SLOTS,
                 "pair_slots": ECB_OPT_PAIR_SLOTS, "grid_ctas": ECB_OPT_GRID_CTAS,
                 "hot_cache": ECB_OPT_HOT_CACHE, "verify_keys": ECB_OPT_VERIFY_KEYS,
-                "chunk_len": ECB_OPT_CHUNK_LEN, "pageable_results": ECB_OPT_PAGEABLE_RESULTS}
+                "chunk_len": ECB_OPT_CHUNK_LEN, "pageable_results": ECB_OPT_PAGEABLE_RESULTS,
+                "bam_window": ECB_OPT_BAM_WINDOW}
 
     def _check(self, rc):
         if rc != 0:
@@ -389,6 +415,86 @@ class EcBuilder(object):
         if self._ctx:
             self._lib.ecb_destroy(self._ctx)
             self._ctx = ctypes.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class BamDecoder(object):
+    """Device decode of one single-sample BAM file on `builder`'s context (ecb_bam_* in include/ecb200.h): BGZF
+    blocks in, the columns bamcols_emit produces out, in device memory.  Malformed input raises ValueError, as the
+    host reader (bamcols) does for the same file."""
+
+    def __init__(self, builder, tid_target, tid_hap, track_ranges=False):
+        self._lib = builder._lib
+        self._builder = builder                   # the decoder lives in the builder's context: keep it alive
+        self._h = ctypes.c_void_p()
+        self.n_references = len(tid_target)
+        tt = np.ascontiguousarray(tid_target, dtype=np.int32)
+        th = np.ascontiguousarray(tid_hap, dtype=np.int32)
+        self._check(self._lib.ecb_bam_create(builder._ctx, tt.ctypes.data, th.ctypes.data, len(tt),
+                                             1 if track_ranges else 0, ctypes.byref(self._h)))
+
+    def _check(self, rc):
+        if rc == 0:
+            return
+        msg = self._lib.ecb_last_error(self._builder._ctx).decode()
+        if rc == ECB_ERR_FORMAT:
+            raise ValueError(msg)
+        raise EcbError(rc, msg)
+
+    def decode(self, data, payload_off, payload_len, isize, skip=0, last=False, n_bytes=None):
+        """data: compressed bytes (pinned uint8 tensor preferred, or a numpy array / bytes); the block table as from
+        BamColumnReader.blocks().  -> (read_group, target_idx, hap_idx): int32 torch views of the device rows of
+        every read closed so far, valid until the next call."""
+        import torch
+        if isinstance(data, (bytes, bytearray)):
+            data = np.frombuffer(data, dtype=np.uint8)
+        ptr = data.data_ptr() if hasattr(data, "data_ptr") else data.ctypes.data
+        n_bytes = int(data.shape[0]) if n_bytes is None else int(n_bytes)
+        off = np.ascontiguousarray(payload_off, dtype=np.int64)
+        length = np.ascontiguousarray(payload_len, dtype=np.int32)
+        size = np.ascontiguousarray(isize, dtype=np.int32)
+        rg, tg, hp = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_void_p()
+        rows = ctypes.c_int64()
+        self._check(self._lib.ecb_bam_decode(self._h, ptr, n_bytes, off.ctypes.data, length.ctypes.data, size.ctypes.data,
+                                             len(off), int(skip), 1 if last else 0, ctypes.byref(rg), ctypes.byref(tg),
+                                             ctypes.byref(hp), ctypes.byref(rows)))
+        n = int(rows.value)
+        dev = torch.device("cuda", self._builder.device)   # the rows live on the builder's GPU
+        return tuple(_device_view(p.value, (n,), "<i4", torch.int32, dev) for p in (rg, tg, hp))
+
+    def counters(self):
+        """-> (all_alignments, n_groups): records seen so far and reads started."""
+        a, g = ctypes.c_int64(), ctypes.c_int64()
+        self._check(self._lib.ecb_bam_counters(self._h, ctypes.byref(a), ctypes.byref(g)))
+        return int(a.value), int(g.value)
+
+    def ranges(self):
+        """(min_pos, max_pos) int32 arrays per reference, as BamColumnReader.ranges()."""
+        lo = np.empty(self.n_references, dtype=np.int32)
+        hi = np.empty(self.n_references, dtype=np.int32)
+        self._check(self._lib.ecb_bam_ranges(self._h, lo.ctypes.data, hi.ctypes.data))
+        return lo, hi
+
+    def stats(self):
+        st = EcbBamStats()
+        self._check(self._lib.ecb_bam_get_stats(self._h, ctypes.byref(st)))
+        return st.as_dict()
+
+    def close(self):
+        if self._h:
+            self._lib.ecb_bam_destroy(self._h)
+            self._h = ctypes.c_void_p()
 
     def __enter__(self):
         return self

@@ -286,7 +286,7 @@ def convert_rank(bam_filename, ec_filename, emase_filename, num_chunks=0, number
 
 
 def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_processes=-1, temp_dir=None,
-            range_filename=None, sample=None, target_filename=None, device=0, devices=None):
+            range_filename=None, sample=None, target_filename=None, device=0, devices=None, decode=None):
     """Convert a name-grouped BAM file into an EC binary file and/or an EMASE file.
 
     Arguments keep the reference's meaning.  num_chunks / number_processes only shape the host decode
@@ -294,9 +294,19 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
     temporary BAM is written.  `device` selects the GPU.  devices=N (or the environment variable
     ALNTOOLS_GPUS=N) shards the file over N GPUs of this machine, one worker process per GPU (convert_rank);
     the same happens without either when the call is made inside a one-process-per-GPU job (torchrun).
-    The EC file does not depend on the number of GPUs.
+    The EC file does not depend on the number of GPUs.  decode="device" (or ALNTOOLS_B200_DECODE=device) inflates
+    and decodes the BAM file on the GPU (one GPU, native emitter); "host" (the default) decodes it on the CPU.
+    The outputs do not depend on it.
     """
     start_time = time.time()
+    mode = emitter.decode_mode(decode)
+    if mode == "device":
+        if utils.under_launcher() or utils.requested_gpus(devices) > 1:
+            raise NotImplementedError("device BAM decode runs on one GPU; the multi-GPU convert has no device decode yet "
+                                      "(use decode='host' / unset ALNTOOLS_B200_DECODE)")
+        if emitter.use_python_emitter():
+            raise NotImplementedError("device BAM decode replaces the native emitter; it does not combine with "
+                                      "ALNTOOLS_B200_EMITTER=python")
     job = dict(bam_filename=bam_filename, ec_filename=ec_filename, emase_filename=emase_filename, num_chunks=num_chunks,
                number_processes=number_processes, temp_dir=temp_dir, range_filename=range_filename, sample=sample,
                target_filename=target_filename)
@@ -360,7 +370,7 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
     import torch
     with bamcols.BamColumnReader(bam_filename, n_threads=num_processes) as reader:
         tables = reader.build_tables(target_filename)       # native statement of header.TargetTables
-        if range_filename is not None:
+        if range_filename is not None and mode == "host":
             reader.track_ranges(True)
         LOG.info("File parsed in {}, total time: {}".format(utils.format_time(temp_time, time.time()),
                                                             utils.format_time(start_time, time.time())))
@@ -369,16 +379,20 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
         # grows it ahead of later ones; one finalize per context, so results skip the pinning cost
         with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=False, alignments_hint=0,
                        device=device, pageable_results=1) as builder:
-            chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(bam_filename) // 2)))   # 24 MB of columns per piece
-            valid = emitter.stream_single(reader, builder, chunk_rows=chunk_rows, pinned=torch.cuda.is_available())
+            if mode == "device":
+                valid, _, ranges, _ = emitter.stream_single_device(bam_filename, reader, builder, tables,
+                                                                range_filename is not None)
+            else:
+                chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(bam_filename) // 2)))   # 24 MB of columns per piece
+                valid = emitter.stream_single(reader, builder, chunk_rows=chunk_rows, pinned=torch.cuda.is_available())
+                ranges = reader.ranges() if range_filename is not None else None
             if valid == 0:
                 # the reference ends up with zero ECs and APM() raises (Sparse3DMatrix.py:45-46)
                 raise RuntimeError("The shape must be a tuple of three positive integers.")
             # the files are written straight from the library's result buffers (no intermediate copies)
             summary = save(builder.finalize(copy=False), tables, valid, temp_time)
         if range_filename is not None:                         # bam_utils.py:735-766
-            lo, hi = reader.ranges()
             utils.write_range_file(range_filename, list(tables.main_targets.keys()), tables.haplotypes,
-                                   reader.references, lo, hi)
+                                   reader.references, ranges[0], ranges[1])
     return summary
 

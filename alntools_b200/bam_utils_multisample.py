@@ -289,6 +289,9 @@ def convert_files(bam_files, ec_filename, emase_filename, minimum_count, target_
     (bam_utils_multisample.py:503-560).  devices=N (or the environment variable ALNTOOLS_GPUS=N) spreads the
     files over N GPUs of this machine, one worker process per GPU (convert_files_rank); the same happens without
     either inside a one-process-per-GPU job (torchrun).  The EC file does not depend on the number of GPUs."""
+    if emitter.decode_mode() == "device":
+        raise NotImplementedError("the per-cell (--multisample) conversion has no device BAM decode yet: it needs a GPU "
+                                  "cell-name dictionary (unset ALNTOOLS_B200_DECODE)")
     job = dict(bam_files=list(bam_files), ec_filename=ec_filename, emase_filename=emase_filename,
                minimum_count=minimum_count, target_filename=target_filename, range_filename=range_filename)
     if utils.under_launcher() or utils.requested_gpus(devices) > 1:

@@ -45,6 +45,8 @@ SIGNATURES = {
     "bamcols_ranges": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p)]),
     "bamcols_phase_seconds": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_double)]),
     "bamcols_target_section": (ctypes.c_int64, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_void_p)]),
+    "bamcols_blocks": (ctypes.c_int64, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p,
+                                        ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64)]),
     "bamcols_inflate_raw": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int]),
 }
 
@@ -264,6 +266,20 @@ class BamColumnReader(object):
         rc = self._lib.bamcols_set_range(self._h, int(vbegin), int(vend))
         if rc != 0:
             _raise(rc, self._lib.bamcols_last_error(self._h).decode())
+
+    def blocks(self, c_begin, max_bytes, max_blocks=1 << 16):
+        """The BGZF blocks from compressed offset c_begin on, without inflating them: at most max_blocks blocks whose
+        compressed bytes fit in max_bytes (at least one while any is left).  -> (payload_off int64 [counted from
+        c_begin], payload_len int32, isize int32, c_end); no blocks at the end of the file."""
+        off = np.empty(int(max_blocks), dtype=np.int64)
+        length = np.empty(int(max_blocks), dtype=np.int32)
+        isize = np.empty(int(max_blocks), dtype=np.int32)
+        end = ctypes.c_int64()
+        n = self._lib.bamcols_blocks(self._h, int(c_begin), int(max_bytes), int(max_blocks), off.ctypes.data,
+                                     length.ctypes.data, isize.ctypes.data, ctypes.byref(end))
+        if n < 0:
+            _raise(int(n), self._lib.bamcols_last_error(self._h).decode())
+        return off[:n], length[:n], isize[:n], int(end.value)
 
     def track_ranges(self, enable=True):
         rc = self._lib.bamcols_track_ranges(self._h, 1 if enable else 0)

@@ -1637,6 +1637,29 @@ int bamcols_ranges(const bamcols* r, const int32_t** min_pos, const int32_t** ma
   return (int)r->range_min.size();
 }
 
+int64_t bamcols_blocks(bamcols* r, int64_t c_begin, int64_t max_bytes, int64_t max_blocks, int64_t* payload_off,
+                       int32_t* payload_len, int32_t* isize, int64_t* c_end) {
+  if (!r || !payload_off || !payload_len || !isize || !c_end || c_begin < 0 || max_bytes < 1 || max_blocks < 1)
+    return BAMCOLS_ERR_INVALID;
+  if ((size_t)c_begin > r->file_size) return fail(r, BAMCOLS_ERR_INVALID, "offset %lld beyond the end of the file", (long long)c_begin);
+  size_t c = (size_t)c_begin;
+  int64_t n = 0;
+  while (n < max_blocks) {
+    BlockJob job;
+    size_t bsize = 0;
+    const int rc = parse_block(r, c, &job, &bsize);
+    if (rc < 0) return rc;
+    if (rc == 1 || (n > 0 && c + bsize - (size_t)c_begin > (size_t)max_bytes)) break;
+    payload_off[n] = (int64_t)((size_t)(job.src - r->file) - (size_t)c_begin);
+    payload_len[n] = (int32_t)job.src_len;
+    isize[n] = (int32_t)job.isize;
+    ++n;
+    c += bsize;
+  }
+  *c_end = (int64_t)c;
+  return n;
+}
+
 int bamcols_inflate_raw(const uint8_t* src, int64_t src_len, uint8_t* dst, int64_t dst_len, int mode) {
   if (!src || (!dst && dst_len) || src_len < 0 || dst_len < 0) return BAMCOLS_ERR_INVALID;
   if (mode == 2) {   // the whole-buffer decoder alone: 1 = decoded, 0 = declined

@@ -17,6 +17,7 @@
 #include "ecb_cells.cuh"
 #include "ecb_exchange.cuh"
 #include "ecb_cells_exchange.cuh"
+#include "ecb_bam.cuh"
 
 namespace {
 
@@ -42,6 +43,7 @@ struct ecb_ctx {
   int use_cache = 1;
   int verify_keys = 0;
   int pageable_results = 0;
+  int64_t opt_bam_window = 0;
   // EC table
   DevBuf table;
   u32 table_slots = 0;
@@ -549,7 +551,7 @@ void cells_release(ecb_ctx* c) {
 
 extern "C" {
 
-int ecb_version(void) { return 2001; }
+int ecb_version(void) { return 2002; }
 
 const char* ecb_last_error(const ecb_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
@@ -624,6 +626,9 @@ int ecb_set_option(ecb_ctx* c, int option, int64_t value) {
     case ECB_OPT_PAGEABLE_RESULTS:
       if (c->h_res) return fail(c, ECB_ERR_STATE, "result buffers already allocated");
       c->pageable_results = value ? 1 : 0; break;
+    case ECB_OPT_BAM_WINDOW:
+      if (value < 0) return fail(c, ECB_ERR_INVALID, "negative window");
+      c->opt_bam_window = value; break;
     default: return fail(c, ECB_ERR_INVALID, "unknown option %d", option);
   }
   return ECB_OK;
@@ -1665,6 +1670,355 @@ int ecb_destroy(ecb_ctx* c) {
   }
   if (c->pool) cudaMemPoolDestroy(c->pool);
   delete c;
+  return ECB_OK;
+}
+
+}  // extern "C"
+
+// ---- device decode of single-sample BAM files (kernels in ecb_bam.cuh) ----------------------------------------
+struct ecb_bam {
+  ecb_ctx* c = nullptr;
+  int32_t n_ref = 0;
+  bool track = false;
+  DevBuf tid_target, tid_hap, range_min, range_max;
+  DevBuf comp, blocks;
+  DevBuf win[2];                  // inflated window; the bytes left after its last whole record move to the other one
+  int cur = 0;
+  u64 carry = 0;                  // bytes at the front of win[cur]: the start of a record that continues
+  DevBuf seg_start, seg_cnt, seg_state, seg_land[2];
+  DevBuf off, valid, rowpos, vrec, starts, starts_x;
+  DevBuf rows[2][3];              // read_group, target_idx, hap_idx; the open read moves to the other set
+  int rcur = 0;
+  u64 n_rows = 0, open_row = 0;   // rows held in rows[rcur]; first row of the read that is still open
+  int64_t all_alignments = 0, group = -1;
+  bool failed = false, finished = false;
+  BamDevState* d_st = nullptr;
+  BamDevState* h_st = nullptr;    // pinned mirror
+  std::vector<BamBlock> h_blocks;
+  cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  ecb_bam_stats stats{};
+};
+
+namespace {
+
+#define ECB_BAM_AUTO_WINDOW (1ll << 30)
+
+int bam_sync_state(ecb_bam* d) {
+  ecb_ctx* c = d->c;
+  CK(cudaMemcpyAsync(d->h_st, d->d_st, sizeof(BamDevState), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return ECB_OK;
+}
+
+double bam_ms(cudaEvent_t a, cudaEvent_t b) {
+  float ms = 0;
+  cudaEventElapsedTime(&ms, a, b);
+  return ms;
+}
+
+void bam_release(ecb_bam* d) {
+  ecb_ctx* c = d->c;
+  DevBuf* bufs[] = {&d->tid_target, &d->tid_hap, &d->range_min, &d->range_max, &d->comp, &d->blocks, &d->win[0], &d->win[1],
+                    &d->seg_start, &d->seg_cnt, &d->seg_state, &d->seg_land[0], &d->seg_land[1], &d->off, &d->valid,
+                    &d->rowpos, &d->vrec, &d->starts, &d->starts_x};
+  for (DevBuf* b : bufs) release(c, *b);
+  for (auto& set : d->rows)
+    for (DevBuf& b : set) release(c, b);
+  cudaStreamSynchronize(c->stream);
+  if (d->d_st) cudaFree(d->d_st);
+  if (d->h_st) cudaFreeHost(d->h_st);
+  for (auto& e : d->ev)
+    if (e) cudaEventDestroy(e);
+  delete d;
+}
+
+// The records of win[cur][p0, carry + wbytes) after blocks [b0, b1) of the call were inflated behind the carry.
+int bam_window(ecb_bam* d, long long b0, long long b1, u64 wbytes, u32 p0) {
+  ecb_ctx* c = d->c;
+  const u64 wend64 = d->carry + wbytes;
+  if (wend64 >= (u64)ECB_BAM_NONE) return fail(c, ECB_ERR_LIMIT, "a BAM window of %llu inflated bytes (a record longer than 4 GiB?)", wend64);
+  const u32 wend = (u32)wend64;
+  CKR(ensure(c, d->win[d->cur], wend64 + 16, true));   // keeps the carried bytes
+  uint8_t* win = (uint8_t*)d->win[d->cur].p;
+  CK(cudaEventRecord(d->ev[2], c->stream));
+  if (b1 > b0) {
+    ecb_bam_inflate_kernel<<<(unsigned)((b1 - b0 + ECB_BAM_INFLATE_THREADS - 1) / ECB_BAM_INFLATE_THREADS), ECB_BAM_INFLATE_THREADS,
+                             0, c->stream>>>((const uint8_t*)d->comp.p, (const BamBlock*)d->blocks.p, b0, b1, win + d->carry, d->d_st);
+    LAUNCH_CHECK("bam_inflate");
+  }
+  CK(cudaEventRecord(d->ev[3], c->stream));
+  // a rejected block leaves its output range partly unwritten: report it before anything hops over that range
+  CKR(bam_sync_state(d));
+  if (d->h_st->error & BAM_ERR_INFLATE)
+    return fail(c, ECB_ERR_FORMAT, "corrupt BGZF block (inflate failed): block %lld of this call", d->h_st->bad_block);
+
+  // record hop: guesses, join rounds, offsets
+  const u32 n_seg = wend > p0 ? (wend - p0 + ECB_BAM_SEG - 1) / ECB_BAM_SEG : 1u;
+  CKR(ensure(c, d->seg_start, (size_t)n_seg * 4));
+  CKR(ensure(c, d->seg_cnt, (size_t)n_seg * 4));
+  CKR(ensure(c, d->seg_state, (size_t)n_seg * 4));
+  CKR(ensure(c, d->seg_land[0], (size_t)n_seg * 4));
+  CKR(ensure(c, d->seg_land[1], (size_t)n_seg * 4));
+  BamHop H{win, p0, wend, n_seg, d->n_ref, (u32*)d->seg_start.p, (u32*)d->seg_cnt.p, (u32*)d->seg_state.p};
+  u32* land[2] = {(u32*)d->seg_land[0].p, (u32*)d->seg_land[1].p};
+  const int grid = (int)((n_seg + 127) / 128);
+  ecb_bam_guess_kernel<<<grid, 128, 0, c->stream>>>(H, land[0]);
+  LAUNCH_CHECK("bam_guess");
+  int a = 0;
+  for (;;) {
+    CK(cudaMemsetAsync(&d->d_st->changed, 0, sizeof(u32), c->stream));
+    ecb_bam_round_kernel<<<grid, 128, 0, c->stream>>>(H, land[a], land[1 - a], &d->d_st->changed);
+    LAUNCH_CHECK("bam_round");
+    a = 1 - a;
+    d->stats.hop_rounds++;
+    CKR(bam_sync_state(d));
+    if (d->h_st->changed == 0) break;
+  }
+  u64 n_rec64 = 0;
+  CKR(device_scan<false>(c, H.cnt, H.cnt, n_seg, 0, &n_rec64));
+  const u32 n_rec = (u32)n_rec64;
+  CKR(ensure(c, d->off, (size_t)n_rec * 4 + 4));
+  ecb_bam_offsets_kernel<<<grid, 128, 0, c->stream>>>(H, H.cnt, land[a], (u32*)d->off.p, d->d_st);
+  LAUNCH_CHECK("bam_offsets");
+  CK(cudaEventRecord(d->ev[4], c->stream));
+  CKR(bam_sync_state(d));
+  if (d->h_st->hop_state == BAM_HOP_BAD) return fail(c, ECB_ERR_FORMAT, "BAM record with block_size %u", d->h_st->hop_bs);
+  const u32 land_at = d->h_st->hop_land;
+
+  // rules and rows
+  if (n_rec) {
+    BamRules R{win, (const u32*)d->off.p, n_rec, d->n_ref, (const int32_t*)d->tid_target.p, (const int32_t*)d->tid_hap.p,
+               d->track ? (int32_t*)d->range_min.p : nullptr, d->track ? (int32_t*)d->range_max.p : nullptr, d->d_st};
+    CKR(ensure(c, d->valid, (size_t)n_rec * 4));
+    CKR(ensure(c, d->rowpos, (size_t)n_rec * 4));
+    const int rgrid = (int)((n_rec + 255) / 256);
+    ecb_bam_validity_kernel<<<rgrid, 256, 0, c->stream>>>(R, (u32*)d->valid.p);
+    LAUNCH_CHECK("bam_validity");
+    u64 n_valid64 = 0;
+    CKR(device_scan<false>(c, (const u32*)d->valid.p, (u32*)d->rowpos.p, n_rec, 0, &n_valid64));
+    CKR(bam_sync_state(d));
+    if (d->h_st->error & BAM_ERR_NAME) return fail(c, ECB_ERR_FORMAT, "BAM record with a bad read-name length");
+    if (d->h_st->error & BAM_ERR_TID)
+      return fail(c, ECB_ERR_FORMAT, "alignment with reference id %d outside the header's %d references", d->h_st->bad_tid, d->n_ref);
+    const u32 n_valid = (u32)n_valid64;
+    if (n_valid) {
+      CKR(ensure(c, d->vrec, (size_t)n_valid * 4));
+      CKR(ensure(c, d->starts, (size_t)n_valid * 4));
+      CKR(ensure(c, d->starts_x, (size_t)n_valid * 4));
+      for (DevBuf& b : d->rows[d->rcur]) CKR(ensure(c, b, (size_t)(d->n_rows + n_valid) * 4, true));
+      ecb_bam_compact_kernel<<<rgrid, 256, 0, c->stream>>>(R, (const u32*)d->valid.p, (const u32*)d->rowpos.p, (u32*)d->vrec.p);
+      LAUNCH_CHECK("bam_compact");
+      const int vgrid = (int)((n_valid + 255) / 256);
+      ecb_bam_starts_kernel<<<vgrid, 256, 0, c->stream>>>(win, (const u32*)d->vrec.p, n_valid, d->d_st, (u32*)d->starts.p);
+      LAUNCH_CHECK("bam_starts");
+      u64 n_starts = 0;
+      CKR(device_scan<false>(c, (const u32*)d->starts.p, (u32*)d->starts_x.p, n_valid, 0, &n_starts));
+      ecb_bam_rows_kernel<<<vgrid, 256, 0, c->stream>>>(R, (const u32*)d->vrec.p, n_valid, (const u32*)d->starts.p,
+                                                         (const u32*)d->starts_x.p, d->group, d->n_rows,
+                                                         (int32_t*)d->rows[d->rcur][0].p, (int32_t*)d->rows[d->rcur][1].p,
+                                                         (int32_t*)d->rows[d->rcur][2].p);
+      LAUNCH_CHECK("bam_rows");
+      d->n_rows += n_valid;
+      d->group += (int64_t)n_starts;
+    }
+    d->all_alignments += n_rec;
+    d->stats.records += n_rec;
+  }
+  CK(cudaEventRecord(d->ev[5], c->stream));
+
+  // what follows the last whole record starts the next window
+  const u64 keep = wend - land_at;
+  if (keep) {
+    CKR(ensure(c, d->win[1 - d->cur], keep + 16));
+    CK(cudaMemcpyAsync(d->win[1 - d->cur].p, win + land_at, keep, cudaMemcpyDeviceToDevice, c->stream));
+    d->cur = 1 - d->cur;
+  }
+  d->carry = keep;
+  CK(cudaEventSynchronize(d->ev[5]));
+  d->stats.inflate_ms += bam_ms(d->ev[2], d->ev[3]);
+  d->stats.hop_ms += bam_ms(d->ev[3], d->ev[4]);
+  d->stats.rules_ms += bam_ms(d->ev[4], d->ev[5]);
+  d->stats.windows++;
+  return ECB_OK;
+}
+
+int bam_decode(ecb_bam* d, const uint8_t* bytes, int64_t n_bytes, const int64_t* block_off, const int32_t* block_len,
+               const int32_t* block_isize, int64_t n_blocks, int64_t skip, int last, const int32_t** read_group,
+               const int32_t** target_idx, const int32_t** hap_idx, int64_t* rows) {
+  ecb_ctx* c = d->c;
+  if (n_bytes < 0 || n_blocks < 0 || skip < 0) return fail(c, ECB_ERR_INVALID, "negative size");
+  if ((n_blocks > 0 && (!block_off || !block_len || !block_isize)) || (n_bytes > 0 && !bytes))
+    return fail(c, ECB_ERR_INVALID, "NULL block table or bytes");
+  if (skip > 0 && d->carry) return fail(c, ECB_ERR_INVALID, "skip is only meaningful before the first record");
+  // the block table comes from outside the library: every block must lie inside `bytes`
+  d->h_blocks.resize((size_t)n_blocks);
+  int64_t total = 0;
+  for (int64_t i = 0; i < n_blocks; ++i) {
+    if (block_off[i] < 0 || block_len[i] < 0 || block_off[i] > n_bytes || block_len[i] > n_bytes - block_off[i])
+      return fail(c, ECB_ERR_INVALID, "block %lld lies outside the %lld bytes given", (long long)i, (long long)n_bytes);
+    if (block_isize[i] < 0 || block_isize[i] > 65536)
+      return fail(c, ECB_ERR_FORMAT, "BGZF block %lld of this call claims %u inflated bytes; the device decoder takes at most 65536",
+                  (long long)i, (unsigned)block_isize[i]);
+    d->h_blocks[(size_t)i] = BamBlock{(u64)block_off[i], (u32)block_len[i], (u32)block_isize[i], 0};
+    total += block_isize[i];
+  }
+  if (skip > total) return fail(c, ECB_ERR_INVALID, "skip %lld beyond the %lld inflated bytes of the call", (long long)skip, (long long)total);
+  CK(cudaSetDevice(c->device));
+
+  // rows of the read the previous call left open go to the front
+  if (d->open_row > 0) {
+    const u64 keep = d->n_rows - d->open_row;
+    const int other = 1 - d->rcur;
+    for (int j = 0; j < 3; ++j) {
+      CKR(ensure(c, d->rows[other][j], (size_t)keep * 4 + 4));
+      if (keep)
+        CK(cudaMemcpyAsync(d->rows[other][j].p, (const int32_t*)d->rows[d->rcur][j].p + d->open_row, (size_t)keep * 4,
+                           cudaMemcpyDeviceToDevice, c->stream));
+    }
+    d->rcur = other;
+    d->n_rows = keep;
+    d->open_row = 0;
+    CK(cudaMemsetAsync(&d->d_st->open_row, 0, sizeof(unsigned long long), c->stream));
+  }
+
+  // windows of whole blocks, at most ECB_OPT_BAM_WINDOW inflated bytes each (at least one block)
+  const int64_t wmax = c->opt_bam_window > 0 ? c->opt_bam_window : ECB_BAM_AUTO_WINDOW;
+  std::vector<int64_t> cut{0};
+  std::vector<u64> wbytes;
+  {
+    u64 acc = 0;
+    for (int64_t i = 0; i < n_blocks; ++i) {
+      const u64 sz = d->h_blocks[(size_t)i].isize;
+      if (i > cut.back() && acc + sz > (u64)wmax) {
+        cut.push_back(i);
+        wbytes.push_back(acc);
+        acc = 0;
+      }
+      d->h_blocks[(size_t)i].dst_off = acc;
+      acc += sz;
+    }
+    if (n_blocks > 0) {
+      cut.push_back(n_blocks);
+      wbytes.push_back(acc);
+    }
+  }
+  if (!wbytes.empty() && (u64)skip > wbytes[0]) return fail(c, ECB_ERR_INVALID, "skip %lld beyond the first window", (long long)skip);
+
+  CK(cudaEventRecord(d->ev[0], c->stream));
+  if (n_blocks > 0) {
+    CKR(ensure(c, d->comp, (size_t)n_bytes + 16));
+    CKR(ensure(c, d->blocks, (size_t)n_blocks * sizeof(BamBlock)));
+    CK(cudaMemcpyAsync(d->comp.p, bytes, (size_t)n_bytes, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(d->blocks.p, d->h_blocks.data(), (size_t)n_blocks * sizeof(BamBlock), cudaMemcpyHostToDevice, c->stream));
+    d->stats.h2d_bytes += n_bytes;
+    d->stats.blocks += n_blocks;
+    d->stats.inflated_bytes += total;
+  }
+  CK(cudaEventRecord(d->ev[1], c->stream));
+  for (size_t w = 0; w < wbytes.size(); ++w)
+    CKR(bam_window(d, cut[w], cut[w + 1], wbytes[w], w == 0 ? (u32)skip : 0u));
+  CKR(bam_sync_state(d));
+  d->stats.h2d_ms += bam_ms(d->ev[0], d->ev[1]);
+  if (last) {
+    if (d->carry) return fail(c, ECB_ERR_FORMAT, "truncated BAM record at the end of the file");
+    d->finished = true;
+    d->open_row = d->n_rows;   // the end of the file closes the last read
+  } else {
+    d->open_row = d->h_st->open_row;
+  }
+  *read_group = (const int32_t*)d->rows[d->rcur][0].p;
+  *target_idx = (const int32_t*)d->rows[d->rcur][1].p;
+  *hap_idx = (const int32_t*)d->rows[d->rcur][2].p;
+  *rows = (int64_t)d->open_row;
+  return ECB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ecb_bam_create(ecb_ctx* c, const int32_t* tid_target, const int32_t* tid_hap, int32_t n_references, int track_ranges,
+                   ecb_bam** out) {
+  if (!c || !out) return ECB_ERR_INVALID;
+  *out = nullptr;
+  if (n_references < 0 || (n_references > 0 && (!tid_target || !tid_hap))) return fail(c, ECB_ERR_INVALID, "bad reference tables");
+  if (c->with_cells) return fail(c, ECB_ERR_INVALID, "the device BAM decoder covers the single-sample path only");
+  CK(cudaSetDevice(c->device));
+  ecb_bam* d = new ecb_bam();
+  d->c = c;
+  d->n_ref = n_references;
+  d->track = track_ranges != 0;
+  auto bail = [&](int code) {
+    bam_release(d);
+    return code;
+  };
+  const size_t tb = (size_t)n_references * 4 + 4;
+  int rc = ECB_OK;
+  for (DevBuf* b : {&d->tid_target, &d->tid_hap, &d->range_min, &d->range_max})
+    if (rc == ECB_OK) rc = ensure(c, *b, tb);
+  if (rc != ECB_OK) return bail(rc);
+  std::vector<int32_t> lo((size_t)n_references + 1, INT32_MAX);
+  if (cudaMalloc(&d->d_st, sizeof(BamDevState)) != cudaSuccess || cudaMallocHost(&d->h_st, sizeof(BamDevState)) != cudaSuccess)
+    return bail(fail(c, ECB_ERR_CUDA, "decoder state allocation failed"));
+  for (auto& e : d->ev)
+    if (cudaEventCreate(&e) != cudaSuccess) return bail(fail(c, ECB_ERR_CUDA, "cudaEventCreate failed"));
+  memset(d->h_st, 0, sizeof(BamDevState));
+  d->h_st->bad_block = 0x7FFFFFFFFFFFFFFFll;
+  const cudaMemcpyKind h2d = cudaMemcpyHostToDevice;
+  if (n_references > 0 &&
+      (cudaMemcpyAsync(d->tid_target.p, tid_target, (size_t)n_references * 4, h2d, c->stream) != cudaSuccess ||
+       cudaMemcpyAsync(d->tid_hap.p, tid_hap, (size_t)n_references * 4, h2d, c->stream) != cudaSuccess))
+    return bail(fail(c, ECB_ERR_CUDA, "table copy failed"));
+  if (cudaMemcpyAsync(d->range_min.p, lo.data(), tb, h2d, c->stream) != cudaSuccess ||
+      cudaMemsetAsync(d->range_max.p, 0xFF, tb, c->stream) != cudaSuccess ||
+      cudaMemcpyAsync(d->d_st, d->h_st, sizeof(BamDevState), h2d, c->stream) != cudaSuccess ||
+      cudaStreamSynchronize(c->stream) != cudaSuccess)
+    return bail(fail(c, ECB_ERR_CUDA, "decoder initialisation failed"));
+  *out = d;
+  return ECB_OK;
+}
+
+int ecb_bam_decode(ecb_bam* d, const uint8_t* bytes, int64_t n_bytes, const int64_t* block_off, const int32_t* block_len,
+                   const int32_t* block_isize, int64_t n_blocks, int64_t skip, int last, const int32_t** read_group,
+                   const int32_t** target_idx, const int32_t** hap_idx, int64_t* rows) {
+  if (!d || !read_group || !target_idx || !hap_idx || !rows) return ECB_ERR_INVALID;
+  if (d->failed) return fail(d->c, ECB_ERR_STATE, "this decoder failed earlier; create a new one");
+  if (d->finished) return fail(d->c, ECB_ERR_STATE, "this decoder has had its last call");
+  const int rc = bam_decode(d, bytes, n_bytes, block_off, block_len, block_isize, n_blocks, skip, last, read_group,
+                            target_idx, hap_idx, rows);
+  if (rc != ECB_OK) d->failed = true;
+  return rc;
+}
+
+int ecb_bam_counters(const ecb_bam* d, int64_t* all_alignments, int64_t* n_groups) {
+  if (!d || !all_alignments || !n_groups) return ECB_ERR_INVALID;
+  *all_alignments = d->all_alignments;
+  *n_groups = d->group + 1;
+  return ECB_OK;
+}
+
+int ecb_bam_ranges(ecb_bam* d, int32_t* range_min, int32_t* range_max) {
+  if (!d || (d->n_ref > 0 && (!range_min || !range_max))) return ECB_ERR_INVALID;
+  ecb_ctx* c = d->c;
+  if (!d->track) return fail(c, ECB_ERR_STATE, "ranges were not tracked");
+  if (d->n_ref == 0) return ECB_OK;
+  CK(cudaSetDevice(c->device));
+  CK(cudaMemcpyAsync(range_min, d->range_min.p, (size_t)d->n_ref * 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(range_max, d->range_max.p, (size_t)d->n_ref * 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return ECB_OK;
+}
+
+int ecb_bam_get_stats(const ecb_bam* d, ecb_bam_stats* out) {
+  if (!d || !out) return ECB_ERR_INVALID;
+  *out = d->stats;
+  return ECB_OK;
+}
+
+int ecb_bam_destroy(ecb_bam* d) {
+  if (!d) return ECB_OK;
+  cudaSetDevice(d->c->device);
+  bam_release(d);
   return ECB_OK;
 }
 

@@ -109,6 +109,17 @@ def use_python_emitter():
     return os.environ.get("ALNTOOLS_B200_EMITTER", "native").lower() == "python"
 
 
+def decode_mode(decode=None):
+    """Where a single-sample convert() decodes the BAM file: `decode`, else the environment variable
+    ALNTOOLS_B200_DECODE (the CLI keeps the reference's options, so the environment is its only way to say it):
+    "host" (default: libbamcols on the CPU threads) or "device" (BGZF inflate and the record pass on the GPU)."""
+    import os
+    mode = decode if decode is not None else os.environ.get("ALNTOOLS_B200_DECODE", "host")
+    if str(mode).lower() not in ("host", "device"):
+        raise ValueError("the BAM decode must be 'host' or 'device' (decode= / ALNTOOLS_B200_DECODE), not %r" % (mode,))
+    return str(mode).lower()
+
+
 _PINNED_POOL = []      # pinned buffer sets of finished conversions, reused by the next one in this process
 
 
@@ -207,6 +218,88 @@ def stream_single(reader, builder, chunk_rows=1 << 21, pinned=True, depth=3):
         worker.join()
         _release_buffers(all_sets, pinned)
     return pushed
+
+
+_PINNED_BYTES = []     # pinned read buffers of finished device decodes, reused by the next one in this process
+
+
+def stream_single_device(path, reader, builder, tables, track_ranges, max_bytes=128 << 20, depth=3):
+    """Decode the single-sample BAM file `path` on the GPU (_native.BamDecoder on `builder`'s context) and push
+    its columns.  `reader` (bamcols.BamColumnReader of the same file) lists the BGZF blocks; a worker thread reads
+    runs of whole blocks (up to max_bytes) into a small ring of pinned buffers while the previous run is decoded.
+    order_base = rows pushed so far, so the result equals stream_single's.  A call's blocks are inflated one thread
+    per block, so runs are large: a 128 MiB run holds a few thousand blocks.
+    Returns (valid alignments, (all_alignments, n_groups), (range_min, range_max) or None, decoder stats)."""
+    import queue
+    import threading
+    import torch
+    from ._native import BamDecoder
+    first = reader.plan_shards(1)[0]                      # virtual offset of the first record
+    free, full = queue.Queue(), queue.Queue()
+    cap = int(max_bytes) + (1 << 17)                      # a run holds at least one block (< 64 KiB + header)
+    bufs = []
+    while _PINNED_BYTES and len(bufs) < depth:           # pinning costs about as much as reading the bytes
+        b = _PINNED_BYTES.pop()
+        if int(b.shape[0]) >= cap:
+            bufs.append(b)
+    bufs += [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(depth - len(bufs))]
+    for b in bufs:
+        free.put(b)
+    stop = threading.Event()
+
+    def produce():
+        try:
+            c = first >> 16
+            with open(path, "rb") as fh:
+                while not stop.is_set():
+                    off, length, isize, c_end = reader.blocks(c, max_bytes)
+                    if len(off) == 0:
+                        full.put((None, 0, None, None))
+                        return
+                    buf = None
+                    while buf is None and not stop.is_set():
+                        try:
+                            buf = free.get(timeout=0.05)
+                        except queue.Empty:
+                            pass
+                    if buf is None:
+                        return
+                    n = c_end - c
+                    fh.seek(c)
+                    if fh.readinto(memoryview(buf.numpy())[:n]) != n:
+                        raise IOError("%s changed while it was read" % path)
+                    full.put((buf, n, (off, length, isize), None))
+                    c = c_end
+        except BaseException as exc:                      # re-raised by the consumer
+            full.put((None, 0, None, exc))
+
+    pushed = 0
+    with BamDecoder(builder, tables.tid_target, tables.tid_hap, track_ranges) as dec:
+        worker = threading.Thread(target=produce, daemon=True)
+        worker.start()
+        try:
+            skip = first & 0xFFFF
+            while True:
+                buf, n, table, exc = full.get()
+                if exc is not None:
+                    raise exc
+                if buf is None:
+                    rg, tg, hp = dec.decode(np.zeros(0, np.uint8), [], [], [], last=True)
+                else:
+                    rg, tg, hp = dec.decode(buf, *table, skip=skip, n_bytes=n)
+                    skip = 0
+                rows = int(rg.shape[0])
+                if rows:
+                    builder.push(rg, tg, hp, order_base=pushed, n=rows)
+                    pushed += rows
+                if buf is None:
+                    break
+                free.put(buf)
+        finally:
+            stop.set()
+            worker.join()
+            _PINNED_BYTES.extend(bufs)
+        return pushed, dec.counters(), dec.ranges() if track_ranges else None, dec.stats()
 
 
 def read_bam(filename):

@@ -106,3 +106,53 @@ def columns_to_bam(filename, cols, n_targets, n_haps, level=1):
     tids = cols["target_idx"].astype(np.int64) * n_haps + cols["hap_idx"]
     bam_io.write_bam_columns(filename, reference_names(n_targets, n_haps), cols["read_group"],
                              np.zeros(len(tids), dtype=np.uint16), tids, level=level)
+
+
+def columns_to_bam_seq(filename, cols, n_targets, n_haps, read_len=100, level=1, seed=0):
+    """columns_to_bam with the record shape of a real aligner's output: every record carries a CIGAR of one
+    read_len-M operation, the packed sequence and the base qualities (seeded random bases and qualities)."""
+    from . import bam_io
+    import struct
+    tids = cols["target_idx"].astype(np.int64) * n_haps + cols["hap_idx"]
+    ids = np.asarray(cols["read_group"], dtype=np.int64)
+    n = len(tids)
+    name_len = len("read%09d" % 0) + 1
+    seq_len = (read_len + 1) // 2
+    body = 32 + name_len + 4 + seq_len + read_len
+    rec_len = 4 + body
+    raw = np.zeros((n, rec_len), dtype=np.uint8)
+    raw[:, 0:4] = np.frombuffer(struct.pack("<i", body), dtype=np.uint8)
+    core = np.zeros(n, dtype=np.dtype([("tid", "<i4"), ("pos", "<i4"), ("l_name", "u1"), ("mapq", "u1"),
+                                       ("bin", "<u2"), ("ncig", "<u2"), ("flag", "<u2"), ("lseq", "<i4"),
+                                       ("ntid", "<i4"), ("npos", "<i4"), ("tlen", "<i4")]))
+    core["tid"] = tids
+    core["pos"] = 10
+    core["l_name"] = name_len
+    core["mapq"] = 255
+    core["bin"] = 4680
+    core["ncig"] = 1
+    core["lseq"] = read_len
+    core["ntid"] = -1
+    core["npos"] = -1
+    raw[:, 4:36] = core.view(np.uint8).reshape(n, 32)
+    raw[:, 36:40] = np.frombuffer(b"read", dtype=np.uint8)
+    rem = ids.copy()
+    for d in range(8, -1, -1):
+        raw[:, 40 + d] = (rem % 10 + 48).astype(np.uint8)
+        rem //= 10
+    at = 36 + name_len
+    raw[:, at:at + 4] = np.frombuffer(struct.pack("<I", read_len << 4), dtype=np.uint8)
+    rng = np.random.default_rng(seed)
+    bases = np.array([1, 2, 4, 8], dtype=np.uint8)                 # A C G T in BAM's 4-bit code
+    seq = bases[rng.integers(0, 4, (n, 2 * seq_len))]
+    raw[:, at + 4:at + 4 + seq_len] = (seq[:, 0::2] << 4) | seq[:, 1::2]
+    raw[:, at + 4 + seq_len:] = rng.integers(2, 41, (n, read_len), dtype=np.uint8)
+    flat = raw.reshape(-1)
+    per_block = max(1, 60000 // rec_len) * rec_len
+    with open(filename, "wb") as fh:
+        header = bam_io.bam_header_bytes(reference_names(n_targets, n_haps))
+        for off in range(0, len(header), 60000):
+            fh.write(bam_io.bgzf_block(header[off:off + 60000], level))
+        for off in range(0, flat.size, per_block):
+            fh.write(bam_io.bgzf_block(flat[off:off + per_block].tobytes(), level))
+        fh.write(bam_io.BGZF_EOF)

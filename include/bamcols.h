@@ -100,6 +100,14 @@ int64_t bamcols_emit(bamcols* r, bamcols_cells* cells, int32_t* read_group, int3
 int bamcols_plan_shards(bamcols* r, int n_shards, int64_t* voffsets);
 int bamcols_set_range(bamcols* r, int64_t vbegin, int64_t vend);
 
+/* The BGZF blocks from compressed offset c_begin on, without inflating them (the block table of the device decoder,
+ * ecb_bam_decode in include/ecb200.h): at most max_blocks blocks whose compressed bytes fit in max_bytes - at least
+ * one block whenever one is left.  payload_off[i] = offset of block i's raw DEFLATE payload counted from c_begin,
+ * payload_len[i] its length, isize[i] its inflated size; *c_end = offset behind the last listed block.  Returns the
+ * number of blocks (0 at the end of the file) or BAMCOLS_ERR_FORMAT with the messages of the reader. */
+int64_t bamcols_blocks(bamcols* r, int64_t c_begin, int64_t max_bytes, int64_t max_blocks, int64_t* payload_off,
+                       int32_t* payload_len, int32_t* isize, int64_t* c_end);
+
 /* Counters so far: records seen (valid or not) and reads started. */
 int64_t bamcols_all_alignments(const bamcols* r);
 int64_t bamcols_n_groups(const bamcols* r);

@@ -43,7 +43,8 @@ enum ecb_status {
   ECB_ERR_LIMIT = -4,       /* a format limit was exceeded (int32 file fields, read too long, ...) */
   ECB_ERR_EMPTY = -5,       /* finalize with zero equivalence classes (the reference raises too:
                                alntools/matrix/Sparse3DMatrix.py:45-46) */
-  ECB_ERR_STATE = -6        /* call sequence error */
+  ECB_ERR_STATE = -6,       /* call sequence error */
+  ECB_ERR_FORMAT = -7       /* malformed BAM input of the device decoder (ecb_bam_decode; since version 2002) */
 };
 
 /* Longest read (alignments sharing one name) whose canonical row can be built. */
@@ -65,6 +66,8 @@ enum ecb_option {
   ECB_OPT_CHUNK_LEN = 7,        /* alignments per work chunk of the grouping kernel (0 = automatic) */
   ECB_OPT_PAGEABLE_RESULTS = 8, /* 1: host results go to ordinary (malloc) memory instead of pinned memory:
                                    cheaper for a context that finalizes once, slower when reused */
+  ECB_OPT_BAM_WINDOW = 9,       /* inflated bytes per window of the device BAM decoder (0 = automatic, 1 GiB);
+                                   a window always takes at least one block */
 };
 
 typedef struct ecb_result {
@@ -265,6 +268,55 @@ typedef struct ecb_cells_slice {
 } ecb_cells_slice;
 int ecb_cells_order_build(ecb_ctx* owner_ctx, const ecb_ctx* local_ctx, int64_t shard_lo, int64_t shard_hi, int64_t n_samples,
                           ecb_cells_slice* out);
+
+/* ---- device decode of single-sample BAM files (since version 2002) ------------------------------------------
+ * The GPU form of libbamcols' single-sample path (include/bamcols.h): BGZF inflate, the record hop, the filters of
+ * alntools/bam_utils.py:264-270, name trimming (:301-304) and the name-change test (:306), producing in device
+ * memory the columns bamcols_emit produces, ready for ecb_push(..., on_device = 1).  A decoder is bound to one
+ * context and uses its device, stream and memory pool; destroy it before the context.  A decoder that has
+ * failed refuses further calls: create a fresh one (after ecb_reset when the context's pushes are abandoned).
+ *
+ * ecb_bam_create: tid_target / tid_hap[n_references] as for bamcols_set_tables (copied); track_ranges = 1
+ * records the smallest and largest pos of the valid alignments of every reference (--rangefile).
+ *
+ * ecb_bam_decode: one call per run of whole BGZF blocks, in file order.
+ *   bytes[n_bytes]      compressed bytes on the host (pinned preferred), copied to the device
+ *   block_off[i]        offset in bytes of block i's raw DEFLATE payload, block_len[i] its length,
+ *   block_isize[i]      its inflated size (ISIZE; at most 65 536, larger blocks are refused with ECB_ERR_FORMAT)
+ *                       - the table bamcols_blocks lists
+ *   skip                inflated bytes of the first block before the first record (the low 16 bits of the first
+ *                       record's virtual offset); 0 after the first call
+ *   last                1 on the final call: the last read is closed, and bytes left after the last whole record
+ *                       are a truncated record
+ * Returns DEVICE pointers to the rows of every read closed by this call (valid until the next call on the decoder);
+ * read_group continues from call to call as bamcols_emit's does.  The blocks are inflated in windows of
+ * ECB_OPT_BAM_WINDOW bytes; records and reads may span blocks, windows and calls.  Corrupt blocks, truncated
+ * records, block_size < 32 and bad read-name lengths fail with ECB_ERR_FORMAT, and so does a valid alignment whose
+ * refID lies outside the header (with its own message). */
+typedef struct ecb_bam ecb_bam;
+typedef struct ecb_bam_stats {
+  int64_t h2d_bytes;       /* compressed bytes copied host->device                                            */
+  int64_t inflated_bytes;
+  int64_t blocks;
+  int64_t windows;
+  int64_t hop_rounds;      /* join rounds of the record hop (1 per window when every segment guessed right)     */
+  int64_t records;         /* = all_alignments                                                                 */
+  double h2d_ms;           /* stream time between CUDA events around each phase, summed over the calls: the  */
+  double inflate_ms;       /* hop and rules phases include the host round trips of their count read-backs    */
+  double hop_ms;
+  double rules_ms;
+} ecb_bam_stats;
+int ecb_bam_create(ecb_ctx* ctx, const int32_t* tid_target, const int32_t* tid_hap, int32_t n_references,
+                   int track_ranges, ecb_bam** out);
+int ecb_bam_decode(ecb_bam* d, const uint8_t* bytes, int64_t n_bytes, const int64_t* block_off, const int32_t* block_len,
+                   const int32_t* block_isize, int64_t n_blocks, int64_t skip, int last, const int32_t** read_group,
+                   const int32_t** target_idx, const int32_t** hap_idx, int64_t* rows);
+/* records seen so far (valid or not) and reads started */
+int ecb_bam_counters(const ecb_bam* d, int64_t* all_alignments, int64_t* n_groups);
+/* host int32[n_references] each; min > max where no valid alignment was seen (as bamcols_ranges) */
+int ecb_bam_ranges(ecb_bam* d, int32_t* range_min, int32_t* range_max);
+int ecb_bam_get_stats(const ecb_bam* d, ecb_bam_stats* out);
+int ecb_bam_destroy(ecb_bam* d);
 
 #ifdef __cplusplus
 }
