@@ -21,6 +21,8 @@ ECB_OPT_VERIFY_KEYS = 6
 ECB_OPT_CHUNK_LEN = 7
 ECB_OPT_PAGEABLE_RESULTS = 8
 ECB_OPT_BAM_WINDOW = 9
+ECB_OPT_COLLATE_SLOTS = 10
+ECB_OPT_COLLATE_PIECE = 11
 
 ECB_ERR_EMPTY = -5
 ECB_ERR_FORMAT = -7
@@ -79,6 +81,18 @@ class EcbBamStats(ctypes.Structure):
         return {name: getattr(self, name) for name, _ in self._fields_}
 
 
+class EcbCollateStats(ctypes.Structure):
+    _fields_ = [
+        ("alignments", ctypes.c_int64), ("reads", ctypes.c_int64), ("table_slots", ctypes.c_int64),
+        ("table_grows", ctypes.c_int64), ("pieces", ctypes.c_int64), ("device_bytes", ctypes.c_int64),
+        ("h2d_bytes", ctypes.c_int64), ("add_ms", ctypes.c_double), ("table_ms", ctypes.c_double),
+        ("order_ms", ctypes.c_double), ("layout_ms", ctypes.c_double), ("push_ms", ctypes.c_double),
+    ]
+
+    def as_dict(self):
+        return {name: getattr(self, name) for name, _ in self._fields_}
+
+
 # every symbol include/ecb200.h declares, with its ctypes signature
 SIGNATURES = {
     "ecb_version": (ctypes.c_int, []),
@@ -129,6 +143,12 @@ SIGNATURES = {
     "ecb_bam_ranges": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "ecb_bam_get_stats": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbBamStats)]),
     "ecb_bam_destroy": (ctypes.c_int, [ctypes.c_void_p]),
+    "ecb_collate_create": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_void_p)]),
+    "ecb_collate_add": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                       ctypes.c_int64, ctypes.c_int]),
+    "ecb_collate_push": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64)]),
+    "ecb_collate_get_stats": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbCollateStats)]),
+    "ecb_collate_destroy": (ctypes.c_int, [ctypes.c_void_p]),
 }
 
 _lib = None
@@ -215,7 +235,8 @@ class EcBuilder(object):
                 "pair_slots": ECB_OPT_PAIR_SLOTS, "grid_ctas": ECB_OPT_GRID_CTAS,
                 "hot_cache": ECB_OPT_HOT_CACHE, "verify_keys": ECB_OPT_VERIFY_KEYS,
                 "chunk_len": ECB_OPT_CHUNK_LEN, "pageable_results": ECB_OPT_PAGEABLE_RESULTS,
-                "bam_window": ECB_OPT_BAM_WINDOW}
+                "bam_window": ECB_OPT_BAM_WINDOW, "collate_slots": ECB_OPT_COLLATE_SLOTS,
+                "collate_piece": ECB_OPT_COLLATE_PIECE}
 
     def _check(self, rc):
         if rc != 0:
@@ -494,6 +515,73 @@ class BamDecoder(object):
     def close(self):
         if self._h:
             self._lib.ecb_bam_destroy(self._h)
+            self._h = ctypes.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _column_ptr(x, dtypes):
+    """Address of a contiguous numpy array or torch tensor (host or device) of one of `dtypes` (numpy dtype names)."""
+    if isinstance(x, np.ndarray):
+        if x.dtype.name not in dtypes or not x.flags["C_CONTIGUOUS"]:
+            raise TypeError("expected a C-contiguous array of %s, got %s" % ("/".join(dtypes), x.dtype))
+        return x.ctypes.data
+    if hasattr(x, "data_ptr"):
+        if str(x.dtype).replace("torch.", "") not in dtypes or not x.is_contiguous():
+            raise TypeError("expected a contiguous tensor of %s, got %s" % ("/".join(dtypes), x.dtype))
+        return x.data_ptr()
+    raise TypeError("unsupported column type %r" % type(x))
+
+
+class Collator(object):
+    """Collation by read name on `builder`'s context (ecb_collate_* in include/ecb200.h): add() the rows of
+    BamColumnReader.emit_keys in file order, then push() regroups them on the GPU and pushes them into the builder as
+    name-grouped reads."""
+
+    def __init__(self, builder):
+        self._lib = builder._lib
+        self._builder = builder                   # the collator lives in the builder's context: keep it alive
+        self._h = ctypes.c_void_p()
+        self._check(self._lib.ecb_collate_create(builder._ctx, ctypes.byref(self._h)))
+
+    def _check(self, rc):
+        if rc != 0:
+            raise EcbError(rc, self._lib.ecb_last_error(self._builder._ctx).decode())
+
+    def add(self, key_lo, key_hi, target_idx, hap_idx, n=None):
+        """key_lo / key_hi: uint64 (numpy) or int64 / uint64 (torch) columns; target_idx / hap_idx: int32.  numpy
+        arrays, pinned host tensors or device tensors on the builder's GPU; the first n rows (default: all)."""
+        if n is None:
+            n = int(key_lo.shape[0])
+        wide = ("uint64", "int64")
+        self._check(self._lib.ecb_collate_add(self._h, _column_ptr(key_lo, wide), _column_ptr(key_hi, wide),
+                                              _column_ptr(target_idx, ("int32",)), _column_ptr(hap_idx, ("int32",)),
+                                              int(n), 1 if _on_device(key_lo) else 0))
+
+    def push(self):
+        """Regroup everything added and push it into the builder; -> number of reads."""
+        n_reads = ctypes.c_int64()
+        self._check(self._lib.ecb_collate_push(self._h, ctypes.byref(n_reads)))
+        return int(n_reads.value)
+
+    def stats(self):
+        st = EcbCollateStats()
+        self._check(self._lib.ecb_collate_get_stats(self._h, ctypes.byref(st)))
+        return st.as_dict()
+
+    def close(self):
+        if self._h:
+            self._lib.ecb_collate_destroy(self._h)
             self._h = ctypes.c_void_p()
 
     def __enter__(self):

@@ -154,14 +154,15 @@ def _job_plan(num_chunks, number_processes):
     return num_chunks, min(num_processes, num_chunks)
 
 
-def _convert_python_emitter(bam_filename, target_filename, device, start_time):
-    """The same build fed by the record-level Python emitter (ALNTOOLS_B200_EMITTER=python)."""
+def _convert_python_emitter(bam_filename, target_filename, device, start_time, collate=False):
+    """The same build fed by the record-level Python emitter (ALNTOOLS_B200_EMITTER=python); collate: reads by name
+    over the whole file (emitter.emit_collated)."""
     temp_time = time.time()
     header, records = emitter.read_bam(bam_filename)
     tables = TargetTables(header.references, header.lengths, target_filename)
     LOG.info("File parsed in {}, total time: {}".format(utils.format_time(temp_time, time.time()),
                                                         utils.format_time(start_time, time.time())))
-    cols = emitter.emit_single(records, tables)
+    cols = emitter.emit_collated(records, tables) if collate else emitter.emit_single(records, tables)
     if cols.valid_alignments == 0:
         raise RuntimeError("The shape must be a tuple of three positive integers.")
     with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=False,
@@ -286,7 +287,7 @@ def convert_rank(bam_filename, ec_filename, emase_filename, num_chunks=0, number
 
 
 def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_processes=-1, temp_dir=None,
-            range_filename=None, sample=None, target_filename=None, device=0, devices=None, decode=None):
+            range_filename=None, sample=None, target_filename=None, device=0, devices=None, decode=None, collate=None):
     """Convert a name-grouped BAM file into an EC binary file and/or an EMASE file.
 
     Arguments keep the reference's meaning.  num_chunks / number_processes only shape the host decode
@@ -297,9 +298,14 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
     The EC file does not depend on the number of GPUs.  decode="device" (or ALNTOOLS_B200_DECODE=device) inflates
     and decodes the BAM file on the GPU (one GPU, native emitter); "host" (the default) decodes it on the CPU.
     The outputs do not depend on it.
+    collate=True (or ALNTOOLS_B200_COLLATE=1) takes a file that is not grouped by read name: a read is every valid
+    alignment with one trimmed name, wherever it lies, and reads are ordered by their first alignment (one GPU, host
+    decode).  The outputs are those of the default convert() of the file regrouped that way; for a grouped file they
+    are the default's.
     """
     start_time = time.time()
     mode = emitter.decode_mode(decode)
+    collate = emitter.collate_mode(collate)
     if mode == "device":
         if utils.under_launcher() or utils.requested_gpus(devices) > 1:
             raise NotImplementedError("device BAM decode runs on one GPU; the multi-GPU convert has no device decode yet "
@@ -307,6 +313,13 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
         if emitter.use_python_emitter():
             raise NotImplementedError("device BAM decode replaces the native emitter; it does not combine with "
                                       "ALNTOOLS_B200_EMITTER=python")
+    if collate:
+        if utils.under_launcher() or utils.requested_gpus(devices) > 1:
+            raise NotImplementedError("collation by read name runs on one GPU: reads span the shards of a multi-GPU "
+                                      "convert (unset ALNTOOLS_B200_COLLATE or use one GPU)")
+        if mode == "device":
+            raise NotImplementedError("collation by read name takes the host decode (use decode='host' / unset "
+                                      "ALNTOOLS_B200_DECODE)")
     job = dict(bam_filename=bam_filename, ec_filename=ec_filename, emase_filename=emase_filename, num_chunks=num_chunks,
                number_processes=number_processes, temp_dir=temp_dir, range_filename=range_filename, sample=sample,
                target_filename=target_filename)
@@ -364,7 +377,7 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
     LOG.info("Parsing file information ...")
     temp_time = time.time()
     if emitter.use_python_emitter():
-        res, tables, valid = _convert_python_emitter(bam_filename, target_filename, device, start_time)
+        res, tables, valid = _convert_python_emitter(bam_filename, target_filename, device, start_time, collate)
         return save(res, tables, valid, temp_time)
     # native emitter: inflate threads + one record pass, streamed to the GPU in read-aligned chunks
     import torch
@@ -379,11 +392,14 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
         # grows it ahead of later ones; one finalize per context, so results skip the pinning cost
         with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=False, alignments_hint=0,
                        device=device, pageable_results=1) as builder:
+            chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(bam_filename) // 2)))   # 24 MB of columns per piece
             if mode == "device":
                 valid, _, ranges, _ = emitter.stream_single_device(bam_filename, reader, builder, tables,
                                                                 range_filename is not None)
+            elif collate:
+                valid, _, _ = emitter.stream_collated(reader, builder, chunk_rows=chunk_rows, pinned=torch.cuda.is_available())
+                ranges = reader.ranges() if range_filename is not None else None
             else:
-                chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(bam_filename) // 2)))   # 24 MB of columns per piece
                 valid = emitter.stream_single(reader, builder, chunk_rows=chunk_rows, pinned=torch.cuda.is_available())
                 ranges = reader.ranges() if range_filename is not None else None
             if valid == 0:

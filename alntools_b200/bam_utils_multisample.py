@@ -283,6 +283,12 @@ def _assemble(parts, n_ec):
     return a_csr, (n_indptr.astype(np.int32), idx, dat)
 
 
+def _refuse_collation():
+    if emitter.collate_mode():
+        raise NotImplementedError("the per-cell (--multisample) conversion has no collation by read name: its rules "
+                                  "depend on consecutive records (unset ALNTOOLS_B200_COLLATE)")
+
+
 def convert_files(bam_files, ec_filename, emase_filename, minimum_count, target_filename=None, device=0,
                   range_filename=None, devices=None):
     """The reference's convert() after its glob: files are merged in the given order
@@ -292,6 +298,7 @@ def convert_files(bam_files, ec_filename, emase_filename, minimum_count, target_
     if emitter.decode_mode() == "device":
         raise NotImplementedError("the per-cell (--multisample) conversion has no device BAM decode yet: it needs a GPU "
                                   "cell-name dictionary (unset ALNTOOLS_B200_DECODE)")
+    _refuse_collation()
     job = dict(bam_files=list(bam_files), ec_filename=ec_filename, emase_filename=emase_filename,
                minimum_count=minimum_count, target_filename=target_filename, range_filename=range_filename)
     if utils.under_launcher() or utils.requested_gpus(devices) > 1:
@@ -377,6 +384,7 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks, minimum_count
             range_filename, target_filename, device=0, devices=None):
     """The reference's per-cell convert: every *.bam of the directory, in filesystem order.  devices /
     ALNTOOLS_GPUS: as convert_files."""
+    _refuse_collation()
     if os.path.isfile(bam_filename):                          # :375-377
         LOG.error('bam file must be a directory')
         return None

@@ -37,6 +37,8 @@ SIGNATURES = {
     "bamcols_emit": (ctypes.c_int64, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                       ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
                                       ctypes.POINTER(ctypes.c_int)]),
+    "bamcols_emit_keys": (ctypes.c_int64, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                           ctypes.c_void_p, ctypes.c_int64, ctypes.POINTER(ctypes.c_int)]),
     "bamcols_all_alignments": (ctypes.c_int64, [ctypes.c_void_p]),
     "bamcols_n_groups": (ctypes.c_int64, [ctypes.c_void_p]),
     "bamcols_plan_shards": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_int64)]),
@@ -245,6 +247,30 @@ class BamColumnReader(object):
         if cells is not None:
             out["cell_idx"] = cols[3]
         return out
+
+    def emit_keys(self, key_lo, key_hi, target_idx, hap_idx):
+        """Fill the given arrays (uint64 / int32 numpy arrays or pinned torch tensors of int64 / int32) with the next
+        valid alignments as (name key, target, haplotype) rows, for collation.  Returns (rows, done)."""
+        cap = int(key_lo.shape[0])
+        done = ctypes.c_int(0)
+        ptr = lambda a: a.ctypes.data if isinstance(a, np.ndarray) else a.data_ptr()
+        n = self._lib.bamcols_emit_keys(self._h, ptr(key_lo), ptr(key_hi), ptr(target_idx), ptr(hap_idx), cap,
+                                        ctypes.byref(done))
+        if n < 0:
+            _raise(int(n), self._lib.bamcols_last_error(self._h).decode())
+        return int(n), bool(done.value)
+
+    def read_all_keys(self, chunk=1 << 20):
+        """The whole file as numpy columns: dict(key_lo, key_hi (uint64), target_idx, hap_idx (int32))."""
+        parts = []
+        while True:
+            bufs = [np.empty(chunk, dtype=np.uint64), np.empty(chunk, dtype=np.uint64),
+                    np.empty(chunk, dtype=np.int32), np.empty(chunk, dtype=np.int32)]
+            n, done = self.emit_keys(*bufs)
+            parts.append([b[:n] for b in bufs])
+            if done:
+                break
+        return {k: np.concatenate([p[i] for p in parts]) for i, k in enumerate(("key_lo", "key_hi", "target_idx", "hap_idx"))}
 
     @property
     def all_alignments(self):

@@ -207,7 +207,8 @@ struct bamcols {
   int64_t all_alignments = 0;
   // single-sample batch path: rows of the current inflated window, produced by all worker threads
   RawBuf<int32_t> st_rg, st_tg, st_hp, st_cell;
-  size_t pending_row = 0;        // per-cell: stage row whose cell is resolved by the next valid alignment
+  RawBuf<uint64_t> st_klo, st_khi;   // key mode (bamcols_emit_keys): 128-bit name keys in place of read_group
+  size_t pending_row = 0;       // per-cell: stage row whose cell is resolved by the next valid alignment
   // per-cell scratch, kept between windows (fresh allocations of this size are page-faulted in every time)
   std::vector<size_t> sc_openers;
   std::vector<std::vector<size_t>> sc_mine;
@@ -220,7 +221,7 @@ struct bamcols {
   size_t st_whole = 0;           // rows [st_pos, st_whole) are whole reads; [st_whole, size) is the open last read
   std::vector<size_t> rec_off;   // scratch: record offsets of the window
   std::vector<uint8_t> rec_flag; // scratch: bit 0 valid, bit 1 starts a read
-  int mode = 0;                  // 0 undecided, 1 single-sample, 2 per-cell
+  int mode = 0;                  // 0 undecided, 1 single-sample, 2 per-cell, 3 name keys
   size_t grain = 4096;           // records per worker thread below which no further thread is used
   double phase_s[6] = {0, 0, 0, 0, 0, 0};  // inflate, record hop, validity, read starts, rows, copy-out
   // --rangefile (bam_utils.py:282-286): smallest / largest reference_start of the valid alignments per tid
@@ -433,6 +434,44 @@ inline size_t trimmed_len(const char* s, size_t n) {
   if (!sp) return n;
   const size_t i = (const char*)sp - s;
   return i > 0 ? i : n;
+}
+
+// 128-bit key of a trimmed read name (bamcols_emit_keys): two multiply-fold hashes with different seeds and
+// constants over the 8-byte words of the name (the last one zero-padded), the length folded into both seeds,
+// each finished with the murmur3 64-bit mix.  All ones is the empty slot of the device table: mapped away.
+inline uint64_t mum64(uint64_t x, uint64_t k) {
+  const unsigned __int128 p = (unsigned __int128)x * k;
+  return (uint64_t)p ^ (uint64_t)(p >> 64);
+}
+inline uint64_t fmix64(uint64_t h) {
+  h ^= h >> 33;
+  h *= 0xff51afd7ed558ccdull;
+  h ^= h >> 33;
+  h *= 0xc4ceb9fe1a85ec53ull;
+  h ^= h >> 33;
+  return h;
+}
+inline void name_key(const char* s, size_t n, uint64_t* lo, uint64_t* hi) {
+  uint64_t a = 0x9E3779B97F4A7C15ull ^ ((uint64_t)n * 0xD6E8FEB86659FD93ull);
+  uint64_t b = 0x243F6A8885A308D3ull + ((uint64_t)n * 0xA0761D6478BD642Full);
+  size_t i = 0;
+  for (; i + 8 <= n; i += 8) {
+    uint64_t w;
+    memcpy(&w, s + i, 8);
+    a = mum64(a ^ w, 0xE7037ED1A0B428DBull);
+    b = mum64(b ^ w, 0x8EBC6AF09C88C6E3ull) + w;
+  }
+  if (i < n) {
+    uint64_t w = 0;
+    memcpy(&w, s + i, n - i);
+    a = mum64(a ^ w, 0xE7037ED1A0B428DBull);
+    b = mum64(b ^ w, 0x8EBC6AF09C88C6E3ull) + w;
+  }
+  a = fmix64(a);
+  b = fmix64(b);
+  if ((a & b) == ~0ull) a = 0;
+  *lo = a;
+  *hi = b;
 }
 
 // Field 14 of name.split('|||') (bam_utils_multisample.py:273): separators are found left to right and
@@ -663,17 +702,23 @@ int find_records(bamcols* r, std::vector<size_t>& off, size_t* next) {
 // per record, (3) "starts a read" per valid record = its trimmed name differs from the previous valid
 // record's, (4) rows written at their final position (prefix sums over the threads).  The open last
 // read is held back (st_whole) until the next window or the end of the file closes it.
-int process_window_single(bamcols* r) {
+// keys: the rows of bamcols_emit_keys instead - step (3) is skipped, every valid record gets the 128-bit key of its
+// trimmed name in place of a read_group, and every row is handed out at once (there are no reads to keep whole).
+int process_window_single(bamcols* r, bool keys = false) {
   // rows still waiting from the previous window go to the front
-  const size_t left = r->st_rg.size() - r->st_pos;
-  if (r->st_pos > 0) {
-    memmove(r->st_rg.data(), r->st_rg.data() + r->st_pos, left * 4);
-    memmove(r->st_tg.data(), r->st_tg.data() + r->st_pos, left * 4);
-    memmove(r->st_hp.data(), r->st_hp.data() + r->st_pos, left * 4);
+  const size_t left = r->st_tg.size() - r->st_pos;
+  auto shift = [&](auto& buf) {
+    if (r->st_pos > 0) memmove(buf.data(), buf.data() + r->st_pos, left * sizeof(buf[0]));
+    buf.resize(left);
+  };
+  if (keys) {
+    shift(r->st_klo);
+    shift(r->st_khi);
+  } else {
+    shift(r->st_rg);
   }
-  r->st_rg.resize(left);
-  r->st_tg.resize(left);
-  r->st_hp.resize(left);
+  shift(r->st_tg);
+  shift(r->st_hp);
   r->st_whole -= r->st_pos;
   r->st_pos = 0;
 
@@ -697,7 +742,7 @@ int process_window_single(bamcols* r) {
     if (r->file_done) {
       if (r->wend != r->wpos) return fail(r, BAMCOLS_ERR_FORMAT, "truncated BAM record at the end of the file");
       r->records_done = true;
-      r->st_whole = r->st_rg.size();  // the end of the file closes the last read
+      r->st_whole = r->st_tg.size();  // the end of the file closes the last read
     }
     return 0;
   }
@@ -737,7 +782,7 @@ int process_window_single(bamcols* r) {
   const bool had_prev = r->started;
   const std::string prev_name = r->current;
   timer = new PhaseTimer(&r->phase_s[3]);
-  parallel_for(nt, [&](int t) {
+  if (!keys) parallel_for(nt, [&](int t) {
     const char* pn = nullptr;  // trimmed name of the previous valid record
     size_t pl = 0;
     bool have = false;
@@ -776,7 +821,31 @@ int process_window_single(bamcols* r) {
     n_start[t + 1] += n_start[t];
   }
   const size_t rows = n_valid[nt];
-  if (rows) {
+  if (rows && keys) {
+    const size_t row0 = r->st_tg.size();
+    for (auto* b : {&r->st_klo, &r->st_khi}) b->resize(row0 + rows);
+    for (auto* b : {&r->st_tg, &r->st_hp}) b->resize(row0 + rows);
+    uint64_t* klo = r->st_klo.data() + row0;
+    uint64_t* khi = r->st_khi.data() + row0;
+    int32_t* tg = r->st_tg.data() + row0;
+    int32_t* hp = r->st_hp.data() + row0;
+    // (4) rows: name keys instead of read starts
+    PhaseTimer rows_timer(&r->phase_s[4]);
+    parallel_for(nt, [&](int t) {
+      size_t k = n_valid[t];
+      for (size_t i = lo(t); i < lo(t + 1); ++i) {
+        if (!fl[i]) continue;
+        const uint8_t* q = base + off[i] + 4;
+        const char* nm = (const char*)q + 32;
+        name_key(nm, trimmed_len(nm, (size_t)q[8] - 1), &klo[k], &khi[k]);
+        const int32_t tid = (int32_t)le32(q);
+        tg[k] = r->tid_target[tid];
+        hp[k] = r->tid_hap[tid];
+        ++k;
+      }
+    });
+    r->st_whole = r->st_tg.size();
+  } else if (rows) {
     const size_t row0 = r->st_rg.size();
     r->st_rg.resize(row0 + rows);
     r->st_tg.resize(row0 + rows);
@@ -1174,6 +1243,34 @@ int64_t emit_single(bamcols* r, bamcols_cells* cells, int32_t* read_group, int32
       return rows;
     }
     const int rc = cells ? process_window_cells(r, cells) : process_window_single(r);
+    if (rc < 0) return rc;
+  }
+}
+
+int64_t emit_keys(bamcols* r, uint64_t* key_lo, uint64_t* key_hi, int32_t* target_idx, int32_t* hap_idx, int64_t capacity,
+                  int* done) {
+  int64_t rows = 0;
+  for (;;) {
+    const size_t take = std::min<size_t>(r->st_whole - r->st_pos, (size_t)(capacity - rows));
+    if (take > 0) {
+      PhaseTimer timer(&r->phase_s[5]);
+      void* dst[4] = {key_lo + rows, key_hi + rows, target_idx + rows, hap_idx + rows};
+      const void* src[4] = {r->st_klo.data() + r->st_pos, r->st_khi.data() + r->st_pos, r->st_tg.data() + r->st_pos,
+                            r->st_hp.data() + r->st_pos};
+      const size_t width[4] = {8, 8, 4, 4};
+      parallel_for(take < (1u << 18) ? 1 : 4, [&](int t) {
+        for (int c = t; c < 4; c += (take < (1u << 18) ? 1 : 4)) memcpy(dst[c], src[c], take * width[c]);
+      });
+      rows += (int64_t)take;
+      r->st_pos += take;
+      if (rows == capacity) return rows;
+      continue;
+    }
+    if (r->records_done) {
+      *done = 1;
+      return rows;
+    }
+    const int rc = process_window_single(r, true);
     if (rc < 0) return rc;
   }
 }
@@ -1693,6 +1790,7 @@ int64_t bamcols_emit(bamcols* r, bamcols_cells* cells, int32_t* read_group, int3
   }
   const int want_mode = cells ? 2 : 1;
   if (r->mode == 0) r->mode = want_mode;
+  if (r->mode == 3) return fail(r, BAMCOLS_ERR_INVALID, "a reader that has emitted name keys cannot switch to read groups");
   if (r->mode != want_mode) return fail(r, BAMCOLS_ERR_INVALID, "a reader cannot switch between single-sample and per-cell rules");
   if (!cells || !r->sequential_cells) {
     try {   // no exception may cross the C ABI
@@ -1796,6 +1894,24 @@ int64_t bamcols_emit(bamcols* r, bamcols_cells* cells, int32_t* read_group, int3
     r->cur.tg.push_back(r->tid_target[tid]);
     r->cur.hp.push_back(r->tid_hap[tid]);
     if (cells) r->cur.cell.push_back(r->cell);
+  }
+}
+
+int64_t bamcols_emit_keys(bamcols* r, uint64_t* key_lo, uint64_t* key_hi, int32_t* target_idx, int32_t* hap_idx,
+                          int64_t capacity, int* done) {
+  if (!r || !key_lo || !key_hi || !target_idx || !hap_idx || !done || capacity < 1) return BAMCOLS_ERR_INVALID;
+  if (r->tid_target.empty() && !r->ref_names.empty()) return fail(r, BAMCOLS_ERR_INVALID, "bamcols_set_tables was not called");
+  *done = 0;
+  if (r->prefetch.joinable()) {
+    r->prefetch.join();
+    if (r->prefetch_rc < 0) return r->prefetch_rc;
+  }
+  if (r->mode == 0) r->mode = 3;
+  if (r->mode != 3) return fail(r, BAMCOLS_ERR_INVALID, "a reader that has emitted read groups cannot switch to name keys");
+  try {
+    return emit_keys(r, key_lo, key_hi, target_idx, hap_idx, capacity, done);
+  } catch (const std::bad_alloc&) {
+    return fail(r, BAMCOLS_ERR_IO, "out of memory while decoding the window");
   }
 }
 

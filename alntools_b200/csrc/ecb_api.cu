@@ -18,6 +18,9 @@
 #include "ecb_exchange.cuh"
 #include "ecb_cells_exchange.cuh"
 #include "ecb_bam.cuh"
+#include "ecb_collate.cuh"
+
+#define ECB_PUSH_LIMIT (0x7FFFFFFFll - 8192)   // alignments of one ecb_push
 
 namespace {
 
@@ -44,6 +47,7 @@ struct ecb_ctx {
   int verify_keys = 0;
   int pageable_results = 0;
   int64_t opt_bam_window = 0;
+  int64_t opt_collate_slots = 0, opt_collate_piece = 0;
   // EC table
   DevBuf table;
   u32 table_slots = 0;
@@ -551,7 +555,7 @@ void cells_release(ecb_ctx* c) {
 
 extern "C" {
 
-int ecb_version(void) { return 2002; }
+int ecb_version(void) { return 2003; }
 
 const char* ecb_last_error(const ecb_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
@@ -629,6 +633,12 @@ int ecb_set_option(ecb_ctx* c, int option, int64_t value) {
     case ECB_OPT_BAM_WINDOW:
       if (value < 0) return fail(c, ECB_ERR_INVALID, "negative window");
       c->opt_bam_window = value; break;
+    case ECB_OPT_COLLATE_SLOTS:
+      if (value < 0) return fail(c, ECB_ERR_INVALID, "negative slot count");
+      c->opt_collate_slots = value; break;
+    case ECB_OPT_COLLATE_PIECE:
+      if (value < 0 || value > ECB_PUSH_LIMIT) return fail(c, ECB_ERR_INVALID, "collate piece %lld outside [0, %lld]", (long long)value, (long long)ECB_PUSH_LIMIT);
+      c->opt_collate_piece = value; break;
     default: return fail(c, ECB_ERR_INVALID, "unknown option %d", option);
   }
   return ECB_OK;
@@ -822,7 +832,7 @@ int ecb_push(ecb_ctx* c, const int32_t* read_group, const int32_t* target_idx, c
              const int32_t* cell_idx, int64_t n, int64_t order_base, int drop_last_group, int on_device) {
   if (!c) return ECB_ERR_INVALID;
   if (n < 0 || order_base < 0) return fail(c, ECB_ERR_INVALID, "negative n or order_base");
-  if (n > 0x7FFFFFFFll - 8192) return fail(c, ECB_ERR_LIMIT, "a push is limited to 2^31-8192 alignments; split it");
+  if (n > ECB_PUSH_LIMIT) return fail(c, ECB_ERR_LIMIT, "a push is limited to 2^31-8192 alignments; split it");
   if (n > 0 && (!read_group || !target_idx || !hap_idx)) return fail(c, ECB_ERR_INVALID, "NULL column");
   if (c->with_cells && n > 0 && !cell_idx) return fail(c, ECB_ERR_INVALID, "context has cells but cell_idx is NULL");
   if (!c->with_cells && cell_idx) return fail(c, ECB_ERR_INVALID, "cell_idx given but context was created without cells");
@@ -2019,6 +2029,213 @@ int ecb_bam_destroy(ecb_bam* d) {
   if (!d) return ECB_OK;
   cudaSetDevice(d->c->device);
   bam_release(d);
+  return ECB_OK;
+}
+
+}  // extern "C"
+
+// ---- collation of alignments by read name (kernels in ecb_collate.cuh) -----------------------------------------
+struct ecb_collate {
+  ecb_ctx* c = nullptr;
+  u64 n = 0;                          // alignments added
+  DevBuf key_lo, key_hi, tg_in, hp_in;   // the added columns, in file order
+  DevBuf table, slot_of, bitmap, word_rank, count, cursor, rg, tg, hp, cuts;
+  u32 slots = 0;
+  bool pushed = false;
+  cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  ecb_collate_stats stats{};
+};
+
+namespace {
+
+int64_t collate_bytes(const ecb_collate* k) {
+  const DevBuf* bufs[] = {&k->key_lo, &k->key_hi, &k->tg_in, &k->hp_in, &k->table, &k->slot_of, &k->bitmap, &k->word_rank,
+                          &k->count, &k->cursor, &k->rg, &k->tg, &k->hp, &k->cuts};
+  int64_t total = 0;
+  for (const DevBuf* b : bufs) total += (int64_t)b->bytes;
+  return total;
+}
+
+void collate_release(ecb_collate* k) {
+  ecb_ctx* c = k->c;
+  DevBuf* bufs[] = {&k->key_lo, &k->key_hi, &k->tg_in, &k->hp_in, &k->table, &k->slot_of, &k->bitmap, &k->word_rank,
+                    &k->count, &k->cursor, &k->rg, &k->tg, &k->hp, &k->cuts};
+  for (DevBuf* b : bufs) release(c, *b);
+  cudaStreamSynchronize(c->stream);
+  for (auto& e : k->ev)
+    if (e) cudaEventDestroy(e);
+  delete k;
+}
+
+// The name table over every added alignment.  A table that runs out of probes is replaced by one four times
+// larger and the insert runs again from the start: positions are file-order indices, so a rerun gives the same
+// slots' contents whatever happened before.
+int collate_table(ecb_collate* k) {
+  ecb_ctx* c = k->c;
+  u64 want = c->opt_collate_slots > 0 ? (u64)c->opt_collate_slots : k->n + k->n / 2;
+  k->slots = std::max<u32>(1u << 10, pow2_ceil(want));
+  CKR(ensure(c, k->slot_of, (size_t)k->n * 4));
+  for (;;) {
+    CKR(ensure(c, k->table, (size_t)k->slots * sizeof(EcbEntry)));
+    CK(cudaMemsetAsync(k->table.p, 0xFF, (size_t)k->slots * sizeof(EcbEntry), c->stream));
+    CK(cudaMemsetAsync(c->d_ctr->scratch, 0, 2 * sizeof(u32), c->stream));
+    CollateParams P{(const u64*)k->key_lo.p, (const u64*)k->key_hi.p, k->n, (EcbEntry*)k->table.p, k->slots - 1,
+                    (u32*)k->slot_of.p, c->d_ctr};
+    ecb_collate_insert_kernel<<<grid_for(k->n, 256, c->sm_count * 8), 256, 0, c->stream>>>(P);
+    LAUNCH_CHECK("collate_insert");
+    CKR(sync_counters(c));
+    if (c->h_ctr->scratch[1] == 0) break;
+    if (k->slots >= (1u << 31)) return fail(c, ECB_ERR_LIMIT, "the name table cannot grow beyond 2^31 slots");
+    k->slots = k->slots <= (1u << 29) ? k->slots * 4u : (1u << 31);
+    k->stats.table_grows++;
+  }
+  k->stats.table_slots = k->slots;
+  k->stats.reads = c->h_ctr->scratch[0];
+  return ECB_OK;
+}
+
+int collate_push(ecb_collate* k, int64_t* n_reads) {
+  ecb_ctx* c = k->c;
+  const u64 n = k->n;
+  *n_reads = 0;
+  if (n == 0) return ECB_OK;
+  float ms = 0;
+  CK(cudaEventRecord(k->ev[0], c->stream));
+  CKR(collate_table(k));
+  const u32 R = (u32)k->stats.reads;
+  CK(cudaEventRecord(k->ev[1], c->stream));
+
+  // read order: first positions -> bitmap -> word ranks -> read ids; alignments per read -> read offsets
+  const size_t words = (size_t)(n / 32) + 1;
+  CKR(ensure(c, k->bitmap, words * 4));
+  CKR(ensure(c, k->word_rank, words * 4));
+  CKR(ensure(c, k->count, (size_t)R * 4));
+  CKR(ensure(c, k->cursor, (size_t)R * 4));
+  CK(cudaMemsetAsync(k->bitmap.p, 0, words * 4, c->stream));
+  const int g_slots = grid_for(k->slots, 256, c->sm_count * 8);
+  ecb_collate_mark_kernel<<<g_slots, 256, 0, c->stream>>>((const EcbEntry*)k->table.p, k->slots, (u32*)k->bitmap.p);
+  LAUNCH_CHECK("collate_mark");
+  CKR(device_scan<true>(c, (const u32*)k->bitmap.p, (u32*)k->word_rank.p, words, 0, nullptr));
+  ecb_collate_ids_kernel<<<g_slots, 256, 0, c->stream>>>((EcbEntry*)k->table.p, k->slots, (const u32*)k->bitmap.p,
+                                                         (const u32*)k->word_rank.p, (u32*)k->count.p);
+  LAUNCH_CHECK("collate_ids");
+  u64 total = 0;
+  CKR(device_scan<false>(c, (const u32*)k->count.p, (u32*)k->cursor.p, R, 0, &total));
+  if (total != n) return fail(c, ECB_ERR_INVALID, "collation lost alignments (%llu of %llu placed)", (unsigned long long)total,
+                              (unsigned long long)n);
+  CK(cudaEventRecord(k->ev[2], c->stream));
+
+  // layout: the regrouped columns, then the pieces
+  CKR(ensure(c, k->rg, (size_t)n * 4));
+  CKR(ensure(c, k->tg, (size_t)n * 4));
+  CKR(ensure(c, k->hp, (size_t)n * 4));
+  ecb_collate_scatter_kernel<<<grid_for(n, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+      (const u32*)k->slot_of.p, (const EcbEntry*)k->table.p, (const int32_t*)k->tg_in.p, (const int32_t*)k->hp_in.p, n,
+      (u32*)k->cursor.p, (int32_t*)k->rg.p, (int32_t*)k->tg.p, (int32_t*)k->hp.p);
+  LAUNCH_CHECK("collate_scatter");
+  const u64 piece = c->opt_collate_piece > 0 ? (u64)c->opt_collate_piece : (u64)ECB_PUSH_LIMIT;
+  const size_t max_cuts = (size_t)(2 * (n / piece) + 4);   // two neighbouring pieces hold more than `piece` alignments
+  CKR(ensure(c, k->cuts, (max_cuts + 2) * 4));
+  ecb_collate_cuts_kernel<<<1, 32, 0, c->stream>>>((const u32*)k->cursor.p, R, n, piece, (u32*)k->cuts.p);
+  LAUNCH_CHECK("collate_cuts");
+  std::vector<u32> cuts(max_cuts + 2);
+  CK(cudaMemcpyAsync(cuts.data(), k->cuts.p, cuts.size() * 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaEventRecord(k->ev[3], c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  const u32 pieces = cuts[0];
+  if (pieces == 0 || pieces > max_cuts || cuts[1 + pieces] != n)
+    return fail(c, ECB_ERR_INVALID, "collation cut %u pieces", pieces);
+  k->stats.device_bytes = collate_bytes(k);
+
+  // push: the columns never leave the device; order_base = the piece's offset in collated order
+  CK(cudaEventRecord(k->ev[4], c->stream));
+  for (u32 j = 0; j < pieces; ++j) {
+    const u64 a = cuts[1 + j], b = cuts[2 + j];
+    CKR(ecb_push(c, (const int32_t*)k->rg.p + a, (const int32_t*)k->tg.p + a, (const int32_t*)k->hp.p + a, nullptr,
+                 (int64_t)(b - a), (int64_t)a, 0, 1));
+    k->stats.pieces++;
+  }
+  CK(cudaEventRecord(k->ev[5], c->stream));
+  CK(cudaEventSynchronize(k->ev[5]));
+  CK(cudaEventElapsedTime(&ms, k->ev[0], k->ev[1])); k->stats.table_ms = ms;
+  CK(cudaEventElapsedTime(&ms, k->ev[1], k->ev[2])); k->stats.order_ms = ms;
+  CK(cudaEventElapsedTime(&ms, k->ev[2], k->ev[3])); k->stats.layout_ms = ms;
+  CK(cudaEventElapsedTime(&ms, k->ev[4], k->ev[5])); k->stats.push_ms = ms;
+  *n_reads = (int64_t)R;
+  return ECB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ecb_collate_create(ecb_ctx* c, ecb_collate** out) {
+  if (!c || !out) return ECB_ERR_INVALID;
+  *out = nullptr;
+  if (c->with_cells) return fail(c, ECB_ERR_INVALID, "collation covers the single-sample path only");
+  CK(cudaSetDevice(c->device));
+  ecb_collate* k = new ecb_collate();
+  k->c = c;
+  for (auto& e : k->ev)
+    if (cudaEventCreate(&e) != cudaSuccess) {
+      collate_release(k);
+      return fail(c, ECB_ERR_CUDA, "cudaEventCreate failed");
+    }
+  *out = k;
+  return ECB_OK;
+}
+
+int ecb_collate_add(ecb_collate* k, const uint64_t* key_lo, const uint64_t* key_hi, const int32_t* target_idx,
+                    const int32_t* hap_idx, int64_t n, int on_device) {
+  if (!k) return ECB_ERR_INVALID;
+  ecb_ctx* c = k->c;
+  if (k->pushed) return fail(c, ECB_ERR_STATE, "this collator has pushed; create a new one");
+  if (n < 0) return fail(c, ECB_ERR_INVALID, "negative n");
+  if (n == 0) return ECB_OK;
+  if (!key_lo || !key_hi || !target_idx || !hap_idx) return fail(c, ECB_ERR_INVALID, "NULL column");
+  if (k->n + (u64)n >= 0xFFFFFFFFull) return fail(c, ECB_ERR_LIMIT, "a collator takes fewer than 2^32 - 1 alignments");
+  CK(cudaSetDevice(c->device));
+  const u64 total = k->n + (u64)n;
+  CKR(ensure(c, k->key_lo, (size_t)total * 8, true));
+  CKR(ensure(c, k->key_hi, (size_t)total * 8, true));
+  CKR(ensure(c, k->tg_in, (size_t)total * 4, true));
+  CKR(ensure(c, k->hp_in, (size_t)total * 4, true));
+  const cudaMemcpyKind kind = on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+  CK(cudaEventRecord(k->ev[0], c->stream));
+  CK(cudaMemcpyAsync((u64*)k->key_lo.p + k->n, key_lo, (size_t)n * 8, kind, c->stream));
+  CK(cudaMemcpyAsync((u64*)k->key_hi.p + k->n, key_hi, (size_t)n * 8, kind, c->stream));
+  CK(cudaMemcpyAsync((int32_t*)k->tg_in.p + k->n, target_idx, (size_t)n * 4, kind, c->stream));
+  CK(cudaMemcpyAsync((int32_t*)k->hp_in.p + k->n, hap_idx, (size_t)n * 4, kind, c->stream));
+  CK(cudaEventRecord(k->ev[1], c->stream));
+  CK(cudaEventSynchronize(k->ev[1]));   // the caller's buffers are free again
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, k->ev[0], k->ev[1]));
+  k->stats.add_ms += ms;
+  if (!on_device) k->stats.h2d_bytes += n * 24;
+  k->n = total;
+  k->stats.alignments = (int64_t)total;
+  return ECB_OK;
+}
+
+int ecb_collate_push(ecb_collate* k, int64_t* n_reads) {
+  if (!k || !n_reads) return ECB_ERR_INVALID;
+  if (k->pushed) return fail(k->c, ECB_ERR_STATE, "this collator has pushed already");
+  ecb_ctx* c = k->c;
+  k->pushed = true;
+  CK(cudaSetDevice(c->device));
+  return collate_push(k, n_reads);
+}
+
+int ecb_collate_get_stats(const ecb_collate* k, ecb_collate_stats* out) {
+  if (!k || !out) return ECB_ERR_INVALID;
+  *out = k->stats;
+  return ECB_OK;
+}
+
+int ecb_collate_destroy(ecb_collate* k) {
+  if (!k) return ECB_OK;
+  cudaSetDevice(k->c->device);
+  collate_release(k);
   return ECB_OK;
 }
 

@@ -120,6 +120,35 @@ def decode_mode(decode=None):
     return str(mode).lower()
 
 
+def collate_mode(collate=None):
+    """Whether a single-sample convert() collates alignments by read name: `collate`, else the environment variable
+    ALNTOOLS_B200_COLLATE ("0", the default, or "1"; the CLI keeps the reference's options, so the environment is
+    its only way to say it)."""
+    import os
+    if collate is not None:
+        return bool(collate)
+    value = os.environ.get("ALNTOOLS_B200_COLLATE", "0").strip()
+    if value not in ("0", "1"):
+        raise ValueError("ALNTOOLS_B200_COLLATE must be 0 or 1, not %r" % (value,))
+    return value == "1"
+
+
+def emit_collated(records, tables):
+    """The rows convert(collate=True) builds from: a read is every valid alignment whose trimmed name (as emit_single
+    trims it) is the same, wherever it lies in the file; reads are ordered by their first valid alignment, and each
+    read's alignments follow in file order.  So the result is emit_single of the file regrouped that way."""
+    reads = {}                                            # trimmed name -> tids; dicts keep insertion order
+    total = 0
+    for qname, flag, tid, _pos, ntid, npos in records:
+        total += 1
+        if _valid(flag, tid, ntid, npos):
+            reads.setdefault(_trim(qname), []).append(tid)
+    rg = np.repeat(np.arange(len(reads), dtype=np.int32), [len(t) for t in reads.values()])
+    tids = np.asarray([t for ts in reads.values() for t in ts], dtype=np.int64)
+    return Columns(rg, tables.tid_target[tids] if len(tids) else [], tables.tid_hap[tids] if len(tids) else [],
+                   None, total, len(reads))
+
+
 _PINNED_POOL = []      # pinned buffer sets of finished conversions, reused by the next one in this process
 
 
@@ -218,6 +247,75 @@ def stream_single(reader, builder, chunk_rows=1 << 21, pinned=True, depth=3):
         worker.join()
         _release_buffers(all_sets, pinned)
     return pushed
+
+
+_PINNED_KEYS = []      # pinned key buffer sets of finished collations, reused by the next one in this process
+
+
+def stream_collated(reader, builder, chunk_rows=1 << 21, pinned=True, depth=3):
+    """Collate the valid alignments of `reader` (bamcols.BamColumnReader, tables set) by read name on the GPU and
+    push them into `builder` as name-grouped reads (_native.Collator).  A worker thread fills a small ring of pinned
+    buffers from emit_keys while the previous buffer is added.  Returns (valid alignments, reads, collator stats)."""
+    import queue
+    import threading
+    from ._native import Collator
+    free, full = queue.Queue(), queue.Queue()
+    sets = []
+    for _ in range(depth):
+        bufs = None
+        if pinned:
+            import torch
+            while _PINNED_KEYS and bufs is None:
+                b = _PINNED_KEYS.pop()
+                if int(b[0].shape[0]) >= chunk_rows:
+                    bufs = b
+            if bufs is None:
+                bufs = [torch.empty(chunk_rows, dtype=torch.int64, pin_memory=True) for _ in range(2)] + \
+                       [torch.empty(chunk_rows, dtype=torch.int32, pin_memory=True) for _ in range(2)]
+        else:
+            bufs = [np.empty(chunk_rows, np.uint64), np.empty(chunk_rows, np.uint64), np.empty(chunk_rows, np.int32),
+                    np.empty(chunk_rows, np.int32)]
+        sets.append(bufs)
+        free.put(bufs)
+    stop = threading.Event()
+
+    def produce():
+        try:
+            while not stop.is_set():
+                try:
+                    bufs = free.get(timeout=0.05)
+                except queue.Empty:
+                    continue
+                n, done = reader.emit_keys(*bufs)
+                full.put((bufs, n, done, None))
+                if done:
+                    return
+        except BaseException as exc:                      # re-raised by the consumer
+            full.put((None, 0, True, exc))
+
+    added = 0
+    with Collator(builder) as col:
+        worker = threading.Thread(target=produce, daemon=True)
+        worker.start()
+        try:
+            while True:
+                bufs, n, done, exc = full.get()
+                if exc is not None:
+                    raise exc
+                if n:
+                    col.add(*bufs, n=n)
+                    added += n
+                free.put(bufs)
+                if done:
+                    break
+        finally:
+            # the producer leaves native code before the caller may close the reader (as in stream_single)
+            stop.set()
+            worker.join()
+            if pinned:
+                _PINNED_KEYS.extend(sets)
+        reads = col.push()
+        return added, reads, col.stats()
 
 
 _PINNED_BYTES = []     # pinned read buffers of finished device decodes, reused by the next one in this process

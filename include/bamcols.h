@@ -88,6 +88,17 @@ const char* bamcols_cells_name(const bamcols_cells* c, int64_t idx);
 int64_t bamcols_emit(bamcols* r, bamcols_cells* cells, int32_t* read_group, int32_t* target_idx, int32_t* hap_idx,
                      int32_t* cell_idx, int64_t capacity, int* done);
 
+/* The rows of collation (ecb_collate_add in include/ecb200.h): one row per VALID alignment in file order, with the
+ * filters, errors, all_alignments counter and --rangefile tracking of the single-sample rules, but no read_group:
+ *     key_lo, key_hi  128-bit key of the read name trimmed at its first blank unless that blank is its first
+ *                     character (alntools/bam_utils.py:301-304); equal names give equal keys, and no key is all
+ *                     ones (the device table's empty slot)
+ *     target_idx, hap_idx  as for bamcols_emit
+ * Up to `capacity` rows per call; a call may end anywhere, since reads are formed later over the whole file.  *done
+ * is set once the file is exhausted.  A reader that has used bamcols_emit refuses this call, and the other way round. */
+int64_t bamcols_emit_keys(bamcols* r, uint64_t* key_lo, uint64_t* key_hi, int32_t* target_idx, int32_t* hap_idx,
+                          int64_t capacity, int* done);
+
 /* Shards of ONE file for several readers (one per GPU / process), without temporary files.  The reference plans
  * chunks as BGZF virtual offsets at read boundaries (alntools/bam_utils.py:1174-1304) and then copies every
  * chunk into its own temporary BAM (:157-195); here every reader opens the same file and confines itself to

@@ -68,6 +68,9 @@ enum ecb_option {
                                    cheaper for a context that finalizes once, slower when reused */
   ECB_OPT_BAM_WINDOW = 9,       /* inflated bytes per window of the device BAM decoder (0 = automatic, 1 GiB);
                                    a window always takes at least one block */
+  ECB_OPT_COLLATE_SLOTS = 10,   /* initial slots of a collator's name table (0 = automatic: 1.5 x the alignments
+                                   added, rounded up to a power of two); the table grows when it runs out of probes */
+  ECB_OPT_COLLATE_PIECE = 11,   /* most alignments one push of a collator carries (0 = the push limit, 2^31 - 8192) */
 };
 
 typedef struct ecb_result {
@@ -317,6 +320,44 @@ int ecb_bam_counters(const ecb_bam* d, int64_t* all_alignments, int64_t* n_group
 int ecb_bam_ranges(ecb_bam* d, int32_t* range_min, int32_t* range_max);
 int ecb_bam_get_stats(const ecb_bam* d, ecb_bam_stats* out);
 int ecb_bam_destroy(ecb_bam* d);
+
+/* ---- collation of alignments by read name (since version 2003) ----------------------------------------------
+ * For files that are not grouped by read name.  A read is the set of valid alignments that share a trimmed name,
+ * wherever they lie in the file; reads are ordered by their first alignment.  The result equals ecb_push of the same
+ * alignments regrouped that way (each read contiguous, reads in that order).  A collator is bound to one
+ * single-sample context and uses its device, stream and memory pool; destroy it before the context.
+ *
+ * ecb_collate_add: append n alignments in file order - the rows of bamcols_emit_keys (include/bamcols.h): 128-bit
+ *   name key (never all ones), target_idx, hap_idx.  on_device 0: host pointers (pinned preferred), 1: device
+ *   pointers of the context's device.  Copied; the buffers may be reused after return.  Fewer than 2^32 - 1
+ *   alignments in all.  Two names with equal keys are one read (DESIGN.md section 6.2).
+ * ecb_collate_push: regroup everything added in device memory and push it into the context (ecb_push with
+ *   on_device = 1, order_base = offset in collated order, in pieces of at most ECB_OPT_COLLATE_PIECE alignments that
+ *   end at read ends; a longer read is a piece of its own).  Once per collator; *n_reads = reads formed.  The
+ *   context's limits apply: a read of more than ECB_MAX_READ_ALIGNMENTS alignments fails with ECB_ERR_LIMIT.
+ * Device memory: 88 to 144 bytes per added alignment with the automatic table (DESIGN.md section 6.2), held until
+ * ecb_collate_destroy.  Running out of it fails the call with ECB_ERR_CUDA and the allocator's message. */
+typedef struct ecb_collate ecb_collate;
+typedef struct ecb_collate_stats {
+  int64_t alignments;      /* added                                                                            */
+  int64_t reads;           /* reads formed (after the push)                                                    */
+  int64_t table_slots;     /* name table slots at the end                                                      */
+  int64_t table_grows;     /* times the name table was replaced by a larger one                                */
+  int64_t pieces;          /* pushes into the context                                                          */
+  int64_t device_bytes;    /* device memory held by the collator after the layout                              */
+  int64_t h2d_bytes;       /* bytes the add calls copied host->device                                          */
+  double add_ms;           /* stream time of the add copies, summed                                            */
+  double table_ms;         /* name table, growth included                                                      */
+  double order_ms;         /* bitmap, ranks, read ids and offsets (with one host round trip)                   */
+  double layout_ms;        /* scatter to collated order and the piece cuts (with one host round trip)          */
+  double push_ms;          /* the pushes into the context                                                      */
+} ecb_collate_stats;
+int ecb_collate_create(ecb_ctx* ctx, ecb_collate** out);
+int ecb_collate_add(ecb_collate* c, const uint64_t* key_lo, const uint64_t* key_hi, const int32_t* target_idx,
+                    const int32_t* hap_idx, int64_t n, int on_device);
+int ecb_collate_push(ecb_collate* c, int64_t* n_reads);
+int ecb_collate_get_stats(const ecb_collate* c, ecb_collate_stats* out);
+int ecb_collate_destroy(ecb_collate* c);
 
 #ifdef __cplusplus
 }
