@@ -11,7 +11,7 @@ import time
 
 import numpy as np
 
-from . import bamcols, bin_utils, emase, emitter, utils
+from . import bamcols, bin_utils, emitter, utils
 from ._native import EcBuilder
 from .header import TargetTables
 
@@ -181,20 +181,12 @@ def convert_rank(bam_filename, ec_filename, emase_filename, num_chunks=0, number
     groups its own on its GPU, is moved to its global position in read order (ecb_rebase: the position is
     known once every rank has counted its alignments), and the ranks merge through the exchange of
     multi_gpu.distributed_finalize.  The final matrices stay partitioned by EC-id range; every rank writes its
-    byte ranges of the EC file.  Returns the totals on rank 0, None elsewhere."""
+    byte ranges of the EC file (multi_gpu.save_rank_outputs).  Returns the totals on rank 0, None elsewhere."""
     import torch
     import torch.distributed as dist
     from . import multi_gpu
     start_time = time.time()
-    rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
-    local_rank = int(os.environ.get("LOCAL_RANK", rank))
-    utils.bind_to_gpu_numa_node(local_rank)          # pinned buffers next to this rank's GPU
-    torch.cuda.set_device(local_rank)
-    device = torch.device("cuda", local_rank)
-    own_group = not dist.is_initialized()
-    if own_group:
-        dist.init_process_group("nccl", device_id=device)
-    try:
+    with multi_gpu.rank_process() as (rank, world, device):
         _, num_processes = _job_plan(num_chunks, number_processes)
         num_processes = max(1, num_processes // world)          # the host threads are shared by the ranks
         if sample is None:
@@ -205,7 +197,7 @@ def convert_rank(bam_filename, ec_filename, emase_filename, num_chunks=0, number
             reader.set_range(plan[rank], plan[rank + 1])
             if range_filename is not None:
                 reader.track_ranges(True)
-            opts = dict(with_cells=False, alignments_hint=0, device=local_rank, result_on_device=1)
+            opts = dict(with_cells=False, alignments_hint=0, device=device.index, result_on_device=1)
             with EcBuilder(tables.num_targets, tables.num_haplotypes, **opts) as builder, \
                     EcBuilder(tables.num_targets, tables.num_haplotypes, **opts) as owner:
                 chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(bam_filename) // 2)))   # 24 MB of columns per piece
@@ -219,71 +211,24 @@ def convert_rank(bam_filename, ec_filename, emase_filename, num_chunks=0, number
                     raise RuntimeError("The shape must be a tuple of three positive integers.")
                 builder.rebase(sum(r[0] for r in every[:rank]))
                 out = multi_gpu.distributed_finalize(builder, lambda: owner, device, result_on="slices")
-                n_ec, id_base, n_local, nnz_local = int(out["n_ec"]), int(out["id_base"]), int(out["n_ec_local"]), int(out["nnz_local"])
-                sizes = [torch.empty(2, dtype=torch.int64, device=device) for _ in range(world)]
-                dist.all_gather(sizes, torch.tensor([n_local, nnz_local], dtype=torch.int64, device=device))
-                sizes = torch.stack(sizes).tolist()
-                nnz_base, nnz_total = sum(r[1] for r in sizes[:rank]), sum(r[1] for r in sizes)
-                a_indptr = out["a_indptr"][:n_local + 1].cpu().numpy()
-                a_indices = out["a_indices"][:nnz_local].cpu().numpy()
-                a_data = out["a_data"][:nnz_local].cpu().numpy()
-                counts = out["n_data"][:n_local].cpu().numpy()
-                reads = torch.tensor([int(counts.astype(np.int64).sum())], dtype=torch.int64, device=device)
+                reads = out["n_data"][:int(out["n_ec_local"])].to(torch.int64).sum().reshape(1)
                 dist.all_reduce(reads)
-            section = tables.target_section()
-            target_names = list(tables.main_targets.keys()) if (emase_filename or section is None) else None
-            if ec_filename:
-                header = bin_utils.ec_header_bytes(tables.haplotypes, target_names, tables.lengths, [sample],
-                                                   target_section=section, n_targets=tables.num_targets)
-                args = (ec_filename, header, n_ec, nnz_total, id_base, nnz_base, a_indptr, a_indices, a_data, counts)
-                if rank == 0:
-                    try:
-                        os.remove(ec_filename)
-                    except OSError:
-                        pass
-                    bin_utils.ecsave2_slice(*args, create=True)
-                dist.barrier()                                    # the file is laid out
-                if rank != 0:
-                    bin_utils.ecsave2_slice(*args, create=False)
-                dist.barrier()
-            if emase_filename:                                    # one writer: the slices travel to rank 0
-                parts = [None] * world
-                dist.all_gather_object(parts, (a_indptr, a_indices, a_data, counts))
-                if rank == 0:
-                    indptr = np.concatenate([[0]] + [p[0][1:].astype(np.int64) + sum(len(q[1]) for q in parts[:i])
-                                                     for i, p in enumerate(parts)]).astype(np.int32)
-                    a_csr = (indptr, np.concatenate([p[1] for p in parts]), np.concatenate([p[2] for p in parts]))
-                    n_counts = np.concatenate([p[3] for p in parts])
-                    n_csc = (np.array([0, n_ec], dtype=np.int32), np.arange(n_ec, dtype=np.int32), n_counts)
-                    try:
-                        os.remove(emase_filename)
-                    except OSError:
-                        pass
-                    emase.save_emase(emase_filename, "bam2ec", (tables.num_targets, tables.num_haplotypes, n_ec),
-                                     tables.haplotypes, target_names, tables.lengths, [sample], a_csr, n_csc,
-                                     incidence_only=True)
-            if range_filename is not None:                        # bam_utils.py:735-766, over all shards
-                lo, hi = reader.ranges()
-                lo_t, hi_t = torch.from_numpy(lo.copy()).to(device), torch.from_numpy(hi.copy()).to(device)
-                dist.all_reduce(lo_t, op=dist.ReduceOp.MIN)
-                dist.all_reduce(hi_t, op=dist.ReduceOp.MAX)
-                if rank == 0:
-                    utils.write_range_file(range_filename, list(tables.main_targets.keys()), tables.haplotypes,
-                                           reader.references, lo_t.cpu().numpy(), hi_t.cpu().numpy())
+                track = range_filename is not None
+                nnz_a = multi_gpu.save_rank_outputs(out, tables, tables.target_section(), [sample], ec_filename,
+                                                    emase_filename, range_filename, reader.references if track else None,
+                                                    reader.ranges() if track else None)
         if rank != 0:
             return None
+        n_ec = int(out["n_ec"])
         LOG.info("# Valid Alignments: {:,}".format(total_valid))
         LOG.info("# Main Targets: {:,}".format(tables.num_targets))
         LOG.info("# Haplotypes: {:,}".format(tables.num_haplotypes))
         LOG.info("# Equivalence Classes: {:,}".format(n_ec))
         LOG.info("# Unique Reads: {:,}".format(int(reads.item())))
         LOG.info("{} GPUs, total time: {}".format(world, utils.format_time(start_time, time.time())))
-        return {"n_ec": n_ec, "nnz_a": nnz_total, "n_samples": 1, "nnz_n": n_ec, "n_reads": int(reads.item()),
+        return {"n_ec": n_ec, "nnz_a": nnz_a, "n_samples": 1, "nnz_n": n_ec, "n_reads": int(reads.item()),
                 "n_alignments": total_valid, "n_gpus": world,
                 "alignments_per_gpu": [r[0] for r in every]}
-    finally:
-        if own_group and dist.is_initialized():
-            dist.destroy_process_group()
 
 
 def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_processes=-1, temp_dir=None,
@@ -304,41 +249,20 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
     are the default's.
     """
     start_time = time.time()
-    mode = emitter.decode_mode(decode)
-    collate = emitter.collate_mode(collate)
-    if mode == "device":
-        if utils.under_launcher() or utils.requested_gpus(devices) > 1:
-            raise NotImplementedError("device BAM decode runs on one GPU; the multi-GPU convert has no device decode yet "
-                                      "(use decode='host' / unset ALNTOOLS_B200_DECODE)")
-        if emitter.use_python_emitter():
-            raise NotImplementedError("device BAM decode replaces the native emitter; it does not combine with "
-                                      "ALNTOOLS_B200_EMITTER=python")
-    if collate:
-        if utils.under_launcher() or utils.requested_gpus(devices) > 1:
-            raise NotImplementedError("collation by read name runs on one GPU: reads span the shards of a multi-GPU "
-                                      "convert (unset ALNTOOLS_B200_COLLATE or use one GPU)")
-        if mode == "device":
-            raise NotImplementedError("collation by read name takes the host decode (use decode='host' / unset "
-                                      "ALNTOOLS_B200_DECODE)")
+    mode = emitter.resolve_mode(False, devices, decode, collate, range_filename is not None)
     job = dict(bam_filename=bam_filename, ec_filename=ec_filename, emase_filename=emase_filename, num_chunks=num_chunks,
                number_processes=number_processes, temp_dir=temp_dir, range_filename=range_filename, sample=sample,
                target_filename=target_filename)
-    if utils.under_launcher():
-        if emitter.use_python_emitter():
-            raise NotImplementedError("the multi-GPU path needs the native emitter (unset ALNTOOLS_B200_EMITTER)")
+    if mode.launcher:
         return convert_rank(**job)
-    if utils.requested_gpus(devices) > 1:
-        if emitter.use_python_emitter():
-            raise NotImplementedError("the multi-GPU path needs the native emitter (unset ALNTOOLS_B200_EMITTER)")
-        return utils.spawn_ranks(utils.requested_gpus(devices), job)
-    if range_filename is not None and emitter.use_python_emitter():
-        raise NotImplementedError("--rangefile needs the native emitter (unset ALNTOOLS_B200_EMITTER)")
+    if mode.gpus > 1:
+        return utils.spawn_ranks(mode.gpus, job)
     num_chunks, num_processes = _job_plan(num_chunks, number_processes)
     if sample is None:                                        # bam_utils.py:552-554
         sample = os.path.basename(bam_filename)
         LOG.info("Sample not supplied, using filename: {}".format(sample))
 
-    def save(res, tables, valid, temp_time):
+    def save(res, tables, valid, temp_time, references=None, ranges=None):
         """Log the totals and write the outputs from the result arrays (bam_utils.py:726-876)."""
         LOG.info("All results combined in {}, total time: {}".format(utils.format_time(temp_time, time.time()),
                                                                      utils.format_time(start_time, time.time())))
@@ -347,28 +271,14 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
         LOG.info("# Haplotypes: {:,}".format(tables.num_haplotypes))
         LOG.info("# Equivalence Classes: {:,}".format(res["n_ec"]))
         LOG.info("# Unique Reads: {:,}".format(res["n_reads"]))
-        a_csr = (res["a_indptr"], res["a_indices"], res["a_data"])
-        n_csc = (res["n_indptr"], res["n_indices"], res["n_data"])
-        section = tables.target_section() if hasattr(tables, "target_section") else None   # native tables only
-        target_names = list(tables.main_targets.keys()) if (emase_filename or section is None) else None
-        if emase_filename:
-            LOG.info("Saving to {}...".format(emase_filename))
-            try:
-                os.remove(emase_filename)
-            except OSError:
-                pass
-            emase.save_emase(emase_filename, "bam2ec", (tables.num_targets, tables.num_haplotypes, res["n_ec"]),
-                             tables.haplotypes, target_names, tables.lengths, [sample], a_csr, n_csc,
-                             incidence_only=True)
+        for name in (emase_filename, ec_filename):
+            if name:
+                LOG.info("Saving to {}...".format(name))
+        temp_time = time.time()
+        bin_utils.save_outputs(tables, tables.target_section(), [sample], (res["a_indptr"], res["a_indices"], res["a_data"]),
+                               (res["n_indptr"], res["n_indices"], res["n_data"]), False, ec_filename, emase_filename,
+                               range_filename, references, ranges)
         if ec_filename:
-            LOG.info("Saving to {}...".format(ec_filename))
-            try:
-                os.remove(ec_filename)
-            except OSError:
-                pass
-            temp_time = time.time()
-            bin_utils.ecsave2_arrays(ec_filename, tables.haplotypes, target_names, tables.lengths, [sample],
-                                     a_csr, n_csc, target_section=section, n_targets=tables.num_targets)
             LOG.info("{} created in {}, total time: {}".format(ec_filename,
                                                                utils.format_time(temp_time, time.time()),
                                                                utils.format_time(start_time, time.time())))
@@ -376,14 +286,14 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
 
     LOG.info("Parsing file information ...")
     temp_time = time.time()
-    if emitter.use_python_emitter():
-        res, tables, valid = _convert_python_emitter(bam_filename, target_filename, device, start_time, collate)
+    if mode.python:
+        res, tables, valid = _convert_python_emitter(bam_filename, target_filename, device, start_time, mode.collate)
         return save(res, tables, valid, temp_time)
     # native emitter: inflate threads + one record pass, streamed to the GPU in read-aligned chunks
     import torch
     with bamcols.BamColumnReader(bam_filename, n_threads=num_processes) as reader:
         tables = reader.build_tables(target_filename)       # native statement of header.TargetTables
-        if range_filename is not None and mode == "host":
+        if range_filename is not None and mode.decode == "host":
             reader.track_ranges(True)
         LOG.info("File parsed in {}, total time: {}".format(utils.format_time(temp_time, time.time()),
                                                             utils.format_time(start_time, time.time())))
@@ -393,10 +303,10 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
         with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=False, alignments_hint=0,
                        device=device, pageable_results=1) as builder:
             chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(bam_filename) // 2)))   # 24 MB of columns per piece
-            if mode == "device":
+            if mode.decode == "device":
                 valid, _, ranges, _ = emitter.stream_single_device(bam_filename, reader, builder, tables,
                                                                 range_filename is not None)
-            elif collate:
+            elif mode.collate:
                 valid, _, _ = emitter.stream_collated(reader, builder, chunk_rows=chunk_rows, pinned=torch.cuda.is_available())
                 ranges = reader.ranges() if range_filename is not None else None
             else:
@@ -406,9 +316,5 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
                 # the reference ends up with zero ECs and APM() raises (Sparse3DMatrix.py:45-46)
                 raise RuntimeError("The shape must be a tuple of three positive integers.")
             # the files are written straight from the library's result buffers (no intermediate copies)
-            summary = save(builder.finalize(copy=False), tables, valid, temp_time)
-        if range_filename is not None:                         # bam_utils.py:735-766
-            utils.write_range_file(range_filename, list(tables.main_targets.keys()), tables.haplotypes,
-                                   reader.references, ranges[0], ranges[1])
-    return summary
-
+            return save(builder.finalize(copy=False), tables, valid, temp_time,
+                        reader.references if range_filename is not None else None, ranges)

@@ -253,6 +253,31 @@ def ecload_arrays(ec_filename):
             "a": mats[0], "n": mats[1]}
 
 
+def save_outputs(tables, section, sample_names, a_csr, n_csc, cells, ec_filename=None, emase_filename=None,
+                 range_filename=None, references=None, ranges=None):
+    """Write the outputs of a conversion that were asked for, each in place of an old file of that name: the EMASE
+    and EC files from the final host matrices a_csr / n_csc (as alntools/bam_utils.py:726-876 does), and the
+    --rangefile report from the header's reference names and the (range_min, range_max) arrays per reference.
+    section: the targets section the native header tables built (TargetTables.target_section(), read while their
+    reader is open), or None; without an EMASE file, which needs the name list anyway, it saves building the names.
+    cells: the per-cell converter, whose EMASE file is titled "Multisample APM" and keeps the counts; the
+    single-sample one is titled "bam2ec" and is incidence only."""
+    from . import emase, utils
+    target_names = list(tables.main_targets.keys()) if (emase_filename or section is None) else None
+    if emase_filename:
+        utils.delete_file(emase_filename)
+        emase.save_emase(emase_filename, "Multisample APM" if cells else "bam2ec",
+                         (tables.num_targets, tables.num_haplotypes, len(a_csr[0]) - 1), tables.haplotypes,
+                         target_names, tables.lengths, sample_names, a_csr, n_csc, incidence_only=not cells)
+    if ec_filename:
+        utils.delete_file(ec_filename)
+        ecsave2_arrays(ec_filename, tables.haplotypes, target_names, tables.lengths, sample_names, a_csr, n_csc,
+                       target_section=section, n_targets=tables.num_targets)
+    if range_filename is not None:
+        utils.write_range_file(range_filename, list(tables.main_targets.keys()), tables.haplotypes, references,
+                               ranges[0], ranges[1])
+
+
 def ec2emase(ec_filename, emase_filename):
     """EC binary file -> EMASE (.h5) file (alntools/bin_utils.py:979-995: ecload, then APM.save with the title
     'Converted from <ec file>' and the data arrays included).  Needs PyTables like every EMASE output."""

@@ -9,9 +9,11 @@ name-change test (:306).  Per VALID alignment it emits
                 (bam_utils_multisample.py:270-280)
 Everything after that - grouping, de-duplication, counting, ordering, matrix build - runs on the GPU.
 """
+import collections
+
 import numpy as np
 
-from . import bam_io
+from . import bam_io, bamcols, utils
 
 
 def _trim(name):
@@ -133,6 +135,49 @@ def collate_mode(collate=None):
     return value == "1"
 
 
+Mode = collections.namedtuple("Mode", ["python", "decode", "collate", "launcher", "gpus"])
+
+
+def resolve_mode(cells, devices=None, decode=None, collate=None, range_file=False):
+    """The settings of one conversion, read once from the arguments and the environment: the emitter
+    (use_python_emitter), the decode (decode_mode), collation (collate_mode), whether this process is one rank of a
+    one-process-per-GPU job (utils.under_launcher) and otherwise how many GPUs to spread the job over
+    (utils.requested_gpus; 1 under a launcher, which has started the ranks).  cells: the per-cell converter, whose
+    decode and collation come from the environment only.  Refuses what no converter runs - ValueError for a value it
+    does not know, NotImplementedError for a combination - before any file is opened or any GPU is touched."""
+    python = use_python_emitter()
+    decode = decode_mode(decode)
+    if cells and decode == "device":
+        raise NotImplementedError("the per-cell (--multisample) conversion has no device BAM decode yet: it needs a GPU "
+                                  "cell-name dictionary (unset ALNTOOLS_B200_DECODE)")
+    collate = collate_mode(collate)
+    if cells and collate:
+        raise NotImplementedError("the per-cell (--multisample) conversion has no collation by read name: its rules "
+                                  "depend on consecutive records (unset ALNTOOLS_B200_COLLATE)")
+    launcher = utils.under_launcher()
+    gpus = 1 if launcher else utils.requested_gpus(devices)
+    multi = launcher or gpus > 1
+    if decode == "device":
+        if multi:
+            raise NotImplementedError("device BAM decode runs on one GPU; the multi-GPU convert has no device decode yet "
+                                      "(use decode='host' / unset ALNTOOLS_B200_DECODE)")
+        if python:
+            raise NotImplementedError("device BAM decode replaces the native emitter; it does not combine with "
+                                      "ALNTOOLS_B200_EMITTER=python")
+    if collate:
+        if multi:
+            raise NotImplementedError("collation by read name runs on one GPU: reads span the shards of a multi-GPU "
+                                      "convert (unset ALNTOOLS_B200_COLLATE or use one GPU)")
+        if decode == "device":
+            raise NotImplementedError("collation by read name takes the host decode (use decode='host' / unset "
+                                      "ALNTOOLS_B200_DECODE)")
+    if python and multi:
+        raise NotImplementedError("the multi-GPU path needs the native emitter (unset ALNTOOLS_B200_EMITTER)")
+    if python and range_file:
+        raise NotImplementedError("--rangefile needs the native emitter (unset ALNTOOLS_B200_EMITTER)")
+    return Mode(python, decode, collate, launcher, gpus)
+
+
 def emit_collated(records, tables):
     """The rows convert(collate=True) builds from: a read is every valid alignment whose trimmed name (as emit_single
     trims it) is the same, wherever it lies in the file; reads are ordered by their first valid alignment, and each
@@ -149,28 +194,73 @@ def emit_collated(records, tables):
                    None, total, len(reads))
 
 
-_PINNED_POOL = []      # pinned buffer sets of finished conversions, reused by the next one in this process
+_PINNED = []      # pinned buffer sets of finished streams, reused by later streams of this process
 
 
-def _column_buffers(rows, with_cells, pinned):
-    n = 4 if with_cells else 3
-    if pinned:
-        import torch
-        # pinning host memory costs about as much as decoding it: a set that an earlier convert() of this
-        # process has pinned is taken again when it is large enough
-        for i, bufs in enumerate(_PINNED_POOL):
-            if len(bufs) == n and int(bufs[0].shape[0]) >= rows:
-                return _PINNED_POOL.pop(i)
-        return [torch.empty(rows, dtype=torch.int32, pin_memory=True) for _ in range(n)]
-    return [np.empty(rows, dtype=np.int32) for _ in range(n)]
+def _buffers(rows, dtypes, pinned):
+    """A set of host buffers of `rows` elements, one per dtype name in `dtypes`; pinned: page-locked torch tensors.
+    Pinning host memory costs about as much as decoding into it, so a pinned set of the same dtypes that an earlier
+    stream of this process left in the pool is taken again when it is large enough."""
+    if not pinned:
+        return [np.empty(rows, dtype=d) for d in dtypes]
+    import torch
+    dtypes = [getattr(torch, d) for d in dtypes]
+    for i, bufs in enumerate(_PINNED):
+        if [b.dtype for b in bufs] == dtypes and int(bufs[0].shape[0]) >= rows:
+            return _PINNED.pop(i)
+    return [torch.empty(rows, dtype=d, pin_memory=True) for d in dtypes]
 
 
-def _release_buffers(sets, pinned):
-    """Buffer sets of a finished stream go back to the pool (at most 8 sets are kept)."""
-    if pinned:
-        for bufs in sets:
-            if len(_PINNED_POOL) < 8:
-                _PINNED_POOL.append(bufs)
+def _release(sets):
+    """Pinned buffer sets of a finished stream go back to the pool (at most 8 sets of the same dtypes are kept)."""
+    for bufs in sets:
+        kind = [b.dtype for b in bufs]
+        if sum([b.dtype for b in held] == kind for held in _PINNED) < 8:
+            _PINNED.append(bufs)
+
+
+def _feed(fill, consume, depth):
+    """Run `fill` on a worker thread up to `depth` buffers ahead of `consume`, which runs in the calling thread.
+
+    fill(buf) fills a buffer and returns (buf, item, done): the buffer it was given (None until the ring holds `depth`
+    buffers: fill makes one then) or one it made in its place, and what consume(buf, item) needs to use it.  Buffers
+    reach consume in the order they were filled and go back to fill once consumed; nothing is filled after the item
+    with done=True.  An exception raised in fill is raised here.  However this returns, the thread has stopped
+    first, so the caller may free what fill works on (bamcols_close frees what bamcols_emit works on)."""
+    import queue
+    import threading
+    free, full = queue.Queue(), queue.Queue()
+    for _ in range(depth):
+        free.put(None)
+    stop = threading.Event()
+
+    def produce():
+        try:
+            done = False
+            while not done and not stop.is_set():
+                try:
+                    buf = free.get(timeout=0.05)
+                except queue.Empty:
+                    continue
+                buf, item, done = fill(buf)
+                full.put((buf, item, done, None))
+        except BaseException as exc:                      # re-raised by the consumer
+            full.put((None, None, True, exc))
+
+    worker = threading.Thread(target=produce, daemon=True)
+    worker.start()
+    try:
+        done = False
+        while not done:
+            buf, item, done, exc = full.get()
+            if exc is not None:
+                raise exc
+            consume(buf, item)
+            item = None                                   # not kept alive while the next one is waited for
+            free.put(buf)
+    finally:
+        stop.set()
+        worker.join()
 
 
 def stream_single(reader, builder, chunk_rows=1 << 21, pinned=True, depth=3):
@@ -178,147 +268,65 @@ def stream_single(reader, builder, chunk_rows=1 << 21, pinned=True, depth=3):
     pinned buffers and push every filled buffer to the GPU while the next one is being decoded.
     Chunks end on read boundaries (bamcols_emit never splits a read), order_base = rows pushed so far,
     so the result equals one push of the whole file.  Returns the number of valid alignments."""
-    import queue
-    import threading
-    free, full = queue.Queue(), queue.Queue()
-    allocated = [0]
-    all_sets = []
-    stop = threading.Event()
-    rows = [int(chunk_rows)]
+    rows, sets, pushed = int(chunk_rows), [], 0
 
-    def next_buffers():
-        """A free buffer set; a new one is pinned only when all existing ones are in flight."""
-        while not stop.is_set():
-            try:
-                bufs = free.get_nowait()
-            except queue.Empty:
-                if allocated[0] < depth:
-                    allocated[0] += 1
-                    bufs = _column_buffers(rows[0], False, pinned)
-                    all_sets.append(bufs)
-                    return bufs
-                try:
-                    bufs = free.get(timeout=0.05)
-                except queue.Empty:
-                    continue
-            if int(bufs[0].shape[0]) >= rows[0]:
-                return bufs
-            allocated[0] -= 1                             # a set from before the buffers grew: let it go
-        return None
-
-    def produce():
-        try:
-            while not stop.is_set():
-                bufs = next_buffers()
-                if bufs is None:
-                    return
-                try:
-                    n, done = reader.emit(bufs[0], bufs[1], bufs[2])
-                except ValueError as exc:                 # a read longer than the buffers hold: grow and retry
-                    if "buffers hold" in str(exc) and rows[0] < (1 << 28):   # (as BamColumnReader.read_all does)
-                        rows[0] *= 4
-                        allocated[0] -= 1
-                        continue
-                    raise
-                full.put((bufs, n, done, None))
-                if done:
-                    return
-        except BaseException as exc:                      # re-raised by the consumer
-            full.put((None, 0, True, exc))
-
-    worker = threading.Thread(target=produce, daemon=True)
-    worker.start()
-    pushed = 0
-    try:
+    def fill(bufs):
+        nonlocal rows
         while True:
-            bufs, n, done, exc = full.get()
-            if exc is not None:
-                raise exc
-            if n:
-                builder.push(bufs[0], bufs[1], bufs[2], order_base=pushed, n=n)
-                pushed += n
-            free.put(bufs)
-            if done:
-                break
+            if bufs is None or int(bufs[0].shape[0]) < rows:   # none yet, or one from before the buffers grew
+                bufs = _buffers(rows, ("int32",) * 3, pinned)
+                sets.append(bufs)
+            try:
+                n, done = reader.emit(bufs[0], bufs[1], bufs[2])
+                return bufs, n, done
+            except ValueError as exc:                     # a read longer than the buffers hold: grow and retry
+                if "buffers hold" in str(exc) and rows < (1 << 28):   # (as BamColumnReader.read_all does)
+                    rows *= 4
+                    continue
+                raise
+
+    def consume(bufs, n):
+        nonlocal pushed
+        if n:
+            builder.push(bufs[0], bufs[1], bufs[2], order_base=pushed, n=n)
+            pushed += n
+
+    try:
+        _feed(fill, consume, depth)
     finally:
-        # whatever happened, the producer has left native code before the caller may close the reader:
-        # bamcols_close frees what bamcols_emit is working on
-        stop.set()
-        worker.join()
-        _release_buffers(all_sets, pinned)
+        if pinned:
+            _release(sets)
     return pushed
-
-
-_PINNED_KEYS = []      # pinned key buffer sets of finished collations, reused by the next one in this process
 
 
 def stream_collated(reader, builder, chunk_rows=1 << 21, pinned=True, depth=3):
     """Collate the valid alignments of `reader` (bamcols.BamColumnReader, tables set) by read name on the GPU and
     push them into `builder` as name-grouped reads (_native.Collator).  A worker thread fills a small ring of pinned
     buffers from emit_keys while the previous buffer is added.  Returns (valid alignments, reads, collator stats)."""
-    import queue
-    import threading
     from ._native import Collator
-    free, full = queue.Queue(), queue.Queue()
-    sets = []
-    for _ in range(depth):
-        bufs = None
-        if pinned:
-            import torch
-            while _PINNED_KEYS and bufs is None:
-                b = _PINNED_KEYS.pop()
-                if int(b[0].shape[0]) >= chunk_rows:
-                    bufs = b
-            if bufs is None:
-                bufs = [torch.empty(chunk_rows, dtype=torch.int64, pin_memory=True) for _ in range(2)] + \
-                       [torch.empty(chunk_rows, dtype=torch.int32, pin_memory=True) for _ in range(2)]
-        else:
-            bufs = [np.empty(chunk_rows, np.uint64), np.empty(chunk_rows, np.uint64), np.empty(chunk_rows, np.int32),
-                    np.empty(chunk_rows, np.int32)]
-        sets.append(bufs)
-        free.put(bufs)
-    stop = threading.Event()
+    sets, added = [], 0
 
-    def produce():
-        try:
-            while not stop.is_set():
-                try:
-                    bufs = free.get(timeout=0.05)
-                except queue.Empty:
-                    continue
-                n, done = reader.emit_keys(*bufs)
-                full.put((bufs, n, done, None))
-                if done:
-                    return
-        except BaseException as exc:                      # re-raised by the consumer
-            full.put((None, 0, True, exc))
+    def fill(bufs):
+        if bufs is None:
+            bufs = _buffers(chunk_rows, ("int64", "int64", "int32", "int32"), pinned)
+            sets.append(bufs)
+        n, done = reader.emit_keys(*bufs)
+        return bufs, n, done
 
-    added = 0
     with Collator(builder) as col:
-        worker = threading.Thread(target=produce, daemon=True)
-        worker.start()
+        def consume(bufs, n):
+            nonlocal added
+            if n:
+                col.add(*bufs, n=n)
+                added += n
+
         try:
-            while True:
-                bufs, n, done, exc = full.get()
-                if exc is not None:
-                    raise exc
-                if n:
-                    col.add(*bufs, n=n)
-                    added += n
-                free.put(bufs)
-                if done:
-                    break
+            _feed(fill, consume, depth)
         finally:
-            # the producer leaves native code before the caller may close the reader (as in stream_single)
-            stop.set()
-            worker.join()
             if pinned:
-                _PINNED_KEYS.extend(sets)
+                _release(sets)
         reads = col.push()
         return added, reads, col.stats()
-
-
-_PINNED_BYTES = []     # pinned read buffers of finished device decodes, reused by the next one in this process
 
 
 def stream_single_device(path, reader, builder, tables, track_ranges, max_bytes=128 << 20, depth=3):
@@ -328,76 +336,77 @@ def stream_single_device(path, reader, builder, tables, track_ranges, max_bytes=
     order_base = rows pushed so far, so the result equals stream_single's.  A call's blocks are inflated one thread
     per block, so runs are large: a 128 MiB run holds a few thousand blocks.
     Returns (valid alignments, (all_alignments, n_groups), (range_min, range_max) or None, decoder stats)."""
-    import queue
-    import threading
-    import torch
     from ._native import BamDecoder
     first = reader.plan_shards(1)[0]                      # virtual offset of the first record
-    free, full = queue.Queue(), queue.Queue()
     cap = int(max_bytes) + (1 << 17)                      # a run holds at least one block (< 64 KiB + header)
-    bufs = []
-    while _PINNED_BYTES and len(bufs) < depth:           # pinning costs about as much as reading the bytes
-        b = _PINNED_BYTES.pop()
-        if int(b.shape[0]) >= cap:
-            bufs.append(b)
-    bufs += [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(depth - len(bufs))]
-    for b in bufs:
-        free.put(b)
-    stop = threading.Event()
+    c, skip, pushed, sets = first >> 16, first & 0xFFFF, 0, []
+    with BamDecoder(builder, tables.tid_target, tables.tid_hap, track_ranges) as dec, open(path, "rb") as fh:
+        def fill(buf):
+            nonlocal c
+            off, length, isize, c_end = reader.blocks(c, max_bytes)
+            if len(off) == 0:
+                return buf, None, True
+            if buf is None:
+                buf = _buffers(cap, ("uint8",), True)
+                sets.append(buf)
+            n = c_end - c
+            fh.seek(c)
+            if fh.readinto(memoryview(buf[0].numpy())[:n]) != n:
+                raise IOError("%s changed while it was read" % path)
+            c = c_end
+            return buf, (n, (off, length, isize)), False
 
-    def produce():
-        try:
-            c = first >> 16
-            with open(path, "rb") as fh:
-                while not stop.is_set():
-                    off, length, isize, c_end = reader.blocks(c, max_bytes)
-                    if len(off) == 0:
-                        full.put((None, 0, None, None))
-                        return
-                    buf = None
-                    while buf is None and not stop.is_set():
-                        try:
-                            buf = free.get(timeout=0.05)
-                        except queue.Empty:
-                            pass
-                    if buf is None:
-                        return
-                    n = c_end - c
-                    fh.seek(c)
-                    if fh.readinto(memoryview(buf.numpy())[:n]) != n:
-                        raise IOError("%s changed while it was read" % path)
-                    full.put((buf, n, (off, length, isize), None))
-                    c = c_end
-        except BaseException as exc:                      # re-raised by the consumer
-            full.put((None, 0, None, exc))
+        def consume(buf, run):
+            nonlocal skip, pushed
+            if run is None:                               # the end of the file
+                rg, tg, hp = dec.decode(np.zeros(0, np.uint8), [], [], [], last=True)
+            else:
+                rg, tg, hp = dec.decode(buf[0], *run[1], skip=skip, n_bytes=run[0])
+                skip = 0
+            rows = int(rg.shape[0])
+            if rows:
+                builder.push(rg, tg, hp, order_base=pushed, n=rows)
+                pushed += rows
 
-    pushed = 0
-    with BamDecoder(builder, tables.tid_target, tables.tid_hap, track_ranges) as dec:
-        worker = threading.Thread(target=produce, daemon=True)
-        worker.start()
         try:
-            skip = first & 0xFFFF
-            while True:
-                buf, n, table, exc = full.get()
-                if exc is not None:
-                    raise exc
-                if buf is None:
-                    rg, tg, hp = dec.decode(np.zeros(0, np.uint8), [], [], [], last=True)
-                else:
-                    rg, tg, hp = dec.decode(buf, *table, skip=skip, n_bytes=n)
-                    skip = 0
-                rows = int(rg.shape[0])
-                if rows:
-                    builder.push(rg, tg, hp, order_base=pushed, n=rows)
-                    pushed += rows
-                if buf is None:
-                    break
-                free.put(buf)
+            _feed(fill, consume, depth)
         finally:
-            stop.set()
-            worker.join()
-            _PINNED_BYTES.extend(bufs)
+            _release(sets)
         return pushed, dec.counters(), dec.ranges() if track_ranges else None, dec.stats()
+
+
+def stream_files(bam_files, tables, cells, builder, order_base=0, n_threads=0, track_ranges=False):
+    """Decode the per-cell BAM files in order on a worker thread, one file ahead of the push, so that at most two
+    decoded files are in host memory, and push every file whole into `builder` (with cells) at order keys from
+    `order_base` on.  One push per file: the file is part of the (file, EC, cell) key and its last read is dropped
+    (drop_last_group; bam_utils_multisample.py:306-308).  tables: the job's target tables; cells: the
+    bamcols.CellDictionary that gives the cell ids.
+    Returns (alignments pushed, (range_min, range_max) over the files or None without track_ranges or files)."""
+    todo = collections.deque(bam_files)
+    pushed, lo, hi = 0, None, None
+
+    def fill(_):
+        with bamcols.BamColumnReader(todo.popleft(), n_threads=n_threads) as reader:
+            reader.set_tables(tables)
+            if track_ranges:
+                reader.track_ranges(True)
+            cols = reader.read_all(cells=cells, chunk=1 << 23)
+            ranges = reader.ranges() if track_ranges else None
+        return None, (cols, ranges), not todo
+
+    def consume(_, item):
+        nonlocal pushed, lo, hi
+        cols, ranges = item
+        builder.push(cols["read_group"], cols["target_idx"], cols["hap_idx"], cols["cell_idx"],
+                     order_base=order_base + pushed, drop_last_group=True)
+        pushed += len(cols["read_group"])
+        if ranges is not None:                            # merged over the files (bam_utils_multisample.py:568-576)
+            lo = ranges[0] if lo is None else np.minimum(lo, ranges[0])
+            hi = ranges[1] if hi is None else np.maximum(hi, ranges[1])
+
+    if todo:
+        _feed(fill, consume, 2)
+    return pushed, None if lo is None else (lo, hi)
 
 
 def read_bam(filename):

@@ -52,6 +52,11 @@ class TargetTables(object):
         self.lengths = np.zeros((len(main_targets), len(self.haplotypes)), dtype=np.int32)  # :605
         self.lengths[self.tid_target, self.tid_hap] = np.asarray(ref_lengths, dtype=np.int32)  # :615-633
 
+    def target_section(self):
+        """The EC file's targets section as bytes, which only the native tables (bamcols) build: None here, and the
+        writer builds it from main_targets and lengths."""
+        return None
+
     @property
     def num_targets(self):
         return len(self.main_targets)

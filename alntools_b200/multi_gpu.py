@@ -22,11 +22,15 @@ of include/ecb200.h.
 torch.distributed is the plumbing (process group, collectives on device tensors); every compute
 step is a libecb200 kernel behind the C ABI.
 """
+import contextlib
 import os
 import time
 
+import numpy as np
 import torch
 import torch.distributed as dist
+
+from . import bin_utils, utils
 
 _TIMING = bool(os.environ.get("ECB_MGPU_TIMING"))
 LAST_PHASES = {}   # with ECB_MGPU_TIMING: the (phase, ms) rows of the last call of each exchange, for tools
@@ -292,6 +296,111 @@ def distributed_finalize_cells(local, make_owner, device, min_count, cell_map, n
             "cell_order": cell_order, "n_ec": sum(r[0] for r in rows), "id_base": sum(rows[r][0] for r in front),
             "n_ec_local": sl["n_ec"], "nnz_local": sl["nnz"], "nnz_a": sum(r[1] for r in rows),
             "nnz_n": int(n_indptr[-1]), "n_samples": n_samples}
+
+
+@contextlib.contextmanager
+def rank_process():
+    """This process as one rank of a one-process-per-GPU job (RANK / WORLD_SIZE / LOCAL_RANK / MASTER_* in the
+    environment, as torchrun sets them): bound to the CPUs next to its GPU, so that the host buffers it pins land in
+    that GPU's NUMA node, with that GPU current, and in a NCCL process group, which is created here unless one
+    exists and then destroyed on the way out.  Yields (rank, world size, device)."""
+    rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
+    local_rank = int(os.environ.get("LOCAL_RANK", rank))
+    utils.bind_to_gpu_numa_node(local_rank)
+    torch.cuda.set_device(local_rank)
+    device = torch.device("cuda", local_rank)
+    own_group = not dist.is_initialized()
+    if own_group:
+        dist.init_process_group("nccl", device_id=device)
+    try:
+        yield rank, world, device
+    finally:
+        if own_group and dist.is_initialized():
+            dist.destroy_process_group()
+
+
+def save_rank_outputs(out, tables, section, sample_names, ec_filename, emase_filename, range_filename=None,
+                      references=None, ranges=None):
+    """Write the outputs of a multi-GPU convert; every rank calls it with its slice `out` of the final matrices, as
+    distributed_finalize or, for the per-cell converter, distributed_finalize_cells returned it.  First, on every
+    rank and before any file is touched, the global sizes are checked against the EC file's int32 fields.  The ranks
+    write their byte ranges of the EC file once rank 0 has laid it out; rank 0 assembles the EMASE file from every
+    rank's slice, and writes the range file from the ranges (range_min, range_max) of every rank's input (None for a
+    rank without input) over the header's reference names `references`.  section, sample_names: as
+    bin_utils.save_outputs.  -> non-zeros of A over all ranks."""
+    rank, world = dist.get_rank(), dist.get_world_size()
+    device = out["a_indptr"].device
+    cells = "n_indptr" in out                             # distributed_finalize_cells' result
+    n_ec, id_base, n_local, nnz_local = (int(out[k]) for k in ("n_ec", "id_base", "n_ec_local", "nnz_local"))
+    rows = torch.empty(3 * world, dtype=torch.int64, device=device)
+    dist.all_gather_into_tensor(rows, torch.tensor([id_base, n_local, nnz_local], dtype=torch.int64, device=device))
+    rows = rows.view(world, 3).tolist()
+    nnz_a = sum(r[2] for r in rows)
+    nnz_base = sum(r[2] for r in rows if r[1] and r[0] < id_base)   # the slices in front of this one in id order
+    nnz_n = int(out["nnz_n"]) if cells else n_ec
+    if n_ec + 1 > 0x7FFFFFFF or nnz_a > 0x7FFFFFFF or nnz_n > 0x7FFFFFFF:
+        raise RuntimeError("the EC file's int32 fields cannot hold %d ECs, %d A and %d N non-zeros" % (n_ec, nnz_a, nnz_n))
+    host = lambda t: t.cpu().numpy()
+    a = (host(out["a_indptr"][:n_local + 1]), host(out["a_indices"][:nnz_local]), host(out["a_data"][:nnz_local]))
+    if cells:
+        n = tuple(host(out[k]) for k in ("n_indptr", "n_col_counts", "n_col_offset", "n_indices", "n_data"))
+    else:
+        n = (host(out["n_data"][:n_local]),)
+    if ec_filename:
+        header = bin_utils.ec_header_bytes(tables.haplotypes, list(tables.main_targets.keys()) if section is None else None,
+                                           tables.lengths, sample_names, target_section=section,
+                                           n_targets=tables.num_targets)
+        write = bin_utils.ecsave2_cells_slice if cells else bin_utils.ecsave2_slice
+        args = (ec_filename, header, n_ec, nnz_a, id_base, nnz_base) + a + n
+        if rank == 0:
+            utils.delete_file(ec_filename)
+            write(*args, create=True)
+        dist.barrier()                                    # the file is laid out
+        if rank != 0:
+            write(*args, create=False)
+        dist.barrier()
+    a_csr = n_csc = None
+    if emase_filename:                                    # one writer: the slices travel to rank 0
+        parts = [None] * world
+        dist.all_gather_object(parts, (id_base, a, n))
+        if rank == 0:
+            a_csr, n_csc = _assemble(parts, n_ec, cells)
+    if range_filename is not None:                        # over every rank's input
+        if ranges is None:                                # neutral elements
+            ranges = (np.full(len(references), np.iinfo(np.int64).max), np.full(len(references), np.iinfo(np.int64).min))
+        lo, hi = (torch.from_numpy(np.asarray(x, dtype=np.int64)).to(device) for x in ranges)
+        dist.all_reduce(lo, op=dist.ReduceOp.MIN)
+        dist.all_reduce(hi, op=dist.ReduceOp.MAX)
+        ranges = (lo.cpu().numpy(), hi.cpu().numpy())
+    if rank == 0:
+        bin_utils.save_outputs(tables, section, sample_names, a_csr, n_csc, cells, emase_filename=emase_filename,
+                               range_filename=range_filename, references=references, ranges=ranges)
+    return nnz_a
+
+
+def _assemble(parts, n_ec, cells):
+    """The whole matrices from every rank's (id_base, A pieces, N pieces), in id order (for the EMASE file)."""
+    parts = sorted((p for p in parts if len(p[1][0]) > 1), key=lambda p: p[0])
+    indptr, at = [np.zeros(1, dtype=np.int64)], 0
+    for _, (ip, ix, _d), _n in parts:
+        indptr.append(ip[1:].astype(np.int64) + at)
+        at += len(ix)
+    a_csr = (np.concatenate(indptr).astype(np.int32), np.concatenate([p[1][1] for p in parts]).astype(np.int32),
+             np.concatenate([p[1][2] for p in parts]).astype(np.int32))
+    if not cells:                                         # one sample: N holds every EC's count
+        return a_csr, (np.array([0, n_ec], dtype=np.int32), np.arange(n_ec, dtype=np.int32),
+                       np.concatenate([p[2][0] for p in parts]))
+    n_indptr = parts[0][2][0] if parts else np.zeros(1, dtype=np.int32)
+    nnz = int(n_indptr[-1])
+    idx, dat = np.empty(nnz, dtype=np.int32), np.empty(nnz, dtype=np.int32)
+    for id_base, _a, (ptr, counts, offset, ix, d) in parts:
+        counts = counts.astype(np.int64)
+        starts = np.cumsum(counts) - counts
+        col = np.repeat(np.arange(len(counts)), counts)
+        dest = ptr[col].astype(np.int64) + offset[col] + (np.arange(len(ix)) - starts[col])
+        idx[dest] = ix + id_base
+        dat[dest] = d
+    return a_csr, (n_indptr.astype(np.int32), idx, dat)
 
 
 def shard_bounds(read_group, world):

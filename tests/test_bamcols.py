@@ -478,16 +478,17 @@ def test_native_target_section_equals_the_python_one(tmp_path):
 
 
 class _StubBuilder(object):
-    """Stands in for EcBuilder: collects what stream_single pushes (host logic only, no GPU)."""
+    """Stands in for EcBuilder: collects what stream_single / stream_files push (host logic only, no GPU)."""
 
     def __init__(self, fail_at=None):
-        self.parts, self.bases, self.fail_at = [], [], fail_at
+        self.parts, self.bases, self.drops, self.fail_at = [], [], [], fail_at
 
-    def push(self, rg, tg, hp, order_base=0, n=None):
+    def push(self, rg, tg, hp, cell=None, order_base=0, n=None, drop_last_group=False):
         if self.fail_at is not None and len(self.parts) >= self.fail_at:
             raise RuntimeError("push failed")
-        self.parts.append([np.array(x[:n]) for x in (rg, tg, hp)])
+        self.parts.append([np.array(x[:n]) for x in (rg, tg, hp) + (() if cell is None else (cell,))])
         self.bases.append(order_base)
+        self.drops.append(drop_last_group)
 
 
 def test_stream_single_pipeline(tmp_path):
@@ -520,6 +521,48 @@ def test_stream_single_pipeline(tmp_path):
         with pytest.raises(RuntimeError, match="push failed"):
             emitter.stream_single(r, _StubBuilder(fail_at=3), chunk_rows=64, pinned=False)
         assert threading.active_count() == before                   # the producer was joined
+
+
+def test_stream_files_pipeline(tmp_path):
+    """emitter.stream_files, the per-cell decode-ahead: one push per file, in order, with drop_last_group and order
+    keys from order_base on, equal to decoding the files one after another, and the ranges merged over the files.
+    When the consumer fails, or a file cannot be read in the decode thread, the error reaches the caller once that
+    thread has been joined."""
+    import threading
+    from alntools_b200 import bam_utils_multisample
+    case = max(golden_cases("multisample"), key=lambda c: len(c["file_order"]))
+    files = [os.path.join(GOLDEN, case["dir"], fn) for fn in case["file_order"]] * 2   # more files than the ring holds
+    tables, _, _ = bam_utils_multisample._tables(files[0], None, False)
+    want, lo, hi = [], None, None
+    ref_cells = bamcols.CellDictionary()
+    for path in files:
+        with bamcols.BamColumnReader(path) as r:
+            r.set_tables(tables)
+            r.track_ranges(True)
+            want.append(r.read_all(cells=ref_cells))
+            l, h = r.ranges()
+        lo, hi = (l, h) if lo is None else (np.minimum(lo, l), np.maximum(hi, h))
+    ref_cells.close()
+    stub, cells = _StubBuilder(), bamcols.CellDictionary()
+    n, ranges = emitter.stream_files(files, tables, cells, stub, order_base=3 << 40, track_ranges=True)
+    cells.close()
+    sizes = [len(w["read_group"]) for w in want]
+    assert n == sum(sizes) and stub.drops == [True] * len(files)
+    assert stub.bases == [(3 << 40) + int(s) for s in np.cumsum([0] + sizes[:-1])]
+    for got, w in zip(stub.parts, want):
+        for g, key in zip(got, ("read_group", "target_idx", "hap_idx", "cell_idx")):
+            assert np.array_equal(g, w[key])
+    assert np.array_equal(ranges[0], lo) and np.array_equal(ranges[1], hi)
+    assert emitter.stream_files([], tables, None, stub) == (0, None)
+    before = threading.active_count()
+    missing = str(tmp_path / "missing.bam")
+    for paths, builder, err in ((files, _StubBuilder(fail_at=1), RuntimeError),
+                                (files[:1] + [missing] + files[1:], _StubBuilder(), OSError)):
+        cells = bamcols.CellDictionary()
+        with pytest.raises(err):
+            emitter.stream_files(paths, tables, cells, builder)
+        assert threading.active_count() == before               # the decode thread was joined
+        cells.close()
 
 
 @pytest.mark.parametrize("payload,n_shards", [(300, 2), (300, 5), (4000, 3), (60000, 4), (70, 7)])

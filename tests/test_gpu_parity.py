@@ -399,6 +399,45 @@ def test_multigpu_convert_writes_the_golden_files(native):
     assert "multigpu convert check: ok" in out.stdout
 
 
+def _single_rank_body_world1(bam, out, target_filename=None, range_filename=None):
+    """bam_utils.convert_rank as the only rank of a job (the orchestration of the multi-GPU convert - shard plan,
+    decode, rebase, exchange, header, slice writes, range all-reduce - on one GPU)."""
+    import json
+    import subprocess
+    import sys
+    from conftest import ROOT
+    code = ("import json, sys; sys.path.insert(0, %r); from alntools_b200 import bam_utils; a = json.loads(sys.argv[1]); "
+            "bam_utils.convert_rank(a[0], a[1], None, range_filename=a[2], target_filename=a[3])" % ROOT)
+    env = dict(os.environ, RANK="0", WORLD_SIZE="1", LOCAL_RANK="0", MASTER_ADDR="127.0.0.1", MASTER_PORT="29545")
+    subprocess.check_call([sys.executable, "-c", code, json.dumps([bam, out, range_filename, target_filename])], env=env,
+                          cwd=ROOT, timeout=600)
+
+
+def test_single_rank_body_matches_one_gpu_file(native, tmp_path):
+    """The single-sample multi-GPU rank body at world 1 writes every golden EC file (and the golden range files), and
+    on a generated 1.5 M-read file the same EC and range files as the one-GPU convert()."""
+    from alntools_b200 import bam_utils, synth
+    for case in golden_cases("single"):
+        out, rng = str(tmp_path / (case["name"] + ".rank.bin")), str(tmp_path / (case["name"] + ".rank.range"))
+        tfile = os.path.join(GOLDEN, case["targets"]) if case["targets"] else None
+        _single_rank_body_world1(os.path.join(GOLDEN, case["bam"]), out, tfile, rng if case.get("range") else None)
+        with open(out, "rb") as a, open(os.path.join(GOLDEN, case["ec"]), "rb") as b:
+            assert a.read() == b.read(), case["name"]
+        if case.get("range"):
+            with open(rng) as a, open(os.path.join(GOLDEN, case["range"])) as b:
+                assert a.read() == b.read(), case["name"]
+    cols = synth.make_columns(1_500_000, 20000, 2, seed=77, mode="diploid", dup_rate=0.01)
+    bam = str(tmp_path / "big.bam")
+    synth.columns_to_bam(bam, cols, 20000, 2)
+    one, one_rng = str(tmp_path / "big.1.bin"), str(tmp_path / "big.1.range")
+    bam_utils.convert(bam, one, None, range_filename=one_rng)
+    out, out_rng = str(tmp_path / "big.rank.bin"), str(tmp_path / "big.rank.range")
+    _single_rank_body_world1(bam, out, range_filename=out_rng)
+    for x, y in ((out, one), (out_rng, one_rng)):
+        with open(x, "rb") as a, open(y, "rb") as b:
+            assert a.read() == b.read(), x
+
+
 def test_rebase_moves_the_order_keys(native):
     """ecb_rebase: pushes made with order_base counted from 0 and then moved by a delta give the result of
     pushes made at their final positions (two contexts merged through the single-GPU exchange emulation would

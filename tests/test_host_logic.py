@@ -164,6 +164,29 @@ def test_convert_writes_the_same_file_with_native_and_python_target_sections(tmp
     assert len(outputs["native"][0]) > 60 and len(outputs["native"][1]) > 60
 
 
+@pytest.mark.parametrize("emitter_mode", ["native", "python"])
+def test_convert_files_without_files_raises(tmp_path, monkeypatch, emitter_mode):
+    """convert_files([]) has no file to take the target tables from: it raises ValueError at once, with either
+    emitter, instead of waiting for tables that never come."""
+    import threading
+    from alntools_b200 import bam_utils_multisample
+    monkeypatch.setenv("ALNTOOLS_B200_EMITTER", emitter_mode)
+    outcome = []
+
+    def run():
+        try:
+            bam_utils_multisample.convert_files([], str(tmp_path / "x.bin"), None, 1)
+        except Exception as exc:     # noqa: BLE001 - checked below
+            outcome.append(exc)
+
+    worker = threading.Thread(target=run, daemon=True)
+    worker.start()
+    worker.join(1.0)
+    assert not worker.is_alive(), "convert_files([]) did not return within a second"
+    assert len(outcome) == 1 and isinstance(outcome[0], ValueError), outcome
+    assert not os.path.exists(str(tmp_path / "x.bin"))
+
+
 def test_sliced_ec_file_writer_reproduces_the_golden_bytes(tmp_path):
     """bin_utils.ecsave2_slice: the EC file written in EC-id ranges by several writers (what the ranks of the
     multi-GPU convert do) is the file ecsave2 writes, for 1, 2, 3 and 5 writers, empty slices included."""
