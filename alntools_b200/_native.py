@@ -23,6 +23,7 @@ ECB_OPT_PAGEABLE_RESULTS = 8
 ECB_OPT_BAM_WINDOW = 9
 ECB_OPT_COLLATE_SLOTS = 10
 ECB_OPT_COLLATE_PIECE = 11
+ECB_OPT_COLLATE_BUDGET = 12
 
 ECB_ERR_EMPTY = -5
 ECB_ERR_FORMAT = -7
@@ -87,6 +88,8 @@ class EcbCollateStats(ctypes.Structure):
         ("table_grows", ctypes.c_int64), ("pieces", ctypes.c_int64), ("device_bytes", ctypes.c_int64),
         ("h2d_bytes", ctypes.c_int64), ("add_ms", ctypes.c_double), ("table_ms", ctypes.c_double),
         ("order_ms", ctypes.c_double), ("layout_ms", ctypes.c_double), ("push_ms", ctypes.c_double),
+        ("spills", ctypes.c_int64), ("groups", ctypes.c_int64), ("host_bytes", ctypes.c_int64),
+        ("d2h_bytes", ctypes.c_int64), ("spill_ms", ctypes.c_double),
     ]
 
     def as_dict(self):
@@ -236,7 +239,7 @@ class EcBuilder(object):
                 "hot_cache": ECB_OPT_HOT_CACHE, "verify_keys": ECB_OPT_VERIFY_KEYS,
                 "chunk_len": ECB_OPT_CHUNK_LEN, "pageable_results": ECB_OPT_PAGEABLE_RESULTS,
                 "bam_window": ECB_OPT_BAM_WINDOW, "collate_slots": ECB_OPT_COLLATE_SLOTS,
-                "collate_piece": ECB_OPT_COLLATE_PIECE}
+                "collate_piece": ECB_OPT_COLLATE_PIECE, "collate_budget": ECB_OPT_COLLATE_BUDGET}
 
     def _check(self, rc):
         if rc != 0:

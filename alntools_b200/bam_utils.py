@@ -246,10 +246,12 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
     collate=True (or ALNTOOLS_B200_COLLATE=1) takes a file that is not grouped by read name: a read is every valid
     alignment with one trimmed name, wherever it lies, and reads are ordered by their first alignment (one GPU, host
     decode).  The outputs are those of the default convert() of the file regrouped that way; for a grouped file they
-    are the default's.
+    are the default's.  ALNTOOLS_B200_COLLATE_BUDGET caps the device bytes of the collation (emitter.collate_budget);
+    a file whose rows do not fit is collated in passes through host memory, with the same outputs.
     """
     start_time = time.time()
     mode = emitter.resolve_mode(False, devices, decode, collate, range_filename is not None)
+    budget = emitter.collate_budget() if mode.collate else 0
     job = dict(bam_filename=bam_filename, ec_filename=ec_filename, emase_filename=emase_filename, num_chunks=num_chunks,
                number_processes=number_processes, temp_dir=temp_dir, range_filename=range_filename, sample=sample,
                target_filename=target_filename)
@@ -301,7 +303,7 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
         # no alignment count is known up front: the library sizes its table from the first chunk and
         # grows it ahead of later ones; one finalize per context, so results skip the pinning cost
         with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=False, alignments_hint=0,
-                       device=device, pageable_results=1) as builder:
+                       device=device, pageable_results=1, collate_budget=budget) as builder:
             chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(bam_filename) // 2)))   # 24 MB of columns per piece
             if mode.decode == "device":
                 valid, _, ranges, _ = emitter.stream_single_device(bam_filename, reader, builder, tables,

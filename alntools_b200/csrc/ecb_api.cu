@@ -1,9 +1,11 @@
 // ecb_api.cu — context management and the C ABI of libecb200.so (see include/ecb200.h).
 #include <algorithm>
+#include <chrono>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -47,7 +49,7 @@ struct ecb_ctx {
   int verify_keys = 0;
   int pageable_results = 0;
   int64_t opt_bam_window = 0;
-  int64_t opt_collate_slots = 0, opt_collate_piece = 0;
+  int64_t opt_collate_slots = 0, opt_collate_piece = 0, opt_collate_budget = 0;
   // EC table
   DevBuf table;
   u32 table_slots = 0;
@@ -555,7 +557,7 @@ void cells_release(ecb_ctx* c) {
 
 extern "C" {
 
-int ecb_version(void) { return 2003; }
+int ecb_version(void) { return 2004; }
 
 const char* ecb_last_error(const ecb_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
@@ -639,6 +641,9 @@ int ecb_set_option(ecb_ctx* c, int option, int64_t value) {
     case ECB_OPT_COLLATE_PIECE:
       if (value < 0 || value > ECB_PUSH_LIMIT) return fail(c, ECB_ERR_INVALID, "collate piece %lld outside [0, %lld]", (long long)value, (long long)ECB_PUSH_LIMIT);
       c->opt_collate_piece = value; break;
+    case ECB_OPT_COLLATE_BUDGET:
+      if (value < 0) return fail(c, ECB_ERR_INVALID, "negative collate budget");
+      c->opt_collate_budget = value; break;
     default: return fail(c, ECB_ERR_INVALID, "unknown option %d", option);
   }
   return ECB_OK;
@@ -2035,53 +2040,263 @@ int ecb_bam_destroy(ecb_bam* d) {
 }  // extern "C"
 
 // ---- collation of alignments by read name (kernels in ecb_collate.cuh) -----------------------------------------
+// Rows of one spill in host memory: by fine bucket, file order inside a bucket.
+struct CollateSpill {
+  u64 m = 0;
+  std::vector<u32> offs;                   // [COLLATE_BUCKETS + 1]
+  std::unique_ptr<u64[]> lo, hi;           // dropped after the names pass
+  std::unique_ptr<int32_t[]> tg, hp;
+  std::unique_ptr<u32[]> pos;              // file-order position; after the names pass the first position of its read
+};
+
+// Rows placed in collated order, in host memory: by piece.
+struct CollateChunk {
+  std::vector<u32> offs;                   // [pieces + 1]
+  std::unique_ptr<u32[]> id, place;
+  std::unique_ptr<int32_t[]> tg, hp;
+};
+
 struct ecb_collate {
   ecb_ctx* c = nullptr;
   u64 n = 0;                          // alignments added
-  DevBuf key_lo, key_hi, tg_in, hp_in;   // the added columns, in file order
+  DevBuf key_lo, key_hi, tg_in, hp_in;   // the added columns, in file order (after a spill: the staging area)
   DevBuf table, slot_of, bitmap, word_rank, count, cursor, rg, tg, hp, cuts;
+  // after a spill: positions / first positions / places, ids, the partition's outputs and scratch, read lists
+  DevBuf pos, idv, o_lo, o_hi, o_tg, o_hp, o_pos, o_id, part_counts, list;
   u32 slots = 0;
   bool pushed = false;
   cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   ecb_collate_stats stats{};
+  // the budget and the spill state
+  int64_t budget = 0;
+  bool spilling = false;
+  u64 stage = 0, res = 0, spilled = 0;   // rows the staging area takes, rows in it, rows already spilled
+  std::vector<CollateSpill> spills;
+  std::vector<CollateChunk> chunks;
+  int64_t host_now = 0;
+  void* ring[2] = {nullptr, nullptr};    // pinned staging ring of the host copies
+  cudaEvent_t ring_ev[2] = {nullptr, nullptr};
+  int ring_next = 0;
 };
 
 namespace {
 
-int64_t collate_bytes(const ecb_collate* k) {
-  const DevBuf* bufs[] = {&k->key_lo, &k->key_hi, &k->tg_in, &k->hp_in, &k->table, &k->slot_of, &k->bitmap, &k->word_rank,
-                          &k->count, &k->cursor, &k->rg, &k->tg, &k->hp, &k->cuts};
+#define COLLATE_RING_BYTES ((size_t)8 << 20)
+#define COLLATE_MIN_STAGE 32
+
+template <class F>
+void for_each_buf(ecb_collate* k, F f) {
+  DevBuf* all[] = {&k->key_lo, &k->key_hi, &k->tg_in, &k->hp_in, &k->table, &k->slot_of, &k->bitmap, &k->word_rank,
+                   &k->count, &k->cursor, &k->rg, &k->tg, &k->hp, &k->cuts, &k->pos, &k->idv, &k->o_lo, &k->o_hi,
+                   &k->o_tg, &k->o_hp, &k->o_pos, &k->o_id, &k->part_counts, &k->list};
+  for (DevBuf* b : all) f(*b);
+}
+
+int64_t collate_bytes(ecb_collate* k) {
   int64_t total = 0;
-  for (const DevBuf* b : bufs) total += (int64_t)b->bytes;
+  for_each_buf(k, [&](DevBuf& b) { total += (int64_t)b.bytes; });
   return total;
 }
 
 void collate_release(ecb_collate* k) {
   ecb_ctx* c = k->c;
-  DevBuf* bufs[] = {&k->key_lo, &k->key_hi, &k->tg_in, &k->hp_in, &k->table, &k->slot_of, &k->bitmap, &k->word_rank,
-                    &k->count, &k->cursor, &k->rg, &k->tg, &k->hp, &k->cuts};
-  for (DevBuf* b : bufs) release(c, *b);
+  for_each_buf(k, [&](DevBuf& b) { release(c, b); });
   cudaStreamSynchronize(c->stream);
   for (auto& e : k->ev)
     if (e) cudaEventDestroy(e);
+  for (int s = 0; s < 2; ++s) {
+    if (k->ring[s]) cudaFreeHost(k->ring[s]);
+    if (k->ring_ev[s]) cudaEventDestroy(k->ring_ev[s]);
+  }
   delete k;
 }
 
-// The name table over every added alignment.  A table that runs out of probes is replaced by one four times
-// larger and the insert runs again from the start: positions are file-order indices, so a rerun gives the same
-// slots' contents whatever happened before.
-int collate_table(ecb_collate* k) {
+void note_peak(ecb_collate* k) { k->stats.device_bytes = std::max(k->stats.device_bytes, collate_bytes(k)); }
+
+void note_host(ecb_collate* k, int64_t delta) {
+  k->host_now += delta;
+  k->stats.host_bytes = std::max(k->stats.host_bytes, k->host_now);
+}
+
+// Exactly `bytes` (rounded up to 256) unless the buffer already holds as many: the budgeted buffers of a spilled
+// collation take none of ensure()'s growth slack.
+int need(ecb_collate* k, DevBuf& b, size_t bytes) {
+  if (b.bytes >= bytes) return ECB_OK;
+  release(k->c, b);
+  CKR(ensure(k->c, b, bytes));
+  note_peak(k);
+  return ECB_OK;
+}
+
+size_t round256(size_t bytes) { return (bytes + 255) & ~(size_t)255; }
+
+// Device bytes of the one-pass collation of n alignments: rows (24 B, half of the growth slack of the add counted),
+// slot, regrouped columns, bitmap and ranks, counts and offsets with R <= n, and the table.
+u64 one_pass_bytes(const ecb_ctx* c, u64 n) {
+  const u64 want = c->opt_collate_slots > 0 ? (u64)c->opt_collate_slots : n + n / 2;
+  const u64 slots = std::max<u64>(1u << 10, pow2_ceil(want));
+  return 36 * n + 4 * n + 12 * n + 8 * (n / 32 + 1) + 8 * n + 32 * slots;
+}
+
+u32 group_slots(u64 g) { return std::max<u32>(64u, pow2_ceil(g + g / 2)); }
+
+// Device bytes of the names pass of a group of g rows: keys, positions, slots, read list, table.
+u64 names_pass_bytes(u64 g) {
+  return round256(8 * g) * 2 + round256(4 * g) * 2 + round256(8 * g) + 32 * (u64)group_slots(g);
+}
+
+u32 part_tiles(u64 m) { return (u32)std::max<u64>(1, (m + COLLATE_TILE - 1) / COLLATE_TILE); }
+
+int ring_init(ecb_collate* k) {
   ecb_ctx* c = k->c;
-  u64 want = c->opt_collate_slots > 0 ? (u64)c->opt_collate_slots : k->n + k->n / 2;
-  k->slots = std::max<u32>(1u << 10, pow2_ceil(want));
-  CKR(ensure(c, k->slot_of, (size_t)k->n * 4));
+  for (int s = 0; s < 2; ++s) {
+    if (!k->ring[s]) CK(cudaHostAlloc(&k->ring[s], COLLATE_RING_BYTES, cudaHostAllocDefault));
+    if (!k->ring_ev[s]) CK(cudaEventCreateWithFlags(&k->ring_ev[s], cudaEventDisableTiming));
+  }
+  return ECB_OK;
+}
+
+// host -> device through the pinned ring, stream-ordered: work queued after it on the stream sees the bytes.
+int ring_h2d(ecb_collate* k, void* dst, const void* src, size_t bytes) {
+  ecb_ctx* c = k->c;
+  for (size_t off = 0; off < bytes; off += COLLATE_RING_BYTES) {
+    const size_t len = std::min(COLLATE_RING_BYTES, bytes - off);
+    const int s = k->ring_next;
+    k->ring_next ^= 1;
+    CK(cudaEventSynchronize(k->ring_ev[s]));
+    memcpy(k->ring[s], (const char*)src + off, len);
+    CK(cudaMemcpyAsync((char*)dst + off, k->ring[s], len, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaEventRecord(k->ring_ev[s], c->stream));
+  }
+  k->stats.h2d_bytes += (int64_t)bytes;
+  return ECB_OK;
+}
+
+// device -> host through the pinned ring; returns with the bytes in dst.  The copy of one slot overlaps the host
+// copy out of the other.
+int ring_d2h(ecb_collate* k, void* dst, const void* src, size_t bytes) {
+  ecb_ctx* c = k->c;
+  int pend = -1;
+  size_t pend_off = 0, pend_len = 0;
+  for (size_t off = 0; off < bytes; off += COLLATE_RING_BYTES) {
+    const size_t len = std::min(COLLATE_RING_BYTES, bytes - off);
+    const int s = k->ring_next;
+    k->ring_next ^= 1;
+    CK(cudaEventSynchronize(k->ring_ev[s]));
+    CK(cudaMemcpyAsync(k->ring[s], (const char*)src + off, len, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaEventRecord(k->ring_ev[s], c->stream));
+    if (pend >= 0) {
+      CK(cudaEventSynchronize(k->ring_ev[pend]));
+      memcpy((char*)dst + pend_off, k->ring[pend], pend_len);
+    }
+    pend = s, pend_off = off, pend_len = len;
+  }
+  if (pend >= 0) {
+    CK(cudaEventSynchronize(k->ring_ev[pend]));
+    memcpy((char*)dst + pend_off, k->ring[pend], pend_len);
+  }
+  k->stats.d2h_bytes += (int64_t)bytes;
+  return ECB_OK;
+}
+
+// Stable partition of rows [0, m) by `P` into nb buckets; offs (host) <- the bucket offsets [nb + 1], which are the
+// scanned counters of tile 0 (one strided copy).
+template <class Part>
+int partition(ecb_collate* k, const Part& P, u64 m, u32 nb, std::vector<u32>& offs) {
+  ecb_ctx* c = k->c;
+  const u32 tiles = part_tiles(m);
+  CKR(need(k, k->part_counts, (size_t)nb * tiles * 4));
+  ecb_part_count_kernel<Part><<<tiles, 256, 0, c->stream>>>(P, m, nb, tiles, (u32*)k->part_counts.p);
+  LAUNCH_CHECK("collate_part_count");
+  CKR(device_scan<false>(c, (const u32*)k->part_counts.p, (u32*)k->part_counts.p, (u64)nb * tiles, 0, nullptr));
+  ecb_part_scatter_kernel<Part><<<tiles, 256, 0, c->stream>>>(P, m, nb, tiles, (const u32*)k->part_counts.p);
+  LAUNCH_CHECK("collate_part_scatter");
+  offs.resize((size_t)nb + 1);
+  CK(cudaMemcpy2DAsync(offs.data(), 4, k->part_counts.p, (size_t)tiles * 4, 4, nb, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  offs[nb] = (u32)m;
+  k->stats.d2h_bytes += (int64_t)nb * 4;
+  return ECB_OK;
+}
+
+// Move the rows of the staging area to host storage, partitioned by fine bucket.
+int collate_spill(ecb_collate* k) {
+  const u64 m = k->res;
+  if (m == 0) return ECB_OK;
+  const auto t0 = std::chrono::steady_clock::now();
+  CKR(need(k, k->o_lo, (size_t)m * 8));
+  CKR(need(k, k->o_hi, (size_t)m * 8));
+  CKR(need(k, k->o_tg, (size_t)m * 4));
+  CKR(need(k, k->o_hp, (size_t)m * 4));
+  CKR(need(k, k->o_pos, (size_t)m * 4));
+  SpillPart P{(const u64*)k->key_lo.p, (const u64*)k->key_hi.p, (const int32_t*)k->tg_in.p, (const int32_t*)k->hp_in.p,
+              k->spilled, (u64*)k->o_lo.p, (u64*)k->o_hi.p, (int32_t*)k->o_tg.p, (int32_t*)k->o_hp.p, (u32*)k->o_pos.p};
+  CollateSpill sp;
+  sp.m = m;
+  CKR(partition(k, P, m, COLLATE_BUCKETS, sp.offs));
+  sp.lo.reset(new u64[m]);
+  sp.hi.reset(new u64[m]);
+  sp.tg.reset(new int32_t[m]);
+  sp.hp.reset(new int32_t[m]);
+  sp.pos.reset(new u32[m]);
+  note_host(k, (int64_t)(28 * m + sp.offs.size() * 4));
+  CKR(ring_d2h(k, sp.lo.get(), k->o_lo.p, m * 8));
+  CKR(ring_d2h(k, sp.hi.get(), k->o_hi.p, m * 8));
+  CKR(ring_d2h(k, sp.tg.get(), k->o_tg.p, m * 4));
+  CKR(ring_d2h(k, sp.hp.get(), k->o_hp.p, m * 4));
+  CKR(ring_d2h(k, sp.pos.get(), k->o_pos.p, m * 4));
+  k->spills.push_back(std::move(sp));
+  k->spilled += m;
+  k->res = 0;
+  k->stats.spills++;
+  k->stats.spill_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  return ECB_OK;
+}
+
+// The add that would pass the budget: the rows held so far are spilled, and from then on device memory is a fixed
+// staging area of `stage` rows (the rows, the partition's outputs and its counters).
+int collate_start_spilling(ecb_collate* k) {
+  ecb_ctx* c = k->c;
+  CKR(ring_init(k));
+  k->res = k->n;
+  CKR(collate_spill(k));
+  DevBuf* staged[] = {&k->key_lo, &k->key_hi, &k->tg_in, &k->hp_in, &k->o_lo, &k->o_hi, &k->o_tg, &k->o_hp, &k->o_pos,
+                      &k->part_counts};
+  for (DevBuf* b : staged) release(c, *b);
+  const int64_t fixed = (int64_t)COLLATE_BUCKETS * 4 + 10 * 256;
+  const int64_t per_row = 24 + 28 + 4 * COLLATE_BUCKETS / COLLATE_TILE;
+  const int64_t stage = (k->budget - fixed) / per_row;
+  if (stage < COLLATE_MIN_STAGE)
+    return fail(c, ECB_ERR_LIMIT, "the collate budget of %lld bytes cannot hold a staging area of %d alignments",
+                (long long)k->budget, COLLATE_MIN_STAGE);
+  k->stage = (u64)stage;
+  CKR(need(k, k->key_lo, (size_t)stage * 8));
+  CKR(need(k, k->key_hi, (size_t)stage * 8));
+  CKR(need(k, k->tg_in, (size_t)stage * 4));
+  CKR(need(k, k->hp_in, (size_t)stage * 4));
+  CKR(need(k, k->o_lo, (size_t)stage * 8));
+  CKR(need(k, k->o_hi, (size_t)stage * 8));
+  CKR(need(k, k->o_tg, (size_t)stage * 4));
+  CKR(need(k, k->o_hp, (size_t)stage * 4));
+  CKR(need(k, k->o_pos, (size_t)stage * 4));
+  CKR(need(k, k->part_counts, (size_t)COLLATE_BUCKETS * part_tiles(stage) * 4));
+  k->spilling = true;
+  return ECB_OK;
+}
+
+// The name table over rows [0, n) (positions from `pos`, or the row index).  A table that runs out of probes is
+// replaced by one four times larger and the insert runs again from the start: positions are file-order indices, so
+// a rerun gives the same slots' contents whatever happened before.  exact: budgeted allocation (need).
+int collate_table(ecb_collate* k, const u64* lo, const u64* hi, const u32* pos, u64 n, u32 slots, bool exact) {
+  ecb_ctx* c = k->c;
+  k->slots = slots;
+  CKR(exact ? need(k, k->slot_of, (size_t)n * 4) : ensure(c, k->slot_of, (size_t)n * 4));
   for (;;) {
-    CKR(ensure(c, k->table, (size_t)k->slots * sizeof(EcbEntry)));
+    CKR(exact ? need(k, k->table, (size_t)k->slots * sizeof(EcbEntry)) : ensure(c, k->table, (size_t)k->slots * sizeof(EcbEntry)));
     CK(cudaMemsetAsync(k->table.p, 0xFF, (size_t)k->slots * sizeof(EcbEntry), c->stream));
     CK(cudaMemsetAsync(c->d_ctr->scratch, 0, 2 * sizeof(u32), c->stream));
-    CollateParams P{(const u64*)k->key_lo.p, (const u64*)k->key_hi.p, k->n, (EcbEntry*)k->table.p, k->slots - 1,
-                    (u32*)k->slot_of.p, c->d_ctr};
-    ecb_collate_insert_kernel<<<grid_for(k->n, 256, c->sm_count * 8), 256, 0, c->stream>>>(P);
+    CollateParams P{lo, hi, pos, n, (EcbEntry*)k->table.p, k->slots - 1, (u32*)k->slot_of.p, c->d_ctr};
+    ecb_collate_insert_kernel<<<grid_for(n, 256, c->sm_count * 8), 256, 0, c->stream>>>(P);
     LAUNCH_CHECK("collate_insert");
     CKR(sync_counters(c));
     if (c->h_ctr->scratch[1] == 0) break;
@@ -2089,8 +2304,7 @@ int collate_table(ecb_collate* k) {
     k->slots = k->slots <= (1u << 29) ? k->slots * 4u : (1u << 31);
     k->stats.table_grows++;
   }
-  k->stats.table_slots = k->slots;
-  k->stats.reads = c->h_ctr->scratch[0];
+  k->stats.table_slots = std::max<int64_t>(k->stats.table_slots, k->slots);
   return ECB_OK;
 }
 
@@ -2101,7 +2315,10 @@ int collate_push(ecb_collate* k, int64_t* n_reads) {
   if (n == 0) return ECB_OK;
   float ms = 0;
   CK(cudaEventRecord(k->ev[0], c->stream));
-  CKR(collate_table(k));
+  const u64 want = c->opt_collate_slots > 0 ? (u64)c->opt_collate_slots : k->n + k->n / 2;
+  CKR(collate_table(k, (const u64*)k->key_lo.p, (const u64*)k->key_hi.p, nullptr, k->n,
+                    std::max<u32>(1u << 10, pow2_ceil(want)), false));
+  k->stats.reads = c->h_ctr->scratch[0];
   const u32 R = (u32)k->stats.reads;
   CK(cudaEventRecord(k->ev[1], c->stream));
 
@@ -2145,7 +2362,7 @@ int collate_push(ecb_collate* k, int64_t* n_reads) {
   const u32 pieces = cuts[0];
   if (pieces == 0 || pieces > max_cuts || cuts[1 + pieces] != n)
     return fail(c, ECB_ERR_INVALID, "collation cut %u pieces", pieces);
-  k->stats.device_bytes = collate_bytes(k);
+  note_peak(k);
 
   // push: the columns never leave the device; order_base = the piece's offset in collated order
   CK(cudaEventRecord(k->ev[4], c->stream));
@@ -2165,6 +2382,243 @@ int collate_push(ecb_collate* k, int64_t* n_reads) {
   return ECB_OK;
 }
 
+// ---- collation after a spill (DESIGN.md section 6.2): names per group, order once, layout per chunk, push per piece
+// 1. names: the rows of a group of fine buckets go up (keys and positions), the group's name table marks the global
+//    bitmap, and the group's reads (first position, alignments) and every row's read's first position come back.
+int spilled_names(ecb_collate* k, std::vector<uint2>& reads) {
+  ecb_ctx* c = k->c;
+  const u64 n = k->n;
+  const size_t words = (size_t)(n / 32) + 1;
+  const int64_t avail = k->budget - (int64_t)round256(words * 4);
+  if (avail <= 0)
+    return fail(c, ECB_ERR_LIMIT, "the collate budget of %lld bytes cannot hold the bitmap of %llu alignments (%llu bytes)",
+                (long long)k->budget, (unsigned long long)n, (unsigned long long)round256(words * 4));
+  // groups of consecutive buckets whose names pass fits next to the bitmap
+  std::vector<u64> rows(COLLATE_BUCKETS, 0);
+  for (const CollateSpill& sp : k->spills)
+    for (u32 b = 0; b < COLLATE_BUCKETS; ++b) rows[b] += sp.offs[b + 1] - sp.offs[b];
+  std::vector<u32> bounds{0};
+  u64 g = 0;
+  for (u32 b = 0; b < COLLATE_BUCKETS; ++b) {
+    if (names_pass_bytes(rows[b]) > (u64)avail)
+      return fail(c, ECB_ERR_LIMIT, "a name bucket of %llu alignments does not fit the collate budget of %lld bytes",
+                  (unsigned long long)rows[b], (long long)k->budget);
+    if (g > 0 && names_pass_bytes(g + rows[b]) > (u64)avail) {
+      bounds.push_back(b);
+      g = 0;
+    }
+    g += rows[b];
+  }
+  bounds.push_back(COLLATE_BUCKETS);
+  k->stats.groups = (int64_t)bounds.size() - 1;
+
+  CKR(need(k, k->bitmap, words * 4));
+  CK(cudaMemsetAsync(k->bitmap.p, 0, words * 4, c->stream));
+  for (size_t gi = 0; gi + 1 < bounds.size(); ++gi) {
+    const u32 b0 = bounds[gi], b1 = bounds[gi + 1];
+    u64 m = 0;
+    for (const CollateSpill& sp : k->spills) m += sp.offs[b1] - sp.offs[b0];
+    if (m == 0) continue;
+    CKR(need(k, k->key_lo, (size_t)m * 8));
+    CKR(need(k, k->key_hi, (size_t)m * 8));
+    CKR(need(k, k->pos, (size_t)m * 4));
+    CKR(need(k, k->list, (size_t)m * 8));
+    // spill after spill: the rows of one name stay in file order
+    u64 off = 0;
+    for (const CollateSpill& sp : k->spills) {
+      const u64 a = sp.offs[b0], e = sp.offs[b1];
+      if (e == a) continue;
+      CKR(ring_h2d(k, (u64*)k->key_lo.p + off, sp.lo.get() + a, (e - a) * 8));
+      CKR(ring_h2d(k, (u64*)k->key_hi.p + off, sp.hi.get() + a, (e - a) * 8));
+      CKR(ring_h2d(k, (u32*)k->pos.p + off, sp.pos.get() + a, (e - a) * 4));
+      off += e - a;
+    }
+    CKR(collate_table(k, (const u64*)k->key_lo.p, (const u64*)k->key_hi.p, (const u32*)k->pos.p, m, group_slots(m), true));
+    const u32 group_reads = c->h_ctr->scratch[0];
+    const int g_slots = grid_for(k->slots, 256, c->sm_count * 8);
+    ecb_collate_mark_kernel<<<g_slots, 256, 0, c->stream>>>((const EcbEntry*)k->table.p, k->slots, (u32*)k->bitmap.p);
+    LAUNCH_CHECK("collate_mark");
+    CK(cudaMemsetAsync(&c->d_ctr->scratch[2], 0, sizeof(u32), c->stream));
+    ecb_collate_list_kernel<<<g_slots, 256, 0, c->stream>>>((const EcbEntry*)k->table.p, k->slots, (uint2*)k->list.p,
+                                                            &c->d_ctr->scratch[2]);
+    LAUNCH_CHECK("collate_list");
+    ecb_collate_first_kernel<<<grid_for(m, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+        (const u32*)k->slot_of.p, (const EcbEntry*)k->table.p, m, (u32*)k->pos.p);
+    LAUNCH_CHECK("collate_first");
+    const size_t r0 = reads.size();
+    reads.resize(r0 + group_reads);
+    note_host(k, (int64_t)group_reads * 8);
+    CKR(ring_d2h(k, reads.data() + r0, k->list.p, (size_t)group_reads * 8));
+    off = 0;
+    for (CollateSpill& sp : k->spills) {
+      const u64 a = sp.offs[b0], e = sp.offs[b1];
+      if (e == a) continue;
+      CKR(ring_d2h(k, sp.pos.get() + a, (const u32*)k->pos.p + off, (e - a) * 4));
+      off += e - a;
+    }
+  }
+  for (CollateSpill& sp : k->spills) {   // the keys are done with
+    sp.lo.reset();
+    sp.hi.reset();
+    note_host(k, -(int64_t)(16 * sp.m));
+  }
+  DevBuf* done[] = {&k->key_lo, &k->key_hi, &k->pos, &k->list, &k->slot_of, &k->table};
+  for (DevBuf* b : done) release(c, *b);
+  return ECB_OK;
+}
+
+int collate_push_spilled(ecb_collate* k, int64_t* n_reads) {
+  ecb_ctx* c = k->c;
+  const u64 n = k->n;
+  *n_reads = 0;
+  CKR(collate_spill(k));   // the rows still in the staging area
+  DevBuf* staged[] = {&k->key_lo, &k->key_hi, &k->tg_in, &k->hp_in, &k->o_lo, &k->o_hi, &k->o_tg, &k->o_hp, &k->o_pos,
+                      &k->part_counts};
+  for (DevBuf* b : staged) release(c, *b);
+  float ms = 0;
+  CK(cudaEventRecord(k->ev[0], c->stream));
+
+  // 1. names
+  std::vector<uint2> reads;
+  CKR(spilled_names(k, reads));
+  const u64 R = reads.size();
+  k->stats.reads = (int64_t)R;
+  CK(cudaEventRecord(k->ev[1], c->stream));
+
+  // 2. order: word ranks of the bitmap, alignments per read id from the read lists, read offsets, piece cuts
+  const size_t words = (size_t)(n / 32) + 1;
+  const int64_t global = (int64_t)(round256(words * 4) * 2 + round256(R * 4) + round256((R + 1) * 4));
+  if (global + 2 * 256 >= k->budget)
+    return fail(c, ECB_ERR_LIMIT, "the collate budget of %lld bytes cannot hold the read order of %llu alignments in %llu "
+                "reads (%lld bytes)", (long long)k->budget, (unsigned long long)n, (unsigned long long)R, (long long)global);
+  CKR(need(k, k->word_rank, words * 4));
+  CKR(device_scan<true>(c, (const u32*)k->bitmap.p, (u32*)k->word_rank.p, words, 0, nullptr));
+  CKR(need(k, k->count, (size_t)R * 4));
+  CKR(need(k, k->cursor, (size_t)(R + 1) * 4));
+  const u64 per_upload = std::max<u64>(1, std::min<u64>(R, (u64)(k->budget - global - 256) / 8));
+  CKR(need(k, k->list, (size_t)per_upload * 8));
+  for (u64 a = 0; a < R; a += per_upload) {
+    const u64 len = std::min(per_upload, R - a);
+    CKR(ring_h2d(k, k->list.p, reads.data() + a, len * 8));
+    ecb_collate_list_ids_kernel<<<grid_for(len, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+        (const uint2*)k->list.p, len, (const u32*)k->bitmap.p, (const u32*)k->word_rank.p, (u32*)k->count.p);
+    LAUNCH_CHECK("collate_list_ids");
+  }
+  release(c, k->list);
+  std::vector<uint2>().swap(reads);
+  note_host(k, -(int64_t)R * 8);
+  u64 total = 0;
+  CKR(device_scan<false>(c, (const u32*)k->count.p, (u32*)k->cursor.p, R, 0, &total));
+  if (total != n) return fail(c, ECB_ERR_INVALID, "collation lost alignments (%llu of %llu placed)", (unsigned long long)total,
+                              (unsigned long long)n);
+  const u32 n32 = (u32)n;   // cursor[R] = n: cursor + 1 are the read ends
+  CK(cudaMemcpyAsync((u32*)k->cursor.p + R, &n32, 4, cudaMemcpyHostToDevice, c->stream));
+  // a piece's columns and its upload area (28 B per alignment) fit the budget; at most COLLATE_MAX_PARTS pieces
+  const u64 fit = (u64)std::max<int64_t>(1, (k->budget - 8 * 256) / 28);
+  const u64 piece = std::min<u64>(c->opt_collate_piece > 0 ? (u64)c->opt_collate_piece : (u64)ECB_PUSH_LIMIT, fit);
+  const size_t max_cuts = (size_t)(2 * (n / piece) + 4);
+  if (max_cuts > COLLATE_MAX_PARTS)
+    return fail(c, ECB_ERR_LIMIT, "pieces of %llu alignments cut %llu alignments into more than %d pieces (collate budget "
+                "%lld bytes)", (unsigned long long)piece, (unsigned long long)n, COLLATE_MAX_PARTS, (long long)k->budget);
+  CKR(need(k, k->cuts, (max_cuts + 2) * 4));
+  ecb_collate_cuts_kernel<<<1, 32, 0, c->stream>>>((const u32*)k->cursor.p + 1, (u32)R, n, piece, (u32*)k->cuts.p);
+  LAUNCH_CHECK("collate_cuts");
+  std::vector<u32> cuts(max_cuts + 2);
+  CK(cudaMemcpyAsync(cuts.data(), k->cuts.p, cuts.size() * 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  k->stats.d2h_bytes += (int64_t)cuts.size() * 4;
+  const u32 pieces = cuts[0];
+  if (pieces == 0 || pieces > max_cuts || cuts[1 + pieces] != n)
+    return fail(c, ECB_ERR_INVALID, "collation cut %u pieces", pieces);
+  CK(cudaEventRecord(k->ev[2], c->stream));
+
+  // 3. layout: every row takes its read id and its place in collated order, and the rows are partitioned by piece
+  const int64_t fixed = global + (int64_t)round256((max_cuts + 2) * 4) + 4 * (int64_t)pieces + 10 * 256;
+  const int64_t per_row = 32 + (4 * (int64_t)pieces + COLLATE_TILE - 1) / COLLATE_TILE;
+  const u64 chunk = (u64)std::max<int64_t>(0, (k->budget - fixed) / per_row);
+  if (chunk == 0)
+    return fail(c, ECB_ERR_LIMIT, "the collate budget of %lld bytes cannot hold the read order and a layout chunk",
+                (long long)k->budget);
+  for (CollateSpill& sp : k->spills) {
+    for (u64 a = 0; a < sp.m; a += chunk) {
+      const u64 m = std::min(chunk, sp.m - a);
+      DevBuf* cols[] = {&k->tg_in, &k->hp_in, &k->pos, &k->idv, &k->o_tg, &k->o_hp, &k->o_pos, &k->o_id};
+      for (DevBuf* b : cols) CKR(need(k, *b, (size_t)m * 4));
+      CKR(ring_h2d(k, k->tg_in.p, sp.tg.get() + a, m * 4));
+      CKR(ring_h2d(k, k->hp_in.p, sp.hp.get() + a, m * 4));
+      CKR(ring_h2d(k, k->pos.p, sp.pos.get() + a, m * 4));
+      ecb_collate_place_kernel<<<grid_for(m, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+          (u32*)k->pos.p, m, (const u32*)k->bitmap.p, (const u32*)k->word_rank.p, (u32*)k->cursor.p, (u32*)k->idv.p);
+      LAUNCH_CHECK("collate_place");
+      PiecePart P{(const u32*)k->idv.p, (const u32*)k->pos.p, (const int32_t*)k->tg_in.p, (const int32_t*)k->hp_in.p,
+                  (const u32*)k->cuts.p + 1, pieces, (u32*)k->o_id.p, (u32*)k->o_pos.p, (int32_t*)k->o_tg.p,
+                  (int32_t*)k->o_hp.p};
+      CollateChunk ch;
+      CKR(partition(k, P, m, pieces, ch.offs));
+      ch.id.reset(new u32[m]);
+      ch.place.reset(new u32[m]);
+      ch.tg.reset(new int32_t[m]);
+      ch.hp.reset(new int32_t[m]);
+      note_host(k, (int64_t)(16 * m + ch.offs.size() * 4));
+      CKR(ring_d2h(k, ch.id.get(), k->o_id.p, m * 4));
+      CKR(ring_d2h(k, ch.place.get(), k->o_pos.p, m * 4));
+      CKR(ring_d2h(k, ch.tg.get(), k->o_tg.p, m * 4));
+      CKR(ring_d2h(k, ch.hp.get(), k->o_hp.p, m * 4));
+      k->chunks.push_back(std::move(ch));
+    }
+    sp.tg.reset();
+    sp.hp.reset();
+    sp.pos.reset();
+    note_host(k, -(int64_t)(12 * sp.m + sp.offs.size() * 4));
+  }
+  k->spills.clear();
+  {
+    DevBuf* done[] = {&k->bitmap, &k->word_rank, &k->count, &k->cursor, &k->cuts, &k->tg_in, &k->hp_in, &k->pos,
+                      &k->idv, &k->o_tg, &k->o_hp, &k->o_pos, &k->o_id, &k->part_counts};
+    for (DevBuf* b : done) release(c, *b);
+  }
+  CK(cudaEventRecord(k->ev[3], c->stream));
+
+  // 4. push: per piece, every chunk's rows of the piece go up and land at place - piece start
+  u64 longest = 0;
+  for (u32 j = 0; j < pieces; ++j) longest = std::max<u64>(longest, cuts[2 + j] - cuts[1 + j]);
+  const u64 upload = std::max<u64>(1, std::min(longest, piece));
+  CKR(need(k, k->rg, (size_t)longest * 4));
+  CKR(need(k, k->tg, (size_t)longest * 4));
+  CKR(need(k, k->hp, (size_t)longest * 4));
+  DevBuf* up[] = {&k->idv, &k->tg_in, &k->hp_in, &k->pos};
+  for (DevBuf* b : up) CKR(need(k, *b, (size_t)upload * 4));
+  for (u32 j = 0; j < pieces; ++j) {
+    const u64 a = cuts[1 + j], b = cuts[2 + j];
+    for (const CollateChunk& ch : k->chunks) {
+      for (u64 s = ch.offs[j]; s < ch.offs[j + 1]; s += upload) {
+        const u64 m = std::min<u64>(upload, ch.offs[j + 1] - s);
+        CKR(ring_h2d(k, k->idv.p, ch.id.get() + s, m * 4));
+        CKR(ring_h2d(k, k->tg_in.p, ch.tg.get() + s, m * 4));
+        CKR(ring_h2d(k, k->hp_in.p, ch.hp.get() + s, m * 4));
+        CKR(ring_h2d(k, k->pos.p, ch.place.get() + s, m * 4));
+        ecb_collate_piece_kernel<<<grid_for(m, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+            (const u32*)k->idv.p, (const int32_t*)k->tg_in.p, (const int32_t*)k->hp_in.p, (const u32*)k->pos.p, m, (u32)a,
+            (int32_t*)k->rg.p, (int32_t*)k->tg.p, (int32_t*)k->hp.p);
+        LAUNCH_CHECK("collate_piece");
+      }
+    }
+    CKR(ecb_push(c, (const int32_t*)k->rg.p, (const int32_t*)k->tg.p, (const int32_t*)k->hp.p, nullptr, (int64_t)(b - a),
+                 (int64_t)a, 0, 1));
+    k->stats.pieces++;
+  }
+  CK(cudaEventRecord(k->ev[4], c->stream));
+  CK(cudaEventSynchronize(k->ev[4]));
+  for (const CollateChunk& ch : k->chunks) note_host(k, -(int64_t)(16 * (u64)ch.offs.back() + ch.offs.size() * 4));
+  k->chunks.clear();
+  CK(cudaEventElapsedTime(&ms, k->ev[0], k->ev[1])); k->stats.table_ms = ms;
+  CK(cudaEventElapsedTime(&ms, k->ev[1], k->ev[2])); k->stats.order_ms = ms;
+  CK(cudaEventElapsedTime(&ms, k->ev[2], k->ev[3])); k->stats.layout_ms = ms;
+  CK(cudaEventElapsedTime(&ms, k->ev[3], k->ev[4])); k->stats.push_ms = ms;
+  *n_reads = (int64_t)R;
+  return ECB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -2174,8 +2628,12 @@ int ecb_collate_create(ecb_ctx* c, ecb_collate** out) {
   *out = nullptr;
   if (c->with_cells) return fail(c, ECB_ERR_INVALID, "collation covers the single-sample path only");
   CK(cudaSetDevice(c->device));
+  size_t free_bytes = 0, total_bytes = 0;
+  CK(cudaMemGetInfo(&free_bytes, &total_bytes));
   ecb_collate* k = new ecb_collate();
   k->c = c;
+  // automatic: half the free memory, the other half is left to the context's EC table and results
+  k->budget = c->opt_collate_budget > 0 ? c->opt_collate_budget : (int64_t)(free_bytes / 2);
   for (auto& e : k->ev)
     if (cudaEventCreate(&e) != cudaSuccess) {
       collate_release(k);
@@ -2196,16 +2654,33 @@ int ecb_collate_add(ecb_collate* k, const uint64_t* key_lo, const uint64_t* key_
   if (k->n + (u64)n >= 0xFFFFFFFFull) return fail(c, ECB_ERR_LIMIT, "a collator takes fewer than 2^32 - 1 alignments");
   CK(cudaSetDevice(c->device));
   const u64 total = k->n + (u64)n;
-  CKR(ensure(c, k->key_lo, (size_t)total * 8, true));
-  CKR(ensure(c, k->key_hi, (size_t)total * 8, true));
-  CKR(ensure(c, k->tg_in, (size_t)total * 4, true));
-  CKR(ensure(c, k->hp_in, (size_t)total * 4, true));
   const cudaMemcpyKind kind = on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+  if (!k->spilling && one_pass_bytes(c, total) > (u64)k->budget) CKR(collate_start_spilling(k));
+  if (!k->spilling) {
+    CKR(ensure(c, k->key_lo, (size_t)total * 8, true));
+    CKR(ensure(c, k->key_hi, (size_t)total * 8, true));
+    CKR(ensure(c, k->tg_in, (size_t)total * 4, true));
+    CKR(ensure(c, k->hp_in, (size_t)total * 4, true));
+  }
   CK(cudaEventRecord(k->ev[0], c->stream));
-  CK(cudaMemcpyAsync((u64*)k->key_lo.p + k->n, key_lo, (size_t)n * 8, kind, c->stream));
-  CK(cudaMemcpyAsync((u64*)k->key_hi.p + k->n, key_hi, (size_t)n * 8, kind, c->stream));
-  CK(cudaMemcpyAsync((int32_t*)k->tg_in.p + k->n, target_idx, (size_t)n * 4, kind, c->stream));
-  CK(cudaMemcpyAsync((int32_t*)k->hp_in.p + k->n, hap_idx, (size_t)n * 4, kind, c->stream));
+  if (!k->spilling) {
+    CK(cudaMemcpyAsync((u64*)k->key_lo.p + k->n, key_lo, (size_t)n * 8, kind, c->stream));
+    CK(cudaMemcpyAsync((u64*)k->key_hi.p + k->n, key_hi, (size_t)n * 8, kind, c->stream));
+    CK(cudaMemcpyAsync((int32_t*)k->tg_in.p + k->n, target_idx, (size_t)n * 4, kind, c->stream));
+    CK(cudaMemcpyAsync((int32_t*)k->hp_in.p + k->n, hap_idx, (size_t)n * 4, kind, c->stream));
+  } else {
+    // the staging area takes what it can; a full one spills
+    for (u64 done = 0; done < (u64)n;) {
+      if (k->res == k->stage) CKR(collate_spill(k));
+      const u64 r = std::min<u64>((u64)n - done, k->stage - k->res);
+      CK(cudaMemcpyAsync((u64*)k->key_lo.p + k->res, key_lo + done, (size_t)r * 8, kind, c->stream));
+      CK(cudaMemcpyAsync((u64*)k->key_hi.p + k->res, key_hi + done, (size_t)r * 8, kind, c->stream));
+      CK(cudaMemcpyAsync((int32_t*)k->tg_in.p + k->res, target_idx + done, (size_t)r * 4, kind, c->stream));
+      CK(cudaMemcpyAsync((int32_t*)k->hp_in.p + k->res, hap_idx + done, (size_t)r * 4, kind, c->stream));
+      k->res += r;
+      done += r;
+    }
+  }
   CK(cudaEventRecord(k->ev[1], c->stream));
   CK(cudaEventSynchronize(k->ev[1]));   // the caller's buffers are free again
   float ms = 0;
@@ -2214,6 +2689,7 @@ int ecb_collate_add(ecb_collate* k, const uint64_t* key_lo, const uint64_t* key_
   if (!on_device) k->stats.h2d_bytes += n * 24;
   k->n = total;
   k->stats.alignments = (int64_t)total;
+  note_peak(k);
   return ECB_OK;
 }
 
@@ -2223,7 +2699,7 @@ int ecb_collate_push(ecb_collate* k, int64_t* n_reads) {
   ecb_ctx* c = k->c;
   k->pushed = true;
   CK(cudaSetDevice(c->device));
-  return collate_push(k, n_reads);
+  return k->spilling ? collate_push_spilled(k, n_reads) : collate_push(k, n_reads);
 }
 
 int ecb_collate_get_stats(const ecb_collate* k, ecb_collate_stats* out) {

@@ -135,6 +135,19 @@ def collate_mode(collate=None):
     return value == "1"
 
 
+def collate_budget():
+    """Device bytes a collator may hold, from the environment variable ALNTOOLS_B200_COLLATE_BUDGET (a non-negative
+    integer; unset or 0: automatic, half of the GPU's free memory).  A collation whose rows do not fit spills them to
+    host memory and works in passes; the outputs do not depend on it.  On a shared GPU it caps what a job takes."""
+    import os
+    value = os.environ.get("ALNTOOLS_B200_COLLATE_BUDGET", "").strip()
+    if not value:
+        return 0
+    if not (value.isascii() and value.isdigit()):
+        raise ValueError("ALNTOOLS_B200_COLLATE_BUDGET must be a non-negative integer (bytes), not %r" % (value,))
+    return int(value)
+
+
 Mode = collections.namedtuple("Mode", ["python", "decode", "collate", "launcher", "gpus"])
 
 

@@ -71,6 +71,9 @@ enum ecb_option {
   ECB_OPT_COLLATE_SLOTS = 10,   /* initial slots of a collator's name table (0 = automatic: 1.5 x the alignments
                                    added, rounded up to a power of two); the table grows when it runs out of probes */
   ECB_OPT_COLLATE_PIECE = 11,   /* most alignments one push of a collator carries (0 = the push limit, 2^31 - 8192) */
+  ECB_OPT_COLLATE_BUDGET = 12,  /* device bytes a collator may hold, read at ecb_collate_create (0 = automatic: half
+                                   of the device's free memory at that moment, the rest is left to the context's EC
+                                   table and results; since version 2004) */
 };
 
 typedef struct ecb_result {
@@ -335,8 +338,17 @@ int ecb_bam_destroy(ecb_bam* d);
  *   on_device = 1, order_base = offset in collated order, in pieces of at most ECB_OPT_COLLATE_PIECE alignments that
  *   end at read ends; a longer read is a piece of its own).  Once per collator; *n_reads = reads formed.  The
  *   context's limits apply: a read of more than ECB_MAX_READ_ALIGNMENTS alignments fails with ECB_ERR_LIMIT.
- * Device memory: 88 to 144 bytes per added alignment with the automatic table (DESIGN.md section 6.2), held until
- * ecb_collate_destroy.  Running out of it fails the call with ECB_ERR_CUDA and the allocator's message. */
+ * Device memory: while the one-pass collation of the alignments added so far fits the budget (ECB_OPT_COLLATE_BUDGET;
+ * 88 to 144 bytes per alignment with the automatic table, DESIGN.md section 6.2), the rows stay on the device as above.
+ * An add that would pass it spills: the rows go to host memory (28 bytes per alignment), partitioned into 4096 buckets
+ * by name key, and from then on the collator holds a fixed staging area.  The push then works in passes over groups of
+ * buckets (names), once over all reads (order), over chunks of rows (layout) and over pieces (push), each within the
+ * budget.  The outputs do not depend on the budget.  A budget that cannot hold the staging area, the bitmap over all
+ * alignments with the per-read counts and offsets (n/4 + 8 bytes per read), or one bucket's names pass fails with
+ * ECB_ERR_LIMIT and a message naming the budget; so does a ECB_OPT_COLLATE_PIECE that cuts a spilled collation into
+ * more than 4096 pieces.  A piece holds at least one read, and a name table that runs out of probes grows, so those
+ * two may pass the budget by what they need.  Running out of device memory otherwise fails with ECB_ERR_CUDA and the
+ * allocator's message. */
 typedef struct ecb_collate ecb_collate;
 typedef struct ecb_collate_stats {
   int64_t alignments;      /* added                                                                            */
@@ -344,13 +356,19 @@ typedef struct ecb_collate_stats {
   int64_t table_slots;     /* name table slots at the end                                                      */
   int64_t table_grows;     /* times the name table was replaced by a larger one                                */
   int64_t pieces;          /* pushes into the context                                                          */
-  int64_t device_bytes;    /* device memory held by the collator after the layout                              */
-  int64_t h2d_bytes;       /* bytes the add calls copied host->device                                          */
-  double add_ms;           /* stream time of the add copies, summed                                            */
+  int64_t device_bytes;    /* peak device memory held by the collator                                          */
+  int64_t h2d_bytes;       /* bytes copied host->device: the add calls, and after a spill the passes           */
+  double add_ms;           /* stream time of the add copies (and the spills inside them), summed               */
   double table_ms;         /* name table, growth included                                                      */
   double order_ms;         /* bitmap, ranks, read ids and offsets (with one host round trip)                   */
   double layout_ms;        /* scatter to collated order and the piece cuts (with one host round trip)          */
   double push_ms;          /* the pushes into the context                                                      */
+  /* since version 2004; after a spill table_ms, order_ms, layout_ms and push_ms time the four passes */
+  int64_t spills;          /* times the staging area went to host memory (0: the one-pass collation ran)       */
+  int64_t groups;          /* groups of name buckets of the names pass                                         */
+  int64_t host_bytes;      /* peak host memory holding spilled rows                                            */
+  int64_t d2h_bytes;       /* bytes copied device->host                                                        */
+  double spill_ms;         /* wall time of the spills, summed                                                  */
 } ecb_collate_stats;
 int ecb_collate_create(ecb_ctx* ctx, ecb_collate** out);
 int ecb_collate_add(ecb_collate* c, const uint64_t* key_lo, const uint64_t* key_hi, const int32_t* target_idx,
