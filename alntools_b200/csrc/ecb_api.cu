@@ -187,13 +187,19 @@ int check_device_error(ecb_ctx* c) {
   return fail(c, ECB_ERR_LIMIT, "device error bits 0x%x", e);
 }
 
+// Device address of the total of a device_scan over n items, valid until the next scan: a copy of it enqueued
+// after the scan reads it without a synchronisation of its own.
+const u64* scan_total(const ecb_ctx* c, u64 n) {
+  return (const u64*)c->scan_partials.p + (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
+}
+
 // Device-wide exclusive scan (in may alias out).  total_out (host) may be NULL.
 template <bool POPC>
 int device_scan(ecb_ctx* c, const u32* in, u32* out, u64 n, u32 base_offset, u64* total_out) {
   const u32 n_blocks = (u32)((n + SCAN_BLOCK - 1) / SCAN_BLOCK);
   CKR(ensure(c, c->scan_partials, ((size_t)n_blocks + 2) * sizeof(u64)));
   u64* partials = (u64*)c->scan_partials.p;
-  u64* d_total = partials + n_blocks;
+  u64* d_total = (u64*)scan_total(c, n);
   if (n_blocks == 0) {
     if (total_out) *total_out = 0;
     return ECB_OK;
@@ -902,8 +908,7 @@ int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
     // single sample: every EC is kept, so E is known; the count of first-occurrence bits is checked against it
     // when the one round trip of this call brings it back (it differs when order_base ranges overlapped)
     CKR(device_scan<true>(c, F.bitmap, (u32*)c->word_rank.p, words, 0, nullptr));
-    const u32 n_blocks = (u32)((words + SCAN_BLOCK - 1) / SCAN_BLOCK);
-    CK(cudaMemcpyAsync(c->h_total + 1, (const u64*)c->scan_partials.p + n_blocks, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(c->h_total + 1, scan_total(c, words), sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
   }
   const u64 E = n_kept;
   if (E + 1 > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "more than 2^31 equivalence classes");
@@ -924,11 +929,8 @@ int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
   // row lengths -> indptr; the rows follow at once: the arena's fill (known on the host since the last push)
   // bounds the number of non-zeros, so the result arrays need not wait for the exact figure
   CKR(device_scan<false>(c, (const u32*)c->r_a_indptr.p, (u32*)c->r_a_indptr.p, E + 1, 0, nullptr));
-  {
-    const u32 n_blocks = (u32)((E + 1 + SCAN_BLOCK - 1) / SCAN_BLOCK);
-    CK(cudaMemcpyAsync(c->h_total, (const u64*)c->scan_partials.p + n_blocks, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
-    c->stats.d2h_bytes += 2 * sizeof(u64);
-  }
+  CK(cudaMemcpyAsync(c->h_total, scan_total(c, E + 1), sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+  c->stats.d2h_bytes += 2 * sizeof(u64);
   const u64 z_bound = std::max<u64>(c->arena_used, 1);
   if (z_bound > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "A matrix may have more than 2^31-1 non-zeros");
   CKR(ensure(c, c->r_a_indices, z_bound * 4));
@@ -1061,14 +1063,38 @@ int ecb_rebase(ecb_ctx* c, int64_t delta) {
   return ECB_OK;
 }
 
-int ecb_arena_create(ecb_ctx* c, int64_t cap_records, void* ipc_handle_out, void** base_out) {
-  if (!c || cap_records < 1 || !base_out) return ECB_ERR_INVALID;
-  if (c->xa_base) return fail(c, ECB_ERR_STATE, "this context already has an arena");
-  CK(cudaSetDevice(c->device));
-  const size_t bytes = ECB_ARENA_HEADER_BYTES + (size_t)cap_records * ECB_KEYREC_WORDS * 8;
-  CK(cudaMalloc(&c->xa_base, bytes));
-  CK(cudaMemset(c->xa_base, 0, ECB_ARENA_HEADER_BYTES));
-  c->xa_cap_ec = cap_records;
+// ---- the exchange over peer memory (see include/ecb200.h and ecb_exchange.cuh) ------------------------------
+
+// An exchange arena: [header | cap_ec EC records | header | cap_pairs pair records], each header {records, unused,
+// overflow}.  A single-sample arena (ecb_arena_create) has no pair part.  Its capacity counts 32-byte dispatch-1
+// records, and the 24-byte records of dispatch 2 share that space; the per-cell capacities count the records of the
+// dispatch at hand (the caller sizes them from exact counts).
+struct ArenaLayout {
+  char* base;
+  int64_t cap_ec, cap_pairs;
+  unsigned long long* ec_hdr() const { return (unsigned long long*)base; }
+  unsigned long long* ec_rec() const { return (unsigned long long*)(base + ECB_ARENA_HEADER_BYTES); }
+  unsigned long long* pair_hdr() const { return ec_rec() + (size_t)cap_ec * ECB_KEYREC_WORDS; }
+  unsigned long long* pair_rec() const { return pair_hdr() + ECB_ARENA_HEADER_BYTES / 8; }
+  size_t bytes() const {
+    return ECB_ARENA_HEADER_BYTES + (size_t)cap_ec * ECB_KEYREC_WORDS * 8 +
+           (cap_pairs ? ECB_ARENA_HEADER_BYTES + (size_t)cap_pairs * ECB_CPAIR1_WORDS * 8 : 0);
+  }
+  // 8-byte words of each record area, as the dispatch kernels' overflow test counts them (order: dispatch 2)
+  u64 ec_words(bool order) const { return (u64)cap_ec * (order && cap_pairs ? ECB_ORDREC_WORDS : ECB_KEYREC_WORDS); }
+  u64 pair_words(bool order) const { return (u64)cap_pairs * (order ? ECB_CPAIR2_WORDS : ECB_CPAIR1_WORDS); }
+};
+
+static ArenaLayout arena_of(const ecb_ctx* c) { return ArenaLayout{(char*)c->xa_base, c->xa_cap_ec, c->xa_cap_pairs}; }
+
+// The arena of an owner context: plain cudaMalloc (exportable through CUDA IPC), headers cleared.
+static int arena_alloc(ecb_ctx* c, int64_t cap_ec, int64_t cap_pairs, void* ipc_handle_out, void** base_out) {
+  CK(cudaMalloc(&c->xa_base, ArenaLayout{nullptr, cap_ec, cap_pairs}.bytes()));
+  c->xa_cap_ec = cap_ec;
+  c->xa_cap_pairs = cap_pairs;
+  const ArenaLayout L = arena_of(c);
+  CK(cudaMemset(L.ec_hdr(), 0, ECB_ARENA_HEADER_BYTES));
+  if (L.cap_pairs) CK(cudaMemset(L.pair_hdr(), 0, ECB_ARENA_HEADER_BYTES));
   if (ipc_handle_out) {
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handles are documented as 64 bytes");
     cudaIpcMemHandle_t h;
@@ -1079,79 +1105,88 @@ int ecb_arena_create(ecb_ctx* c, int64_t cap_records, void* ipc_handle_out, void
   return ECB_OK;
 }
 
-int ecb_arena_open_peer(ecb_ctx* c, const void* ipc_handle, void** base_out) {
-  if (!c || !ipc_handle || !base_out) return ECB_ERR_INVALID;
-  CK(cudaSetDevice(c->device));
-  cudaIpcMemHandle_t h;
-  memcpy(&h, ipc_handle, sizeof h);
-  void* p = nullptr;
-  CK(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
-  c->xa_opened.push_back(p);
-  *base_out = p;
-  return ECB_OK;
+// Both headers of this context's arena in one round trip: the records that arrived (n_pair = 0 without a pair
+// part), ECB_ERR_LIMIT when the last dispatch (order: dispatch 2) found the arena too small.
+static int arena_headers(ecb_ctx* c, bool order, u64* n_ec, u64* n_pair) {
+  const ArenaLayout L = arena_of(c);
+  unsigned long long h[6] = {0, 0, 0, 0, 0, 0};
+  CK(cudaMemcpyAsync(h, L.ec_hdr(), 3 * 8, cudaMemcpyDeviceToHost, c->stream));
+  if (L.cap_pairs) CK(cudaMemcpyAsync(h + 3, L.pair_hdr(), 3 * 8, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  *n_ec = h[0];
+  *n_pair = h[3];
+  const u64 rec_words = order ? ECB_ORDREC_WORDS : ECB_KEYREC_WORDS;
+  if (!h[2] && !h[5] && h[0] * rec_words <= L.ec_words(order) && h[3] <= (u64)L.cap_pairs) return ECB_OK;
+  if (L.cap_pairs)
+    return fail(c, ECB_ERR_LIMIT, "exchange arena too small: %llu ECs and %llu pairs arrived, capacity %lld and %lld", h[0],
+                h[3], (long long)L.cap_ec, (long long)L.cap_pairs);
+  if (order) return fail(c, ECB_ERR_LIMIT, "exchange arena too small for the second dispatch");
+  return fail(c, ECB_ERR_LIMIT, "exchange arena too small: %llu records arrived, capacity %lld", h[0], (long long)L.cap_ec);
 }
 
-int ecb_arena_reset(ecb_ctx* c) {
-  if (!c || !c->xa_base) return ECB_ERR_INVALID;
-  CK(cudaSetDevice(c->device));
-  CK(cudaMemsetAsync(c->xa_base, 0, ECB_ARENA_HEADER_BYTES, c->stream));
-  if (c->xa_cap_pairs)   // the pair area's header
-    CK(cudaMemsetAsync((char*)c->xa_base + ECB_ARENA_HEADER_BYTES + (size_t)c->xa_cap_ec * ECB_KEYREC_WORDS * 8, 0,
-                       ECB_ARENA_HEADER_BYTES, c->stream));
-  // on a caller-provided stream (ecb_set_stream) the call is stream-ordered - a collective on that stream is the
-  // barrier in front of the peers' stores; a context on its own stream synchronises
-  if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));
-  return ECB_OK;
-}
-
-static int arena_targets(ecb_ctx* c, ArenaTargets* A, int world, void* const* bases, int64_t cap_records) {
+// Every rank's arena as seen from this process, as targets of a dispatch (order: dispatch 2): the EC areas, and the
+// pair areas of per-cell arenas (cap_pairs > 0) when P is given.
+static int arena_targets(ecb_ctx* c, int world, void* const* bases, int64_t cap_ec, int64_t cap_pairs, bool order,
+                         ArenaTargets* E, ArenaTargets* P = nullptr) {
   for (int r = 0; r < world; ++r) {
     if (!bases[r]) return fail(c, ECB_ERR_INVALID, "arena base of rank %d is NULL", r);
-    char* b = (char*)bases[r];
-    A->hdr[r] = (unsigned long long*)b;
-    A->rec[r] = (unsigned long long*)(b + ECB_ARENA_HEADER_BYTES);
+    const ArenaLayout L{(char*)bases[r], cap_ec, cap_pairs};
+    E->hdr[r] = L.ec_hdr();
+    E->rec[r] = L.ec_rec();
+    if (P) {
+      P->hdr[r] = L.pair_hdr();
+      P->rec[r] = L.pair_rec();
+    }
   }
-  A->cap_words = (unsigned long long)cap_records * ECB_KEYREC_WORDS;
+  const ArenaLayout L{nullptr, cap_ec, cap_pairs};
+  E->cap_words = L.ec_words(order);
+  if (P) P->cap_words = L.pair_words(order);
   return ECB_OK;
 }
 
-int ecb_export_to_arenas(ecb_ctx* c, int world, void* const* arena_bases, int64_t cap_records, int64_t* min_base,
-                         int64_t* max_end) {
-  if (!c || !arena_bases || cap_records < 1) return ECB_ERR_INVALID;
-  if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
-  if (c->with_cells) return fail(c, ECB_ERR_INVALID, "the multi-GPU exchange covers the single-sample path only");
-  CK(cudaSetDevice(c->device));
-  if (!c->table_slots) CKR(init_table(c));
-  if (min_base) *min_base = c->n_ec ? (int64_t)c->min_base : 0;
-  if (max_end) *max_end = c->n_ec ? (int64_t)c->max_end : 0;
-  if (c->n_ec == 0) return ECB_OK;
-  KeyDispatchParams P{};
-  P.table = (const EcbEntry*)c->table.p;
-  P.ec_slot = (const u32*)c->ec_slot.p;
-  P.n_ec = c->n_ec;
-  P.world = (u32)world;
-  ArenaTargets A{};
-  CKR(arena_targets(c, &A, world, arena_bases, cap_records));
-  ecb_key_dispatch_kernel<false><<<grid_for(c->n_ec, 256, c->sm_count * 8), 256, 0, c->stream>>>(P, A);
-  LAUNCH_CHECK("export_to_arenas");
-  // remote stores are complete (and visible to the owner) when the kernel is.  On a caller-provided stream the
-  // caller's next collective on that stream is the barrier between the stores and the owner's merge - no host
-  // round trip here; a context on its own stream synchronises
-  if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));
+// Shards with alignments, by position, and the rank that holds each (dispatch 2); they must not overlap (one
+// read order over all ranks).
+static int shard_routes(ecb_ctx* c, int world, const int64_t* shard_lo, const int64_t* shard_hi, u64* lo, u32* dest,
+                        u32* n_shards) {
+  std::vector<int> order;
+  for (int r = 0; r < world; ++r)
+    if (shard_hi[r] > shard_lo[r]) order.push_back(r);
+  std::sort(order.begin(), order.end(), [&](int a, int b) { return shard_lo[a] < shard_lo[b]; });
+  if (order.empty()) return fail(c, ECB_ERR_STATE, "no rank has pushed alignments");
+  for (size_t k = 0; k < order.size(); ++k) {
+    if (k && shard_lo[order[k]] < shard_hi[order[k - 1]])
+      return fail(c, ECB_ERR_INVALID, "the ranks' order_base ranges overlap");
+    if (shard_hi[order[k]] - shard_lo[order[k]] > 0xFFFFFFFEll)
+      return fail(c, ECB_ERR_LIMIT, "a rank's alignments span more than 2^32 positions");
+    lo[k] = (u64)shard_lo[order[k]];
+    dest[k] = (u32)order[k];
+  }
+  *n_shards = (u32)order.size();
   return ECB_OK;
 }
 
-static int import_keys(ecb_ctx* c, const unsigned long long* rec, u64 n_rec);
+// The ECs of this context as a dispatch sends them: dispatch 1 (shard_lo NULL), or dispatch 2 with the routes of
+// the shards (when there is an EC to route).
+static int key_dispatch_params(ecb_ctx* c, int world, const int64_t* shard_lo, const int64_t* shard_hi,
+                               KeyDispatchParams* K) {
+  K->table = (const EcbEntry*)c->table.p;
+  K->ec_slot = (const u32*)c->ec_slot.p;
+  K->n_ec = c->table_slots ? c->n_ec : 0;
+  K->world = (u32)world;
+  if (shard_lo && K->n_ec) CKR(shard_routes(c, world, shard_lo, shard_hi, K->lo, K->dest, &K->n_shards));
+  return ECB_OK;
+}
 
-int ecb_import_arena(ecb_ctx* c) {
-  if (!c || !c->xa_base) return ECB_ERR_INVALID;
-  CK(cudaSetDevice(c->device));
-  unsigned long long hdr[3] = {0, 0, 0};
-  CK(cudaMemcpyAsync(hdr, c->xa_base, sizeof hdr, cudaMemcpyDeviceToHost, c->stream));
-  CK(cudaStreamSynchronize(c->stream));
-  if (hdr[2] || hdr[0] > (unsigned long long)c->xa_cap_ec)
-    return fail(c, ECB_ERR_LIMIT, "exchange arena too small: %llu records arrived, capacity %lld", hdr[0], (long long)c->xa_cap_ec);
-  return import_keys(c, (const unsigned long long*)((const char*)c->xa_base + ECB_ARENA_HEADER_BYTES), hdr[0]);
+// The EC records of a dispatch into the EC areas E (order: dispatch 2; kept_only: the per-cell dispatch 2, where
+// ECs without reads in kept cells stay behind).
+static int key_dispatch(ecb_ctx* c, const KeyDispatchParams& K, const ArenaTargets& E, bool order, bool kept_only,
+                        const char* name) {
+  const int g = grid_for(K.n_ec, 256, c->sm_count * 8);
+  if (!order) ecb_key_dispatch_kernel<false><<<g, 256, 0, c->stream>>>(K, E);
+  else if (!kept_only) ecb_key_dispatch_kernel<true><<<g, 256, 0, c->stream>>>(K, E);
+  else ecb_key_dispatch_kernel<true, true><<<g, 256, 0, c->stream>>>(K, E);
+  LAUNCH_CHECK(name);
+  return ECB_OK;
 }
 
 // Owner merge of n_rec dispatch-1 EC records (ecb_import_arena, ecb_cells_import_arena).
@@ -1177,25 +1212,128 @@ static int import_keys(ecb_ctx* c, const unsigned long long* rec, u64 n_rec) {
   return ECB_OK;
 }
 
-// Shards with alignments, by position, and the rank that holds each (dispatch 2); they must not overlap (one
-// read order over all ranks).
-static int shard_routes(ecb_ctx* c, int world, const int64_t* shard_lo, const int64_t* shard_hi, u64* lo, u32* dest,
-                        u32* n_shards) {
-  std::vector<int> order;
-  for (int r = 0; r < world; ++r)
-    if (shard_hi[r] > shard_lo[r]) order.push_back(r);
-  std::sort(order.begin(), order.end(), [&](int a, int b) { return shard_lo[a] < shard_lo[b]; });
-  if (order.empty()) return fail(c, ECB_ERR_STATE, "no rank has pushed alignments");
-  for (size_t k = 0; k < order.size(); ++k) {
-    if (k && shard_lo[order[k]] < shard_hi[order[k - 1]])
-      return fail(c, ECB_ERR_INVALID, "the ranks' order_base ranges overlap");
-    if (shard_hi[order[k]] - shard_lo[order[k]] > 0xFFFFFFFEll)
-      return fail(c, ECB_ERR_LIMIT, "a rank's alignments span more than 2^32 positions");
-    lo[k] = (u64)shard_lo[order[k]];
-    dest[k] = (u32)order[k];
-  }
-  *n_shards = (u32)order.size();
+// The flags of the second dispatch's slice build (ecb_order_mark_kernel, cells_pair_slice_kernel), after a
+// sync_counters.
+static int check_slice_flags(ecb_ctx* c) {
+  const u32 bad = c->h_ctr->scratch[5];
+  if (!bad) return ECB_OK;
+  return fail(c, ECB_ERR_INVALID, "second dispatch: %s",
+              (bad & 4u) ? "an EC arrived that the local context has never seen" : (bad & 2u) ? "two ECs share a first read"
+              : (bad & 1u) ? "a record outside the shard's positions arrived" : (bad & 8u) ? "a pair arrived without its EC"
+                           : "a pair's column is out of range");
+}
+
+// The A part of a slice (ecb_order_build, ecb_cells_order_build) from the n_rec dispatch-2 records at `rec`: an EC's
+// id in the slice is the rank of its bit in a bitmap over the shard's `span` positions, its row comes from the
+// LOCAL context.  Row lengths -> r_a_indptr, merged counts -> counts, rows -> r_a_indices / r_a_data, and *nnz.
+// The lens pass skips every record the mark pass flags; the rows kernel, which indexes with what the lens pass
+// wrote, runs only after one round trip has shown the flags clear and the non-zeros within int32.
+static int build_a_slice(ecb_ctx* c, const ecb_ctx* local, const unsigned long long* rec, u64 n_rec, u64 span,
+                         DevBuf& counts, u64* nnz) {
+  const u32 local_n_ec = local->table_slots ? local->n_ec : 0;
+  if (span > 0xFFFFFFFEull) return fail(c, ECB_ERR_LIMIT, "a rank's alignments span more than 2^32 positions");
+  if (n_rec > span) return fail(c, ECB_ERR_INVALID, "%llu ECs arrived for a shard of %llu positions", n_rec, span);
+  if (n_rec > local_n_ec) return fail(c, ECB_ERR_INVALID, "%llu ECs arrived but the local context holds %u", n_rec, local_n_ec);
+  if (n_rec + 1 > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "slice exceeds the int32 fields of the EC file");
+  const size_t words = (size_t)(span / 32) + 1;
+  CKR(ensure(c, c->bitmap, words * 4));
+  CKR(ensure(c, c->word_rank, words * 4));
+  CKR(ensure(c, c->r_a_indptr, (n_rec + 1) * 4));
+  CKR(ensure(c, counts, std::max<u64>(n_rec, 1) * 4));
+  CKR(ensure(c, c->first_rel, std::max<u64>(n_rec, 1) * 8));   // scratch: local id per record, then per slice id
+  // every row of the slice is a row of the local context: its arena fill bounds the non-zeros
+  const u64 z_bound = std::max<u64>(local->arena_used, 1);
+  CKR(ensure(c, c->r_a_indices, z_bound * 4));
+  CKR(ensure(c, c->r_a_data, z_bound * 4));
+  u32* lid_of_rec = (u32*)c->first_rel.p;
+  u32* lid_of_id = lid_of_rec + n_rec;
+  CK(cudaMemsetAsync(c->bitmap.p, 0, words * 4, c->stream));
+  CK(cudaMemsetAsync(c->r_a_indptr.p, 0, (n_rec + 1) * 4, c->stream));
+  CK(cudaMemsetAsync(&c->d_ctr->scratch[5], 0, sizeof(u32), c->stream));
+  *nnz = 0;
+  if (n_rec == 0) return ECB_OK;
+  const int g = grid_for(n_rec, 256, c->sm_count * 8);
+  ecb_order_mark_kernel<<<g, 256, 0, c->stream>>>(rec, (u32)n_rec, (u32)span, (const EcbEntry*)local->table.p,
+                                                  local->table_slots - 1, (u32*)c->bitmap.p, lid_of_rec, &c->d_ctr->scratch[5]);
+  LAUNCH_CHECK("order_mark");
+  CKR(device_scan<true>(c, (const u32*)c->bitmap.p, (u32*)c->word_rank.p, words, 0, nullptr));
+  ecb_order_lens_kernel<<<g, 256, 0, c->stream>>>(rec, (u32)n_rec, (u32)span, (const u32*)c->bitmap.p,
+                                                  (const u32*)c->word_rank.p, lid_of_rec, (const u32*)local->row_len.p,
+                                                  (int32_t*)c->r_a_indptr.p, (int32_t*)counts.p, lid_of_id);
+  LAUNCH_CHECK("order_lens");
+  CKR(device_scan<false>(c, (const u32*)c->r_a_indptr.p, (u32*)c->r_a_indptr.p, n_rec + 1, 0, nullptr));
+  CK(cudaMemcpyAsync(c->h_total, scan_total(c, n_rec + 1), sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+  c->stats.d2h_bytes += sizeof(u64);
+  CKR(sync_counters(c));
+  CKR(check_slice_flags(c));
+  *nnz = *c->h_total;
+  if (*nnz > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "slice exceeds the int32 fields of the EC file");
+  ecb_order_rows_kernel<<<grid_for(n_rec, 256, c->sm_count * 16), 256, 0, c->stream>>>(
+      lid_of_id, (const u32*)local->row_len.p, (const u32*)local->row_off.p, (const uint2*)local->arena.p,
+      (const int32_t*)c->r_a_indptr.p, (u32)n_rec, (int32_t*)c->r_a_indices.p, (int32_t*)c->r_a_data.p);
+  LAUNCH_CHECK("order_rows");
   return ECB_OK;
+}
+
+int ecb_arena_create(ecb_ctx* c, int64_t cap_records, void* ipc_handle_out, void** base_out) {
+  if (!c || cap_records < 1 || !base_out) return ECB_ERR_INVALID;
+  if (c->xa_base) return fail(c, ECB_ERR_STATE, "this context already has an arena");
+  CK(cudaSetDevice(c->device));
+  return arena_alloc(c, cap_records, 0, ipc_handle_out, base_out);
+}
+
+int ecb_arena_open_peer(ecb_ctx* c, const void* ipc_handle, void** base_out) {
+  if (!c || !ipc_handle || !base_out) return ECB_ERR_INVALID;
+  CK(cudaSetDevice(c->device));
+  cudaIpcMemHandle_t h;
+  memcpy(&h, ipc_handle, sizeof h);
+  void* p = nullptr;
+  CK(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
+  c->xa_opened.push_back(p);
+  *base_out = p;
+  return ECB_OK;
+}
+
+int ecb_arena_reset(ecb_ctx* c) {
+  if (!c || !c->xa_base) return ECB_ERR_INVALID;
+  CK(cudaSetDevice(c->device));
+  const ArenaLayout L = arena_of(c);
+  CK(cudaMemsetAsync(L.ec_hdr(), 0, ECB_ARENA_HEADER_BYTES, c->stream));
+  if (L.cap_pairs) CK(cudaMemsetAsync(L.pair_hdr(), 0, ECB_ARENA_HEADER_BYTES, c->stream));
+  // on a caller-provided stream (ecb_set_stream) the call is stream-ordered - a collective on that stream is the
+  // barrier in front of the peers' stores; a context on its own stream synchronises
+  if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));
+  return ECB_OK;
+}
+
+int ecb_export_to_arenas(ecb_ctx* c, int world, void* const* arena_bases, int64_t cap_records, int64_t* min_base,
+                         int64_t* max_end) {
+  if (!c || !arena_bases || cap_records < 1) return ECB_ERR_INVALID;
+  if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
+  if (c->with_cells) return fail(c, ECB_ERR_INVALID, "the multi-GPU exchange covers the single-sample path only");
+  CK(cudaSetDevice(c->device));
+  if (!c->table_slots) CKR(init_table(c));
+  if (min_base) *min_base = c->n_ec ? (int64_t)c->min_base : 0;
+  if (max_end) *max_end = c->n_ec ? (int64_t)c->max_end : 0;
+  if (c->n_ec == 0) return ECB_OK;
+  KeyDispatchParams K{};
+  ArenaTargets E{};
+  CKR(key_dispatch_params(c, world, nullptr, nullptr, &K));
+  CKR(arena_targets(c, world, arena_bases, cap_records, 0, false, &E));
+  CKR(key_dispatch(c, K, E, false, false, "export_to_arenas"));
+  // remote stores are complete (and visible to the owner) when the kernel is.  On a caller-provided stream the
+  // caller's next collective on that stream is the barrier between the stores and the owner's merge - no host
+  // round trip here; a context on its own stream synchronises
+  if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));
+  return ECB_OK;
+}
+
+int ecb_import_arena(ecb_ctx* c) {
+  if (!c || !c->xa_base) return ECB_ERR_INVALID;
+  CK(cudaSetDevice(c->device));
+  u64 n_ec = 0, n_pair = 0;
+  CKR(arena_headers(c, false, &n_ec, &n_pair));
+  return import_keys(c, arena_of(c).ec_rec(), n_ec);
 }
 
 int ecb_order_dispatch(ecb_ctx* c, int world, void* const* arena_bases, int64_t cap_records, const int64_t* shard_lo,
@@ -1203,17 +1341,12 @@ int ecb_order_dispatch(ecb_ctx* c, int world, void* const* arena_bases, int64_t 
   if (!c || !arena_bases || !shard_lo || !shard_hi || cap_records < 1) return ECB_ERR_INVALID;
   if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
   CK(cudaSetDevice(c->device));
-  if (c->n_ec == 0) return ECB_OK;
-  KeyDispatchParams P{};
-  P.table = (const EcbEntry*)c->table.p;
-  P.ec_slot = (const u32*)c->ec_slot.p;
-  P.n_ec = c->n_ec;
-  P.world = (u32)world;
-  CKR(shard_routes(c, world, shard_lo, shard_hi, P.lo, P.dest, &P.n_shards));
-  ArenaTargets A{};
-  CKR(arena_targets(c, &A, world, arena_bases, cap_records));
-  ecb_key_dispatch_kernel<true><<<grid_for(c->n_ec, 256, c->sm_count * 8), 256, 0, c->stream>>>(P, A);
-  LAUNCH_CHECK("order_dispatch");
+  KeyDispatchParams K{};
+  CKR(key_dispatch_params(c, world, shard_lo, shard_hi, &K));
+  if (K.n_ec == 0) return ECB_OK;
+  ArenaTargets E{};
+  CKR(arena_targets(c, world, arena_bases, cap_records, 0, true, &E));
+  CKR(key_dispatch(c, K, E, true, false, "order_dispatch"));
   if (c->stream == c->own_stream) CK(cudaStreamSynchronize(c->stream));   // (as ecb_export_to_arenas)
   return ECB_OK;
 }
@@ -1223,61 +1356,12 @@ int ecb_order_build(ecb_ctx* c, const ecb_ctx* local, int64_t shard_lo, int64_t 
   if (local->device != c->device) return fail(c, ECB_ERR_INVALID, "the local context lives on another device");
   memset(out, 0, sizeof *out);
   CK(cudaSetDevice(c->device));
-  unsigned long long hdr[3] = {0, 0, 0};
-  CK(cudaMemcpyAsync(hdr, c->xa_base, sizeof hdr, cudaMemcpyDeviceToHost, c->stream));
+  u64 n_ec = 0, n_pair = 0, nnz = 0;
+  CKR(arena_headers(c, true, &n_ec, &n_pair));
+  CKR(build_a_slice(c, local, arena_of(c).ec_rec(), n_ec, (u64)(shard_hi - shard_lo), c->r_n_data, &nnz));
   CK(cudaStreamSynchronize(c->stream));
-  if (hdr[2]) return fail(c, ECB_ERR_LIMIT, "exchange arena too small for the second dispatch");
-  const u64 n_local = hdr[0];
-  const u64 span = (u64)(shard_hi - shard_lo);
-  if (span > 0xFFFFFFFEull) return fail(c, ECB_ERR_LIMIT, "a rank's alignments span more than 2^32 positions");
-  if (n_local > span) return fail(c, ECB_ERR_INVALID, "%llu ECs arrived for a shard of %llu positions", hdr[0], (unsigned long long)span);
-  if (n_local > local->n_ec) return fail(c, ECB_ERR_INVALID, "%llu ECs arrived but the local context holds %u", hdr[0], local->n_ec);
-  if (n_local + 1 > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "slice exceeds the int32 fields of the EC file");
-  const unsigned long long* rec = (const unsigned long long*)((const char*)c->xa_base + ECB_ARENA_HEADER_BYTES);
-  const size_t words = (size_t)(span / 32) + 1;
-  CKR(ensure(c, c->bitmap, words * 4));
-  CKR(ensure(c, c->word_rank, words * 4));
-  CKR(ensure(c, c->r_a_indptr, (n_local + 1) * 4));
-  CKR(ensure(c, c->r_n_data, std::max<u64>(n_local, 1) * 4));
-  CKR(ensure(c, c->first_rel, std::max<u64>(n_local, 1) * 8));   // scratch: local id per record, then per slice id
-  // every row of the slice is a row of the local context: its arena fill bounds the non-zeros
-  const u64 z_bound = std::max<u64>(local->arena_used, 1);
-  CKR(ensure(c, c->r_a_indices, z_bound * 4));
-  CKR(ensure(c, c->r_a_data, z_bound * 4));
-  u32* lid_of_rec = (u32*)c->first_rel.p;
-  u32* lid_of_id = lid_of_rec + n_local;
-  CK(cudaMemsetAsync(c->bitmap.p, 0, words * 4, c->stream));
-  CK(cudaMemsetAsync(c->r_a_indptr.p, 0, (n_local + 1) * 4, c->stream));
-  CK(cudaMemsetAsync(&c->d_ctr->scratch[5], 0, sizeof(u32), c->stream));
-  u64 nnz = 0;
-  if (n_local) {
-    const int g = grid_for(n_local, 256, c->sm_count * 8);
-    ecb_order_mark_kernel<<<g, 256, 0, c->stream>>>(rec, (u32)n_local, (u32)span, (const EcbEntry*)local->table.p,
-                                                    local->table_slots - 1, (u32*)c->bitmap.p, lid_of_rec, &c->d_ctr->scratch[5]);
-    LAUNCH_CHECK("order_mark");
-    CKR(device_scan<true>(c, (const u32*)c->bitmap.p, (u32*)c->word_rank.p, words, 0, nullptr));
-    ecb_order_lens_kernel<<<g, 256, 0, c->stream>>>(rec, (u32)n_local, (u32)span, (const u32*)c->bitmap.p,
-                                                    (const u32*)c->word_rank.p, lid_of_rec, (const u32*)local->row_len.p,
-                                                    (int32_t*)c->r_a_indptr.p, (int32_t*)c->r_n_data.p, lid_of_id);
-    LAUNCH_CHECK("order_lens");
-    CKR(device_scan<false>(c, (const u32*)c->r_a_indptr.p, (u32*)c->r_a_indptr.p, n_local + 1, 0, nullptr));
-    {
-      const u32 n_blocks = (u32)((n_local + 1 + SCAN_BLOCK - 1) / SCAN_BLOCK);
-      CK(cudaMemcpyAsync(c->h_total, (const u64*)c->scan_partials.p + n_blocks, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
-    }
-    ecb_order_rows_kernel<<<grid_for(n_local, 256, c->sm_count * 16), 256, 0, c->stream>>>(
-        lid_of_id, (const u32*)local->row_len.p, (const u32*)local->row_off.p, (const uint2*)local->arena.p,
-        (const int32_t*)c->r_a_indptr.p, (u32)n_local, (int32_t*)c->r_a_indices.p, (int32_t*)c->r_a_data.p);
-    LAUNCH_CHECK("order_rows");
-  }
-  CKR(sync_counters(c));
-  if (c->h_ctr->scratch[5])
-    return fail(c, ECB_ERR_INVALID, "second dispatch: %s", (c->h_ctr->scratch[5] & 4u) ? "an EC arrived that the local context has never seen"
-                : (c->h_ctr->scratch[5] & 2u) ? "two ECs share a first read" : "a record outside the shard's positions arrived");
-  if (n_local) nnz = *c->h_total;
-  if (nnz > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "slice exceeds the int32 fields of the EC file");
   out->id_base = 0;   // the caller knows where this rank's id range starts (the ECs of the shards in front)
-  out->n_ec = (int64_t)n_local;
+  out->n_ec = (int64_t)n_ec;
   out->nnz = (int64_t)nnz;
   out->a_indptr = (const int32_t*)c->r_a_indptr.p;
   out->a_indices = (const int32_t*)c->r_a_indices.p;
@@ -1370,43 +1454,19 @@ int ecb_cells_order(ecb_ctx* c, int world, const uint64_t* cell_keys, const uint
   return ECB_OK;
 }
 
-// Both record areas of every rank's per-cell arena (the same capacities on every rank).  The device-side overflow
-// flag is set by the record width of the dispatch (`order`: dispatch 2), so that it fires at the capacity in
-// records the host checks.
-static int cells_arena_targets(ecb_ctx* c, ArenaTargets* E, ArenaTargets* P, int world, void* const* bases, int64_t cap_ec,
-                               int64_t cap_pairs, bool order) {
-  CKR(arena_targets(c, E, world, bases, cap_ec));
-  E->cap_words = (unsigned long long)cap_ec * (order ? ECB_ORDREC_WORDS : ECB_KEYREC_WORDS);
-  for (int r = 0; r < world; ++r) {
-    char* b = (char*)bases[r] + ECB_ARENA_HEADER_BYTES + (size_t)cap_ec * ECB_KEYREC_WORDS * 8;
-    P->hdr[r] = (unsigned long long*)b;
-    P->rec[r] = (unsigned long long*)(b + ECB_ARENA_HEADER_BYTES);
-  }
-  P->cap_words = (unsigned long long)cap_pairs * (order ? ECB_CPAIR2_WORDS : ECB_CPAIR1_WORDS);
-  return ECB_OK;
-}
-
-static void key_dispatch_params(ecb_ctx* c, int world, KeyDispatchParams* K) {
-  K->table = (const EcbEntry*)c->table.p;
-  K->ec_slot = (const u32*)c->ec_slot.p;
-  K->n_ec = c->table_slots ? c->n_ec : 0;
-  K->world = (u32)world;
-}
-
 int ecb_cells_dispatch_counts(ecb_ctx* c, int world, const int64_t* shard_lo, const int64_t* shard_hi, int64_t* counts) {
   if (!c || !counts || (!shard_lo) != (!shard_hi)) return ECB_ERR_INVALID;
   if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
   CK(cudaSetDevice(c->device));
   CK(cudaMemsetAsync(counts, 0, (size_t)world * 2 * 8, c->stream));
   KeyDispatchParams K{};
-  key_dispatch_params(c, world, &K);
+  CKR(key_dispatch_params(c, world, shard_lo, shard_hi, &K));
   CellPairDispatchParams P{};
   P.ec_table = K.table;
   P.ec_slot = K.ec_slot;
   P.world = (u32)world;
   if (shard_lo) {   // dispatch 2, an owner context
     if (K.n_ec == 0) return ECB_OK;
-    CKR(shard_routes(c, world, shard_lo, shard_hi, K.lo, K.dest, &K.n_shards));
     memcpy(P.lo, K.lo, sizeof P.lo);
     memcpy(P.dest, K.dest, sizeof P.dest);
     P.n_shards = K.n_shards;
@@ -1436,20 +1496,7 @@ int ecb_cells_arena_create(ecb_ctx* c, int64_t cap_ec, int64_t cap_pairs, void* 
   if (c->xa_base) CK(cudaFree(c->xa_base));
   c->xa_base = nullptr;
   c->xa_cap_ec = c->xa_cap_pairs = 0;
-  const size_t pair_hdr = ECB_ARENA_HEADER_BYTES + (size_t)cap_ec * ECB_KEYREC_WORDS * 8;
-  const size_t bytes = pair_hdr + ECB_ARENA_HEADER_BYTES + (size_t)cap_pairs * ECB_CPAIR1_WORDS * 8;
-  CK(cudaMalloc(&c->xa_base, bytes));
-  CK(cudaMemset(c->xa_base, 0, ECB_ARENA_HEADER_BYTES));
-  CK(cudaMemset((char*)c->xa_base + pair_hdr, 0, ECB_ARENA_HEADER_BYTES));
-  c->xa_cap_ec = cap_ec;
-  c->xa_cap_pairs = cap_pairs;
-  if (ipc_handle_out) {
-    cudaIpcMemHandle_t h;
-    CK(cudaIpcGetMemHandle(&h, c->xa_base));
-    memcpy(ipc_handle_out, &h, sizeof h);
-  }
-  *base_out = c->xa_base;
-  return ECB_OK;
+  return arena_alloc(c, cap_ec, cap_pairs, ipc_handle_out, base_out);
 }
 
 int ecb_cells_export_to_arenas(ecb_ctx* c, int world, void* const* arena_bases, int64_t cap_ec, int64_t cap_pairs,
@@ -1464,13 +1511,12 @@ int ecb_cells_export_to_arenas(ecb_ctx* c, int world, void* const* arena_bases, 
   if (n_ec == 0) return ECB_OK;
   if (!c->cx_kept.p) return fail(c, ECB_ERR_STATE, "ecb_cells_order has not run on this context");
   ArenaTargets E{}, A{};
-  CKR(cells_arena_targets(c, &E, &A, world, arena_bases, cap_ec, cap_pairs, false));
+  CKR(arena_targets(c, world, arena_bases, cap_ec, cap_pairs, false, &E, &A));
   // EVERY local EC goes, with the reads it has in kept cells (0 too: this rank may hold its first occurrence)
   KeyDispatchParams K{};
-  key_dispatch_params(c, world, &K);
+  CKR(key_dispatch_params(c, world, nullptr, nullptr, &K));
   K.count_of = (const u32*)c->cx_kept.p;
-  ecb_key_dispatch_kernel<false><<<grid_for(n_ec, 256, c->sm_count * 8), 256, 0, c->stream>>>(K, E);
-  LAUNCH_CHECK("cells_export_ecs");
+  CKR(key_dispatch(c, K, E, false, false, "cells_export_ecs"));
   if (c->cx_n_local_cells) {
     CellPairDispatchParams P{};
     P.pair_table = (const EcbEntry*)c->cells.pair_table.p;
@@ -1485,30 +1531,13 @@ int ecb_cells_export_to_arenas(ecb_ctx* c, int world, void* const* arena_bases, 
   return ECB_OK;
 }
 
-// Both headers {records, unused, overflow} of this context's per-cell arena (one host round trip).
-static int cells_arena_headers(ecb_ctx* c, unsigned long long* h_ec, unsigned long long* h_pair) {
-  CK(cudaMemcpyAsync(h_ec, c->xa_base, 3 * 8, cudaMemcpyDeviceToHost, c->stream));
-  CK(cudaMemcpyAsync(h_pair, (const char*)c->xa_base + ECB_ARENA_HEADER_BYTES + (size_t)c->xa_cap_ec * ECB_KEYREC_WORDS * 8,
-                     3 * 8, cudaMemcpyDeviceToHost, c->stream));
-  CK(cudaStreamSynchronize(c->stream));
-  if (h_ec[2] || h_ec[0] > (unsigned long long)c->xa_cap_ec || h_pair[2] || h_pair[0] > (unsigned long long)c->xa_cap_pairs)
-    return fail(c, ECB_ERR_LIMIT, "exchange arena too small: %llu ECs and %llu pairs arrived, capacity %lld and %lld", h_ec[0],
-                h_pair[0], (long long)c->xa_cap_ec, (long long)c->xa_cap_pairs);
-  return ECB_OK;
-}
-
-static const unsigned long long* cells_pair_records(const ecb_ctx* c) {
-  return (const unsigned long long*)((const char*)c->xa_base + 2 * ECB_ARENA_HEADER_BYTES +
-                                     (size_t)c->xa_cap_ec * ECB_KEYREC_WORDS * 8);
-}
-
 int ecb_cells_import_arena(ecb_ctx* c) {
   if (!c || !c->xa_base || !c->xa_cap_pairs) return ECB_ERR_INVALID;
   CK(cudaSetDevice(c->device));
-  unsigned long long h_ec[3], h_pair[3];
-  CKR(cells_arena_headers(c, h_ec, h_pair));
-  CKR(import_keys(c, (const unsigned long long*)((const char*)c->xa_base + ECB_ARENA_HEADER_BYTES), h_ec[0]));
-  const u64 n_pair = h_pair[0];
+  const ArenaLayout L = arena_of(c);
+  u64 n_ec = 0, n_pair = 0;
+  CKR(arena_headers(c, false, &n_ec, &n_pair));
+  CKR(import_keys(c, L.ec_rec(), n_ec));
   if (n_pair > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "too many records in one import");
   if (n_pair && !c->table_slots) return fail(c, ECB_ERR_INVALID, "pairs arrived without their ECs");
   CellScratch& S = c->cells;
@@ -1517,7 +1546,7 @@ int ecb_cells_import_arena(ecb_ctx* c) {
   CK(cudaMemsetAsync(S.pair_table.p, 0xFF, (size_t)S.pair_slots * sizeof(EcbEntry), c->stream));
   if (n_pair) {
     cells_pair_import_kernel<<<grid_for(n_pair, 256, c->sm_count * 8), 256, 0, c->stream>>>(
-        cells_pair_records(c), (u32)n_pair, (const EcbEntry*)c->table.p, c->table_slots - 1, (EcbEntry*)S.pair_table.p,
+        L.pair_rec(), (u32)n_pair, (const EcbEntry*)c->table.p, c->table_slots - 1, (EcbEntry*)S.pair_table.p,
         S.pair_slots - 1, c->d_ctr);
     LAUNCH_CHECK("cells_import_pairs");
     CKR(sync_counters(c));
@@ -1532,13 +1561,11 @@ int ecb_cells_order_dispatch(ecb_ctx* c, int world, void* const* arena_bases, in
   if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
   CK(cudaSetDevice(c->device));
   KeyDispatchParams K{};
-  key_dispatch_params(c, world, &K);
+  CKR(key_dispatch_params(c, world, shard_lo, shard_hi, &K));
   if (K.n_ec == 0) return ECB_OK;
-  CKR(shard_routes(c, world, shard_lo, shard_hi, K.lo, K.dest, &K.n_shards));
   ArenaTargets E{}, A{};
-  CKR(cells_arena_targets(c, &E, &A, world, arena_bases, cap_ec, cap_pairs, true));
-  ecb_key_dispatch_kernel<true, true><<<grid_for(K.n_ec, 256, c->sm_count * 8), 256, 0, c->stream>>>(K, E);
-  LAUNCH_CHECK("cells_order_dispatch_ecs");
+  CKR(arena_targets(c, world, arena_bases, cap_ec, cap_pairs, true, &E, &A));
+  CKR(key_dispatch(c, K, E, true, true, "cells_order_dispatch_ecs"));
   CellPairDispatchParams P{};
   P.pair_table = (const EcbEntry*)c->cells.pair_table.p;
   P.pair_slots = c->cells.pair_slots;
@@ -1562,61 +1589,14 @@ int ecb_cells_order_build(ecb_ctx* c, const ecb_ctx* local, int64_t shard_lo, in
   if (local->device != c->device) return fail(c, ECB_ERR_INVALID, "the local context lives on another device");
   memset(out, 0, sizeof *out);
   CK(cudaSetDevice(c->device));
-  unsigned long long h_ec[3], h_pair[3];
-  CKR(cells_arena_headers(c, h_ec, h_pair));
-  const u64 n_local = h_ec[0], n_pair = h_pair[0];
+  const ArenaLayout L = arena_of(c);
+  u64 n_ec = 0, n_pair = 0, nnz = 0;
+  CKR(arena_headers(c, true, &n_ec, &n_pair));
+  if (n_pair > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "slice exceeds the int32 fields of the EC file");
   const u64 span = (u64)(shard_hi - shard_lo);
-  const u32 local_n_ec = local->table_slots ? local->n_ec : 0;
-  if (span > 0xFFFFFFFEull) return fail(c, ECB_ERR_LIMIT, "a rank's alignments span more than 2^32 positions");
-  if (n_local > span) return fail(c, ECB_ERR_INVALID, "%llu ECs arrived for a shard of %llu positions", n_local, (unsigned long long)span);
-  if (n_local > local_n_ec) return fail(c, ECB_ERR_INVALID, "%llu ECs arrived but the local context holds %u", n_local, local_n_ec);
-  if (n_local + 1 > 0x7FFFFFFFull || n_pair > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "slice exceeds the int32 fields of the EC file");
-  const unsigned long long* rec = (const unsigned long long*)((const char*)c->xa_base + ECB_ARENA_HEADER_BYTES);
-  const size_t words = (size_t)(span / 32) + 1;
-  CKR(ensure(c, c->bitmap, words * 4));
-  CKR(ensure(c, c->word_rank, words * 4));
-  CKR(ensure(c, c->r_a_indptr, (n_local + 1) * 4));
-  CKR(ensure(c, c->count_of, std::max<u64>(n_local, 1) * 4));     // the merged counts (not part of the slice)
-  CKR(ensure(c, c->first_rel, std::max<u64>(n_local, 1) * 8));   // scratch: local id per record, then per slice id
-  const u64 z_bound = std::max<u64>(local->arena_used, 1);
-  CKR(ensure(c, c->r_a_indices, z_bound * 4));
-  CKR(ensure(c, c->r_a_data, z_bound * 4));
   CKR(ensure(c, c->cx_col_counts, (size_t)n_samples * 4));
-  u32* lid_of_rec = (u32*)c->first_rel.p;
-  u32* lid_of_id = lid_of_rec + n_local;
-  CK(cudaMemsetAsync(c->bitmap.p, 0, words * 4, c->stream));
-  CK(cudaMemsetAsync(c->r_a_indptr.p, 0, (n_local + 1) * 4, c->stream));
   CK(cudaMemsetAsync(c->cx_col_counts.p, 0, (size_t)n_samples * 4, c->stream));
-  CK(cudaMemsetAsync(&c->d_ctr->scratch[5], 0, sizeof(u32), c->stream));
-  auto check_bad = [&]() -> int {
-    CKR(sync_counters(c));
-    const u32 bad = c->h_ctr->scratch[5];
-    if (bad)
-      return fail(c, ECB_ERR_INVALID, "second dispatch: %s",
-                  (bad & 4u) ? "an EC arrived that the local context has never seen" : (bad & 2u) ? "two ECs share a first read"
-                  : (bad & 1u) ? "a record outside the shard's positions arrived" : (bad & 8u) ? "a pair arrived without its EC"
-                               : "a pair's column is out of range");
-    return ECB_OK;
-  };
-  u64 nnz = 0;
-  if (n_local) {
-    const int g = grid_for(n_local, 256, c->sm_count * 8);
-    ecb_order_mark_kernel<<<g, 256, 0, c->stream>>>(rec, (u32)n_local, (u32)span, (const EcbEntry*)local->table.p,
-                                                    local->table_slots - 1, (u32*)c->bitmap.p, lid_of_rec, &c->d_ctr->scratch[5]);
-    LAUNCH_CHECK("order_mark");
-    CKR(check_bad());   // nothing below indexes with what the mark pass produced before it is known to be sound
-    CKR(device_scan<true>(c, (const u32*)c->bitmap.p, (u32*)c->word_rank.p, words, 0, nullptr));
-    ecb_order_lens_kernel<<<g, 256, 0, c->stream>>>(rec, (u32)n_local, (u32)span, (const u32*)c->bitmap.p,
-                                                    (const u32*)c->word_rank.p, lid_of_rec, (const u32*)local->row_len.p,
-                                                    (int32_t*)c->r_a_indptr.p, (int32_t*)c->count_of.p, lid_of_id);
-    LAUNCH_CHECK("order_lens");
-    CKR(device_scan<false>(c, (const u32*)c->r_a_indptr.p, (u32*)c->r_a_indptr.p, n_local + 1, 0, &nnz));
-    if (nnz > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "slice exceeds the int32 fields of the EC file");
-    ecb_order_rows_kernel<<<grid_for(n_local, 256, c->sm_count * 16), 256, 0, c->stream>>>(
-        lid_of_id, (const u32*)local->row_len.p, (const u32*)local->row_off.p, (const uint2*)local->arena.p,
-        (const int32_t*)c->r_a_indptr.p, (u32)n_local, (int32_t*)c->r_a_indices.p, (int32_t*)c->r_a_data.p);
-    LAUNCH_CHECK("order_rows");
-  }
+  CKR(build_a_slice(c, local, L.ec_rec(), n_ec, span, c->count_of, &nnz));   // merged counts: not part of the slice
   CKR(ensure(c, c->r_n_indices, std::max<u64>(n_pair, 1) * 4));
   CKR(ensure(c, c->r_n_data, std::max<u64>(n_pair, 1) * 4));
   if (n_pair) {
@@ -1624,10 +1604,11 @@ int ecb_cells_order_build(ecb_ctx* c, const ecb_ctx* local, int64_t shard_lo, in
     CKR(ensure(c, S.sort_k[0], (size_t)n_pair * 8));
     CKR(ensure(c, S.sort_v[0], (size_t)n_pair * 4));
     cells_pair_slice_kernel<<<grid_for(n_pair, 256, c->sm_count * 8), 256, 0, c->stream>>>(
-        cells_pair_records(c), (u32)n_pair, (u32)span, (u32)n_samples, (const u32*)c->bitmap.p, (const u32*)c->word_rank.p,
+        L.pair_rec(), (u32)n_pair, (u32)span, (u32)n_samples, (const u32*)c->bitmap.p, (const u32*)c->word_rank.p,
         (u64*)S.sort_k[0].p, (u32*)S.sort_v[0].p, &c->d_ctr->scratch[5]);
     LAUNCH_CHECK("cells_pair_slice");
-    CKR(check_bad());
+    CKR(sync_counters(c));   // the sort and the column counts below index with what the pair pass produced
+    CKR(check_slice_flags(c));
     int rb = 0;
     CKR(radix_sort(c, (u32)n_pair, 32 + bits_for((u64)n_samples), &rb));
     cells_slice_csc_kernel<<<grid_for(n_pair, 256, c->sm_count * 8), 256, 0, c->stream>>>(
@@ -1637,7 +1618,7 @@ int ecb_cells_order_build(ecb_ctx* c, const ecb_ctx* local, int64_t shard_lo, in
   }
   CKR(sync_counters(c));
   CKR(check_device_error(c));
-  out->n_ec = (int64_t)n_local;
+  out->n_ec = (int64_t)n_ec;
   out->nnz = (int64_t)nnz;
   out->a_indptr = (const int32_t*)c->r_a_indptr.p;
   out->a_indices = (const int32_t*)c->r_a_indices.p;

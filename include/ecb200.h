@@ -207,7 +207,14 @@ int ecb_export_to_arenas(ecb_ctx* local_ctx, int world, void* const* arena_bases
 int ecb_import_arena(ecb_ctx* owner_ctx);
 
 /* This rank's slice of the final matrices: a_indptr[n_ec + 1] (offsets local to the slice), a_indices, a_data
- * and n_data (read counts), all device memory of the owner context, valid until the next call on it. */
+ * and n_data (read counts), all device memory of the owner context, valid until the next call on it.
+ * Besides bad arguments and CUDA errors, ecb_order_build fails, before any row is copied, with
+ *   ECB_ERR_LIMIT    "exchange arena too small for the second dispatch", a shard of more than 2^32 positions, or a
+ *                    slice beyond the int32 fields of the EC file;
+ *   ECB_ERR_INVALID  more ECs arrived than the shard has positions or the local context holds ECs, or "second
+ *                    dispatch: ..." - an EC the local context has never seen, two ECs with one first position
+ *                    (order_base ranges of one rank's pushes overlapped), or a record outside the shard.
+ * The owner and the local context stay usable. */
 typedef struct ecb_slice {
   int64_t id_base, n_ec, nnz;
   const int32_t *a_indptr, *a_indices, *a_data, *n_data;
