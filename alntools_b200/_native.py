@@ -24,6 +24,7 @@ ECB_OPT_BAM_WINDOW = 9
 ECB_OPT_COLLATE_SLOTS = 10
 ECB_OPT_COLLATE_PIECE = 11
 ECB_OPT_COLLATE_BUDGET = 12
+ECB_OPT_MAX_READ = 13
 
 ECB_ERR_EMPTY = -5
 ECB_ERR_FORMAT = -7
@@ -50,6 +51,7 @@ class EcbStats(ctypes.Structure):
         ("table_used", ctypes.c_int64), ("table_grows", ctypes.c_int64),
         ("overflow_reads", ctypes.c_int64), ("h2d_bytes", ctypes.c_int64),
         ("d2h_bytes", ctypes.c_int64), ("row_entries", ctypes.c_int64),
+        ("long_reads", ctypes.c_int64), ("long_ms", ctypes.c_double),
     ]
 
     def as_dict(self):
@@ -219,7 +221,13 @@ def _on_device(x):
 
 
 class EcBuilder(object):
-    """One context = one GPU.  push() columns, finalize() -> dict of numpy int32 arrays."""
+    """One context = one GPU.  push() columns, finalize() -> dict of numpy int32 arrays.
+
+    Options are the ECB_OPT_* of include/ecb200.h by their names in _OPTIONS.  max_read (ECB_OPT_MAX_READ) is the
+    longest read a push accepts: 16384 alignments by default, 0 for the push limit (2^31 - 8192).  Reads longer than
+    16384 then take a sort-based pass of their own on the GPU, with the same result as the reference.  The default
+    stays at 16384 because in a file grouped by read name a read that long is more often a broken input than a real
+    one, and the error says so early."""
 
     def __init__(self, n_targets, n_haps, with_cells=False, alignments_hint=0, device=0, **options):
         self._lib = load_library()
@@ -239,7 +247,8 @@ class EcBuilder(object):
                 "hot_cache": ECB_OPT_HOT_CACHE, "verify_keys": ECB_OPT_VERIFY_KEYS,
                 "chunk_len": ECB_OPT_CHUNK_LEN, "pageable_results": ECB_OPT_PAGEABLE_RESULTS,
                 "bam_window": ECB_OPT_BAM_WINDOW, "collate_slots": ECB_OPT_COLLATE_SLOTS,
-                "collate_piece": ECB_OPT_COLLATE_PIECE, "collate_budget": ECB_OPT_COLLATE_BUDGET}
+                "collate_piece": ECB_OPT_COLLATE_PIECE, "collate_budget": ECB_OPT_COLLATE_BUDGET,
+                "max_read": ECB_OPT_MAX_READ}
 
     def _check(self, rc):
         if rc != 0:

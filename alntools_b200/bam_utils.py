@@ -114,7 +114,7 @@ def process_convert_bam(cp, device=0):
                 break
             if builder is None:
                 builder = EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=False, alignments_hint=0,
-                                    device=device)
+                                    device=device, max_read=emitter.max_read())
             builder.push(cols["read_group"], cols["target_idx"], cols["hap_idx"], order_base=pushed)
             pushed += n
             ret.valid_alignments += n
@@ -154,9 +154,9 @@ def _job_plan(num_chunks, number_processes):
     return num_chunks, min(num_processes, num_chunks)
 
 
-def _convert_python_emitter(bam_filename, target_filename, device, start_time, collate=False):
+def _convert_python_emitter(bam_filename, target_filename, device, start_time, collate=False, max_read=16384):
     """The same build fed by the record-level Python emitter (ALNTOOLS_B200_EMITTER=python); collate: reads by name
-    over the whole file (emitter.emit_collated)."""
+    over the whole file (emitter.emit_collated); max_read: as emitter.max_read."""
     temp_time = time.time()
     header, records = emitter.read_bam(bam_filename)
     tables = TargetTables(header.references, header.lengths, target_filename)
@@ -166,7 +166,7 @@ def _convert_python_emitter(bam_filename, target_filename, device, start_time, c
     if cols.valid_alignments == 0:
         raise RuntimeError("The shape must be a tuple of three positive integers.")
     with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=False,
-                   alignments_hint=cols.valid_alignments, device=device) as builder:
+                   alignments_hint=cols.valid_alignments, device=device, max_read=max_read) as builder:
         builder.push(cols.read_group, cols.target_idx, cols.hap_idx, order_base=0)
         res = builder.finalize()
     return res, tables, cols.valid_alignments
@@ -186,6 +186,7 @@ def convert_rank(bam_filename, ec_filename, emase_filename, num_chunks=0, number
     import torch.distributed as dist
     from . import multi_gpu
     start_time = time.time()
+    limit = emitter.max_read()
     with multi_gpu.rank_process() as (rank, world, device):
         _, num_processes = _job_plan(num_chunks, number_processes)
         num_processes = max(1, num_processes // world)          # the host threads are shared by the ranks
@@ -198,7 +199,7 @@ def convert_rank(bam_filename, ec_filename, emase_filename, num_chunks=0, number
             if range_filename is not None:
                 reader.track_ranges(True)
             opts = dict(with_cells=False, alignments_hint=0, device=device.index, result_on_device=1)
-            with EcBuilder(tables.num_targets, tables.num_haplotypes, **opts) as builder, \
+            with EcBuilder(tables.num_targets, tables.num_haplotypes, max_read=limit, **opts) as builder, \
                     EcBuilder(tables.num_targets, tables.num_haplotypes, **opts) as owner:
                 chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(bam_filename) // 2)))   # 24 MB of columns per piece
                 valid = emitter.stream_single(reader, builder, chunk_rows=chunk_rows, pinned=True)
@@ -248,10 +249,14 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
     decode).  The outputs are those of the default convert() of the file regrouped that way; for a grouped file they
     are the default's.  ALNTOOLS_B200_COLLATE_BUDGET caps the device bytes of the collation (emitter.collate_budget);
     a file whose rows do not fit is collated in passes through host memory, with the same outputs.
+    ALNTOOLS_B200_MAX_READ raises the longest read accepted from 16384 alignments (emitter.max_read; 0: the push limit),
+    in every mode; longer reads take a sort-based pass on the GPU.  The default stays, because in a file grouped by
+    name a read that long more often means a broken input.
     """
     start_time = time.time()
     mode = emitter.resolve_mode(False, devices, decode, collate, range_filename is not None)
     budget = emitter.collate_budget() if mode.collate else 0
+    limit = emitter.max_read()
     job = dict(bam_filename=bam_filename, ec_filename=ec_filename, emase_filename=emase_filename, num_chunks=num_chunks,
                number_processes=number_processes, temp_dir=temp_dir, range_filename=range_filename, sample=sample,
                target_filename=target_filename)
@@ -289,7 +294,8 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
     LOG.info("Parsing file information ...")
     temp_time = time.time()
     if mode.python:
-        res, tables, valid = _convert_python_emitter(bam_filename, target_filename, device, start_time, mode.collate)
+        res, tables, valid = _convert_python_emitter(bam_filename, target_filename, device, start_time, mode.collate,
+                                                     limit)
         return save(res, tables, valid, temp_time)
     # native emitter: inflate threads + one record pass, streamed to the GPU in read-aligned chunks
     import torch
@@ -303,7 +309,7 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
         # no alignment count is known up front: the library sizes its table from the first chunk and
         # grows it ahead of later ones; one finalize per context, so results skip the pinning cost
         with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=False, alignments_hint=0,
-                       device=device, pageable_results=1, collate_budget=budget) as builder:
+                       device=device, pageable_results=1, collate_budget=budget, max_read=limit) as builder:
             chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(bam_filename) // 2)))   # 24 MB of columns per piece
             if mode.decode == "device":
                 valid, _, ranges, _ = emitter.stream_single_device(bam_filename, reader, builder, tables,

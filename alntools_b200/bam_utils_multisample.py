@@ -75,6 +75,7 @@ def convert_files_rank(bam_files, ec_filename, emase_filename, minimum_count, ta
     import torch.distributed as dist
     from . import multi_gpu
     start_time = time.time()
+    limit = emitter.max_read()
     with multi_gpu.rank_process() as (rank, world, device):
         cuts = partition_files([os.path.getsize(f) for f in bam_files], world)
         n_threads = max(1, (os.cpu_count() or 1) // world)      # the host threads are shared by the ranks
@@ -82,7 +83,7 @@ def convert_files_rank(bam_files, ec_filename, emase_filename, minimum_count, ta
         cells = bamcols.CellDictionary()
         opts = dict(alignments_hint=0, device=device.index, result_on_device=1)
         try:
-            with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=True, **opts) as builder, \
+            with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=True, max_read=limit, **opts) as builder, \
                     EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=False, **opts) as owner:
                 valid, ranges = emitter.stream_files(bam_files[cuts[rank]:cuts[rank + 1]], tables, cells, builder,
                                                      rank * RANK_STRIDE, n_threads, range_filename is not None)
@@ -117,8 +118,10 @@ def convert_files(bam_files, ec_filename, emase_filename, minimum_count, target_
     """The reference's convert() after its glob: files are merged in the given order
     (bam_utils_multisample.py:503-560).  devices=N (or the environment variable ALNTOOLS_GPUS=N) spreads the
     files over N GPUs of this machine, one worker process per GPU (convert_files_rank); the same happens without
-    either inside a one-process-per-GPU job (torchrun).  The EC file does not depend on the number of GPUs."""
+    either inside a one-process-per-GPU job (torchrun).  The EC file does not depend on the number of GPUs.
+    ALNTOOLS_B200_MAX_READ: the longest read accepted, as for the single-sample convert (emitter.max_read)."""
     mode = emitter.resolve_mode(True, devices, range_file=range_filename is not None)
+    limit = emitter.max_read()
     bam_files = list(bam_files)
     if not bam_files:
         raise ValueError("convert_files needs at least one BAM file")
@@ -144,7 +147,7 @@ def convert_files(bam_files, ec_filename, emase_filename, minimum_count, target_
         for name, idx in cell_ids.items():
             cell_names[idx] = name
         with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=True,
-                       alignments_hint=total_valid, device=device) as builder:
+                       alignments_hint=total_valid, device=device, max_read=limit) as builder:
             base = 0
             for cols in per_file:
                 builder.push(cols.read_group, cols.target_idx, cols.hap_idx, cols.cell_idx, order_base=base,
@@ -157,7 +160,7 @@ def convert_files(bam_files, ec_filename, emase_filename, minimum_count, target_
         cells = bamcols.CellDictionary()
         try:
             with EcBuilder(tables.num_targets, tables.num_haplotypes, with_cells=True,
-                           alignments_hint=0, device=device) as builder:
+                           alignments_hint=0, device=device, max_read=limit) as builder:
                 total_valid, ranges = emitter.stream_files(bam_files, tables, cells, builder,
                                                            track_ranges=range_filename is not None)
                 res = builder.finalize(minimum_count)
@@ -184,6 +187,7 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks, minimum_count
     """The reference's per-cell convert: every *.bam of the directory, in filesystem order.  devices /
     ALNTOOLS_GPUS: as convert_files."""
     emitter.resolve_mode(True, devices, range_file=range_filename is not None)   # refusals before the directory is read
+    emitter.max_read()
     if os.path.isfile(bam_filename):                          # :375-377
         LOG.error('bam file must be a directory')
         return None

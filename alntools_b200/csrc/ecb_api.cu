@@ -21,8 +21,12 @@
 #include "ecb_cells_exchange.cuh"
 #include "ecb_bam.cuh"
 #include "ecb_collate.cuh"
+#include "ecb_longread.cuh"
 
 #define ECB_PUSH_LIMIT (0x7FFFFFFFll - 8192)   // alignments of one ecb_push
+// Largest ECB_OPT_MAX_READ, and what 0 stands for: the push limit as documented (2^31 - 8192), one more than the
+// longest push, so that no read is ever above it.
+#define ECB_MAX_READ_LIMIT ((1ll << 31) - 8192)
 
 namespace {
 
@@ -50,6 +54,7 @@ struct ecb_ctx {
   int pageable_results = 0;
   int64_t opt_bam_window = 0;
   int64_t opt_collate_slots = 0, opt_collate_piece = 0, opt_collate_budget = 0;
+  int64_t max_read = ECB_MAX_READ_ALIGNMENTS;   // ECB_OPT_MAX_READ (0 stored as the push limit)
   // EC table
   DevBuf table;
   u32 table_slots = 0;
@@ -74,6 +79,9 @@ struct ecb_ctx {
   cudaStream_t copy_stream = nullptr;
   cudaEvent_t copy_done[2] = {nullptr, nullptr};
   DevBuf overflow_bits;
+  // reads longer than ECB_MAX_READ_ALIGNMENTS (ecb_longread.cuh): the grouping kernel's list, the sorted list with
+  // the prefix of the lengths, the run ranks and the per-read sums
+  DevBuf lr_list, lr_meta, lr_rank, lr_acc;
   DevBuf scan_partials;  // u64 block sums + 1 total
   // push bookkeeping
   u64 min_base = ~0ull, max_end = 0;
@@ -89,7 +97,7 @@ struct ecb_ctx {
   size_t h_res_bytes = 0;
   // stats
   ecb_stats stats{};
-  cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  cudaEvent_t ev[8] = {};
   bool long_attr_set = false;
   // arena of the multi-GPU exchange (plain cudaMalloc: must be exportable through CUDA IPC)
   void* xa_base = nullptr;
@@ -182,7 +190,8 @@ int check_device_error(ecb_ctx* c) {
   if (e & ECB_DEVERR_VALUE_RANGE)
     return fail(c, ECB_ERR_INVALID, "target_idx/hap_idx outside [0,%d) x [0,%d)", c->n_targets, c->n_haps);
   if (e & ECB_DEVERR_READ_TOO_LONG)
-    return fail(c, ECB_ERR_LIMIT, "a read has more than %d alignments", ECB_MAX_READ_ALIGNMENTS);
+    return fail(c, ECB_ERR_LIMIT, "a read has more than %lld alignments%s", (long long)c->max_read,
+                c->max_read == ECB_MAX_READ_ALIGNMENTS ? " (ECB_OPT_MAX_READ raises the limit)" : "");
   if (e & ECB_DEVERR_VERIFY) return fail(c, ECB_ERR_LIMIT, "128-bit key collision detected by verification");
   return fail(c, ECB_ERR_LIMIT, "device error bits 0x%x", e);
 }
@@ -314,6 +323,8 @@ GroupParams make_group_params(ecb_ctx* c, const int32_t* rg, const int32_t* tg, 
   P.ttable = (EcbEntry*)c->ttable.p;
   P.tmask = c->ttable_slots ? c->ttable_slots - 1 : 0;
   P.push_id = push_id;
+  P.max_read = (int)c->max_read;
+  P.deferred = (uint2*)c->lr_list.p;
   return P;
 }
 
@@ -420,6 +431,79 @@ int bits_for(u64 v) {
   int b = 1;
   while (b < 64 && (v >> b)) ++b;
   return b;
+}
+
+// ---- reads longer than ECB_MAX_READ_ALIGNMENTS (ecb_longread.cuh) ----------------------------------------------
+// Key pass and insert of the n_def reads the grouping kernel deferred.  One host round trip brings their list back
+// (sorted by offset here, so that read indices follow the push order), one copy sends it with the prefix of the
+// lengths, and the sort, sums, scan and insert follow on the stream; the caller's sync_counters ends it.
+int long_keys(ecb_ctx* c, const GroupParams& P, const int32_t* tg, const int32_t* hp, u32 n_def, LongParams* L) {
+  std::vector<uint2> list(n_def);
+  CK(cudaMemcpyAsync(list.data(), c->lr_list.p, (size_t)n_def * sizeof(uint2), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  c->stats.d2h_bytes += (int64_t)n_def * sizeof(uint2);
+  std::sort(list.begin(), list.end(), [](const uint2& a, const uint2& b) { return a.x < b.x; });
+  // [n_def] (offset, length), then [n_def + 1] u32 starts
+  std::vector<u32> meta((size_t)n_def * 2 + n_def + 1);
+  memcpy(meta.data(), list.data(), (size_t)n_def * sizeof(uint2));
+  u32* start = meta.data() + (size_t)n_def * 2;
+  u64 total = 0;
+  for (u32 r = 0; r < n_def; ++r) {
+    start[r] = (u32)total;
+    total += list[r].y;
+  }
+  start[n_def] = (u32)total;   // total <= alignments of the push < 2^31
+  CKR(ensure(c, c->lr_meta, meta.size() * 4));
+  CK(cudaMemcpyAsync(c->lr_meta.p, meta.data(), meta.size() * 4, cudaMemcpyHostToDevice, c->stream));
+  c->stats.h2d_bytes += (int64_t)meta.size() * 4;
+  CellScratch& S = c->cells;
+  CKR(ensure(c, S.sort_k[0], (size_t)total * 8));
+  CKR(ensure(c, S.sort_v[0], (size_t)total * 4));
+  CKR(ensure(c, c->lr_rank, ((size_t)total + 1) * 4));
+  CKR(ensure(c, c->lr_acc, (size_t)n_def * sizeof(LongAcc)));
+  LongParams& Q = *L;
+  Q = LongParams{};
+  Q.tg = tg; Q.hp = hp;
+  Q.reads = (const uint2*)c->lr_meta.p;
+  Q.start = (const u32*)c->lr_meta.p + (size_t)n_def * 2;
+  Q.n_reads = n_def;
+  Q.total = (u32)total;
+  Q.n_targets = c->n_targets; Q.n_haps = c->n_haps;
+  Q.keys = (u64*)S.sort_k[0].p;
+  Q.vals = (u32*)S.sort_v[0].p;
+  Q.rank = (u32*)c->lr_rank.p;
+  Q.acc = (LongAcc*)c->lr_acc.p;
+  Q.ctr = c->d_ctr;
+  ecb_long_gather_kernel<<<grid_for(total, ECB_LONG_THREADS, c->sm_count * 8), ECB_LONG_THREADS, 0, c->stream>>>(Q);
+  LAUNCH_CHECK("long_gather");
+  int rb = 0;
+  CKR(radix_sort(c, (u32)total, 31 + (n_def > 1 ? bits_for(n_def - 1) : 0), &rb));
+  Q.sorted = (const u64*)S.sort_k[rb].p;
+  ecb_long_sums_kernel<<<grid_for(total, ECB_LONG_THREADS * 16, c->sm_count * 4), ECB_LONG_THREADS, 0, c->stream>>>(Q);
+  LAUNCH_CHECK("long_sums");
+  CKR(device_scan<false>(c, Q.rank, Q.rank, total + 1, 0, nullptr));
+  ecb_long_insert_kernel<<<grid_for(n_def, ECB_LONG_THREADS, c->sm_count), ECB_LONG_THREADS, 0, c->stream>>>(P, Q);
+  LAUNCH_CHECK("long_insert");
+  return ECB_OK;
+}
+
+// Rows of the ECs the deferred reads claimed (after the harvest, which skipped them), and their verification.
+int long_rows(ecb_ctx* c, const LongParams& L) {
+  const int g_r = grid_for(L.n_reads, ECB_LONG_THREADS, c->sm_count);
+  const int g_i = grid_for(L.total, ECB_LONG_THREADS, c->sm_count * 8);
+  ecb_long_rows_reserve_kernel<<<g_r, ECB_LONG_THREADS, 0, c->stream>>>(L, (u32*)c->row_len.p, (u32*)c->row_off.p);
+  LAUNCH_CHECK("long_rows_reserve");
+  ecb_long_rows_kernel<false><<<g_i, ECB_LONG_THREADS, 0, c->stream>>>(L, (uint2*)c->arena.p);
+  LAUNCH_CHECK("long_rows");
+  ecb_long_rows_kernel<true><<<g_i, ECB_LONG_THREADS, 0, c->stream>>>(L, (uint2*)c->arena.p);
+  LAUNCH_CHECK("long_rows_or");
+  if (c->verify_keys) {
+    ecb_long_verify_kernel<<<std::min<u32>(L.n_reads, (u32)c->sm_count * 4), ECB_LONG_THREADS, 0, c->stream>>>(
+        L, (const EcbEntry*)c->table.p, c->table_slots - 1, (const u32*)c->row_len.p, (const u32*)c->row_off.p,
+        (const uint2*)c->arena.p);
+    LAUNCH_CHECK("long_verify");
+  }
+  return ECB_OK;
 }
 
 CellParams make_cell_params(ecb_ctx* c, const CellResult* cr) {
@@ -563,7 +647,7 @@ void cells_release(ecb_ctx* c) {
 
 extern "C" {
 
-int ecb_version(void) { return 2004; }
+int ecb_version(void) { return 2005; }
 
 const char* ecb_last_error(const ecb_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
@@ -650,6 +734,11 @@ int ecb_set_option(ecb_ctx* c, int option, int64_t value) {
     case ECB_OPT_COLLATE_BUDGET:
       if (value < 0) return fail(c, ECB_ERR_INVALID, "negative collate budget");
       c->opt_collate_budget = value; break;
+    case ECB_OPT_MAX_READ:
+      if (value != 0 && (value < ECB_MAX_READ_ALIGNMENTS || value > ECB_MAX_READ_LIMIT))
+        return fail(c, ECB_ERR_INVALID, "max_read %lld is neither 0 nor in [%d, %lld]", (long long)value,
+                    ECB_MAX_READ_ALIGNMENTS, (long long)ECB_MAX_READ_LIMIT);
+      c->max_read = value ? value : ECB_MAX_READ_LIMIT; break;
     default: return fail(c, ECB_ERR_INVALID, "unknown option %d", option);
   }
   return ECB_OK;
@@ -712,6 +801,7 @@ static int push_one(ecb_ctx* c, const int32_t* read_group, const int32_t* target
   const size_t ov_words = ((size_t)n + 31) / 32;
   CKR(ensure(c, c->overflow_bits, ov_words * 4));
   CK(cudaMemsetAsync(c->overflow_bits.p, 0, ov_words * 4, c->stream));
+  CKR(ensure(c, c->lr_list, ((size_t)n / (ECB_MAX_READ_ALIGNMENTS + 1) + 1) * sizeof(uint2)));
 
   const u32 e_before = c->n_ec;
   CKR(group_prepare_launch(c));
@@ -728,8 +818,21 @@ static int push_one(ecb_ctx* c, const int32_t* read_group, const int32_t* target
   CK(cudaEventRecord(c->ev[2], c->stream));
   CKR(sync_counters(c));
   CKR(check_device_error(c));
+  // reads longer than ECB_MAX_READ_ALIGNMENTS: the sort-based pass (only when the grouping kernel deferred some)
+  const u32 n_def = c->h_ctr->n_deferred;
+  LongParams L{};
+  float long_ms = 0;
+  if (n_def) {
+    CK(cudaEventRecord(c->ev[5], c->stream));
+    CKR(long_keys(c, P, tg, hp, n_def, &L));
+    CK(cudaEventRecord(c->ev[6], c->stream));
+    CKR(sync_counters(c));
+    CKR(check_device_error(c));
+    CK(cudaEventElapsedTime(&long_ms, c->ev[5], c->ev[6]));
+  }
   DevBuf spill_in;
-  while (c->h_ctr->n_overflow || c->h_ctr->n_spill) {  // table too full: grow, then replay just what did not fit
+  // table too full: grow, then replay just what did not fit
+  while (c->h_ctr->n_overflow || c->h_ctr->n_spill || c->h_ctr->n_deferred_fail) {
     c->stats.overflow_reads += c->h_ctr->n_overflow;
     const u32 n_spill = c->h_ctr->n_spill;
     if (c->table_slots >= (1u << 31)) return fail(c, ECB_ERR_LIMIT, "EC table cannot grow beyond 2^31 slots");
@@ -750,6 +853,11 @@ static int push_one(ecb_ctx* c, const int32_t* read_group, const int32_t* target
           P, (const EcbSpill*)spill_in.p, n_spill);
       LAUNCH_CHECK("spill_replay");
     }
+    if (c->h_ctr->n_deferred_fail) {   // the deferred reads still pending go in again; their keys are kept
+      CK(cudaMemsetAsync(&c->d_ctr->n_deferred_fail, 0, sizeof(u32), c->stream));
+      ecb_long_insert_kernel<<<grid_for(n_def, ECB_LONG_THREADS, c->sm_count), ECB_LONG_THREADS, 0, c->stream>>>(P, L);
+      LAUNCH_CHECK("long_insert");
+    }
     CKR(sync_counters(c));
     CKR(check_device_error(c));
   }
@@ -760,6 +868,12 @@ static int push_one(ecb_ctx* c, const int32_t* read_group, const int32_t* target
   CK(cudaEventRecord(c->ev[3], c->stream));
   CKR(harvest_new_rows(c, rg, tg, hp, n, e_before, c->n_ec));
   CK(cudaEventRecord(c->ev[4], c->stream));
+  if (n_def) {
+    CK(cudaEventRecord(c->ev[5], c->stream));
+    CKR(long_rows(c, L));
+    CK(cudaEventRecord(c->ev[6], c->stream));
+    CK(cudaMemsetAsync(&c->d_ctr->n_deferred, 0, sizeof(u32), c->stream));   // the list is empty for the next push
+  }
   if (c->verify_keys) {
     VerifyParams V{};
     V.rg = rg; V.tg = tg; V.hp = hp; V.n = (int)n; V.drop_last = drop_last_group;
@@ -779,7 +893,12 @@ static int push_one(ecb_ctx* c, const int32_t* read_group, const int32_t* target
   float ms = 0;
   CK(cudaEventElapsedTime(&ms, c->ev[1], c->ev[2])); c->stats.group_ms = ms;
   CK(cudaEventElapsedTime(&ms, c->ev[3], c->ev[4])); c->stats.harvest_ms = ms;
-  CK(cudaEventElapsedTime(&ms, c->ev[0], c->ev[4])); c->stats.push_ms = ms;
+  CK(cudaEventElapsedTime(&ms, c->ev[0], n_def ? c->ev[6] : c->ev[4])); c->stats.push_ms = ms;
+  if (n_def) {
+    CK(cudaEventElapsedTime(&ms, c->ev[5], c->ev[6]));
+    c->stats.long_reads += n_def;
+    c->stats.long_ms += long_ms + ms;
+  }
 
   c->min_base = std::min<u64>(c->min_base, (u64)order_base);
   c->max_end = std::max<u64>(c->max_end, (u64)order_base + (u64)n);
@@ -850,6 +969,8 @@ int ecb_push(ecb_ctx* c, const int32_t* read_group, const int32_t* target_idx, c
   CK(cudaSetDevice(c->device));
   if (!c->table_slots) CKR(init_table(c, n));
   const u32 push_id = c->push_count++;
+  c->stats.long_reads = 0;   // "the last push": summed over the pieces of a pipelined push
+  c->stats.long_ms = 0;
   if (n == 0) return ECB_OK;
   if (!on_device && n >= 2 * ECB_PIPE_PIECE)
     return push_pipelined(c, read_group, target_idx, hap_idx, cell_idx, n, order_base, drop_last_group, push_id);
@@ -1637,7 +1758,7 @@ int ecb_destroy(ecb_ctx* c) {
   if (c->stream) cudaStreamSynchronize(c->stream);
   DevBuf* bufs[] = {&c->table, &c->ec_slot, &c->ec_rep, &c->ec_len, &c->spill, &c->row_len, &c->row_off, &c->arena, &c->long_list, &c->mid_list, &c->big_list, &c->count_of,
                     &c->ttable, &c->st_rg, &c->st_tg, &c->st_hp, &c->st_cell, &c->st2_rg, &c->st2_tg, &c->st2_hp, &c->st2_cell,
-                    &c->overflow_bits,
+                    &c->overflow_bits, &c->lr_list, &c->lr_meta, &c->lr_rank, &c->lr_acc,
                     &c->scan_partials, &c->bitmap, &c->word_rank, &c->first_rel, &c->ecid_of, &c->ec_keep,
                     &c->r_a_indptr, &c->r_a_indices, &c->r_a_data, &c->r_n_indptr, &c->r_n_indices,
                     &c->r_n_data, &c->r_cell_order, &c->cx_kept, &c->cx_col_of_cell, &c->cx_col_counts};

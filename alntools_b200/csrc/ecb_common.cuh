@@ -139,6 +139,8 @@ struct EcbCounters {
   u32 chunk_next;     // next unclaimed chunk of the grouping kernel (reset before every launch)
   u64 arena_used;     // (target, mask) pairs in the row arena
   u32 scratch[8];
+  u32 n_deferred;     // reads of the current push longer than ECB_MAX_READ_ALIGNMENTS (ecb_longread.cuh)
+  u32 n_deferred_fail;// ... of them that found the table too full (inserted again after a growth)
 };
 
 #define ECB_DEVERR_EC_CAPACITY 1u   // provisional id space exhausted

@@ -77,6 +77,8 @@ struct GroupParams {
   EcbEntry* ttable;    // (file, EC slot, cell) table, with cells only
   u32 tmask;
   u32 push_id;
+  int max_read;        // longest read accepted (ECB_OPT_MAX_READ)
+  uint2* deferred;     // [ctr->n_deferred] (offset, length) of the reads longer than ECB_MAX_READ_ALIGNMENTS
 };
 
 // Probe for `key` from `slot` on (linear probing, at most max_probe slots): find it or claim the
@@ -385,10 +387,14 @@ struct LongRead {
 
 // Key and length of a read that starts at w and fills a whole window (>= 32 alignments).
 // Warp-cooperative: walks the read in blocks of 32; duplicates inside a block come from one
-// match, duplicates against the earlier blocks of the read from shuffled compares.
+// match, duplicates against the earlier blocks of the read from shuffled compares.  A read longer than
+// ECB_MAX_READ_ALIGNMENTS stops the compares once it passes that length (the walk to its end goes on):
+// up to max_read it is deferred to the sort-based pass of ecb_longread.cuh (its key here is not used),
+// beyond it the push fails.  The read the push drops (its last alignment is drop_pos) is not deferred.
 __device__ __noinline__ LongRead ecb_long_read(const int32_t* __restrict__ rg, const int32_t* __restrict__ tg,
                                                const int32_t* __restrict__ hp, int n, int w, int n_targets,
-                                               int n_haps, EcbCounters* ctr) {
+                                               int n_haps, EcbCounters* ctr, int max_read, int drop_pos,
+                                               uint2* deferred) {
   const int lane = threadIdx.x & 31;
   const u32 lt_mask = (1u << lane) - 1u;
   const int rg0 = rg[w];
@@ -419,7 +425,10 @@ __device__ __noinline__ LongRead ecb_long_read(const int32_t* __restrict__ rg, c
     if (len > ECB_MAX_READ_ALIGNMENTS) too_long = true;
   }
   if (bad) atomicOr(&ctr->error, ECB_DEVERR_VALUE_RANGE);
-  if (too_long && lane == 0) atomicOr(&ctr->error, ECB_DEVERR_READ_TOO_LONG);
+  if (len > ECB_MAX_READ_ALIGNMENTS && lane == 0) {
+    if (len > max_read) atomicOr(&ctr->error, ECB_DEVERR_READ_TOO_LONG);
+    else if (w + len - 1 != drop_pos) deferred[atomicAdd(&ctr->n_deferred, 1u)] = make_uint2((u32)w, (u32)len);
+  }
   sum.a = __reduce_add_sync(ECB_FULL, sum.a);
   sum.b = __reduce_add_sync(ECB_FULL, sum.b);
   sum.c = __reduce_add_sync(ECB_FULL, sum.c);
@@ -512,12 +521,13 @@ __global__ void __launch_bounds__(ECB_GTHREADS, 1) ecb_group_insert_kernel(const
       int wnext;
       if (hb == 1u) {
         // one read fills the window
-        const LongRead lr = ecb_long_read(c_rg, c_tg, c_hp, n, w, P.n_targets, P.n_haps, P.ctr);
+        const LongRead lr = ecb_long_read(c_rg, c_tg, c_hp, n, w, P.n_targets, P.n_haps, P.ctr, P.max_read, drop_pos,
+                                          P.deferred);
         key = lr.key;
         s = (u32)w;
         len = (u32)lr.len;
         wnext = w + lr.len;
-        ins = lane == 0 && wnext - 1 != drop_pos;
+        ins = lane == 0 && wnext - 1 != drop_pos && lr.len <= ECB_MAX_READ_ALIGNMENTS;
       } else {
         const int last_head = 31 - __clz(hb);          // >= 1; lanes below it form complete reads
         const int st = 31 - __clz(hb & le_mask);       // lane of this alignment's read start
@@ -744,6 +754,9 @@ struct VerifyParams {
 __global__ void __launch_bounds__(256) ecb_verify_kernel(const VerifyParams P) {
   for (int s = blockIdx.x * blockDim.x + threadIdx.x; s < P.n; s += gridDim.x * blockDim.x) {
     if (s > 0 && P.rg[s] == P.rg[s - 1]) continue;   // not a read start
+    int end = s + 1;
+    while (end < P.n && P.rg[end] == P.rg[s]) ++end;
+    if (end - s > ECB_MAX_READ_ALIGNMENTS) continue;   // deferred: verified by ecb_long_verify_kernel
     int len = 0;
     const Key128 key = ecb_serial_read_key(P.rg, P.tg, P.hp, P.n, s, &len);
     if (P.drop_last && s + len == P.n) continue;

@@ -84,10 +84,10 @@ __global__ void __launch_bounds__(256) ecb_harvest_short_kernel(const HarvestPar
     const u32 k = in ? P.ec_len[e] : 0u;
     warp_append(P.mid_list, &P.ctr->scratch[1], in && k > 8 && k <= 32, e);
     warp_append(P.big_list, &P.ctr->scratch[3], in && k > 32 && k <= HARVEST_WSORT_MAX, e);
-    if (in && k > HARVEST_WSORT_MAX) {
-      if (k > HARVEST_LONG_MAX) atomicOr(&P.ctr->error, ECB_DEVERR_READ_TOO_LONG);
-      P.long_list[atomicAdd(&P.ctr->n_long, 1u)] = e;
-    }
+    // ECs first met in a read longer than HARVEST_LONG_MAX get their rows from the long-read pass
+    // (ecb_longread.cuh); the grouping kernel has checked every read against the limit
+    const bool deferred = in && k > HARVEST_LONG_MAX;
+    if (in && k > HARVEST_WSORT_MAX && !deferred) P.long_list[atomicAdd(&P.ctr->n_long, 1u)] = e;
     const bool mine = in && k <= 8;
     const int s = (int)(mine ? P.ec_rep[e] : 0u);
     u32 c[8];
@@ -118,9 +118,9 @@ __global__ void __launch_bounds__(256) ecb_harvest_short_kernel(const HarvestPar
     // length as the upper bound of the row length (rows need not be packed: row_off / row_len index them),
     // so those kernels need no reservation of their own - one atomic per EC on the arena cursor was most of
     // their time on heavily multimapping input
-    const u32 want = mine ? cnt : (in ? min(k, (u32)HARVEST_LONG_MAX) : 0u);
+    const u32 want = mine ? cnt : (in && !deferred ? k : 0u);
     const u32 off = harvest_block_reserve(P.ctr, want, s_scan);
-    if (in && !mine) P.row_off[e] = off;
+    if (in && !mine && !deferred) P.row_off[e] = off;
     if (!mine) continue;
     uint2* out = P.arena + off;
     u32 w = 0, prev_t = 0xFFFFFFFFu, mask = 0;

@@ -148,6 +148,22 @@ def collate_budget():
     return int(value)
 
 
+def max_read():
+    """Longest read (alignments with one name) a conversion accepts, from the environment variable
+    ALNTOOLS_B200_MAX_READ (a non-negative integer; unset: 16384, the library's default; 0: no limit below the push
+    limit of 2^31 - 8192).  Reads longer than 16384 alignments then go through a sort-based pass on the GPU.  The
+    default is kept because in a file grouped by name a read that long more often means a broken input; values from 1
+    to 16383 are refused by the library.  The CLI keeps the reference's options, so the environment is its only way to
+    say it."""
+    import os
+    value = os.environ.get("ALNTOOLS_B200_MAX_READ", "").strip()
+    if not value:
+        return 16384
+    if not (value.isascii() and value.isdigit()):
+        raise ValueError("ALNTOOLS_B200_MAX_READ must be a non-negative integer (alignments), not %r" % (value,))
+    return int(value)
+
+
 Mode = collections.namedtuple("Mode", ["python", "decode", "collate", "launcher", "gpus"])
 
 

@@ -47,7 +47,8 @@ enum ecb_status {
   ECB_ERR_FORMAT = -7       /* malformed BAM input of the device decoder (ecb_bam_decode; since version 2002) */
 };
 
-/* Longest read (alignments sharing one name) whose canonical row can be built. */
+/* Longest read (alignments sharing one name) a push accepts by default, and the longest one the grouping kernel
+ * keys inline.  ECB_OPT_MAX_READ raises the limit: longer reads then take a sort-based pass of their own. */
 #define ECB_MAX_READ_ALIGNMENTS 16384
 /* target_idx < 2^26 and hap_idx < 31 (the EC file stores the haplotype mask in an int32,
  * alntools/bin_utils.py:232). */
@@ -74,6 +75,14 @@ enum ecb_option {
   ECB_OPT_COLLATE_BUDGET = 12,  /* device bytes a collator may hold, read at ecb_collate_create (0 = automatic: half
                                    of the device's free memory at that moment, the rest is left to the context's EC
                                    table and results; since version 2004) */
+  ECB_OPT_MAX_READ = 13,        /* longest read a push accepts (default ECB_MAX_READ_ALIGNMENTS; 0 = the push limit,
+                                   2^31 - 8192; other values below ECB_MAX_READ_ALIGNMENTS are ECB_ERR_INVALID).  A
+                                   longer read fails the push with ECB_ERR_LIMIT.  Reads above ECB_MAX_READ_ALIGNMENTS
+                                   are deferred by the grouping kernel and keyed, counted and given their rows by a
+                                   sort of their alignments on the device (24 bytes per such alignment while it
+                                   runs); shorter reads take the inline path either way.  The default stays as it
+                                   is because in a file grouped by name so long a read is more often a broken input
+                                   than a real one.  Since version 2005 */
 };
 
 typedef struct ecb_result {
@@ -105,6 +114,9 @@ typedef struct ecb_stats {
   int64_t h2d_bytes;      /* bytes copied host->device since create/reset                         */
   int64_t d2h_bytes;      /* bytes copied device->host since create/reset                         */
   int64_t row_entries;    /* (target, mask) pairs reserved in the row arena (upper bound of nnz)   */
+  /* since version 2005 */
+  int64_t long_reads;     /* reads longer than ECB_MAX_READ_ALIGNMENTS in the last push (deferred) */
+  double long_ms;         /* device time of the deferred pass of the last push                    */
 } ecb_stats;
 
 /* Library/ABI version (major*1000 + minor). */
@@ -344,7 +356,7 @@ int ecb_bam_destroy(ecb_bam* d);
  * ecb_collate_push: regroup everything added in device memory and push it into the context (ecb_push with
  *   on_device = 1, order_base = offset in collated order, in pieces of at most ECB_OPT_COLLATE_PIECE alignments that
  *   end at read ends; a longer read is a piece of its own).  Once per collator; *n_reads = reads formed.  The
- *   context's limits apply: a read of more than ECB_MAX_READ_ALIGNMENTS alignments fails with ECB_ERR_LIMIT.
+ *   context's limits apply: a read of more than ECB_OPT_MAX_READ alignments fails with ECB_ERR_LIMIT.
  * Device memory: while the one-pass collation of the alignments added so far fits the budget (ECB_OPT_COLLATE_BUDGET;
  * 88 to 144 bytes per alignment with the automatic table, DESIGN.md section 6.2), the rows stay on the device as above.
  * An add that would pass it spills: the rows go to host memory (28 bytes per alignment), partitioned into 4096 buckets
@@ -354,7 +366,8 @@ int ecb_bam_destroy(ecb_bam* d);
  * alignments with the per-read counts and offsets (n/4 + 8 bytes per read), or one bucket's names pass fails with
  * ECB_ERR_LIMIT and a message naming the budget; so does a ECB_OPT_COLLATE_PIECE that cuts a spilled collation into
  * more than 4096 pieces.  A piece holds at least one read, and a name table that runs out of probes grows, so those
- * two may pass the budget by what they need.  Running out of device memory otherwise fails with ECB_ERR_CUDA and the
+ * two may pass the budget by what they need; with ECB_OPT_MAX_READ raised, one long read can pass it by its own
+ * rows and the long-read pass of its push.  Running out of device memory otherwise fails with ECB_ERR_CUDA and the
  * allocator's message. */
 typedef struct ecb_collate ecb_collate;
 typedef struct ecb_collate_stats {
