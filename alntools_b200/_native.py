@@ -55,7 +55,14 @@ class EcbStats(ctypes.Structure):
     ]
 
     def as_dict(self):
-        return {name: getattr(self, name) for name, _ in self._fields_}
+        return {name: getattr(self, name) for cls in reversed(type(self).__mro__)
+                for name, _ in cls.__dict__.get("_fields_", ())}
+
+
+class EcbStatsSamples(EcbStats):
+    """ecb_stats since version 2006: EcbStats (the layout up to version 2005), then the fields of the samples
+    (ecb_sample_close).  ecb_get_stats writes the whole of it."""
+    _fields_ = [("samples", ctypes.c_int64), ("sample_pairs", ctypes.c_int64), ("sample_ms", ctypes.c_double)]
 
 
 class EcbSlice(ctypes.Structure):
@@ -134,6 +141,8 @@ SIGNATURES = {
     "ecb_push": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                 ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int, ctypes.c_int]),
     "ecb_finalize": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.POINTER(EcbResult)]),
+    "ecb_sample_close": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64)]),
+    "ecb_finalize_samples": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbResult)]),
     "ecb_reset": (ctypes.c_int, [ctypes.c_void_p]),
     "ecb_get_stats": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbStats)]),
     "ecb_destroy": (ctypes.c_int, [ctypes.c_void_p]),
@@ -287,8 +296,29 @@ class EcBuilder(object):
         (valid until the next finalize / reset / close): the EC file can be written straight from them."""
         if self._result_on_device:
             raise RuntimeError("finalize() needs host results; use finalize_raw() with result_on_device")
-        res = self.finalize_raw(min_cell_count)
+        return self._host_result(self.finalize_raw(min_cell_count), copy)
 
+    def close_sample(self):
+        """Close the current sample: the alignments pushed since the previous close (or since create / reset) are
+        one column of N.  Later pushes take order_base from 0 again (see ecb_sample_close).  -> the sample's
+        non-zero entries."""
+        nnz = ctypes.c_int64()
+        self._check(self._lib.ecb_sample_close(self._ctx, ctypes.byref(nnz)))
+        return int(nnz.value)
+
+    def finalize_samples_raw(self):
+        res = EcbResult()
+        self._check(self._lib.ecb_finalize_samples(self._ctx, ctypes.byref(res)))
+        return res
+
+    def finalize_samples(self, copy=True):
+        """As finalize(), with N holding one column per closed sample (ecb_finalize_samples)."""
+        if self._result_on_device:
+            raise RuntimeError("finalize_samples() needs host results; use finalize_samples_raw() with "
+                               "result_on_device")
+        return self._host_result(self.finalize_samples_raw(), copy)
+
+    def _host_result(self, res, copy):
         def arr(ptr, n):
             if n == 0:
                 return np.zeros(0, dtype=np.int32)
@@ -440,7 +470,7 @@ class EcBuilder(object):
                 "n_data": view(sl.n_data, sl.nnz_n)}
 
     def stats(self):
-        st = EcbStats()
+        st = EcbStatsSamples()
         self._check(self._lib.ecb_get_stats(self._ctx, ctypes.byref(st)))
         return st.as_dict()
 

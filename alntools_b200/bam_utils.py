@@ -11,7 +11,7 @@ import time
 
 import numpy as np
 
-from . import bamcols, bin_utils, emitter, utils
+from . import bam_io, bamcols, bin_utils, emitter, utils
 from ._native import EcBuilder
 from .header import TargetTables
 
@@ -326,3 +326,116 @@ def convert(bam_filename, ec_filename, emase_filename, num_chunks=0, number_proc
             # the files are written straight from the library's result buffers (no intermediate copies)
             return save(builder.finalize(copy=False), tables, valid, temp_time,
                         reader.references if range_filename is not None else None, ranges)
+
+
+def convert_samples(bam_files, ec_filename, sample_names=None, target_filename=None, range_filename=None, device=0,
+                    decode=None, collate=None, devices=None):
+    """Convert several BAM files, one per sample, into one EC file whose N matrix has one column per file.
+
+    Every file is read with the rules of the single-sample convert() (filters, name trimming, a new read at each
+    change of trimmed name; with collate=True each file is collated on its own), and a read never spans two files.
+    The ECs, their ids and the A matrix are those of convert() over the files' valid alignments back to back, in the
+    given order: an EC id is the rank of its first occurrence over the first file, then the second, and so on.  Entry
+    (e, s) of N is the number of reads of file s in EC e; a file without a valid alignment is an empty column.  So
+    files converted together share one EC index, which separately converted files do not.  With one file the EC
+    file is the bytes convert() writes.
+
+    sample_names: one name per file (default: each file's base name, as convert() names its sample).  Every file must
+    have the @SQ list (names and lengths) of the first; the targets and target_filename apply as in convert().
+    range_filename: the smallest and largest position per reference over all files.  decode / collate and the
+    environment variables ALNTOOLS_B200_DECODE, ALNTOOLS_B200_COLLATE, ALNTOOLS_B200_COLLATE_BUDGET,
+    ALNTOOLS_B200_MAX_READ and ALNTOOLS_B200_EMITTER=python work as for convert().  One GPU (`device`): more than one
+    GPU (devices, ALNTOOLS_GPUS or a launcher) and an EMASE (.h5) output raise NotImplementedError, before any file
+    is opened, as do no files or a number of names that differs from the number of files (ValueError)."""
+    start_time = time.time()
+    bam_files = list(bam_files)
+    if not bam_files:
+        raise ValueError("convert_samples needs at least one BAM file")
+    if sample_names is None:
+        sample_names = [os.path.basename(f) for f in bam_files]
+    sample_names = list(sample_names)
+    if len(sample_names) != len(bam_files):
+        raise ValueError("%d sample names for %d BAM files" % (len(sample_names), len(bam_files)))
+    if str(ec_filename).lower().endswith(".h5"):
+        raise NotImplementedError("convert_samples writes EC files only; an EMASE (.h5) file of several samples is "
+                                  "not supported")
+    mode = emitter.resolve_mode(False, devices, decode, collate, range_filename is not None)
+    if mode.launcher or mode.gpus > 1:
+        raise NotImplementedError("convert_samples runs on one GPU (unset ALNTOOLS_GPUS, or run it outside a "
+                                  "multi-GPU launcher)")
+    budget = emitter.collate_budget() if mode.collate else 0
+    limit = emitter.max_read()
+
+    def header(path):
+        if mode.python:
+            h = bam_io.read_header(path)
+            return h.references, h.lengths
+        with bamcols.BamColumnReader(path, n_threads=1) as reader:
+            return reader.references, reader.lengths
+
+    first = header(bam_files[0])
+    for path in bam_files[1:]:
+        if header(path) != first:
+            raise ValueError("%s does not have the @SQ list (names and lengths) of %s" % (path, bam_files[0]))
+
+    track = range_filename is not None
+    references = ranges = None
+    valid = 0
+    if mode.python:
+        tables = TargetTables(first[0], first[1], target_filename)
+        section = tables.target_section()
+        builder = EcBuilder(tables.num_targets, tables.num_haplotypes, alignments_hint=0, device=device,
+                            pageable_results=1, max_read=limit)
+    else:
+        with bamcols.BamColumnReader(bam_files[0], n_threads=1) as reader:
+            tables = reader.build_tables(target_filename)
+            section = tables.target_section()
+            references = reader.references if track else None
+        builder = EcBuilder(tables.num_targets, tables.num_haplotypes, alignments_hint=0, device=device,
+                            pageable_results=1, collate_budget=budget, max_read=limit)
+    with builder:
+        for path in bam_files:
+            if mode.python:
+                _, records = emitter.read_bam(path)
+                cols = emitter.emit_collated(records, tables) if mode.collate else emitter.emit_single(records, tables)
+                if cols.valid_alignments:
+                    builder.push(cols.read_group, cols.target_idx, cols.hap_idx, order_base=0)
+                n, lo_hi = cols.valid_alignments, None
+            else:
+                n, lo_hi = _stream_sample(path, builder, tables, mode, track)
+            builder.close_sample()                         # later pushes count their order keys from 0 again
+            valid += n
+            if lo_hi is not None:
+                ranges = lo_hi if ranges is None else (np.minimum(ranges[0], lo_hi[0]), np.maximum(ranges[1], lo_hi[1]))
+        if valid == 0:
+            raise RuntimeError("The shape must be a tuple of three positive integers.")   # as convert()
+        res = builder.finalize_samples(copy=False)
+        LOG.info("# Samples: {:,}".format(len(bam_files)))
+        LOG.info("# Valid Alignments: {:,}".format(valid))
+        LOG.info("# Equivalence Classes: {:,}".format(res["n_ec"]))
+        LOG.info("# Unique Reads: {:,}".format(res["n_reads"]))
+        bin_utils.save_outputs(tables, section, sample_names, (res["a_indptr"], res["a_indices"], res["a_data"]),
+                               (res["n_indptr"], res["n_indices"], res["n_data"]), False, ec_filename, None,
+                               range_filename, references, ranges)
+    LOG.info("{} created, total time: {}".format(ec_filename, utils.format_time(start_time, time.time())))
+    return {k: v for k, v in res.items() if not hasattr(v, "shape")}
+
+
+def _stream_sample(path, builder, tables, mode, track_ranges):
+    """One file of convert_samples through the feed convert() uses for `mode`, with order keys from 0.
+    -> (valid alignments, (range_min, range_max) or None)."""
+    import torch
+    pinned = torch.cuda.is_available()
+    with bamcols.BamColumnReader(path, n_threads=0) as reader:
+        reader.set_tables(tables)
+        if track_ranges and mode.decode == "host":
+            reader.track_ranges(True)
+        chunk_rows = int(min(1 << 21, max(1 << 16, os.path.getsize(path) // 2)))
+        if mode.decode == "device":
+            valid, _, ranges, _ = emitter.stream_single_device(path, reader, builder, tables, track_ranges)
+            return valid, ranges
+        if mode.collate:
+            valid, _, _ = emitter.stream_collated(reader, builder, chunk_rows=chunk_rows, pinned=pinned)
+        else:
+            valid = emitter.stream_single(reader, builder, chunk_rows=chunk_rows, pinned=pinned)
+        return valid, reader.ranges() if track_ranges else None

@@ -73,3 +73,22 @@ def ec2emase(ec_file, emase_file, verbose):
     """Convert a binary EC format file (ec_file) to EMASE format (emase_file)"""
     utils.configure_logging(verbose)
     methods.ec2emase(ec_file, emase_file)
+
+
+@cli.command('bam2ec-samples', options_metavar='<options>', short_help='convert several BAM files to one EC file')
+@click.argument('ec_file', metavar='ec_file', type=click.Path(resolve_path=True, dir_okay=False, writable=True))
+@click.argument('bam_files', metavar='bam_file...', nargs=-1, required=True,
+                type=click.Path(exists=True, resolve_path=True, dir_okay=False))
+@click.option('-s', '--sample', 'samples', multiple=True, help="sample identifier, once per bam_file, in order")
+@click.option('--rangefile', type=click.Path(exists=False, resolve_path=True, file_okay=True, dir_okay=False,
+                                             writable=True), help="range file")
+@click.option('-t', '--targets', metavar='FILE', type=click.Path(exists=True, resolve_path=True, file_okay=True,
+                                                               dir_okay=False), help="target file")
+@click.option('-v', '--verbose', count=True, help='enables verbose mode')
+def bam2ec_samples(ec_file, bam_files, samples, rangefile, targets, verbose):
+    """Convert BAM files (bam_file..., one per sample, read as bam2ec reads one) to one binary EC file (ec_file)
+    with one column per sample over one shared EC index"""
+    from . import bam_utils
+    utils.configure_logging(verbose)
+    bam_utils.convert_samples(list(bam_files), ec_file, sample_names=list(samples) or None, target_filename=targets,
+                              range_filename=rangefile)

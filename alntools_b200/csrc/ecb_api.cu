@@ -22,6 +22,7 @@
 #include "ecb_bam.cuh"
 #include "ecb_collate.cuh"
 #include "ecb_longread.cuh"
+#include "ecb_samples.cuh"
 
 #define ECB_PUSH_LIMIT (0x7FFFFFFFll - 8192)   // alignments of one ecb_push
 // Largest ECB_OPT_MAX_READ, and what 0 stands for: the push limit as documented (2^31 - 8192), one more than the
@@ -107,6 +108,15 @@ struct ecb_ctx {
   // per-cell exchange: kept reads per local EC, column of every global cell, entries per column of the slice
   DevBuf cx_kept, cx_col_of_cell, cx_col_counts;
   u32 cx_n_local_cells = 0;
+  // samples (ecb_sample_close): every EC's count at the last close (provisional ids below smp_n_ec), the
+  // (provisional id, reads) pairs of the closed samples, pairs per sample, the order key where the open sample starts
+  // and the alignments pushed into it
+  DevBuf smp_last, smp_pairs;
+  u32 smp_n_ec = 0;
+  u64 smp_n_pairs = 0;
+  std::vector<u32> smp_counts;
+  u64 smp_base = 0;
+  int64_t smp_open = 0;
   std::string err;
 };
 
@@ -636,6 +646,37 @@ int cells_emit(ecb_ctx* c, CellResult* cr, const u32* ecid_of, u64 n_ec_final) {
   return ECB_OK;
 }
 
+// N of ecb_finalize_samples (CSC, one column per closed sample) from the pairs and the final EC ids: the pairs per
+// sample, uploaded and scanned, are n_indptr; the pairs, keyed by (sample, EC id) and sorted, are the entries.
+int samples_emit(ecb_ctx* c, u64 n_ec_final) {
+  CellScratch& S = c->cells;
+  const u32 n_samples = (u32)c->smp_counts.size();
+  const u32 nnz = (u32)c->smp_n_pairs;   // checked against 2^31 - 1 by the caller
+  CKR(ensure(c, c->r_n_indptr, ((size_t)n_samples + 1) * 4));
+  CKR(ensure(c, c->r_n_indices, std::max<size_t>(nnz, 1) * 4));
+  CKR(ensure(c, c->r_n_data, std::max<size_t>(nnz, 1) * 4));
+  CK(cudaMemcpyAsync(c->r_n_indptr.p, c->smp_counts.data(), (size_t)n_samples * 4, cudaMemcpyHostToDevice, c->stream));
+  CK(cudaMemsetAsync((u32*)c->r_n_indptr.p + n_samples, 0, 4, c->stream));
+  c->stats.h2d_bytes += (int64_t)n_samples * 4;
+  CKR(device_scan<false>(c, (const u32*)c->r_n_indptr.p, (u32*)c->r_n_indptr.p, (u64)n_samples + 1, 0, nullptr));
+  if (nnz == 0) return ECB_OK;
+  CKR(ensure(c, S.sort_k[0], (size_t)nnz * 8));
+  CKR(ensure(c, S.sort_v[0], (size_t)nnz * 4));
+  const int ec_bits = bits_for(n_ec_final);
+  const int g = grid_for(nnz, 256, c->sm_count * 8);
+  ecb_sample_keys_kernel<<<g, 256, 0, c->stream>>>((const uint2*)c->smp_pairs.p, nnz, (const int32_t*)c->r_n_indptr.p,
+                                                   n_samples, (const u32*)c->ecid_of.p, ec_bits, (u64*)S.sort_k[0].p,
+                                                   (u32*)S.sort_v[0].p);
+  LAUNCH_CHECK("sample_keys");
+  int rb = 0;
+  CKR(radix_sort(c, nnz, ec_bits + bits_for(n_samples), &rb));
+  ecb_sample_csc_kernel<<<g, 256, 0, c->stream>>>((const u64*)S.sort_k[rb].p, (const u32*)S.sort_v[rb].p, nnz,
+                                                  (1ull << ec_bits) - 1, (int32_t*)c->r_n_indices.p,
+                                                  (int32_t*)c->r_n_data.p);
+  LAUNCH_CHECK("sample_csc");
+  return ECB_OK;
+}
+
 void cells_release(ecb_ctx* c) {
   CellScratch& S = c->cells;
   DevBuf* bufs[] = {&S.fe_table, &S.pair_table, &S.cell_key, &S.cell_total, &S.cell_new, &S.sort_k[0], &S.sort_k[1],
@@ -647,7 +688,7 @@ void cells_release(ecb_ctx* c) {
 
 extern "C" {
 
-int ecb_version(void) { return 2005; }
+int ecb_version(void) { return 2006; }
 
 const char* ecb_last_error(const ecb_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
@@ -972,13 +1013,15 @@ int ecb_push(ecb_ctx* c, const int32_t* read_group, const int32_t* target_idx, c
   c->stats.long_reads = 0;   // "the last push": summed over the pieces of a pipelined push
   c->stats.long_ms = 0;
   if (n == 0) return ECB_OK;
+  c->smp_open += n;
+  order_base += (int64_t)c->smp_base;   // 0 until a sample is closed
   if (!on_device && n >= 2 * ECB_PIPE_PIECE)
     return push_pipelined(c, read_group, target_idx, hap_idx, cell_idx, n, order_base, drop_last_group, push_id);
   return push_one(c, read_group, target_idx, hap_idx, cell_idx, n, order_base, drop_last_group, on_device, push_id);
 }
 
-int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
-  if (!c || !out) return ECB_ERR_INVALID;
+// ecb_finalize, and with samples ecb_finalize_samples: the same A and EC ids, N from the closed samples' pairs.
+static int finalize(ecb_ctx* c, int64_t min_cell_count, bool samples, ecb_result* out) {
   memset(out, 0, sizeof *out);
   CK(cudaSetDevice(c->device));
   if (!c->table_slots || c->n_ec == 0) return fail(c, ECB_ERR_EMPTY, "no equivalence classes (nothing pushed)");
@@ -1036,7 +1079,7 @@ int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
 
   CKR(ensure(c, c->r_a_indptr, (E + 1) * 4));
   F.a_indptr = (int32_t*)c->r_a_indptr.p;
-  if (!c->with_cells) {
+  if (!c->with_cells && !samples) {
     CKR(ensure(c, c->r_n_indptr, 2 * 4));
     CKR(ensure(c, c->r_n_indices, E * 4));
     CKR(ensure(c, c->r_n_data, E * 4));
@@ -1044,7 +1087,7 @@ int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
     F.n_data = (int32_t*)c->r_n_data.p;
   }
   CK(cudaMemsetAsync((int32_t*)c->r_a_indptr.p + E, 0, 4, c->stream));
-  if (c->with_cells) ecb_fin_rank_kernel<false><<<g_ec, 256, 0, c->stream>>>(F);
+  if (c->with_cells || samples) ecb_fin_rank_kernel<false><<<g_ec, 256, 0, c->stream>>>(F);
   else ecb_fin_rank_kernel<true><<<g_ec, 256, 0, c->stream>>>(F);
   LAUNCH_CHECK("fin_rank");
   // row lengths -> indptr; the rows follow at once: the arena's fill (known on the host since the last push)
@@ -1064,6 +1107,7 @@ int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
   LAUNCH_CHECK("fin_rows_long");
   CellResult cr2 = cr;
   if (c->with_cells) CKR(cells_emit(c, &cr2, (const u32*)c->ecid_of.p, E));   // N matrix as CSC
+  else if (samples) CKR(samples_emit(c, E));
   else {
     ecb_set_pair_kernel<<<1, 1, 0, c->stream>>>((int32_t*)c->r_n_indptr.p, 0, (int32_t)E);
     LAUNCH_CHECK("set_pair");
@@ -1080,6 +1124,9 @@ int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
   if (c->with_cells) {
     n_samples = cr2.n_kept_cells;
     nnz_n = cr2.nnz_n;
+  } else if (samples) {
+    n_samples = (int64_t)c->smp_counts.size();
+    nnz_n = (int64_t)c->smp_n_pairs;
   }
 
   out->n_ec = (int64_t)E;
@@ -1139,6 +1186,56 @@ int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
   return ECB_OK;
 }
 
+int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
+  if (!c || !out) return ECB_ERR_INVALID;
+  return finalize(c, min_cell_count, false, out);
+}
+
+int ecb_sample_close(ecb_ctx* c, int64_t* nonzeros) {
+  if (!c) return ECB_ERR_INVALID;
+  if (nonzeros) *nonzeros = 0;
+  if (c->with_cells) return fail(c, ECB_ERR_INVALID, "samples are closed on single-sample contexts only");
+  CK(cudaSetDevice(c->device));
+  const u32 n = c->table_slots ? c->n_ec : 0;   // current on the host: every push ends with a sync
+  u32 added = 0;
+  float ms = 0;
+  if (n) {
+    CKR(ensure(c, c->smp_last, (size_t)n * 4, true));
+    CKR(ensure(c, c->smp_pairs, (size_t)(c->smp_n_pairs + n) * sizeof(uint2), true));
+    CK(cudaEventRecord(c->ev[0], c->stream));
+    CK(cudaMemsetAsync(&c->d_ctr->scratch[6], 0, sizeof(u32), c->stream));
+    ecb_sample_close_kernel<<<grid_for(n, 256, c->sm_count * 8), 256, 0, c->stream>>>(
+        (const EcbEntry*)c->table.p, (const u32*)c->ec_slot.p, n, c->smp_n_ec, (u32*)c->smp_last.p,
+        (uint2*)c->smp_pairs.p + c->smp_n_pairs, &c->d_ctr->scratch[6]);
+    LAUNCH_CHECK("sample_close");
+    CK(cudaEventRecord(c->ev[1], c->stream));
+    CKR(sync_counters(c));   // the call's one round trip brings the pair count back
+    added = c->h_ctr->scratch[6];
+    CK(cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
+  }
+  c->smp_n_ec = n;
+  c->smp_n_pairs += added;
+  c->smp_counts.push_back(added);
+  c->smp_base = c->max_end;   // the next sample's order keys follow this one's
+  c->smp_open = 0;
+  c->stats.samples++;
+  c->stats.sample_pairs += added;
+  c->stats.sample_ms += ms;
+  if (nonzeros) *nonzeros = added;
+  return ECB_OK;
+}
+
+int ecb_finalize_samples(ecb_ctx* c, ecb_result* out) {
+  if (!c || !out) return ECB_ERR_INVALID;
+  memset(out, 0, sizeof *out);
+  if (c->with_cells) return fail(c, ECB_ERR_INVALID, "samples are closed on single-sample contexts only");
+  if (c->smp_open) return fail(c, ECB_ERR_INVALID, "%lld alignments were pushed after the last ecb_sample_close",
+                               (long long)c->smp_open);
+  if (c->smp_n_pairs > 0x7FFFFFFFull)
+    return fail(c, ECB_ERR_LIMIT, "N matrix has %llu non-zeros (more than 2^31-1)", (unsigned long long)c->smp_n_pairs);
+  return finalize(c, 0, true, out);
+}
+
 int ecb_reset(ecb_ctx* c) {
   if (!c) return ECB_ERR_INVALID;
   CK(cudaSetDevice(c->device));
@@ -1155,6 +1252,11 @@ int ecb_reset(ecb_ctx* c) {
   c->max_end = 0;
   c->n_alignments = 0;
   c->push_count = 0;
+  c->smp_n_ec = 0;
+  c->smp_n_pairs = 0;
+  c->smp_counts.clear();
+  c->smp_base = 0;
+  c->smp_open = 0;
   const int64_t slots = c->stats.table_slots;
   c->stats = ecb_stats{};
   c->stats.table_slots = slots;
@@ -1761,7 +1863,8 @@ int ecb_destroy(ecb_ctx* c) {
                     &c->overflow_bits, &c->lr_list, &c->lr_meta, &c->lr_rank, &c->lr_acc,
                     &c->scan_partials, &c->bitmap, &c->word_rank, &c->first_rel, &c->ecid_of, &c->ec_keep,
                     &c->r_a_indptr, &c->r_a_indices, &c->r_a_data, &c->r_n_indptr, &c->r_n_indices,
-                    &c->r_n_data, &c->r_cell_order, &c->cx_kept, &c->cx_col_of_cell, &c->cx_col_counts};
+                    &c->r_n_data, &c->r_cell_order, &c->cx_kept, &c->cx_col_of_cell, &c->cx_col_counts,
+                    &c->smp_last, &c->smp_pairs};
   for (DevBuf* b : bufs) release(c, *b);
   cells_release(c);
   if (c->stream) cudaStreamSynchronize(c->stream);

@@ -91,7 +91,8 @@ typedef struct ecb_result {
   const int32_t* a_indptr;   /* [E+1]  CSR row offsets of the A matrix (E x T)                    */
   const int32_t* a_indices;  /* [Z]    main-target index, ascending inside a row                  */
   const int32_t* a_data;     /* [Z]    haplotype bitmask, bit h = sorted-haplotype index h        */
-  int64_t n_samples;         /* S: 1 without cells; number of kept cells with cells               */
+  int64_t n_samples;         /* S: 1 without cells; number of kept cells with cells; samples closed
+                                by ecb_finalize_samples                                            */
   int64_t nnz_n;
   const int32_t* n_indptr;   /* [S+1]  CSC column offsets of the N matrix (E x S)                 */
   const int32_t* n_indices;  /* [nnz_n] EC ids, ascending inside a column                         */
@@ -117,6 +118,10 @@ typedef struct ecb_stats {
   /* since version 2005 */
   int64_t long_reads;     /* reads longer than ECB_MAX_READ_ALIGNMENTS in the last push (deferred) */
   double long_ms;         /* device time of the deferred pass of the last push                    */
+  /* since version 2006 */
+  int64_t samples;        /* samples closed since create/reset (ecb_sample_close)                  */
+  int64_t sample_pairs;   /* (EC, sample) entries they recorded                                    */
+  double sample_ms;       /* device time of the closes, summed                                     */
 } ecb_stats;
 
 /* Library/ABI version (major*1000 + minor). */
@@ -159,6 +164,32 @@ int ecb_push(ecb_ctx* ctx, const int32_t* read_group, const int32_t* target_idx,
  * Result buffers are library-owned (pinned host memory, or device memory with
  * ECB_OPT_RESULT_ON_DEVICE) and stay valid until the next finalize/reset/destroy. */
 int ecb_finalize(ecb_ctx* ctx, int64_t min_cell_count, ecb_result* out);
+
+/* ---- several samples in one single-sample context (since version 2006) ----------------------------------------
+ * An EC file holds an E x S count matrix N.  Files pushed one after the other into one single-sample context share
+ * its EC table, so EC identity, EC ids and the A matrix are those of one build over the concatenated columns: an EC id
+ * is the rank of the EC's first occurrence over sample 1, then sample 2, and so on.  Every way of pushing works
+ * unchanged inside a sample: host or device columns, several pushes, ecb_bam_decode, a collator, long reads, table
+ * growth and replay.
+ *
+ * ecb_sample_close: the alignments pushed since the previous close (or since create/reset) are one sample; an empty
+ *   sample is allowed.  One kernel compares every EC's count (read through the table after the pushes have completed)
+ *   with its count at the previous close and appends (provisional id, delta) for every delta > 0 to a device list
+ *   with one atomic per warp.  *nonzeros = the sample's pairs, brought back by the call's one host round trip.  From
+ *   then on, order_base of ecb_push counts from the end of the closed samples' order range (the largest
+ *   order_base + n pushed so far), so that every sample can be pushed from order_base 0, as one file on its own is.
+ * ecb_finalize_samples: A, the EC ids and the other fields as ecb_finalize; N (CSC) has one column per closed sample:
+ *   entry (e, s) is the reads of sample s in EC e, zeros are not stored, EC ids ascend inside a column and an empty
+ *   sample is an empty column.  The pairs get their EC ids, the LSD radix sort orders them by (sample, EC id) and the
+ *   scan of the pairs per sample gives n_indptr.  Results are delivered as by ecb_finalize (pinned, pageable or on
+ *   the device, valid until the next finalize/reset/destroy).  Fails with ECB_ERR_INVALID when alignments were
+ *   pushed after the last close, with ECB_ERR_LIMIT for more than 2^31 - 1 entries of N, and with ECB_ERR_EMPTY when
+ *   no sample holds a read.  ecb_finalize still gives the one-sample result of everything pushed.
+ * Both refuse contexts created with cells (ECB_ERR_INVALID).  ecb_reset forgets the samples.  Device memory: 4 bytes
+ * per EC for the counts at the last close and 8 bytes per pair; during ecb_finalize_samples the sort adds 24 bytes
+ * per pair and its histograms. */
+int ecb_sample_close(ecb_ctx* ctx, int64_t* nonzeros);
+int ecb_finalize_samples(ecb_ctx* ctx, ecb_result* out);
 
 /* Forget all pushed data but keep allocations (tables, staging) for the next job. */
 int ecb_reset(ecb_ctx* ctx);
