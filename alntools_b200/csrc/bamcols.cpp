@@ -48,14 +48,6 @@ struct BlockJob {
   size_t dst_off;
 };
 
-// One completed or growing read: its rows (the read_group value is the same for all of them).
-struct GroupRows {
-  std::vector<int32_t> tg, hp, cell;
-  int32_t group = 0;
-  size_t size() const { return tg.size(); }
-  void clear() { tg.clear(); hp.clear(); cell.clear(); }
-};
-
 }  // namespace
 
 // Cell dictionary: ids in order of first appearance (bam_utils_multisample.py:270-280).  Open addressing
@@ -202,10 +194,9 @@ struct bamcols {
   int64_t group = -1;
   bool pending = false;          // per-cell: the current read's cell is resolved at the next valid alignment
   int32_t cell = 0;
-  GroupRows cur, ready;
-  bool records_done = false, all_flushed = false;
+  bool records_done = false;
   int64_t all_alignments = 0;
-  // single-sample batch path: rows of the current inflated window, produced by all worker threads
+  // staged rows of the current inflated window, produced by all worker threads
   RawBuf<int32_t> st_rg, st_tg, st_hp, st_cell;
   RawBuf<uint64_t> st_klo, st_khi;   // key mode (bamcols_emit_keys): 128-bit name keys in place of read_group
   size_t pending_row = 0;       // per-cell: stage row whose cell is resolved by the next valid alignment
@@ -216,11 +207,10 @@ struct bamcols {
   std::vector<size_t> sc_cell_len;
   std::vector<uint64_t> sc_cell_hash;
   std::vector<int32_t> sc_cell_id, sc_group_cell;
-  bool sequential_cells = false; // BAMCOLS_SEQUENTIAL_CELLS: the one-pass statement of the per-cell rules
   size_t st_pos = 0;             // next row to hand out
   size_t st_whole = 0;           // rows [st_pos, st_whole) are whole reads; [st_whole, size) is the open last read
   std::vector<size_t> rec_off;   // scratch: record offsets of the window
-  std::vector<uint8_t> rec_flag; // scratch: bit 0 valid, bit 1 starts a read
+  std::vector<uint8_t> rec_flag; // scratch: per record of the window, see Window::fl
   int mode = 0;                  // 0 undecided, 1 single-sample, 2 per-cell, 3 name keys
   size_t grain = 4096;           // records per worker thread below which no further thread is used
   double phase_s[6] = {0, 0, 0, 0, 0, 0};  // inflate, record hop, validity, read starts, rows, copy-out
@@ -241,11 +231,16 @@ struct bamcols {
 
 namespace {
 
-struct PhaseTimer {
-  double* acc;
+// lap(p) adds the wall time since the previous lap, or since the clock was made, to phase p of bamcols::phase_s.
+struct PhaseClock {
+  double* phase_s;
   std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
-  explicit PhaseTimer(double* a) : acc(a) {}
-  ~PhaseTimer() { *acc += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count(); }
+  explicit PhaseClock(double* s) : phase_s(s) {}
+  void lap(int phase) {
+    const auto now = std::chrono::steady_clock::now();
+    phase_s[phase] += std::chrono::duration<double>(now - t0).count();
+    t0 = now;
+  }
 };
 
 int fail(bamcols* r, int code, const char* fmt, ...) {
@@ -322,7 +317,7 @@ struct Inflater {
 // sets file_done when the file has no more blocks.
 int refill(bamcols* r) {
   if (r->file_done) return 0;
-  PhaseTimer timer(&r->phase_s[0]);
+  PhaseClock clock(r->phase_s);
   // keep the unread tail at the front
   const size_t keep = r->wend - r->wpos;
   if (r->wpos > 0 && keep > 0) memmove(r->win.data(), r->win.data() + r->wpos, keep);
@@ -387,6 +382,7 @@ int refill(bamcols* r) {
   }
   if (bad.load()) return fail(r, BAMCOLS_ERR_FORMAT, "corrupt BGZF block (inflate failed) before offset %zu", r->cpos);
   r->wend = keep + total;
+  clock.lap(0);
   return 0;
 }
 
@@ -697,98 +693,66 @@ int find_records(bamcols* r, std::vector<size_t>& off, size_t* next) {
   return 0;
 }
 
-// Single-sample rules (bam_utils.py:258-328) over every whole record of the inflated window, on all
-// worker threads: (1) one sequential hop over the block_size fields finds the records, (2) validity
-// per record, (3) "starts a read" per valid record = its trimmed name differs from the previous valid
-// record's, (4) rows written at their final position (prefix sums over the threads).  The open last
-// read is held back (st_whole) until the next window or the end of the file closes it.
-// keys: the rows of bamcols_emit_keys instead - step (3) is skipped, every valid record gets the 128-bit key of its
-// trimmed name in place of a read_group, and every row is handed out at once (there are no reads to keep whole).
-int process_window_single(bamcols* r, bool keys = false) {
-  // rows still waiting from the previous window go to the front
-  const size_t left = r->st_tg.size() - r->st_pos;
-  auto shift = [&](auto& buf) {
-    if (r->st_pos > 0) memmove(buf.data(), buf.data() + r->st_pos, left * sizeof(buf[0]));
-    buf.resize(left);
-  };
-  if (keys) {
-    shift(r->st_klo);
-    shift(r->st_khi);
-  } else {
-    shift(r->st_rg);
-  }
-  shift(r->st_tg);
-  shift(r->st_hp);
-  r->st_whole -= r->st_pos;
-  r->st_pos = 0;
+// The reference's filter (bam_utils.py:264-270) with the record checks that come with it, for the record whose
+// block_size field is at `rec`.  The one statement of the filter on the host; ecb_bam_validity_kernel is the device's.
+enum { REC_FILTERED = 0, REC_VALID = 1, REC_BAD_NAME = 2, REC_BAD_TID = 3 };
+inline int record_validity(const uint8_t* rec, int32_t n_ref) {
+  const size_t bs = le32(rec);
+  const uint8_t* q = rec + 4;
+  const int32_t tid = (int32_t)le32(q);
+  const size_t l_name = q[8];
+  const uint32_t flag = le16(q + 14);
+  const int32_t ntid = (int32_t)le32(q + 20), npos = (int32_t)le32(q + 24);
+  if (32 + l_name > bs || l_name == 0) return REC_BAD_NAME;
+  if (flag & 0x4) return REC_FILTERED;
+  if ((flag & 0x1) && ((flag & 0x80) || !(flag & 0x2) || tid != ntid || npos < 0)) return REC_FILTERED;
+  if (tid < 0 || tid >= n_ref) return REC_BAD_TID;
+  return REC_VALID;
+}
 
-  // (1) records of the window
-  if (r->wend - r->wpos < 4 || r->wend - r->wpos < 4 + (size_t)le32(r->win.data() + r->wpos)) {
-    const int rc = refill(r);
-    if (rc < 0) return rc;
+// fn(column) for every staged column of the reader's mode, in the order of the caller's buffers:
+// read_group or the two key halves, target_idx, hap_idx, and cell_idx in per-cell mode.
+template <class F>
+void for_staged(bamcols* r, F fn) {
+  if (r->mode == 3) {
+    fn(r->st_klo);
+    fn(r->st_khi);
+  } else {
+    fn(r->st_rg);
   }
-  const uint8_t* base = r->win.data();
-  std::vector<size_t>& off = r->rec_off;
-  off.clear();
-  size_t p = r->wpos;
-  {
-    PhaseTimer timer(&r->phase_s[1]);
-    const int rc = find_records(r, off, &p);
-    if (rc < 0) return rc;
-  }
-  r->wpos = p;
-  const size_t n = off.size();
-  if (n == 0) {
-    if (r->file_done) {
-      if (r->wend != r->wpos) return fail(r, BAMCOLS_ERR_FORMAT, "truncated BAM record at the end of the file");
-      r->records_done = true;
-      r->st_whole = r->st_tg.size();  // the end of the file closes the last read
-    }
-    return 0;
-  }
-  r->all_alignments += (int64_t)n;
-  std::vector<uint8_t>& fl = r->rec_flag;
-  fl.assign(n, 0);
-  const int nt = (int)std::max<size_t>(1, std::min<size_t>((size_t)r->n_threads, n / r->grain + 1));
-  const int32_t n_ref = (int32_t)r->tid_target.size();
-  std::vector<size_t> n_valid(nt + 1, 0), n_start(nt + 1, 0);
-  std::atomic<int> bad(0);
-  auto lo = [&](int t) { return n * (size_t)t / (size_t)nt; };
-  // (2) validity (bam_utils.py:264-270)
-  PhaseTimer* timer = new PhaseTimer(&r->phase_s[2]);
-  parallel_for(nt, [&](int t) {
-    size_t cnt = 0;
-    for (size_t i = lo(t); i < lo(t + 1); ++i) {
-      const uint8_t* q = base + off[i] + 4;
-      const size_t bs = le32(base + off[i]);
-      const int32_t tid = (int32_t)le32(q);
-      const size_t l_name = q[8];
-      const uint32_t flag = le16(q + 14);
-      const int32_t ntid = (int32_t)le32(q + 20), npos = (int32_t)le32(q + 24);
-      if (32 + l_name > bs || l_name == 0) { bad.store(1); continue; }
-      if (flag & 0x4) continue;
-      if ((flag & 0x1) && ((flag & 0x80) || !(flag & 0x2) || tid != ntid || npos < 0)) continue;
-      if (tid < 0 || tid >= n_ref) { bad.store(2); continue; }
-      if (r->track_ranges) note_position(r, tid, (int32_t)le32(q + 4));
-      fl[i] = 1;
-      ++cnt;
-    }
-    n_valid[t + 1] = cnt;
-  });
-  delete timer;
-  if (bad.load() == 1) return fail(r, BAMCOLS_ERR_FORMAT, "BAM record with a bad read-name length");
-  if (bad.load() == 2) return fail(r, BAMCOLS_ERR_TID, "alignment with a reference id outside the header's %d references", n_ref);
-  // (3) read starts (bam_utils.py:301-306)
+  fn(r->st_tg);
+  fn(r->st_hp);
+  if (r->mode == 2) fn(r->st_cell);
+}
+
+// The whole records of one inflated window after the validity pass.  Worker t of nt takes the records
+// [lo(t), lo(t + 1)); their valid ones become rows n_valid[t] ... n_valid[t + 1] - 1 of the window, and in the
+// read-group modes they open reads n_start[t] + 1 ... n_start[t + 1], counted from the read that is open when
+// the window begins.
+struct Window {
+  const uint8_t* base;
+  const std::vector<size_t>& off;
+  std::vector<uint8_t>& fl;   // bit 0 valid, bit 3 starts a read (per-cell: bits 1 and 2 hold its two comparisons)
+  size_t n;
+  int nt;
+  std::vector<size_t> n_valid, n_start;
+  size_t lo(int t) const { return n * (size_t)t / (size_t)nt; }
+};
+
+// Single-sample read starts (bam_utils.py:301-306): a valid record starts a read iff its trimmed name differs
+// from the previous valid record's; the last valid record's trimmed name is remembered for the next window.
+void single_starts(bamcols* r, Window& w) {
+  const uint8_t* base = w.base;
+  std::vector<uint8_t>& fl = w.fl;
   const bool had_prev = r->started;
-  const std::string prev_name = r->current;
-  timer = new PhaseTimer(&r->phase_s[3]);
-  if (!keys) parallel_for(nt, [&](int t) {
+  const std::string& prev_name = r->current;
+  parallel_for(w.nt, [&](int t) {
     const char* pn = nullptr;  // trimmed name of the previous valid record
     size_t pl = 0;
     bool have = false;
-    for (size_t j = lo(t); j-- > 0;)
+    for (size_t j = w.lo(t); j-- > 0;)
       if (fl[j]) {
-        const uint8_t* q = base + off[j] + 4;
+        const uint8_t* q = base + w.off[j] + 4;
         pn = (const char*)q + 32;
         pl = trimmed_len(pn, (size_t)q[8] - 1);
         have = true;
@@ -800,188 +764,56 @@ int process_window_single(bamcols* r, bool keys = false) {
       have = true;
     }
     size_t cnt = 0;
-    for (size_t i = lo(t); i < lo(t + 1); ++i) {
+    for (size_t i = w.lo(t); i < w.lo(t + 1); ++i) {
       if (!fl[i]) continue;
-      const uint8_t* q = base + off[i] + 4;
+      const uint8_t* q = base + w.off[i] + 4;
       const char* nm = (const char*)q + 32;
       const size_t nl = trimmed_len(nm, (size_t)q[8] - 1);
       if (!have || nl != pl || memcmp(nm, pn, nl) != 0) {
-        fl[i] |= 2;
+        fl[i] |= 8;
         ++cnt;
       }
       pn = nm;
       pl = nl;
       have = true;
     }
-    n_start[t + 1] = cnt;
+    w.n_start[t + 1] = cnt;
   });
-  delete timer;
-  for (int t = 0; t < nt; ++t) {
-    n_valid[t + 1] += n_valid[t];
-    n_start[t + 1] += n_start[t];
-  }
-  const size_t rows = n_valid[nt];
-  if (rows && keys) {
-    const size_t row0 = r->st_tg.size();
-    for (auto* b : {&r->st_klo, &r->st_khi}) b->resize(row0 + rows);
-    for (auto* b : {&r->st_tg, &r->st_hp}) b->resize(row0 + rows);
-    uint64_t* klo = r->st_klo.data() + row0;
-    uint64_t* khi = r->st_khi.data() + row0;
-    int32_t* tg = r->st_tg.data() + row0;
-    int32_t* hp = r->st_hp.data() + row0;
-    // (4) rows: name keys instead of read starts
-    PhaseTimer rows_timer(&r->phase_s[4]);
-    parallel_for(nt, [&](int t) {
-      size_t k = n_valid[t];
-      for (size_t i = lo(t); i < lo(t + 1); ++i) {
-        if (!fl[i]) continue;
-        const uint8_t* q = base + off[i] + 4;
-        const char* nm = (const char*)q + 32;
-        name_key(nm, trimmed_len(nm, (size_t)q[8] - 1), &klo[k], &khi[k]);
-        const int32_t tid = (int32_t)le32(q);
-        tg[k] = r->tid_target[tid];
-        hp[k] = r->tid_hap[tid];
-        ++k;
-      }
-    });
-    r->st_whole = r->st_tg.size();
-  } else if (rows) {
-    const size_t row0 = r->st_rg.size();
-    r->st_rg.resize(row0 + rows);
-    r->st_tg.resize(row0 + rows);
-    r->st_hp.resize(row0 + rows);
-    const int64_t group0 = r->group;  // id of the read that is open when the window begins (-1: none)
-    int32_t* rg = r->st_rg.data() + row0;
-    int32_t* tg = r->st_tg.data() + row0;
-    int32_t* hp = r->st_hp.data() + row0;
-    // (4) rows
-    PhaseTimer rows_timer(&r->phase_s[4]);
-    parallel_for(nt, [&](int t) {
-      size_t k = n_valid[t];
-      int64_t g = group0 + (int64_t)n_start[t];
-      for (size_t i = lo(t); i < lo(t + 1); ++i) {
-        if (!fl[i]) continue;
-        if (fl[i] & 2) ++g;
-        const int32_t tid = (int32_t)le32(base + off[i] + 4);
-        rg[k] = (int32_t)g;
-        tg[k] = r->tid_target[tid];
-        hp[k] = r->tid_hap[tid];
-        ++k;
-      }
-    });
-    r->group = group0 + (int64_t)n_start[nt];
-    // remember the last valid record's trimmed name for the next window
-    for (size_t j = n; j-- > 0;)
-      if (fl[j]) {
-        const uint8_t* q = base + off[j] + 4;
-        const char* nm = (const char*)q + 32;
-        r->current.assign(nm, trimmed_len(nm, (size_t)q[8] - 1));
-        break;
-      }
-    r->started = true;
-    // whole reads = everything before the start of the last read
-    size_t w = r->st_rg.size();
-    const int32_t last = r->st_rg[w - 1];
-    while (w > 0 && r->st_rg[w - 1] == last) --w;
-    r->st_whole = w;
-  }
-  return 0;
+  for (int t = 0; t < w.nt; ++t) w.n_start[t + 1] += w.n_start[t];
+  for (size_t j = w.n; j-- > 0;)
+    if (fl[j]) {
+      const uint8_t* q = base + w.off[j] + 4;
+      const char* nm = (const char*)q + 32;
+      r->current.assign(nm, trimmed_len(nm, (size_t)q[8] - 1));
+      break;
+    }
 }
 
-// Per-cell rules (bam_utils_multisample.py:258-300) over the records of the inflated window, in
-// parallel except for two cheap sequential passes.  With P the previous valid record, a record B
-// starts a read iff the remembered name differs from trim(B), and the remembered name is
+// Per-cell rules (bam_utils_multisample.py:258-300) over the valid records of the window, in parallel except
+// for two cheap sequential passes.  With P the previous valid record, a record B starts a read iff the
+// remembered name differs from trim(B), and the remembered name is
 //   - trim(first record of the file) until the first switch,
 //   - the UNTRIMMED name of the record that made the last switch (:292) afterwards,
-// which, because every record inside a read matches the remembered name, is trim(P) if P did not
-// switch and P's untrimmed name if it did.  So both outcomes are computed per record in parallel
-// ("differs from trim(P)", "differs from P untrimmed") and one pass over two bits per record picks.
-// The cell of a read is field 14 of its remembered name, looked up when the NEXT valid alignment
-// arrives (dictionary ids follow that order; a read that ends the file alone is never looked up).
-int process_window_cells(bamcols* r, bamcols_cells* cells) {
-  const size_t left = r->st_rg.size() - r->st_pos;
-  if (r->st_pos > 0) {
-    memmove(r->st_rg.data(), r->st_rg.data() + r->st_pos, left * 4);
-    memmove(r->st_tg.data(), r->st_tg.data() + r->st_pos, left * 4);
-    memmove(r->st_hp.data(), r->st_hp.data() + r->st_pos, left * 4);
-    memmove(r->st_cell.data(), r->st_cell.data() + r->st_pos, left * 4);
-  }
-  r->st_rg.resize(left);
-  r->st_tg.resize(left);
-  r->st_hp.resize(left);
-  r->st_cell.resize(left);
-  r->st_whole -= r->st_pos;
-  if (r->pending) r->pending_row -= r->st_pos;
-  r->st_pos = 0;
-
-  if (r->wend - r->wpos < 4 || r->wend - r->wpos < 4 + (size_t)le32(r->win.data() + r->wpos)) {
-    const int rc = refill(r);
-    if (rc < 0) return rc;
-  }
-  auto lap_t0 = std::chrono::steady_clock::now();
-  auto lap = [&](int phase) {   // time since the previous lap goes to `phase`
-    const auto now = std::chrono::steady_clock::now();
-    r->phase_s[phase] += std::chrono::duration<double>(now - lap_t0).count();
-    lap_t0 = now;
-  };
-  const uint8_t* base = r->win.data();
-  std::vector<size_t>& off = r->rec_off;
-  off.clear();
-  size_t p = r->wpos;
-  {
-    const int rc = find_records(r, off, &p);
-    if (rc < 0) return rc;
-  }
-  r->wpos = p;
-  lap(1);
-  const size_t n = off.size();
-  if (n == 0) {
-    if (r->file_done) {
-      if (r->wend != r->wpos) return fail(r, BAMCOLS_ERR_FORMAT, "truncated BAM record at the end of the file");
-      r->records_done = true;
-      r->st_whole = r->st_rg.size();
-    }
-    return 0;
-  }
-  r->all_alignments += (int64_t)n;
-  std::vector<uint8_t>& fl = r->rec_flag;   // bit 0 valid, bit 1 differs from trim(P), bit 2 differs from P untrimmed
-  fl.assign(n, 0);
-  const int nt = (int)std::max<size_t>(1, std::min<size_t>((size_t)r->n_threads, n / r->grain + 1));
-  const int32_t n_ref = (int32_t)r->tid_target.size();
-  std::vector<size_t> n_valid(nt + 1, 0), n_start(nt + 1, 0);
-  std::atomic<int> bad(0);
-  auto lo = [&](int t) { return n * (size_t)t / (size_t)nt; };
+// which, because every record inside a read matches the remembered name, is trim(P) if P did not switch and P's
+// untrimmed name if it did.  So both outcomes are computed per record in parallel ("differs from trim(P)",
+// "differs from P untrimmed") and one pass over two bits per record picks.
+// The cell of a read is field 14 of its remembered name, looked up when the NEXT valid alignment arrives
+// (dictionary ids follow that order; a read that ends the file alone is never looked up).  Leaves the cell of
+// the window's k-th read in sc_group_cell[k] (k = 0: the read open when the window begins).
+int cell_starts(bamcols* r, bamcols_cells* cells, Window& w, size_t row0) {
+  const uint8_t* base = w.base;
+  const std::vector<size_t>& off = w.off;
+  std::vector<uint8_t>& fl = w.fl;
+  const size_t n = w.n;
+  const int nt = w.nt;
+  std::vector<size_t>& n_start = w.n_start;
+  auto lo = [&](int t) { return w.lo(t); };
   auto name_of = [&](size_t i, const char** nm, size_t* full, size_t* trimmed) {
     const uint8_t* q = base + off[i] + 4;
     *nm = (const char*)q + 32;
     *full = (size_t)q[8] - 1;
     *trimmed = trimmed_len(*nm, *full);
   };
-  parallel_for(nt, [&](int t) {
-    size_t cnt = 0;
-    for (size_t i = lo(t); i < lo(t + 1); ++i) {
-      const uint8_t* q = base + off[i] + 4;
-      const size_t bs = le32(base + off[i]);
-      const int32_t tid = (int32_t)le32(q);
-      const size_t l_name = q[8];
-      const uint32_t flag = le16(q + 14);
-      const int32_t ntid = (int32_t)le32(q + 20), npos = (int32_t)le32(q + 24);
-      if (32 + l_name > bs || l_name == 0) { bad.store(1); continue; }
-      if (flag & 0x4) continue;
-      if ((flag & 0x1) && ((flag & 0x80) || !(flag & 0x2) || tid != ntid || npos < 0)) continue;
-      if (tid < 0 || tid >= n_ref) { bad.store(2); continue; }
-      if (r->track_ranges) note_position(r, tid, (int32_t)le32(q + 4));
-      fl[i] = 1;
-      ++cnt;
-    }
-    n_valid[t + 1] = cnt;
-  });
-  if (bad.load() == 1) return fail(r, BAMCOLS_ERR_FORMAT, "BAM record with a bad read-name length");
-  if (bad.load() == 2) return fail(r, BAMCOLS_ERR_TID, "alignment with a reference id outside the header's %d references", n_ref);
-  for (int t = 0; t < nt; ++t) n_valid[t + 1] += n_valid[t];
-  const size_t rows = n_valid[nt];
-  lap(2);
-  if (rows == 0) return 0;
 
   // both comparison outcomes per valid record, against the previous valid record of the window
   parallel_for(nt, [&](int t) {
@@ -1142,11 +974,6 @@ int process_window_cells(bamcols* r, bamcols_cells* cells) {
   }
 
   // dictionary pass, in the order the reference resolves cells
-  const size_t row0 = r->st_rg.size();
-  r->st_rg.resize(row0 + rows);
-  r->st_tg.resize(row0 + rows);
-  r->st_hp.resize(row0 + rows);
-  r->st_cell.resize(row0 + rows);
   std::vector<int32_t>& group_cell = r->sc_group_cell;
   if (group_cell.size() < n_open + 1) group_cell.resize(n_open + 1);
   group_cell[0] = r->cell;   // the read that is open when the window begins
@@ -1161,29 +988,6 @@ int process_window_cells(bamcols* r, bamcols_cells* cells) {
     if (cell_id[k] == -2) return fail(r, BAMCOLS_ERR_CELL_FIELD, "list index out of range");
     group_cell[k + 1] = cell_id[k] >= 0 ? cell_id[k] : cells->id_of(cell_ptr[k], cell_len[k], cell_hash[k]);
   }
-
-  lap(3);
-  // rows
-  const int64_t group0 = r->group;
-  int32_t* rg = r->st_rg.data() + row0;
-  int32_t* tg = r->st_tg.data() + row0;
-  int32_t* hp = r->st_hp.data() + row0;
-  int32_t* cc = r->st_cell.data() + row0;
-  parallel_for(nt, [&](int t) {
-    size_t k = n_valid[t];
-    size_t g = n_start[t];
-    for (size_t i = lo(t); i < lo(t + 1); ++i) {
-      if (!fl[i]) continue;
-      if (fl[i] & 8) ++g;
-      const int32_t tid = (int32_t)le32(base + off[i] + 4);
-      rg[k] = (int32_t)(group0 + (int64_t)g);
-      tg[k] = r->tid_target[tid];
-      hp[k] = r->tid_hap[tid];
-      cc[k] = group_cell[g];
-      ++k;
-    }
-  });
-  r->group = group0 + (int64_t)n_open;
   if (n_open) {
     const char* nm;
     size_t nf, ntm;
@@ -1191,48 +995,200 @@ int process_window_cells(bamcols* r, bamcols_cells* cells) {
     r->current.assign(nm, (file_first_here && n_open == 1) ? ntm : nf);
     r->cell = group_cell[n_open];
     r->pending = pending_now;
-    if (pending_now) r->pending_row = row0 + rows - 1;   // that read's only row is the window's last row
+    if (pending_now) r->pending_row = row0 + w.n_valid[nt] - 1;   // that read's only row is the window's last row
   }
-  r->started = true;
-  lap(4);
-  size_t w = r->st_rg.size();
-  const int32_t last = r->st_rg[w - 1];
-  while (w > 0 && r->st_rg[w - 1] == last) --w;
-  r->st_whole = w;
   return 0;
 }
 
-int64_t emit_single(bamcols* r, bamcols_cells* cells, int32_t* read_group, int32_t* target_idx, int32_t* hap_idx,
-                    int32_t* cell_idx, int64_t capacity, int* done) {
+// Rows of the read-group modes, written at their final positions: read_group counts on from the read open
+// when the window begins; per-cell mode adds the cell of each read (cell_starts).
+template <bool CELLS>
+void group_rows(bamcols* r, const Window& w, size_t row0) {
+  const int64_t group0 = r->group;
+  int32_t* rg = r->st_rg.data() + row0;
+  int32_t* tg = r->st_tg.data() + row0;
+  int32_t* hp = r->st_hp.data() + row0;
+  int32_t* cc = CELLS ? r->st_cell.data() + row0 : nullptr;
+  const int32_t* group_cell = r->sc_group_cell.data();
+  parallel_for(w.nt, [&](int t) {
+    size_t k = w.n_valid[t];
+    size_t g = w.n_start[t];
+    for (size_t i = w.lo(t); i < w.lo(t + 1); ++i) {
+      if (!w.fl[i]) continue;
+      if (w.fl[i] & 8) ++g;
+      const int32_t tid = (int32_t)le32(w.base + w.off[i] + 4);
+      rg[k] = (int32_t)(group0 + (int64_t)g);
+      tg[k] = r->tid_target[tid];
+      hp[k] = r->tid_hap[tid];
+      if (CELLS) cc[k] = group_cell[g];
+      ++k;
+    }
+  });
+  r->group = group0 + (int64_t)w.n_start[w.nt];
+}
+
+// Rows of name-key mode (bamcols_emit_keys): every valid record gets the 128-bit key of its trimmed name in
+// place of a read_group.
+void key_rows(bamcols* r, const Window& w, size_t row0) {
+  uint64_t* klo = r->st_klo.data() + row0;
+  uint64_t* khi = r->st_khi.data() + row0;
+  int32_t* tg = r->st_tg.data() + row0;
+  int32_t* hp = r->st_hp.data() + row0;
+  parallel_for(w.nt, [&](int t) {
+    size_t k = w.n_valid[t];
+    for (size_t i = w.lo(t); i < w.lo(t + 1); ++i) {
+      if (!w.fl[i]) continue;
+      const uint8_t* q = w.base + w.off[i] + 4;
+      const char* nm = (const char*)q + 32;
+      name_key(nm, trimmed_len(nm, (size_t)q[8] - 1), &klo[k], &khi[k]);
+      const int32_t tid = (int32_t)le32(q);
+      tg[k] = r->tid_target[tid];
+      hp[k] = r->tid_hap[tid];
+      ++k;
+    }
+  });
+}
+
+// End of the whole reads among the staged rows: everything before the first row of the last read.
+size_t whole_reads_end(const bamcols* r) {
+  size_t w = r->st_rg.size();
+  const int32_t last = r->st_rg[w - 1];
+  while (w > 0 && r->st_rg[w - 1] == last) --w;
+  return w;
+}
+
+// The rules of the reader's mode over every whole record of the inflated window, on all worker threads:
+// (1) the record boundaries (find_records), (2) validity per record, (3) per mode: "starts a read" per valid
+// record, or nothing in name-key mode, (4) rows written at their final positions (prefix sums over the threads).
+// The open last read is held back (st_whole) until the next window or the end of the file closes it; name-key
+// mode has no reads to keep whole and hands out every row at once.
+int process_window(bamcols* r, bamcols_cells* cells) {
+  // rows still waiting from the previous window go to the front
+  const size_t left = r->st_tg.size() - r->st_pos;
+  for_staged(r, [&](auto& buf) {
+    if (r->st_pos > 0) memmove(buf.data(), buf.data() + r->st_pos, left * sizeof(buf[0]));
+    buf.resize(left);
+  });
+  r->st_whole -= r->st_pos;
+  if (r->pending) r->pending_row -= r->st_pos;
+  r->st_pos = 0;
+
+  // (1) records of the window
+  if (r->wend - r->wpos < 4 || r->wend - r->wpos < 4 + (size_t)le32(r->win.data() + r->wpos)) {
+    const int rc = refill(r);
+    if (rc < 0) return rc;
+  }
+  PhaseClock clock(r->phase_s);
+  std::vector<size_t>& off = r->rec_off;
+  size_t p = r->wpos;
+  {
+    const int rc = find_records(r, off, &p);
+    if (rc < 0) return rc;
+  }
+  r->wpos = p;
+  clock.lap(1);
+  const size_t n = off.size();
+  if (n == 0) {
+    if (r->file_done) {
+      if (r->wend != r->wpos) return fail(r, BAMCOLS_ERR_FORMAT, "truncated BAM record at the end of the file");
+      r->records_done = true;
+      r->st_whole = r->st_tg.size();  // the end of the file closes the last read
+    }
+    return 0;
+  }
+  r->all_alignments += (int64_t)n;
+  r->rec_flag.assign(n, 0);
+  const int nt = (int)std::max<size_t>(1, std::min<size_t>((size_t)r->n_threads, n / r->grain + 1));
+  Window w{r->win.data(), off, r->rec_flag, n, nt, std::vector<size_t>(nt + 1, 0), std::vector<size_t>(nt + 1, 0)};
+
+  // (2) validity
+  const int32_t n_ref = (int32_t)r->tid_target.size();
+  std::atomic<int> bad(0);
+  parallel_for(nt, [&](int t) {
+    size_t cnt = 0;
+    for (size_t i = w.lo(t); i < w.lo(t + 1); ++i) {
+      const uint8_t* rec = w.base + off[i];
+      const int v = record_validity(rec, n_ref);
+      if (v != REC_VALID) {
+        if (v != REC_FILTERED) bad.store(v);
+        continue;
+      }
+      if (r->track_ranges) note_position(r, (int32_t)le32(rec + 4), (int32_t)le32(rec + 8));
+      w.fl[i] = 1;
+      ++cnt;
+    }
+    w.n_valid[t + 1] = cnt;
+  });
+  if (bad.load() == REC_BAD_NAME) return fail(r, BAMCOLS_ERR_FORMAT, "BAM record with a bad read-name length");
+  if (bad.load() == REC_BAD_TID)
+    return fail(r, BAMCOLS_ERR_TID, "alignment with a reference id outside the header's %d references", n_ref);
+  for (int t = 0; t < nt; ++t) w.n_valid[t + 1] += w.n_valid[t];
+  const size_t rows = w.n_valid[nt];
+  clock.lap(2);
+  if (rows == 0) return 0;
+  const size_t row0 = r->st_tg.size();
+  for_staged(r, [&](auto& buf) { buf.resize(row0 + rows); });
+
+  if (r->mode == 3) {   // (4) rows: name keys instead of read starts
+    key_rows(r, w, row0);
+    r->st_whole = r->st_tg.size();
+    clock.lap(4);
+    return 0;
+  }
+  // (3) read starts; per-cell mode also resolves the cells here
+  if (r->mode == 2) {
+    const int rc = cell_starts(r, cells, w, row0);
+    if (rc < 0) return rc;
+  } else {
+    single_starts(r, w);
+  }
+  clock.lap(3);
+  // (4) rows
+  if (r->mode == 2) group_rows<true>(r, w, row0); else group_rows<false>(r, w, row0);
+  r->started = true;
+  r->st_whole = whole_reads_end(r);
+  clock.lap(4);
+  return 0;
+}
+
+// Hands the staged rows of the reader's mode to the caller's buffers dst[] (in for_staged order) until they are
+// full or the file ends.  In the read-group modes a call stops at the start of a read, so no read is split
+// between two calls.
+int64_t emit_rows(bamcols* r, bamcols_cells* cells, void* const* dst, int64_t capacity, int* done) {
   int64_t rows = 0;
   for (;;) {
     const size_t avail = r->st_whole - r->st_pos;
     if (avail > 0) {
       size_t take = std::min<size_t>(avail, (size_t)(capacity - rows));
-      if (take < avail)  // stop at the start of a read
+      if (take < avail && r->mode != 3)  // stop at the start of a read
         while (take > 0 && r->st_rg[r->st_pos + take] == r->st_rg[r->st_pos + take - 1]) --take;
       if (take == 0) {
         if (rows == 0) return fail(r, BAMCOLS_ERR_INVALID, "a read has more alignments than the buffers hold (%lld rows)", (long long)capacity);
         return rows;
       }
-      PhaseTimer timer(&r->phase_s[5]);
-      {
-        // columns x slices on the worker threads (one memcpy stream does not fill the memory system)
-        int32_t* dst[4] = {read_group + rows, target_idx + rows, hap_idx + rows, cells ? cell_idx + rows : nullptr};
-        const int32_t* src[4] = {r->st_rg.data() + r->st_pos, r->st_tg.data() + r->st_pos, r->st_hp.data() + r->st_pos,
-                                 cells ? r->st_cell.data() + r->st_pos : nullptr};
-        const int ncol = cells ? 4 : 3;
+      PhaseClock clock(r->phase_s);
+      // columns x slices on the worker threads (one memcpy stream does not fill the memory system)
+      uint8_t* to[4];
+      const uint8_t* from[4];
+      size_t width[4];
+      int ncol = 0;
+      for_staged(r, [&](auto& buf) {
+        width[ncol] = sizeof(buf[0]);
+        to[ncol] = (uint8_t*)dst[ncol] + (size_t)rows * width[ncol];
+        from[ncol] = (const uint8_t*)(buf.data() + r->st_pos);
+        ++ncol;
+      });
+      if (take < (1u << 18)) {   // small: not worth a thread
+        for (int c = 0; c < ncol; ++c) memcpy(to[c], from[c], take * width[c]);
+      } else {
         const int slices = (int)std::max<size_t>(1, std::min<size_t>((size_t)std::max(1, r->n_threads / ncol), take / (1u << 18)));
-        parallel_for(take < (1u << 18) ? 1 : ncol * slices, [&](int t) {
-          if (take < (1u << 18)) {   // small: not worth a thread
-            for (int c = 0; c < ncol; ++c) memcpy(dst[c], src[c], take * 4);
-            return;
-          }
+        parallel_for(ncol * slices, [&](int t) {
           const int c = t / slices, k = t % slices;
           const size_t a = take * (size_t)k / (size_t)slices, b = take * (size_t)(k + 1) / (size_t)slices;
-          memcpy(dst[c] + a, src[c] + a, (b - a) * 4);
+          memcpy(to[c] + a * width[c], from[c] + a * width[c], (b - a) * width[c]);
         });
       }
+      clock.lap(5);
       rows += (int64_t)take;
       r->st_pos += take;
       if (rows == capacity) return rows;
@@ -1242,35 +1198,7 @@ int64_t emit_single(bamcols* r, bamcols_cells* cells, int32_t* read_group, int32
       *done = 1;
       return rows;
     }
-    const int rc = cells ? process_window_cells(r, cells) : process_window_single(r);
-    if (rc < 0) return rc;
-  }
-}
-
-int64_t emit_keys(bamcols* r, uint64_t* key_lo, uint64_t* key_hi, int32_t* target_idx, int32_t* hap_idx, int64_t capacity,
-                  int* done) {
-  int64_t rows = 0;
-  for (;;) {
-    const size_t take = std::min<size_t>(r->st_whole - r->st_pos, (size_t)(capacity - rows));
-    if (take > 0) {
-      PhaseTimer timer(&r->phase_s[5]);
-      void* dst[4] = {key_lo + rows, key_hi + rows, target_idx + rows, hap_idx + rows};
-      const void* src[4] = {r->st_klo.data() + r->st_pos, r->st_khi.data() + r->st_pos, r->st_tg.data() + r->st_pos,
-                            r->st_hp.data() + r->st_pos};
-      const size_t width[4] = {8, 8, 4, 4};
-      parallel_for(take < (1u << 18) ? 1 : 4, [&](int t) {
-        for (int c = t; c < 4; c += (take < (1u << 18) ? 1 : 4)) memcpy(dst[c], src[c], take * width[c]);
-      });
-      rows += (int64_t)take;
-      r->st_pos += take;
-      if (rows == capacity) return rows;
-      continue;
-    }
-    if (r->records_done) {
-      *done = 1;
-      return rows;
-    }
-    const int rc = process_window_single(r, true);
+    const int rc = process_window(r, cells);
     if (rc < 0) return rc;
   }
 }
@@ -1308,7 +1236,6 @@ int bamcols_open(bamcols** out, const char* path, int n_threads) {
   }
   r->file = (const uint8_t*)m;
   madvise(m, r->file_size, MADV_SEQUENTIAL);
-  r->sequential_cells = getenv("BAMCOLS_SEQUENTIAL_CELLS") != nullptr;
   if (const char* b = getenv("BAMCOLS_BATCH_BLOCKS")) r->batch_blocks = (size_t)std::max(1L, atol(b));  // tests: many small windows
   if (const char* g = getenv("BAMCOLS_GRAIN")) r->grain = (size_t)std::max(1L, atol(g));  // tests: split tiny inputs too
   const unsigned hw = std::thread::hardware_concurrency();
@@ -1792,108 +1719,11 @@ int64_t bamcols_emit(bamcols* r, bamcols_cells* cells, int32_t* read_group, int3
   if (r->mode == 0) r->mode = want_mode;
   if (r->mode == 3) return fail(r, BAMCOLS_ERR_INVALID, "a reader that has emitted name keys cannot switch to read groups");
   if (r->mode != want_mode) return fail(r, BAMCOLS_ERR_INVALID, "a reader cannot switch between single-sample and per-cell rules");
-  if (!cells || !r->sequential_cells) {
-    try {   // no exception may cross the C ABI
-      return emit_single(r, cells, read_group, target_idx, hap_idx, cell_idx, capacity, done);
-    } catch (const std::bad_alloc&) {
-      return fail(r, BAMCOLS_ERR_IO, "out of memory while decoding the window");
-    }
-  }
-  // ---- per-cell rules as ONE sequential pass (BAMCOLS_SEQUENTIAL_CELLS): the plain statement of
-  // bam_utils_multisample.py:258-300 that the parallel window code above is tested against -------------
-  const int32_t n_ref = (int32_t)r->tid_target.size();
-  int64_t rows = 0;
-  for (;;) {
-    // a finished read waits for room in the caller's buffers
-    if (r->ready.size()) {
-      const int64_t k = (int64_t)r->ready.size();
-      if (rows + k > capacity) {
-        if (rows == 0) return fail(r, BAMCOLS_ERR_INVALID, "a read has %lld alignments but the buffers hold %lld rows", (long long)k, (long long)capacity);
-        return rows;
-      }
-      for (int64_t i = 0; i < k; ++i) read_group[rows + i] = r->ready.group;
-      memcpy(target_idx + rows, r->ready.tg.data(), (size_t)k * 4);
-      memcpy(hap_idx + rows, r->ready.hp.data(), (size_t)k * 4);
-      if (cells) memcpy(cell_idx + rows, r->ready.cell.data(), (size_t)k * 4);
-      rows += k;
-      r->ready.clear();
-    }
-    if (r->records_done) {
-      if (!r->all_flushed) {  // the last read of the file
-        r->all_flushed = true;
-        std::swap(r->cur, r->ready);
-        continue;
-      }
-      *done = 1;
-      return rows;
-    }
-    // ---- next record --------------------------------------------------------------------------------
-    int rc = ensure_bytes(r, 4);
-    if (rc < 0) return rc;
-    if (rc == 0) {
-      if (r->wend != r->wpos) return fail(r, BAMCOLS_ERR_FORMAT, "truncated BAM record at the end of the file");
-      r->records_done = true;
-      continue;
-    }
-    const size_t bs = le32(r->win.data() + r->wpos);
-    if (bs < 32) return fail(r, BAMCOLS_ERR_FORMAT, "BAM record with block_size %zu", bs);
-    rc = ensure_bytes(r, 4 + bs);
-    if (rc < 0) return rc;
-    if (rc == 0) return fail(r, BAMCOLS_ERR_FORMAT, "truncated BAM record at the end of the file");
-    const uint8_t* p = r->win.data() + r->wpos + 4;
-    r->wpos += 4 + bs;
-    r->all_alignments++;
-    const int32_t tid = (int32_t)le32(p);
-    const size_t l_name = p[8];
-    const uint32_t flag = le16(p + 14);
-    const int32_t ntid = (int32_t)le32(p + 20), npos = (int32_t)le32(p + 24);
-    if (32 + l_name > bs || l_name == 0) return fail(r, BAMCOLS_ERR_FORMAT, "BAM record with a bad read-name length");
-    // bam_utils.py:264-270
-    if (flag & 0x4) continue;
-    if ((flag & 0x1) && ((flag & 0x80) || !(flag & 0x2) || tid != ntid || npos < 0)) continue;
-    const char* qname = (const char*)p + 32;
-    const size_t qlen = l_name - 1;  // the stored name without its terminating NUL
-    const size_t tlen = trimmed_len(qname, qlen);
-    if (tid < 0 || tid >= n_ref) return fail(r, BAMCOLS_ERR_TID, "alignment with reference id %d outside the header's %d references", tid, n_ref);
-    if (r->track_ranges) note_position(r, tid, (int32_t)le32(p + 4));
-
-    bool sw;
-    if (!cells) {
-      // bam_utils.py:301-306
-      sw = !r->started || r->current.size() != tlen || memcmp(r->current.data(), qname, tlen) != 0;
-      if (sw) r->current.assign(qname, tlen);
-    } else {
-      // bam_utils_multisample.py:258-300 (see alntools_b200/emitter.py:emit_multisample)
-      const char* cf;
-      size_t cl;
-      if (!r->started) {
-        r->current.assign(qname, tlen);
-        if (!cell_field(r->current, &cf, &cl)) return fail(r, BAMCOLS_ERR_CELL_FIELD, "list index out of range");
-        r->cell = cells->id_of(cf, cl);
-      } else if (r->pending) {
-        if (!cell_field(r->current, &cf, &cl)) return fail(r, BAMCOLS_ERR_CELL_FIELD, "list index out of range");
-        r->cell = cells->id_of(cf, cl);
-        r->cur.cell.back() = r->cell;  // the row that opened the read (always the last one written)
-        r->pending = false;
-      }
-      sw = r->started && (r->current.size() != tlen || memcmp(r->current.data(), qname, tlen) != 0);
-      if (sw) {
-        r->current.assign(qname, qlen);  // :292 keeps the untrimmed name
-        r->pending = true;
-        r->cell = 0;
-      }
-      if (!r->started) sw = true;  // opens read 0 (no pending cell: it was resolved above)
-    }
-    if (sw) {
-      if (r->started) std::swap(r->cur, r->ready);  // the previous read is complete
-      r->cur.clear();
-      r->started = true;
-      r->group++;
-      r->cur.group = (int32_t)r->group;
-    }
-    r->cur.tg.push_back(r->tid_target[tid]);
-    r->cur.hp.push_back(r->tid_hap[tid]);
-    if (cells) r->cur.cell.push_back(r->cell);
+  try {   // no exception may cross the C ABI
+    void* const dst[4] = {read_group, target_idx, hap_idx, cell_idx};
+    return emit_rows(r, cells, dst, capacity, done);
+  } catch (const std::bad_alloc&) {
+    return fail(r, BAMCOLS_ERR_IO, "out of memory while decoding the window");
   }
 }
 
@@ -1909,7 +1739,8 @@ int64_t bamcols_emit_keys(bamcols* r, uint64_t* key_lo, uint64_t* key_hi, int32_
   if (r->mode == 0) r->mode = 3;
   if (r->mode != 3) return fail(r, BAMCOLS_ERR_INVALID, "a reader that has emitted read groups cannot switch to name keys");
   try {
-    return emit_keys(r, key_lo, key_hi, target_idx, hap_idx, capacity, done);
+    void* const dst[4] = {key_lo, key_hi, target_idx, hap_idx};
+    return emit_rows(r, nullptr, dst, capacity, done);
   } catch (const std::bad_alloc&) {
     return fail(r, BAMCOLS_ERR_IO, "out of memory while decoding the window");
   }

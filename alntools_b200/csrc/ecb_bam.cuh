@@ -1,5 +1,5 @@
 // ecb_bam.cuh — device decode of single-sample BAM windows (ecb_bam_* in include/ecb200.h): BGZF inflate, the
-// record hop, and the single-sample rules of libbamcols' process_window_single (bamcols.cpp), producing the same
+// record hop, and the single-sample rules of libbamcols' process_window (bamcols.cpp), producing the same
 // int32 columns bamcols_emit produces.
 //
 // A window is a run of whole BGZF blocks inflated behind the bytes the previous window left over (the start of a
@@ -198,7 +198,7 @@ struct BamRules {
   BamDevState* st;
 };
 
-// bamcols.cpp:716-730 per record: valid[i] = 1 for a valid alignment.
+// bamcols.cpp:record_validity per record: valid[i] = 1 for a valid alignment.
 __global__ void ecb_bam_validity_kernel(BamRules R, u32* __restrict__ valid) {
   const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= R.n_rec) return;
@@ -236,7 +236,7 @@ __global__ void ecb_bam_compact_kernel(BamRules R, const u32* __restrict__ valid
   vrec[rowpos[i]] = R.off[i];
 }
 
-// starts[k] = 1 iff valid record k's trimmed name differs from the previous valid record's (bamcols.cpp:736-772)
+// starts[k] = 1 iff valid record k's trimmed name differs from the previous valid record's (bamcols.cpp:single_starts)
 __global__ void ecb_bam_starts_kernel(const uint8_t* __restrict__ win, const u32* __restrict__ vrec, u32 n_valid,
                                       const BamDevState* st, u32* __restrict__ starts) {
   const u32 k = blockIdx.x * blockDim.x + threadIdx.x;

@@ -424,35 +424,25 @@ def test_randomised_per_cell_bams(tmp_path, monkeypatch):
             _multisample_both(path, tables, cell_ids, cells, n_threads=int(rng.choice([1, 2, 5])))
 
 
-def test_per_cell_parallel_equals_sequential_statement(tmp_path, monkeypatch):
-    """BAMCOLS_SEQUENTIAL_CELLS selects the one-pass C++ statement of the per-cell rules; both must agree,
-    including on WHERE a short name raises (only when a later valid alignment exists)."""
+def test_per_cell_short_name_raises_where_the_python_statement_does(tmp_path, monkeypatch):
+    """A short name raises only when a later valid alignment exists, as in the record-level Python emitter;
+    with every record on its own worker thread and with the window unsplit."""
     ok = [(_cell_name("a", "C1"), 0, 0), (_cell_name("a", "C1"), 0, 1), (_cell_name("b", "C2"), 0, 2)]
     tail_bad = ok + [("short|||name", 0, 3)]                      # ends the file alone: never looked up
     mid_bad = ok + [("short|||name", 0, 3), (_cell_name("c", "C3"), 0, 4)]
     tables = TargetTables([r[0] for r in REFS], [r[1] for r in REFS], None)
-    for name, alns, raises in (("ok", ok, False), ("tail", tail_bad, False), ("mid", mid_bad, True)):
-        path = _write(tmp_path, alns, name + ".bam")
-        results = []
-        for seq in (False, True):
-            if seq:
-                monkeypatch.setenv("BAMCOLS_SEQUENTIAL_CELLS", "1")
-            else:
-                monkeypatch.delenv("BAMCOLS_SEQUENTIAL_CELLS", raising=False)
-            cells = bamcols.CellDictionary()
-            with bamcols.BamColumnReader(path) as r:
-                r.set_tables(tables)
-                if raises:
-                    with pytest.raises(IndexError):
-                        r.read_all(cells=cells)
-                    continue
-                got = r.read_all(cells=cells)
-            results.append((got["read_group"].tolist(), got["cell_idx"].tolist(), cells.names()))
-        if not raises:
-            assert results[0] == results[1]
-            header, recs = load_records(path)
-            want = emitter.emit_multisample(recs, tables, {})
-            assert results[0][0] == want.read_group.tolist() and results[0][1] == want.cell_idx.tolist()
+    for grain in (1, 4096):
+        monkeypatch.setenv("BAMCOLS_GRAIN", str(grain))
+        for name, alns in (("ok", ok), ("tail", tail_bad)):
+            _multisample_both(_write(tmp_path, alns, name + ".bam"), tables, {}, bamcols.CellDictionary(), n_threads=4)
+        path = _write(tmp_path, mid_bad, "mid.bam")
+        header, recs = load_records(path)
+        with pytest.raises(IndexError):
+            emitter.emit_multisample(recs, tables, {})
+        with bamcols.BamColumnReader(path, n_threads=4) as r:
+            r.set_tables(tables)
+            with pytest.raises(IndexError):
+                r.read_all(cells=bamcols.CellDictionary())
 
 
 def test_native_target_section_equals_the_python_one(tmp_path):
