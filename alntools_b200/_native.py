@@ -26,7 +26,9 @@ ECB_OPT_COLLATE_PIECE = 11
 ECB_OPT_COLLATE_BUDGET = 12
 ECB_OPT_MAX_READ = 13
 
+ECB_ERR_LIMIT = -4
 ECB_ERR_EMPTY = -5
+ECB_ERR_STATE = -6
 ECB_ERR_FORMAT = -7
 
 _i32p = ctypes.POINTER(ctypes.c_int32)
@@ -63,6 +65,12 @@ class EcbStatsSamples(EcbStats):
     """ecb_stats since version 2006: EcbStats (the layout up to version 2005), then the fields of the samples
     (ecb_sample_close).  ecb_get_stats writes the whole of it."""
     _fields_ = [("samples", ctypes.c_int64), ("sample_pairs", ctypes.c_int64), ("sample_ms", ctypes.c_double)]
+
+
+class EcbStatsEcRows(EcbStatsSamples):
+    """ecb_stats since version 2007: EcbStatsSamples, then the fields of the EC-row pushes (ecb_push_ecs)."""
+    _fields_ = [("ec_pushes", ctypes.c_int64), ("ec_rows", ctypes.c_int64), ("ec_claimed", ctypes.c_int64),
+                ("ec_ms", ctypes.c_double), ("ec_check_ms", ctypes.c_double)]
 
 
 class EcbSlice(ctypes.Structure):
@@ -143,6 +151,10 @@ SIGNATURES = {
     "ecb_finalize": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.POINTER(EcbResult)]),
     "ecb_sample_close": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64)]),
     "ecb_finalize_samples": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbResult)]),
+    "ecb_push_ecs": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
+                                    ctypes.c_int64, ctypes.c_int64, ctypes.c_int]),
+    "ecb_sample_append": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                         ctypes.c_int64, ctypes.c_int64, ctypes.c_int, ctypes.POINTER(ctypes.c_int64)]),
     "ecb_reset": (ctypes.c_int, [ctypes.c_void_p]),
     "ecb_get_stats": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbStats)]),
     "ecb_destroy": (ctypes.c_int, [ctypes.c_void_p]),
@@ -304,6 +316,28 @@ class EcBuilder(object):
         non-zero entries."""
         nnz = ctypes.c_int64()
         self._check(self._lib.ecb_sample_close(self._ctx, ctypes.byref(nnz)))
+        return int(nnz.value)
+
+    def push_ecs(self, a_indptr, a_indices, a_data, order_base=0):
+        """The rows of one EC file's A matrix (CSR, int32: indptr, target indices, haplotype masks) as ECs of this
+        context, first occurrences at order_base + row (see ecb_push_ecs).  No read is counted.  numpy arrays or
+        torch tensors, all on the host or all on this builder's GPU."""
+        n_ec = int(a_indptr.shape[0]) - 1
+        if n_ec < 0:
+            raise ValueError("a_indptr needs at least one entry")
+        self._check(self._lib.ecb_push_ecs(self._ctx, _ptr(a_indptr), _ptr(a_indices), _ptr(a_data), n_ec,
+                                           int(a_indices.shape[0]), int(order_base), 1 if _on_device(a_indptr) else 0))
+
+    def append_samples(self, n_indptr, n_indices, n_data):
+        """Columns of counts (CSC, int32) over the rows of the last push_ecs, closed as samples at once (see
+        ecb_sample_append).  -> the non-zero entries added."""
+        n_samples = int(n_indptr.shape[0]) - 1
+        if n_samples < 0:
+            raise ValueError("n_indptr needs at least one entry")
+        nnz = ctypes.c_int64()
+        self._check(self._lib.ecb_sample_append(self._ctx, _ptr(n_indptr), _ptr(n_indices), _ptr(n_data), n_samples,
+                                                int(n_indices.shape[0]), 1 if _on_device(n_indptr) else 0,
+                                                ctypes.byref(nnz)))
         return int(nnz.value)
 
     def finalize_samples_raw(self):
@@ -470,7 +504,7 @@ class EcBuilder(object):
                 "n_data": view(sl.n_data, sl.nnz_n)}
 
     def stats(self):
-        st = EcbStatsSamples()
+        st = EcbStatsEcRows()
         self._check(self._lib.ecb_get_stats(self._ctx, ctypes.byref(st)))
         return st.as_dict()
 

@@ -25,6 +25,8 @@ def _name_bytes(name):
     """The bytes ecsave2 writes for a name: pack('<{len(name)}s', name.encode()) keeps len(name) BYTES, so a
     non-ASCII name is cut inside its UTF-8 encoding (bin_utils.py:131-135,153-159,177-180).  Same here, so the
     file stays byte-identical and the length prefix always matches what follows."""
+    if isinstance(name, bytes):                      # a name as read from an EC file: written as it was
+        return name
     return name.encode("utf-8")[:len(name)]
 
 
@@ -291,3 +293,177 @@ def ec2emase(ec_filename, emase_filename):
     shape = (len(ec["targets"]), len(ec["haplotypes"]), len(ec["a"][0]) - 1)
     emase.save_emase(emase_filename, "Converted from {}".format(ec_filename), shape, ec["haplotypes"], ec["targets"],
                      ec["lengths"], ec["samples"], ec["a"], ec["n"], incidence_only=False, as_ecload=True)
+
+
+def _ec_sections(path, first=None):
+    """Where the sections of EC file `path` (format 2) lie, read without its matrices: -> dict(header: the bytes from
+    the format word to the end of the targets section, haplotypes: their names as bytes, n_targets, section: the bytes
+    of the targets after their count, samples: names as bytes, matrices_at, n_ec, nnz_a, n_cols, nnz_n, size).
+    `first`: the sections of the first file of a merge, whose header this file must repeat byte for byte.  Raises
+    ValueError naming the file when it is not a well-formed file of format 2 or has no sample."""
+    import mmap
+    size = os.path.getsize(path)
+    with open(path, "rb") as fh:
+        if size < 4:
+            raise ValueError("%s: truncated EC file" % path)
+        with mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ) as mm:
+            pos = [0]
+
+            def i32():
+                if pos[0] + 4 > size:
+                    raise ValueError("%s: truncated EC file" % path)
+                v = struct.unpack_from("<i", mm, pos[0])[0]
+                pos[0] += 4
+                return v
+
+            def skip(n, what):
+                if n < 0 or pos[0] + n > size:
+                    raise ValueError("%s: truncated EC file (%s)" % (path, what))
+                start = pos[0]
+                pos[0] += n
+                return start
+
+            def name(what):
+                n = i32()
+                return bytes(mm[skip(n, what):pos[0]])
+
+            fmt = i32()
+            if fmt != 2:
+                raise ValueError("%s: not an EC file of format 2 (format %d)" % (path, fmt))
+            if first is not None:
+                h = first["header"]
+                if size < len(h):
+                    raise ValueError("%s: truncated EC file (header)" % path)
+                if mm[:len(h)] != h:
+                    raise ValueError("%s: its haplotype or target section differs from that of %s" % (path, first["path"]))
+                pos[0] = len(h)
+                out = dict(first)
+            else:
+                n_haps = i32()
+                if n_haps < 0:
+                    raise ValueError("%s: negative number of haplotypes" % path)
+                haplotypes = [name("haplotype names") for _ in range(n_haps)]
+                n_targets = i32()
+                if n_targets < 0:
+                    raise ValueError("%s: negative number of targets" % path)
+                section_at = pos[0]
+                for _ in range(n_targets):
+                    skip(i32(), "target names")
+                    skip(4 * n_haps, "target lengths")
+                out = {"header": bytes(mm[:pos[0]]), "haplotypes": haplotypes, "n_targets": n_targets,
+                       "section": bytes(mm[section_at:pos[0]])}
+            n_samples = i32()
+            if n_samples <= 0:
+                raise ValueError("%s: an EC file needs at least one sample, found %d" % (path, n_samples))
+            samples = [name("sample names") for _ in range(n_samples)]
+            matrices_at = pos[0]
+            a_ptr, nnz_a = i32(), i32()
+            if a_ptr < 1 or nnz_a < 0:
+                raise ValueError("%s: inconsistent A sizes (%d offsets, %d entries)" % (path, a_ptr, nnz_a))
+            skip(4 * (a_ptr + 2 * nnz_a), "A matrix")
+            n_ptr, nnz_n = i32(), i32()
+            if n_ptr != n_samples + 1 or nnz_n < 0:
+                raise ValueError("%s: inconsistent N sizes (%d offsets for %d samples, %d entries)"
+                                 % (path, n_ptr, n_samples, nnz_n))
+            skip(4 * (n_ptr + 2 * nnz_n), "N matrix")
+            if pos[0] != size:
+                raise ValueError("%s: trailing bytes in EC file (%d)" % (path, size - pos[0]))
+    out.update(path=path, samples=samples, matrices_at=matrices_at, n_ec=a_ptr - 1, nnz_a=nnz_a, n_cols=n_samples,
+               nnz_n=nnz_n, size=size)
+    return out
+
+
+def _ec_matrices(sec):
+    """The A and N arrays of a file described by _ec_sections, read at once: int32 views of one buffer."""
+    buf = np.fromfile(sec["path"], dtype="<i4", count=(sec["size"] - sec["matrices_at"]) // 4, offset=sec["matrices_at"])
+    e, za, s, zn = sec["n_ec"], sec["nnz_a"], sec["n_cols"], sec["nnz_n"]
+    at = [2]
+
+    def take(n):
+        v = buf[at[0]:at[0] + n]
+        at[0] += n
+        return v
+
+    a = (take(e + 1), take(za), take(za))
+    at[0] += 2
+    return a, (take(s + 1), take(zn), take(zn))
+
+
+def merge_ec_files(ec_files, ec_filename, sample_names=None, device=0):
+    """Merge EC files (format 2) into one EC file with one shared EC index, on one GPU.
+
+    Every file must have the first file's haplotype and target sections, byte for byte; the output takes them.  An EC
+    is a distinct A row (a set of (target, haplotype) elements): the output holds every distinct row of the inputs,
+    and its EC ids follow the row's first appearance as (file index, id in that file).  N has the columns of every
+    file in order, each entry moved to the merged id of its row; zeros are not stored and ids ascend in a column.
+    Columns are never joined by name.  The samples are the inputs' sample lists back to back, or sample_names (one per
+    output column).  EC ids being ranks of first occurrence, the merge of convert() outputs of several BAM files is the
+    file convert_samples() writes for those files, and merging is associative.
+
+    Every file is checked (format, sizes, samples, header) before a GPU is touched or the output is written; values
+    the GPU finds malformed (a target out of range, unsorted or empty rows, bad masks, repeated rows, N indices out of
+    range, negative counts) raise ValueError naming the file.  The next file is read on a worker thread while the
+    current one is pushed, so at most two files are in host memory.  One GPU: inside a multi-GPU launcher or with
+    ALNTOOLS_GPUS > 1 it raises NotImplementedError, as it does for an EMASE (.h5) output (ec2emase converts the
+    merged file).  -> dict(n_ec, nnz_a, nnz_n, n_samples, ecs_added (per file), seconds (read, push, finalize, write))."""
+    import time
+    from . import utils
+    from .emitter import _feed
+    ec_files = [str(f) for f in ec_files]
+    if not ec_files:
+        raise ValueError("merge_ec_files needs at least one EC file")
+    if str(ec_filename).lower().endswith(".h5"):
+        raise NotImplementedError("merge_ec_files writes EC files only; convert the merged file with ec2emase")
+    if utils.under_launcher() or utils.requested_gpus(None) > 1:
+        raise NotImplementedError("merge_ec_files runs on one GPU (unset ALNTOOLS_GPUS, or run it outside a multi-GPU "
+                                  "launcher)")
+    secs = [_ec_sections(ec_files[0])]
+    secs += [_ec_sections(f, secs[0]) for f in ec_files[1:]]
+    names = [n for s in secs for n in s["samples"]]
+    if sample_names is not None:
+        sample_names = list(sample_names)
+        if len(sample_names) != len(names):
+            raise ValueError("%d sample names for %d columns" % (len(sample_names), len(names)))
+        names = sample_names
+    first = secs[0]
+    from ._native import ECB_ERR_FORMAT, ECB_ERR_LIMIT, EcBuilder, EcbError
+    seconds = {"read": 0.0, "push": 0.0, "finalize": 0.0, "write": 0.0}
+    added = []
+    todo = list(range(len(secs)))
+
+    def fill(_):
+        t0 = time.perf_counter()
+        k = todo.pop(0)
+        mats = _ec_matrices(secs[k])
+        seconds["read"] += time.perf_counter() - t0
+        return None, (k, mats), not todo
+
+    with EcBuilder(max(first["n_targets"], 1), max(len(first["haplotypes"]), 1), device=device,
+                   pageable_results=1) as builder:
+        def consume(_, item):
+            k, (a, n) = item
+            t0 = time.perf_counter()
+            before = builder.stats()["ec_claimed"]
+            try:
+                builder.push_ecs(*a)
+                builder.append_samples(*n)
+            except EcbError as exc:
+                if exc.code in (ECB_ERR_FORMAT, ECB_ERR_LIMIT):
+                    raise ValueError("%s: %s" % (ec_files[k], str(exc).split(": ", 1)[-1])) from None
+                raise
+            added.append(builder.stats()["ec_claimed"] - before)
+            seconds["push"] += time.perf_counter() - t0
+
+        _feed(fill, consume, 2)
+        t0 = time.perf_counter()
+        res = builder.finalize_samples(copy=False)
+        seconds["finalize"] = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        utils.delete_file(ec_filename)
+        ecsave2_arrays(ec_filename, first["haplotypes"], None, None, names,
+                       (res["a_indptr"], res["a_indices"], res["a_data"]),
+                       (res["n_indptr"], res["n_indices"], res["n_data"]), target_section=first["section"],
+                       n_targets=first["n_targets"])
+        seconds["write"] = time.perf_counter() - t0
+        return {"n_ec": int(res["n_ec"]), "nnz_a": int(res["nnz_a"]), "nnz_n": int(res["nnz_n"]),
+                "n_samples": int(res["n_samples"]), "ecs_added": added, "seconds": seconds}

@@ -92,3 +92,29 @@ def bam2ec_samples(ec_file, bam_files, samples, rangefile, targets, verbose):
     utils.configure_logging(verbose)
     bam_utils.convert_samples(list(bam_files), ec_file, sample_names=list(samples) or None, target_filename=targets,
                               range_filename=rangefile)
+
+
+@click.group()
+def _merge_commands():
+    """commands that work on EC files alone"""
+
+
+@_merge_commands.command('ec-merge', options_metavar='<options>', short_help='merge EC files into one EC file')
+@click.argument('ec_file', metavar='ec_file', type=click.Path(resolve_path=True, dir_okay=False, writable=True))
+@click.argument('in_files', metavar='in_ec_file...', nargs=-1, required=True,
+                type=click.Path(exists=True, resolve_path=True, dir_okay=False))
+@click.option('-s', '--sample', 'samples', multiple=True,
+              help="sample identifier, once per column of the inputs, in order")
+@click.option('-v', '--verbose', count=True, help='enables verbose mode')
+def ec_merge(ec_file, in_files, samples, verbose):
+    """Merge binary EC files (in_ec_file..., with one haplotype and target list) into one binary EC file (ec_file)
+    with every input's columns over one shared EC index"""
+    from . import bin_utils
+    utils.configure_logging(verbose)
+    bin_utils.merge_ec_files(list(in_files), ec_file, sample_names=list(samples) or None)
+
+
+# `python -m alntools_b200`: the converter commands of `cli` and the commands on EC files, in one command line.
+# `cli` keeps exactly the reference's commands and bam2ec-samples.
+main = click.CommandCollection(sources=[cli, _merge_commands], context_settings=dict(help_option_names=['-h', '--help']),
+                               help="alntools bam2ec / bam2emase on a B200")

@@ -23,6 +23,7 @@
 #include "ecb_collate.cuh"
 #include "ecb_longread.cuh"
 #include "ecb_samples.cuh"
+#include "ecb_ecrows.cuh"
 
 #define ECB_PUSH_LIMIT (0x7FFFFFFFll - 8192)   // alignments of one ecb_push
 // Largest ECB_OPT_MAX_READ, and what 0 stands for: the push limit as documented (2^31 - 8192), one more than the
@@ -117,6 +118,15 @@ struct ecb_ctx {
   std::vector<u32> smp_counts;
   u64 smp_base = 0;
   int64_t smp_open = 0;
+  // EC rows (ecb_push_ecs, ecb_ecrows.cuh): per row of the last push its key sums, table slot, provisional EC id and
+  // arena place; the flags / positions of an append's N entries and its column counts.  ecr_rows: rows of the last
+  // push, which await their ecb_sample_append (-1: none); ecr_used: rows were pushed since create/reset; ecr_broken:
+  // a push failed after it had changed the EC table (only ecb_reset recovers)
+  DevBuf ecr_acc, ecr_slot, ecr_ec, ecr_dst, ecr_flag, ecr_cols;
+  DevBuf ecr_seen;           // per provisional id: tag of the last push with a row on the EC (ecr_seen_n set up)
+  u32 ecr_seen_n = 0, ecr_tag = 0;
+  int64_t ecr_rows = -1;
+  bool ecr_used = false, ecr_broken = false;
   std::string err;
 };
 
@@ -688,7 +698,7 @@ void cells_release(ecb_ctx* c) {
 
 extern "C" {
 
-int ecb_version(void) { return 2006; }
+int ecb_version(void) { return 2007; }
 
 const char* ecb_last_error(const ecb_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
@@ -1007,6 +1017,9 @@ int ecb_push(ecb_ctx* c, const int32_t* read_group, const int32_t* target_idx, c
   if (n > 0 && (!read_group || !target_idx || !hap_idx)) return fail(c, ECB_ERR_INVALID, "NULL column");
   if (c->with_cells && n > 0 && !cell_idx) return fail(c, ECB_ERR_INVALID, "context has cells but cell_idx is NULL");
   if (!c->with_cells && cell_idx) return fail(c, ECB_ERR_INVALID, "cell_idx given but context was created without cells");
+  if (c->ecr_broken || c->ecr_rows >= 0)
+    return fail(c, ECB_ERR_STATE, c->ecr_broken ? "an ecb_push_ecs failed after it changed the EC table: ecb_reset first"
+                                                : "the EC rows of the last ecb_push_ecs await ecb_sample_append");
   CK(cudaSetDevice(c->device));
   if (!c->table_slots) CKR(init_table(c, n));
   const u32 push_id = c->push_count++;
@@ -1188,6 +1201,11 @@ static int finalize(ecb_ctx* c, int64_t min_cell_count, bool samples, ecb_result
 
 int ecb_finalize(ecb_ctx* c, int64_t min_cell_count, ecb_result* out) {
   if (!c || !out) return ECB_ERR_INVALID;
+  if (c->ecr_used) {
+    memset(out, 0, sizeof *out);
+    return fail(c, ECB_ERR_STATE, "the context holds ECs given as EC rows (ecb_push_ecs), which carry no reads: "
+                                  "ecb_finalize_samples gives their counts");
+  }
   return finalize(c, min_cell_count, false, out);
 }
 
@@ -1195,6 +1213,9 @@ int ecb_sample_close(ecb_ctx* c, int64_t* nonzeros) {
   if (!c) return ECB_ERR_INVALID;
   if (nonzeros) *nonzeros = 0;
   if (c->with_cells) return fail(c, ECB_ERR_INVALID, "samples are closed on single-sample contexts only");
+  if (c->ecr_broken || c->ecr_rows >= 0)
+    return fail(c, ECB_ERR_STATE, c->ecr_broken ? "an ecb_push_ecs failed after it changed the EC table: ecb_reset first"
+                                                : "the EC rows of the last ecb_push_ecs await ecb_sample_append");
   CK(cudaSetDevice(c->device));
   const u32 n = c->table_slots ? c->n_ec : 0;   // current on the host: every push ends with a sync
   u32 added = 0;
@@ -1231,9 +1252,257 @@ int ecb_finalize_samples(ecb_ctx* c, ecb_result* out) {
   if (c->with_cells) return fail(c, ECB_ERR_INVALID, "samples are closed on single-sample contexts only");
   if (c->smp_open) return fail(c, ECB_ERR_INVALID, "%lld alignments were pushed after the last ecb_sample_close",
                                (long long)c->smp_open);
+  if (c->ecr_broken) return fail(c, ECB_ERR_STATE, "an ecb_push_ecs failed after it changed the EC table: ecb_reset first");
+  if (c->ecr_rows >= 0)
+    return fail(c, ECB_ERR_INVALID, "the %lld EC rows of the last ecb_push_ecs await ecb_sample_append",
+                (long long)c->ecr_rows);
   if (c->smp_n_pairs > 0x7FFFFFFFull)
     return fail(c, ECB_ERR_LIMIT, "N matrix has %llu non-zeros (more than 2^31-1)", (unsigned long long)c->smp_n_pairs);
   return finalize(c, 0, true, out);
+}
+
+// ---- ECs given as EC-file rows (ecb_push_ecs / ecb_sample_append; kernels in ecb_ecrows.cuh) --------------------
+// A host copy of an index pointer of n + 1 entries (copied back when it is device memory), checked before any kernel
+// indexes with it: it runs from 0 to nnz and never decreases; with rows (A) no two entries are equal either, since an
+// empty row is no set of elements.
+static int host_indptr(ecb_ctx* c, const int32_t* p, int64_t n, int64_t nnz, int on_device, bool rows, const char* what,
+                       std::vector<int32_t>& copy, const int32_t** out) {
+  if (on_device) {
+    copy.resize((size_t)n + 1);
+    CK(cudaMemcpyAsync(copy.data(), p, ((size_t)n + 1) * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    c->stats.d2h_bytes += (n + 1) * 4;
+    p = copy.data();
+  }
+  if (p[0] != 0 || p[n] != nnz)
+    return fail(c, ECB_ERR_FORMAT, "%s: %s runs from %d to %d, not from 0 to nnz = %lld", what, rows ? "a_indptr" : "n_indptr",
+                p[0], p[n], (long long)nnz);
+  for (int64_t i = 0; i < n; ++i) {
+    if (p[i + 1] < p[i])
+      return fail(c, ECB_ERR_FORMAT, "%s: %s decreases at %lld (%d after %d)", what, rows ? "a_indptr" : "n_indptr",
+                  (long long)i + 1, p[i + 1], p[i]);
+    if (rows && p[i + 1] == p[i]) return fail(c, ECB_ERR_FORMAT, "%s: row %lld is empty", what, (long long)i);
+  }
+  *out = p;
+  return ECB_OK;
+}
+
+// Device columns of an EC-file array: the caller's when they are device memory, else staged with one copy each.
+static const int32_t* ecr_upload(ecb_ctx* c, DevBuf& st, const int32_t* p, int64_t n, int on_device, int* rc) {
+  *rc = ECB_OK;
+  if (on_device || n == 0) return p;
+  if ((*rc = ensure(c, st, (size_t)n * 4)) != ECB_OK) return nullptr;
+  if (cudaMemcpyAsync(st.p, p, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream) != cudaSuccess) {
+    *rc = fail(c, ECB_ERR_CUDA, "cudaMemcpyAsync of an EC-file array failed");
+    return nullptr;
+  }
+  c->stats.h2d_bytes += n * 4;
+  return (const int32_t*)st.p;
+}
+
+static int ecr_state(ecb_ctx* c) {
+  if (c->with_cells) return fail(c, ECB_ERR_INVALID, "EC rows go into single-sample contexts only");
+  if (c->ecr_broken) return fail(c, ECB_ERR_STATE, "an ecb_push_ecs failed after it changed the EC table: ecb_reset first");
+  return ECB_OK;
+}
+
+int ecb_push_ecs(ecb_ctx* c, const int32_t* a_indptr, const int32_t* a_indices, const int32_t* a_data, int64_t n_ec,
+                 int64_t nnz, int64_t order_base, int on_device) {
+  if (!c) return ECB_ERR_INVALID;
+  CKR(ecr_state(c));
+  if (n_ec < 0 || nnz < 0 || order_base < 0) return fail(c, ECB_ERR_INVALID, "negative n_ec, nnz or order_base");
+  if (n_ec > (1ll << 30) || nnz > 0x7FFFFFFFll)
+    return fail(c, ECB_ERR_LIMIT, "one push of EC rows takes at most 2^30 rows and 2^31 - 1 entries");
+  if (!a_indptr || (nnz > 0 && (!a_indices || !a_data))) return fail(c, ECB_ERR_INVALID, "NULL array");
+  if (c->smp_open)
+    return fail(c, ECB_ERR_STATE, "%lld alignments were pushed after the last ecb_sample_close: close that sample first",
+                (long long)c->smp_open);
+  CK(cudaSetDevice(c->device));
+  std::vector<int32_t> ip_copy;
+  const int32_t* ip = nullptr;
+  CKR(host_indptr(c, a_indptr, n_ec, nnz, on_device, true, "EC rows", ip_copy, &ip));
+  if (!c->table_slots) CKR(init_table(c, n_ec * 8));
+  const u64 base = c->smp_base + (u64)order_base;
+  if (n_ec == 0) {
+    c->ecr_rows = 0;
+    c->ecr_used = true;
+    c->stats.ec_pushes++;
+    return ECB_OK;
+  }
+  CK(cudaEventRecord(c->ev[0], c->stream));
+  int rc = ECB_OK;
+  EcrParams R{};
+  R.indptr = ecr_upload(c, c->st_rg, a_indptr, n_ec + 1, on_device, &rc);
+  CKR(rc);
+  R.indices = ecr_upload(c, c->st_tg, a_indices, nnz, on_device, &rc);
+  CKR(rc);
+  R.data = ecr_upload(c, c->st_hp, a_data, nnz, on_device, &rc);
+  CKR(rc);
+  const u32 n = (u32)n_ec;
+  CKR(ensure(c, c->ecr_acc, (size_t)n * sizeof(Mix4)));
+  CKR(ensure(c, c->ecr_slot, (size_t)n * 4));
+  CKR(ensure(c, c->ecr_ec, (size_t)n * 4));
+  CKR(ensure(c, c->ecr_dst, (size_t)n * 4));
+  CK(cudaMemsetAsync(c->ecr_acc.p, 0, (size_t)n * sizeof(Mix4), c->stream));
+  CK(cudaMemsetAsync(c->d_ctr->ecr_bad, 0xFF, sizeof c->d_ctr->ecr_bad, c->stream));
+  R.n_rows = n;
+  R.nnz = (u32)nnz;
+  R.n_targets = c->n_targets;
+  R.n_haps = c->n_haps;
+  R.base = base;
+  R.acc = (Mix4*)c->ecr_acc.p;
+  R.row_slot = (u32*)c->ecr_slot.p;
+  R.row_ec = (u32*)c->ecr_ec.p;
+  R.row_dst = (u32*)c->ecr_dst.p;
+  R.ctr = c->d_ctr;
+  const int g_z = grid_for(nnz, ECR_THREADS, c->sm_count * 16), g_r = grid_for(n, ECR_THREADS, c->sm_count * 16);
+  ecb_ecr_keys_kernel<<<g_z, ECR_THREADS, 0, c->stream>>>(R);
+  LAUNCH_CHECK("ecr_keys");
+  CKR(sync_counters(c));   // the value checks come back before anything is inserted
+  const u32* bad = c->h_ctr->ecr_bad;
+  auto row_of = [&](u32 i) { return (long long)(std::upper_bound(ip, ip + n_ec + 1, (int32_t)i) - ip) - 1; };
+  if (bad[ECR_BAD_TARGET] != ECB_NONE)
+    return fail(c, ECB_ERR_FORMAT, "EC rows: target outside [0, %d) at entry %u (row %lld)", c->n_targets,
+                bad[ECR_BAD_TARGET], row_of(bad[ECR_BAD_TARGET]));
+  if (bad[ECR_BAD_ORDER] != ECB_NONE)
+    return fail(c, ECB_ERR_FORMAT, "EC rows: targets not strictly ascending at entry %u (row %lld)", bad[ECR_BAD_ORDER],
+                row_of(bad[ECR_BAD_ORDER]));
+  if (bad[ECR_BAD_MASK] != ECB_NONE)
+    return fail(c, ECB_ERR_FORMAT, "EC rows: haplotype mask 0 or with a bit at or above n_haps = %d at entry %u (row %lld)",
+                c->n_haps, bad[ECR_BAD_MASK], row_of(bad[ECR_BAD_MASK]));
+
+  // from here on the table changes: the rows of an earlier push can no longer be appended
+  c->ecr_rows = -1;
+  while ((u64)(c->n_ec + n) * 2 > c->table_slots) {   // at most half full after the insert: no replay path
+    if (c->table_slots >= (1u << 31)) return fail(c, ECB_ERR_LIMIT, "EC table cannot grow beyond 2^31 slots");
+    CKR(grow_table(c, c->table_slots * 2));
+  }
+  const u64 bound = c->arena_used + (u64)nnz;
+  if (bound > 0xFFFFFFFFull) return fail(c, ECB_ERR_LIMIT, "row arena exceeds 2^32 entries");
+  CKR(ensure(c, c->arena, (size_t)bound * sizeof(uint2), true));
+  const u32 ids_bound = c->n_ec + n;
+  if (ids_bound > c->ecr_seen_n) {
+    CKR(ensure(c, c->ecr_seen, (size_t)ids_bound * 4, true));
+    CK(cudaMemsetAsync((u32*)c->ecr_seen.p + c->ecr_seen_n, 0, (size_t)(ids_bound - c->ecr_seen_n) * 4, c->stream));
+    c->ecr_seen_n = ids_bound;
+  }
+  R.seen = (u32*)c->ecr_seen.p;
+  R.tag = ++c->ecr_tag;
+  c->ecr_broken = true;   // until the rows are in
+  const GroupParams P = make_group_params(c, nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0);
+  ecb_ecr_insert_kernel<<<g_r, ECR_THREADS, 0, c->stream>>>(P, R);
+  LAUNCH_CHECK("ecr_insert");
+  ecb_ecr_reserve_kernel<<<g_r, ECR_THREADS, 0, c->stream>>>(R, (const EcbEntry*)c->table.p, (u32*)c->row_len.p,
+                                                             (u32*)c->row_off.p);
+  LAUNCH_CHECK("ecr_reserve");
+  ecb_ecr_copy_kernel<<<g_z, ECR_THREADS, 0, c->stream>>>(R, (uint2*)c->arena.p);
+  LAUNCH_CHECK("ecr_copy");
+  CK(cudaEventRecord(c->ev[2], c->stream));
+  ecb_ecr_check_kernel<<<g_z, ECR_THREADS, 0, c->stream>>>(R, (const u32*)c->row_len.p, (const u32*)c->row_off.p,
+                                                           (const uint2*)c->arena.p);
+  LAUNCH_CHECK("ecr_check");
+  CK(cudaEventRecord(c->ev[3], c->stream));
+  CK(cudaEventRecord(c->ev[1], c->stream));
+  CKR(sync_counters(c));
+  if (bad[ECR_BAD_DUPLICATE] != ECB_NONE)
+    return fail(c, ECB_ERR_FORMAT, "EC rows: row %u holds the set of another row of the same push (duplicate rows)",
+                bad[ECR_BAD_DUPLICATE]);
+  if (bad[ECR_BAD_PROBE] != ECB_NONE) return fail(c, ECB_ERR_LIMIT, "EC rows: the EC table ran out of probes at row %u",
+                                                  bad[ECR_BAD_PROBE]);
+  if (bad[ECR_BAD_COLLISION] != ECB_NONE)
+    return fail(c, ECB_ERR_LIMIT, "EC rows: row %u and a different set share one 128-bit key (key collision)",
+                bad[ECR_BAD_COLLISION]);
+  CKR(check_device_error(c));
+  c->ecr_broken = false;
+  const u32 claimed = c->h_ctr->n_ec - c->n_ec;
+  c->n_ec = c->h_ctr->n_ec;
+  c->min_base = std::min<u64>(c->min_base, base);
+  c->max_end = std::max<u64>(c->max_end, base + n);
+  c->smp_base = c->max_end;   // a later push of rows follows these, whether they get their counts or not
+  c->ecr_rows = n_ec;
+  c->ecr_used = true;
+  float ms = 0, check_ms = 0;
+  CK(cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
+  CK(cudaEventElapsedTime(&check_ms, c->ev[2], c->ev[3]));
+  c->stats.ec_pushes++;
+  c->stats.ec_rows += n_ec;
+  c->stats.ec_claimed += claimed;
+  c->stats.ec_ms += ms;
+  c->stats.ec_check_ms += check_ms;
+  c->stats.table_slots = c->table_slots;
+  c->stats.table_used = c->n_ec;
+  return ECB_OK;
+}
+
+int ecb_sample_append(ecb_ctx* c, const int32_t* n_indptr, const int32_t* n_indices, const int32_t* n_data,
+                      int64_t n_samples, int64_t nnz, int on_device, int64_t* nonzeros) {
+  if (!c) return ECB_ERR_INVALID;
+  if (nonzeros) *nonzeros = 0;
+  CKR(ecr_state(c));
+  if (n_samples < 0 || nnz < 0) return fail(c, ECB_ERR_INVALID, "negative n_samples or nnz");
+  if (n_samples > 0x7FFFFFFFll || nnz > 0x7FFFFFFFll)
+    return fail(c, ECB_ERR_LIMIT, "one append takes at most 2^31 - 1 samples and 2^31 - 1 entries");
+  if (!n_indptr || (nnz > 0 && (!n_indices || !n_data))) return fail(c, ECB_ERR_INVALID, "NULL array");
+  if (c->ecr_rows < 0) return fail(c, ECB_ERR_STATE, "no EC rows await their samples: ecb_push_ecs first");
+  CK(cudaSetDevice(c->device));
+  std::vector<int32_t> ip_copy;
+  const int32_t* ip = nullptr;
+  CKR(host_indptr(c, n_indptr, n_samples, nnz, on_device, false, "N", ip_copy, &ip));
+  const u32 S = (u32)n_samples, z = (u32)nnz;
+  std::vector<u32> cols(S, 0u);
+  float ms = 0;
+  if (z) {
+    CK(cudaEventRecord(c->ev[0], c->stream));
+    int rc = ECB_OK;
+    const int32_t* d_ip = ecr_upload(c, c->st_rg, n_indptr, n_samples + 1, on_device, &rc);
+    CKR(rc);
+    const int32_t* d_ix = ecr_upload(c, c->st_tg, n_indices, nnz, on_device, &rc);
+    CKR(rc);
+    const int32_t* d_v = ecr_upload(c, c->st_hp, n_data, nnz, on_device, &rc);
+    CKR(rc);
+    CKR(ensure(c, c->ecr_flag, ((size_t)z + 1) * 4));
+    CKR(ensure(c, c->ecr_cols, std::max<size_t>(S, 1) * 4));
+    CKR(ensure(c, c->smp_pairs, (size_t)(c->smp_n_pairs + z) * sizeof(uint2), true));
+    CK(cudaMemsetAsync((u32*)c->ecr_flag.p + z, 0, 4, c->stream));
+    CK(cudaMemsetAsync(c->d_ctr->ecr_bad, 0xFF, sizeof c->d_ctr->ecr_bad, c->stream));
+    const int g = grid_for(z, ECR_THREADS, c->sm_count * 16);
+    ecb_ecr_append_flags_kernel<<<g, ECR_THREADS, 0, c->stream>>>(d_ix, d_v, z, (u32)c->ecr_rows, (u32*)c->ecr_flag.p,
+                                                                   c->d_ctr);
+    LAUNCH_CHECK("ecr_append_flags");
+    CKR(device_scan<false>(c, (const u32*)c->ecr_flag.p, (u32*)c->ecr_flag.p, (u64)z + 1, 0, nullptr));
+    ecb_ecr_append_pairs_kernel<<<g, ECR_THREADS, 0, c->stream>>>(
+        d_ip, S, d_ix, d_v, z, (u32)c->ecr_rows, (const u32*)c->ecr_flag.p, (const u32*)c->ecr_ec.p,
+        (uint2*)c->smp_pairs.p + c->smp_n_pairs, (u32*)c->ecr_cols.p);
+    LAUNCH_CHECK("ecr_append_pairs");
+    if (S) CK(cudaMemcpyAsync(cols.data(), c->ecr_cols.p, (size_t)S * 4, cudaMemcpyDeviceToHost, c->stream));
+    c->stats.d2h_bytes += (int64_t)S * 4;
+    CK(cudaEventRecord(c->ev[1], c->stream));
+    CKR(sync_counters(c));   // the call's one round trip: the column counts and the value checks
+    const u32* bad = c->h_ctr->ecr_bad;
+    if (bad[ECR_BAD_N_INDEX] != ECB_NONE)
+      return fail(c, ECB_ERR_FORMAT, "N: EC index outside [0, %lld) at entry %u", (long long)c->ecr_rows,
+                  bad[ECR_BAD_N_INDEX]);
+    if (bad[ECR_BAD_N_COUNT] != ECB_NONE)
+      return fail(c, ECB_ERR_FORMAT, "N: negative count at entry %u", bad[ECR_BAD_N_COUNT]);
+    CK(cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
+  }
+  u64 added = 0;
+  for (u32 v : cols) added += v;
+  // the ECs the rows claimed hold no reads: their count at this "close" is 0
+  const u32 n = c->n_ec;
+  if (n > c->smp_n_ec) {
+    CKR(ensure(c, c->smp_last, (size_t)n * 4, true));
+    CK(cudaMemsetAsync((u32*)c->smp_last.p + c->smp_n_ec, 0, (size_t)(n - c->smp_n_ec) * 4, c->stream));
+  }
+  c->smp_n_ec = n;
+  c->smp_n_pairs += added;
+  c->smp_counts.insert(c->smp_counts.end(), cols.begin(), cols.end());
+  c->ecr_rows = -1;
+  c->stats.samples += n_samples;
+  c->stats.sample_pairs += (int64_t)added;
+  c->stats.sample_ms += ms;
+  if (nonzeros) *nonzeros = (int64_t)added;
+  return ECB_OK;
 }
 
 int ecb_reset(ecb_ctx* c) {
@@ -1257,6 +1526,8 @@ int ecb_reset(ecb_ctx* c) {
   c->smp_counts.clear();
   c->smp_base = 0;
   c->smp_open = 0;
+  c->ecr_rows = -1;
+  c->ecr_used = c->ecr_broken = false;
   const int64_t slots = c->stats.table_slots;
   c->stats = ecb_stats{};
   c->stats.table_slots = slots;
@@ -1534,6 +1805,7 @@ int ecb_export_to_arenas(ecb_ctx* c, int world, void* const* arena_bases, int64_
   if (!c || !arena_bases || cap_records < 1) return ECB_ERR_INVALID;
   if (world < 1 || world > ECB_MAX_WORLD) return fail(c, ECB_ERR_INVALID, "world %d outside [1, %d]", world, ECB_MAX_WORLD);
   if (c->with_cells) return fail(c, ECB_ERR_INVALID, "the multi-GPU exchange covers the single-sample path only");
+  if (c->ecr_used) return fail(c, ECB_ERR_STATE, "the multi-GPU exchange covers reads; this context holds EC rows");
   CK(cudaSetDevice(c->device));
   if (!c->table_slots) CKR(init_table(c));
   if (min_base) *min_base = c->n_ec ? (int64_t)c->min_base : 0;
@@ -1864,7 +2136,8 @@ int ecb_destroy(ecb_ctx* c) {
                     &c->scan_partials, &c->bitmap, &c->word_rank, &c->first_rel, &c->ecid_of, &c->ec_keep,
                     &c->r_a_indptr, &c->r_a_indices, &c->r_a_data, &c->r_n_indptr, &c->r_n_indices,
                     &c->r_n_data, &c->r_cell_order, &c->cx_kept, &c->cx_col_of_cell, &c->cx_col_counts,
-                    &c->smp_last, &c->smp_pairs};
+                    &c->smp_last, &c->smp_pairs, &c->ecr_acc, &c->ecr_slot, &c->ecr_ec, &c->ecr_dst, &c->ecr_flag,
+                    &c->ecr_cols, &c->ecr_seen};
   for (DevBuf* b : bufs) release(c, *b);
   cells_release(c);
   if (c->stream) cudaStreamSynchronize(c->stream);

@@ -141,6 +141,7 @@ struct EcbCounters {
   u32 scratch[8];
   u32 n_deferred;     // reads of the current push longer than ECB_MAX_READ_ALIGNMENTS (ecb_longread.cuh)
   u32 n_deferred_fail;// ... of them that found the table too full (inserted again after a growth)
+  u32 ecr_bad[8];     // EC rows: first bad entry / row of each kind (ecb_ecrows.cuh; ECB_NONE = none)
 };
 
 #define ECB_DEVERR_EC_CAPACITY 1u   // provisional id space exhausted

@@ -44,7 +44,8 @@ enum ecb_status {
   ECB_ERR_EMPTY = -5,       /* finalize with zero equivalence classes (the reference raises too:
                                alntools/matrix/Sparse3DMatrix.py:45-46) */
   ECB_ERR_STATE = -6,       /* call sequence error */
-  ECB_ERR_FORMAT = -7       /* malformed BAM input of the device decoder (ecb_bam_decode; since version 2002) */
+  ECB_ERR_FORMAT = -7       /* malformed BAM input of the device decoder (ecb_bam_decode; since version 2002), or
+                               malformed EC-file arrays (ecb_push_ecs / ecb_sample_append; since version 2007) */
 };
 
 /* Longest read (alignments sharing one name) a push accepts by default, and the longest one the grouping kernel
@@ -122,6 +123,12 @@ typedef struct ecb_stats {
   int64_t samples;        /* samples closed since create/reset (ecb_sample_close)                  */
   int64_t sample_pairs;   /* (EC, sample) entries they recorded                                    */
   double sample_ms;       /* device time of the closes, summed                                     */
+  /* since version 2007 */
+  int64_t ec_pushes;      /* ecb_push_ecs calls since create/reset                                 */
+  int64_t ec_rows;        /* EC rows they pushed                                                   */
+  int64_t ec_claimed;     /* ECs those rows claimed (rows whose set was new to the context)        */
+  double ec_ms;           /* device time of those pushes, summed (incl. H2D when host arrays)      */
+  double ec_check_ms;     /* ... of it spent in the exact check of the rows that found an EC       */
 } ecb_stats;
 
 /* Library/ABI version (major*1000 + minor). */
@@ -190,6 +197,43 @@ int ecb_finalize(ecb_ctx* ctx, int64_t min_cell_count, ecb_result* out);
  * per pair and its histograms. */
 int ecb_sample_close(ecb_ctx* ctx, int64_t* nonzeros);
 int ecb_finalize_samples(ecb_ctx* ctx, ecb_result* out);
+
+/* ---- ECs given as the rows of EC files (since version 2007) ---------------------------------------------------
+ * A merge of EC files feeds each file's A rows and N columns into one single-sample context instead of reads, and
+ * takes the result from ecb_finalize_samples: for every file, ecb_push_ecs, then ecb_sample_append.  EC ids are ranks
+ * of first occurrence, so the merged ids follow (file, row id in that file), and the merge of the convert() outputs of
+ * several BAM files is what the samples of those files give.
+ *
+ * ecb_push_ecs: the n_ec rows of one EC file's A matrix (CSR: a_indptr[n_ec + 1], a_indices = main targets ascending
+ *   inside a row, a_data = haplotype masks) as ECs of this context.  Row e's key is the set hash of its (target,
+ *   haplotype) elements: the key ecb_push gives a read with that set.  Its first occurrence is order_base + e, counted,
+ *   as ecb_push counts after a close, from the end of the closed samples' range.  A new key claims an EC that holds the
+ *   row; a known key is compared element for element with the row its EC holds.  No read is counted.
+ *   The host checks a_indptr (0 to nnz, rising, no empty row; copied back first when it is device memory) before any
+ *   kernel reads it; one pass over the entries then checks the values (target in [0, n_targets), targets strictly
+ *   ascending in a row, mask not 0 and below 1 << n_haps) and sums the keys, and its flags come back before anything
+ *   is inserted: a malformed file leaves the context as it was (ECB_ERR_FORMAT, naming the kind and the first bad
+ *   entry and its row).  After the insert, two rows of one push with one set fail with ECB_ERR_FORMAT, and a row whose
+ *   key an EC with a different row holds (a 128-bit key collision, never merged) with ECB_ERR_LIMIT; after either,
+ *   every call but ecb_reset / ecb_destroy fails with ECB_ERR_STATE.  The table grows before the insert, so that it is
+ *   at most half full after it.  Refused (ECB_ERR_STATE) when alignments were pushed after the last ecb_sample_close.
+ * ecb_sample_append: n_samples samples given as columns (CSC: n_indptr[n_samples + 1], n_indices = row ids of the
+ *   LAST ecb_push_ecs, n_data = counts), closed at once: entry i adds (EC of row n_indices[i], n_data[i]) to the samples'
+ *   pair list, which ecb_finalize_samples sorts into N.  Zeros are dropped; a row index outside the last push or a
+ *   negative count fails with ECB_ERR_FORMAT, before anything is added.  *nonzeros = pairs added.  One pass over the
+ *   entries, one scan and one host round trip, whatever the number of columns.  Later ecb_push / ecb_push_ecs order
+ *   keys count from the end of the pushed rows.
+ * Between the two calls the rows are open input: ecb_push, ecb_sample_close (ECB_ERR_STATE) and ecb_finalize_samples
+ * (ECB_ERR_INVALID) refuse.  A later ecb_push_ecs replaces rows that were not appended (their ECs stay, without
+ * counts, and the later rows follow them in the order).  ecb_finalize refuses a context that received EC rows, and so does the multi-GPU exchange (ECB_ERR_STATE):
+ * they carry no reads.  Both refuse contexts created with cells (ECB_ERR_INVALID).  ecb_reset forgets everything.
+ * Host arrays are copied with one cudaMemcpyAsync each.  Device memory: 28 bytes per row of the largest push and 12 per
+ * A entry (staging of host arrays; 8 of them stay in the row arena for a new row); per N entry 4 bytes of flags and 8
+ * bytes in the pair list, plus 8 of staging for host arrays. */
+int ecb_push_ecs(ecb_ctx* ctx, const int32_t* a_indptr, const int32_t* a_indices, const int32_t* a_data,
+                 int64_t n_ec, int64_t nnz, int64_t order_base, int on_device);
+int ecb_sample_append(ecb_ctx* ctx, const int32_t* n_indptr, const int32_t* n_indices, const int32_t* n_data,
+                      int64_t n_samples, int64_t nnz, int on_device, int64_t* nonzeros);
 
 /* Forget all pushed data but keep allocations (tables, staging) for the next job. */
 int ecb_reset(ecb_ctx* ctx);
