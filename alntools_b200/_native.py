@@ -99,6 +99,17 @@ class EcbBamStats(ctypes.Structure):
         return {name: getattr(self, name) for name, _ in self._fields_}
 
 
+class EcbSamStats(ctypes.Structure):
+    _fields_ = [
+        ("bytes", ctypes.c_int64), ("lines", ctypes.c_int64), ("calls", ctypes.c_int64),
+        ("h2d_ms", ctypes.c_double), ("lines_ms", ctypes.c_double), ("fields_ms", ctypes.c_double),
+        ("rules_ms", ctypes.c_double),
+    ]
+
+    def as_dict(self):
+        return {name: getattr(self, name) for name, _ in self._fields_}
+
+
 class EcbCollateStats(ctypes.Structure):
     _fields_ = [
         ("alignments", ctypes.c_int64), ("reads", ctypes.c_int64), ("table_slots", ctypes.c_int64),
@@ -169,6 +180,15 @@ SIGNATURES = {
     "ecb_bam_ranges": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "ecb_bam_get_stats": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbBamStats)]),
     "ecb_bam_destroy": (ctypes.c_int, [ctypes.c_void_p]),
+    "ecb_sam_create": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p,
+                                      ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.POINTER(ctypes.c_void_p)]),
+    "ecb_sam_parse": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int,
+                                     ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p),
+                                     ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_int64)]),
+    "ecb_sam_counters": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]),
+    "ecb_sam_ranges": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "ecb_sam_get_stats": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(EcbSamStats)]),
+    "ecb_sam_destroy": (ctypes.c_int, [ctypes.c_void_p]),
     "ecb_collate_create": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_void_p)]),
     "ecb_collate_add": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                        ctypes.c_int64, ctypes.c_int]),
@@ -591,6 +611,87 @@ class BamDecoder(object):
     def close(self):
         if self._h:
             self._lib.ecb_bam_destroy(self._h)
+            self._h = ctypes.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class SamDecoder(object):
+    """Device parse of single-sample SAM text on `builder`'s context (ecb_sam_* in include/ecb200.h): whole alignment
+    lines in, the columns BamDecoder gives for the same alignments as BAM out, in device memory.  references: the @SQ
+    names in header order (str); first_line: the line number of the first byte of the first call.  A bad line raises
+    ValueError with "line N: <what>"."""
+
+    def __init__(self, builder, references, tid_target, tid_hap, first_line=1, track_ranges=False):
+        self._lib = builder._lib
+        self._builder = builder                   # the decoder lives in the builder's context: keep it alive
+        self._h = ctypes.c_void_p()
+        self.n_references = len(tid_target)
+        names = [r.encode() for r in references]
+        blob = b"".join(names)
+        off = np.zeros(len(names) + 1, dtype=np.int64)
+        np.cumsum([len(n) for n in names], out=off[1:])
+        tt = np.ascontiguousarray(tid_target, dtype=np.int32)
+        th = np.ascontiguousarray(tid_hap, dtype=np.int32)
+        self._check(self._lib.ecb_sam_create(builder._ctx, blob, off.ctypes.data, len(tt), tt.ctypes.data, th.ctypes.data,
+                                             int(first_line), 1 if track_ranges else 0, ctypes.byref(self._h)))
+
+    def _check(self, rc):
+        if rc == 0:
+            return
+        msg = self._lib.ecb_last_error(self._builder._ctx).decode()
+        if rc == ECB_ERR_FORMAT:
+            raise ValueError(msg)
+        raise EcbError(rc, msg)
+
+    def parse(self, data, n_bytes=None, last=False):
+        """data: text bytes (pinned uint8 tensor preferred, or a numpy array / bytes), its first n_bytes whole lines.
+        -> (read_group, target_idx, hap_idx): int32 torch views of the device rows of every read closed so far, valid
+        until the next call."""
+        import torch
+        if isinstance(data, (bytes, bytearray)):
+            data = np.frombuffer(data, dtype=np.uint8)
+        ptr = data.data_ptr() if hasattr(data, "data_ptr") else data.ctypes.data
+        n_bytes = int(data.shape[0]) if n_bytes is None else int(n_bytes)
+        rg, tg, hp = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_void_p()
+        rows = ctypes.c_int64()
+        self._check(self._lib.ecb_sam_parse(self._h, ptr if n_bytes else None, n_bytes, 1 if last else 0,
+                                            ctypes.byref(rg), ctypes.byref(tg), ctypes.byref(hp), ctypes.byref(rows)))
+        n = int(rows.value)
+        dev = torch.device("cuda", self._builder.device)
+        return tuple(_device_view(p.value, (n,), "<i4", torch.int32, dev) for p in (rg, tg, hp))
+
+    def counters(self):
+        """-> (all_alignments, n_groups): alignment lines seen so far and reads started."""
+        a, g = ctypes.c_int64(), ctypes.c_int64()
+        self._check(self._lib.ecb_sam_counters(self._h, ctypes.byref(a), ctypes.byref(g)))
+        return int(a.value), int(g.value)
+
+    def ranges(self):
+        """(min_pos, max_pos) int32 arrays per reference, as BamDecoder.ranges()."""
+        lo = np.empty(self.n_references, dtype=np.int32)
+        hi = np.empty(self.n_references, dtype=np.int32)
+        self._check(self._lib.ecb_sam_ranges(self._h, lo.ctypes.data, hi.ctypes.data))
+        return lo, hi
+
+    def stats(self):
+        st = EcbSamStats()
+        self._check(self._lib.ecb_sam_get_stats(self._h, ctypes.byref(st)))
+        return st.as_dict()
+
+    def close(self):
+        if self._h:
+            self._lib.ecb_sam_destroy(self._h)
             self._h = ctypes.c_void_p()
 
     def __enter__(self):

@@ -20,6 +20,7 @@
 #include "ecb_exchange.cuh"
 #include "ecb_cells_exchange.cuh"
 #include "ecb_bam.cuh"
+#include "ecb_sam.cuh"
 #include "ecb_collate.cuh"
 #include "ecb_longread.cuh"
 #include "ecb_samples.cuh"
@@ -698,7 +699,7 @@ void cells_release(ecb_ctx* c) {
 
 extern "C" {
 
-int ecb_version(void) { return 2007; }
+int ecb_version(void) { return 2008; }
 
 const char* ecb_last_error(const ecb_ctx* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
@@ -2302,14 +2303,15 @@ int bam_window(ecb_bam* d, long long b0, long long b1, u64 wbytes, u32 p0) {
       ecb_bam_compact_kernel<<<rgrid, 256, 0, c->stream>>>(R, (const u32*)d->valid.p, (const u32*)d->rowpos.p, (u32*)d->vrec.p);
       LAUNCH_CHECK("bam_compact");
       const int vgrid = (int)((n_valid + 255) / 256);
-      ecb_bam_starts_kernel<<<vgrid, 256, 0, c->stream>>>(win, (const u32*)d->vrec.p, n_valid, d->d_st, (u32*)d->starts.p);
+      const BamRecordAt A{win, (const u32*)d->vrec.p};
+      ecb_read_starts_kernel<<<vgrid, 256, 0, c->stream>>>(A, n_valid, &d->d_st->carry, (u32*)d->starts.p);
       LAUNCH_CHECK("bam_starts");
       u64 n_starts = 0;
       CKR(device_scan<false>(c, (const u32*)d->starts.p, (u32*)d->starts_x.p, n_valid, 0, &n_starts));
-      ecb_bam_rows_kernel<<<vgrid, 256, 0, c->stream>>>(R, (const u32*)d->vrec.p, n_valid, (const u32*)d->starts.p,
-                                                         (const u32*)d->starts_x.p, d->group, d->n_rows,
-                                                         (int32_t*)d->rows[d->rcur][0].p, (int32_t*)d->rows[d->rcur][1].p,
-                                                         (int32_t*)d->rows[d->rcur][2].p);
+      ecb_read_rows_kernel<<<vgrid, 256, 0, c->stream>>>(A, n_valid, (const u32*)d->starts.p, (const u32*)d->starts_x.p,
+                                                          d->group, d->n_rows, R.tid_target, R.tid_hap, &d->d_st->carry,
+                                                          (int32_t*)d->rows[d->rcur][0].p, (int32_t*)d->rows[d->rcur][1].p,
+                                                          (int32_t*)d->rows[d->rcur][2].p);
       LAUNCH_CHECK("bam_rows");
       d->n_rows += n_valid;
       d->group += (int64_t)n_starts;
@@ -2371,7 +2373,7 @@ int bam_decode(ecb_bam* d, const uint8_t* bytes, int64_t n_bytes, const int64_t*
     d->rcur = other;
     d->n_rows = keep;
     d->open_row = 0;
-    CK(cudaMemsetAsync(&d->d_st->open_row, 0, sizeof(unsigned long long), c->stream));
+    CK(cudaMemsetAsync(&d->d_st->carry.open_row, 0, sizeof(unsigned long long), c->stream));
   }
 
   // windows of whole blocks, at most ECB_OPT_BAM_WINDOW inflated bytes each (at least one block)
@@ -2417,7 +2419,7 @@ int bam_decode(ecb_bam* d, const uint8_t* bytes, int64_t n_bytes, const int64_t*
     d->finished = true;
     d->open_row = d->n_rows;   // the end of the file closes the last read
   } else {
-    d->open_row = d->h_st->open_row;
+    d->open_row = d->h_st->carry.open_row;
   }
   *read_group = (const int32_t*)d->rows[d->rcur][0].p;
   *target_idx = (const int32_t*)d->rows[d->rcur][1].p;
@@ -2512,6 +2514,313 @@ int ecb_bam_destroy(ecb_bam* d) {
   if (!d) return ECB_OK;
   cudaSetDevice(d->c->device);
   bam_release(d);
+  return ECB_OK;
+}
+
+}  // extern "C"
+
+// ---- device parse of single-sample SAM text (kernels in ecb_sam.cuh) --------------------------------------------
+struct ecb_sam {
+  ecb_ctx* c = nullptr;
+  int32_t n_ref = 0;
+  bool track = false;
+  int64_t next_line = 1;          // line number of the next call's first byte
+  DevBuf tid_target, tid_hap, range_min, range_max;
+  DevBuf slots, blob, name_off;   // the @SQ name table
+  u32 mask = 0;
+  DevBuf text, seg_nl, seg_tab, line_end, tabs_end, lines, valid, rowpos, vline, starts, starts_x;
+  DevBuf rows[2][3];              // read_group, target_idx, hap_idx; the open read moves to the other set
+  int rcur = 0;
+  u64 n_rows = 0, open_row = 0;
+  int64_t all_alignments = 0, group = -1;
+  bool failed = false, finished = false;
+  SamDevState* d_st = nullptr;
+  SamDevState* h_st = nullptr;    // pinned mirror
+  cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+  ecb_sam_stats stats{};
+};
+
+namespace {
+
+int sam_sync_state(ecb_sam* d) {
+  ecb_ctx* c = d->c;
+  CK(cudaMemcpyAsync(d->h_st, d->d_st, sizeof(SamDevState), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return ECB_OK;
+}
+
+void sam_release(ecb_sam* d) {
+  ecb_ctx* c = d->c;
+  DevBuf* bufs[] = {&d->tid_target, &d->tid_hap, &d->range_min, &d->range_max, &d->slots, &d->blob, &d->name_off,
+                    &d->text, &d->seg_nl, &d->seg_tab, &d->line_end, &d->tabs_end, &d->lines, &d->valid, &d->rowpos,
+                    &d->vline, &d->starts, &d->starts_x};
+  for (DevBuf* b : bufs) release(c, *b);
+  for (auto& set : d->rows)
+    for (DevBuf& b : set) release(c, b);
+  cudaStreamSynchronize(c->stream);
+  if (d->d_st) cudaFree(d->d_st);
+  if (d->h_st) cudaFreeHost(d->h_st);
+  for (auto& e : d->ev)
+    if (e) cudaEventDestroy(e);
+  delete d;
+}
+
+// The messages of the SAM_BAD_* kinds; alntools_b200/sam_utils.py raises the same ones.
+int sam_bad_line(ecb_sam* d, int64_t line, u32 kind) {
+  static const char* what[] = {"", "a header line (starting with '@') after the first alignment line",
+                               "fewer than 11 tab-separated fields", "QNAME empty or longer than 254 bytes",
+                               "FLAG not a decimal integer in [0, 65535]", "RNAME not '*' and not an @SQ name",
+                               "POS not a decimal integer in [0, 2147483647]", "RNEXT not '*', '=' or an @SQ name",
+                               "PNEXT not a decimal integer in [0, 2147483647]"};
+  if (kind == SAM_BAD_TID)
+    return fail(d->c, ECB_ERR_FORMAT, "line %lld: alignment with reference id -1 outside the header's %d references",
+                (long long)line, d->n_ref);
+  return fail(d->c, ECB_ERR_FORMAT, "line %lld: %s", (long long)line, kind < SAM_BAD_TID ? what[kind] : "bad line");
+}
+
+int sam_parse(ecb_sam* d, const uint8_t* text, int64_t n_bytes, int last, const int32_t** read_group,
+              const int32_t** target_idx, const int32_t** hap_idx, int64_t* rows) {
+  ecb_ctx* c = d->c;
+  if (n_bytes < 0 || n_bytes > (1ll << 31)) return fail(c, ECB_ERR_INVALID, "a call takes 0 to 2 GiB of text, not %lld bytes", (long long)n_bytes);
+  if (n_bytes > 0 && !text) return fail(c, ECB_ERR_INVALID, "NULL text");
+  const bool open_end = n_bytes > 0 && text[n_bytes - 1] != '\n';
+  if (open_end && !last) return fail(c, ECB_ERR_INVALID, "a call that is not the last must end with a whole line");
+  CK(cudaSetDevice(c->device));
+
+  // rows of the read the previous call left open go to the front
+  if (d->open_row > 0) {
+    const u64 keep = d->n_rows - d->open_row;
+    const int other = 1 - d->rcur;
+    for (int j = 0; j < 3; ++j) {
+      CKR(ensure(c, d->rows[other][j], (size_t)keep * 4 + 4));
+      if (keep)
+        CK(cudaMemcpyAsync(d->rows[other][j].p, (const int32_t*)d->rows[d->rcur][j].p + d->open_row, (size_t)keep * 4,
+                           cudaMemcpyDeviceToDevice, c->stream));
+    }
+    d->rcur = other;
+    d->n_rows = keep;
+    d->open_row = 0;
+    CK(cudaMemsetAsync(&d->d_st->carry.open_row, 0, sizeof(unsigned long long), c->stream));
+  }
+
+  // the text, a '\n' after an open last line, zeros up to a whole segment
+  const u64 n = (u64)n_bytes + (open_end ? 1 : 0);
+  const u32 n_seg = (u32)((n + SAM_SEG - 1) / SAM_SEG);
+  CKR(ensure(c, d->text, (size_t)n_seg * SAM_SEG + 16));
+  uint8_t* txt = (uint8_t*)d->text.p;
+  CK(cudaEventRecord(d->ev[0], c->stream));
+  if (n_bytes > 0) CK(cudaMemcpyAsync(txt, text, (size_t)n_bytes, cudaMemcpyHostToDevice, c->stream));
+  if (open_end) CK(cudaMemsetAsync(txt + n_bytes, '\n', 1, c->stream));
+  if ((u64)n_seg * SAM_SEG > n) CK(cudaMemsetAsync(txt + n, 0, (size_t)n_seg * SAM_SEG - n, c->stream));
+  CK(cudaEventRecord(d->ev[1], c->stream));
+
+  // lines
+  u64 n_lines64 = 0;
+  if (n_seg) {
+    CKR(ensure(c, d->seg_nl, (size_t)n_seg * 4));
+    CKR(ensure(c, d->seg_tab, (size_t)n_seg * 4));
+    const int wgrid = (int)(((u64)n_seg * 32 + 255) / 256);
+    ecb_sam_count_kernel<<<wgrid, 256, 0, c->stream>>>((const uint4*)txt, n_seg, (u32*)d->seg_nl.p, (u32*)d->seg_tab.p);
+    LAUNCH_CHECK("sam_count");
+    CKR(device_scan<false>(c, (const u32*)d->seg_tab.p, (u32*)d->seg_tab.p, n_seg, 0, nullptr));
+    CKR(device_scan<false>(c, (const u32*)d->seg_nl.p, (u32*)d->seg_nl.p, n_seg, 0, &n_lines64));
+    CKR(ensure(c, d->line_end, (size_t)n_lines64 * 4 + 4));
+    CKR(ensure(c, d->tabs_end, (size_t)n_lines64 * 4 + 4));
+    ecb_sam_lines_kernel<<<wgrid, 256, 0, c->stream>>>((const uint4*)txt, n_seg, (const u32*)d->seg_nl.p,
+                                                       (const u32*)d->seg_tab.p, (u32*)d->line_end.p, (u32*)d->tabs_end.p);
+    LAUNCH_CHECK("sam_lines");
+  }
+  const u32 n_lines = (u32)n_lines64;
+  CK(cudaEventRecord(d->ev[2], c->stream));
+
+  // fields, checks and the filter
+  u64 n_valid64 = 0;
+  if (n_lines) {
+    CKR(ensure(c, d->lines, (size_t)n_lines * sizeof(SamLine)));
+    CKR(ensure(c, d->valid, (size_t)n_lines * 4));
+    CKR(ensure(c, d->rowpos, (size_t)n_lines * 4));
+    SamFields F{txt, (const u32*)d->line_end.p, (const u32*)d->tabs_end.p, n_lines,
+                SamNames{(const SamNameSlot*)d->slots.p, d->mask, (const char*)d->blob.p, (const int64_t*)d->name_off.p},
+                d->n_ref, d->track ? (int32_t*)d->range_min.p : nullptr, d->track ? (int32_t*)d->range_max.p : nullptr,
+                d->d_st};
+    ecb_sam_fields_kernel<<<(n_lines + 255) / 256, 256, 0, c->stream>>>(F, (SamLine*)d->lines.p, (u32*)d->valid.p);
+    LAUNCH_CHECK("sam_fields");
+    CKR(device_scan<false>(c, (const u32*)d->valid.p, (u32*)d->rowpos.p, n_lines, 0, &n_valid64));
+    CKR(sam_sync_state(d));
+    if (d->h_st->bad != SAM_NO_ERROR)
+      return sam_bad_line(d, d->next_line + (int64_t)(d->h_st->bad >> 4), (u32)(d->h_st->bad & 15u));
+  }
+  CK(cudaEventRecord(d->ev[3], c->stream));
+
+  // rules and rows
+  const u32 n_valid = (u32)n_valid64;
+  if (n_valid) {
+    CKR(ensure(c, d->vline, (size_t)n_valid * 4));
+    CKR(ensure(c, d->starts, (size_t)n_valid * 4));
+    CKR(ensure(c, d->starts_x, (size_t)n_valid * 4));
+    for (DevBuf& b : d->rows[d->rcur]) CKR(ensure(c, b, (size_t)(d->n_rows + n_valid) * 4, true));
+    ecb_sam_compact_kernel<<<(n_lines + 255) / 256, 256, 0, c->stream>>>((const u32*)d->valid.p, (const u32*)d->rowpos.p,
+                                                                         n_lines, (u32*)d->vline.p);
+    LAUNCH_CHECK("sam_compact");
+    const SamRecordAt A{txt, (const SamLine*)d->lines.p, (const u32*)d->vline.p};
+    const int vgrid = (int)((n_valid + 255) / 256);
+    ecb_read_starts_kernel<<<vgrid, 256, 0, c->stream>>>(A, n_valid, &d->d_st->carry, (u32*)d->starts.p);
+    LAUNCH_CHECK("sam_starts");
+    u64 n_starts = 0;
+    CKR(device_scan<false>(c, (const u32*)d->starts.p, (u32*)d->starts_x.p, n_valid, 0, &n_starts));
+    ecb_read_rows_kernel<<<vgrid, 256, 0, c->stream>>>(A, n_valid, (const u32*)d->starts.p, (const u32*)d->starts_x.p,
+                                                        d->group, d->n_rows, (const int32_t*)d->tid_target.p,
+                                                        (const int32_t*)d->tid_hap.p, &d->d_st->carry,
+                                                        (int32_t*)d->rows[d->rcur][0].p, (int32_t*)d->rows[d->rcur][1].p,
+                                                        (int32_t*)d->rows[d->rcur][2].p);
+    LAUNCH_CHECK("sam_rows");
+    d->n_rows += n_valid;
+    d->group += (int64_t)n_starts;
+  }
+  CK(cudaEventRecord(d->ev[4], c->stream));
+  CKR(sam_sync_state(d));
+  d->all_alignments += n_lines;
+  d->next_line += n_lines;
+  d->stats.bytes += n_bytes;
+  d->stats.lines += n_lines;
+  d->stats.calls++;
+  d->stats.h2d_ms += bam_ms(d->ev[0], d->ev[1]);
+  d->stats.lines_ms += bam_ms(d->ev[1], d->ev[2]);
+  d->stats.fields_ms += bam_ms(d->ev[2], d->ev[3]);
+  d->stats.rules_ms += bam_ms(d->ev[3], d->ev[4]);
+  if (last) {
+    d->finished = true;
+    d->open_row = d->n_rows;   // the end of the text closes the last read
+  } else {
+    d->open_row = d->h_st->carry.open_row;
+  }
+  *read_group = (const int32_t*)d->rows[d->rcur][0].p;
+  *target_idx = (const int32_t*)d->rows[d->rcur][1].p;
+  *hap_idx = (const int32_t*)d->rows[d->rcur][2].p;
+  *rows = (int64_t)d->open_row;
+  return ECB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ecb_sam_create(ecb_ctx* c, const char* ref_names, const int64_t* ref_name_off, int32_t n_references,
+                   const int32_t* tid_target, const int32_t* tid_hap, int64_t first_line, int track_ranges, ecb_sam** out) {
+  if (!c || !out) return ECB_ERR_INVALID;
+  *out = nullptr;
+  if (n_references < 0 || !ref_name_off || (n_references > 0 && (!tid_target || !tid_hap)))
+    return fail(c, ECB_ERR_INVALID, "bad reference tables");
+  if (first_line < 1) return fail(c, ECB_ERR_INVALID, "first_line must be at least 1");
+  if (c->with_cells) return fail(c, ECB_ERR_INVALID, "the device SAM decoder covers the single-sample path only");
+  if (ref_name_off[0] != 0) return fail(c, ECB_ERR_INVALID, "ref_name_off[0] must be 0");
+  for (int32_t i = 0; i < n_references; ++i)
+    if (ref_name_off[i + 1] < ref_name_off[i] || ref_name_off[i + 1] - ref_name_off[i] > 0xFFFFFFFFll)
+      return fail(c, ECB_ERR_INVALID, "ref_name_off is not a list of offsets");
+  const int64_t blob_bytes = ref_name_off[n_references];
+  if (blob_bytes > 0 && !ref_names) return fail(c, ECB_ERR_INVALID, "NULL ref_names");
+
+  // the name table: open addressing on sam_hash, at most half full; the first of two equal names keeps its slot
+  const u32 n_slots = std::max<u32>(16u, pow2_ceil((u64)n_references * 2));
+  std::vector<SamNameSlot> slots(n_slots, SamNameSlot{0ull, -1, 0});
+  for (int32_t t = 0; t < n_references; ++t) {
+    const uint8_t* nm = (const uint8_t*)ref_names + ref_name_off[t];
+    const u32 len = (u32)(ref_name_off[t + 1] - ref_name_off[t]);
+    const unsigned long long h = sam_hash(nm, len);
+    for (u32 i = (u32)h & (n_slots - 1);; i = (i + 1) & (n_slots - 1)) {
+      SamNameSlot& e = slots[i];
+      if (e.tid < 0) {
+        e = SamNameSlot{h, t, 0};
+        break;
+      }
+      if (e.hash == h && ref_name_off[e.tid + 1] - ref_name_off[e.tid] == len &&
+          memcmp(ref_names + ref_name_off[e.tid], nm, len) == 0)
+        break;
+    }
+  }
+
+  CK(cudaSetDevice(c->device));
+  ecb_sam* d = new ecb_sam();
+  d->c = c;
+  d->n_ref = n_references;
+  d->track = track_ranges != 0;
+  d->next_line = first_line;
+  d->mask = n_slots - 1;
+  auto bail = [&](int code) {
+    sam_release(d);
+    return code;
+  };
+  const size_t tb = (size_t)n_references * 4 + 4;
+  int rc = ECB_OK;
+  for (DevBuf* b : {&d->tid_target, &d->tid_hap, &d->range_min, &d->range_max})
+    if (rc == ECB_OK) rc = ensure(c, *b, tb);
+  if (rc == ECB_OK) rc = ensure(c, d->slots, (size_t)n_slots * sizeof(SamNameSlot));
+  if (rc == ECB_OK) rc = ensure(c, d->blob, (size_t)blob_bytes + 16);
+  if (rc == ECB_OK) rc = ensure(c, d->name_off, ((size_t)n_references + 1) * 8);
+  if (rc != ECB_OK) return bail(rc);
+  if (cudaMalloc(&d->d_st, sizeof(SamDevState)) != cudaSuccess || cudaMallocHost(&d->h_st, sizeof(SamDevState)) != cudaSuccess)
+    return bail(fail(c, ECB_ERR_CUDA, "decoder state allocation failed"));
+  for (auto& e : d->ev)
+    if (cudaEventCreate(&e) != cudaSuccess) return bail(fail(c, ECB_ERR_CUDA, "cudaEventCreate failed"));
+  memset(d->h_st, 0, sizeof(SamDevState));
+  d->h_st->bad = SAM_NO_ERROR;
+  std::vector<int32_t> lo((size_t)n_references + 1, INT32_MAX);
+  const cudaMemcpyKind h2d = cudaMemcpyHostToDevice;
+  bool ok = true;
+  if (n_references > 0)
+    ok = cudaMemcpyAsync(d->tid_target.p, tid_target, (size_t)n_references * 4, h2d, c->stream) == cudaSuccess &&
+         cudaMemcpyAsync(d->tid_hap.p, tid_hap, (size_t)n_references * 4, h2d, c->stream) == cudaSuccess;
+  if (ok && blob_bytes > 0) ok = cudaMemcpyAsync(d->blob.p, ref_names, (size_t)blob_bytes, h2d, c->stream) == cudaSuccess;
+  ok = ok && cudaMemcpyAsync(d->name_off.p, ref_name_off, ((size_t)n_references + 1) * 8, h2d, c->stream) == cudaSuccess &&
+       cudaMemcpyAsync(d->slots.p, slots.data(), (size_t)n_slots * sizeof(SamNameSlot), h2d, c->stream) == cudaSuccess &&
+       cudaMemcpyAsync(d->range_min.p, lo.data(), tb, h2d, c->stream) == cudaSuccess &&
+       cudaMemsetAsync(d->range_max.p, 0xFF, tb, c->stream) == cudaSuccess &&
+       cudaMemcpyAsync(d->d_st, d->h_st, sizeof(SamDevState), h2d, c->stream) == cudaSuccess &&
+       cudaStreamSynchronize(c->stream) == cudaSuccess;
+  if (!ok) return bail(fail(c, ECB_ERR_CUDA, "decoder initialisation failed"));
+  *out = d;
+  return ECB_OK;
+}
+
+int ecb_sam_parse(ecb_sam* d, const uint8_t* text, int64_t n_bytes, int last, const int32_t** read_group,
+                  const int32_t** target_idx, const int32_t** hap_idx, int64_t* rows) {
+  if (!d || !read_group || !target_idx || !hap_idx || !rows) return ECB_ERR_INVALID;
+  if (d->failed) return fail(d->c, ECB_ERR_STATE, "this decoder failed earlier; create a new one");
+  if (d->finished) return fail(d->c, ECB_ERR_STATE, "this decoder has had its last call");
+  const int rc = sam_parse(d, text, n_bytes, last, read_group, target_idx, hap_idx, rows);
+  if (rc != ECB_OK) d->failed = true;
+  return rc;
+}
+
+int ecb_sam_counters(const ecb_sam* d, int64_t* all_alignments, int64_t* n_groups) {
+  if (!d || !all_alignments || !n_groups) return ECB_ERR_INVALID;
+  *all_alignments = d->all_alignments;
+  *n_groups = d->group + 1;
+  return ECB_OK;
+}
+
+int ecb_sam_ranges(ecb_sam* d, int32_t* range_min, int32_t* range_max) {
+  if (!d || (d->n_ref > 0 && (!range_min || !range_max))) return ECB_ERR_INVALID;
+  ecb_ctx* c = d->c;
+  if (!d->track) return fail(c, ECB_ERR_STATE, "ranges were not tracked");
+  if (d->n_ref == 0) return ECB_OK;
+  CK(cudaSetDevice(c->device));
+  CK(cudaMemcpyAsync(range_min, d->range_min.p, (size_t)d->n_ref * 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(range_max, d->range_max.p, (size_t)d->n_ref * 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return ECB_OK;
+}
+
+int ecb_sam_get_stats(const ecb_sam* d, ecb_sam_stats* out) {
+  if (!d || !out) return ECB_ERR_INVALID;
+  *out = d->stats;
+  return ECB_OK;
+}
+
+int ecb_sam_destroy(ecb_sam* d) {
+  if (!d) return ECB_OK;
+  cudaSetDevice(d->c->device);
+  sam_release(d);
   return ECB_OK;
 }
 

@@ -31,6 +31,15 @@
 #define BAM_ERR_NAME 2u
 #define BAM_ERR_TID 4u
 
+// What the rows of one call hand to the next: the open read and the trimmed name of the last valid record.  Shared
+// by the BAM and SAM decoders (ecb_sam.cuh).
+struct ReadCarry {
+  unsigned long long open_row;       // first row of the read that is still open
+  int have_name;              // a valid record has been seen
+  u32 name_len;
+  char name[256];             // trimmed name of the last valid record
+};
+
 // One BGZF block of a call: raw DEFLATE payload in the compressed buffer, inflated bytes in the window buffer.
 struct BamBlock {
   u64 src_off;
@@ -46,10 +55,7 @@ struct BamDevState {
   long long bad_block;        // first corrupt block (index among the call's blocks)
   int bad_tid;                // a refID outside the header
   u32 hop_state, hop_land, hop_bs;   // end of the window's hop: state, offset, block_size there
-  unsigned long long open_row;       // first row of the read that is still open
-  int have_name;              // a valid record has been seen
-  u32 name_len;
-  char name[256];             // trimmed name of the last valid record
+  ReadCarry carry;
 };
 
 __device__ __forceinline__ u32 bam_le32(const uint8_t* p) {
@@ -61,6 +67,17 @@ __device__ __forceinline__ u32 bam_trimmed_len(const uint8_t* s, u32 n) {
   for (u32 i = 0; i < n; ++i)
     if (s[i] == ' ') return i > 0 ? i : n;
   return n;
+}
+
+// The single-sample filter (alntools/bam_utils.py:264-270; bamcols.cpp:record_validity and emitter._valid on the
+// host) on one alignment's fields, for both device decoders: ECB_REC_BAD_TID is a valid alignment whose refID lies
+// outside [0, n_ref).
+enum { ECB_REC_FILTERED = 0, ECB_REC_VALID = 1, ECB_REC_BAD_TID = 2 };
+__device__ __forceinline__ int ecb_alignment_rule(u32 flag, int tid, int ntid, int npos, int n_ref) {
+  if (flag & 0x4) return ECB_REC_FILTERED;
+  if ((flag & 0x1) && ((flag & 0x80) || !(flag & 0x2) || tid != ntid || npos < 0)) return ECB_REC_FILTERED;
+  if (tid < 0 || tid >= n_ref) return ECB_REC_BAD_TID;
+  return ECB_REC_VALID;
 }
 
 __global__ void __launch_bounds__(ECB_BAM_INFLATE_THREADS) ecb_bam_inflate_kernel(const uint8_t* __restrict__ comp,
@@ -209,22 +226,22 @@ __global__ void ecb_bam_validity_kernel(BamRules R, u32* __restrict__ valid) {
   const u32 l_name = q[8];
   const u32 flag = bam_le16(q + 14);
   const int ntid = (int)bam_le32(q + 20), npos = (int)bam_le32(q + 24);
-  u32 v = 1;
+  u32 v = 0;
   if (32 + l_name > bs || l_name == 0) {
     atomicOr(&R.st->error, BAM_ERR_NAME);
-    v = 0;
-  } else if (flag & 0x4) {
-    v = 0;
-  } else if ((flag & 0x1) && ((flag & 0x80) || !(flag & 0x2) || tid != ntid || npos < 0)) {
-    v = 0;
-  } else if (tid < 0 || tid >= R.n_ref) {
-    atomicOr(&R.st->error, BAM_ERR_TID);
-    R.st->bad_tid = tid;
-    v = 0;
-  } else if (R.range_min) {
-    const int pos = (int)bam_le32(q + 4);
-    atomicMin(&R.range_min[tid], pos);
-    atomicMax(&R.range_max[tid], pos);
+  } else {
+    const int rule = ecb_alignment_rule(flag, tid, ntid, npos, R.n_ref);
+    if (rule == ECB_REC_BAD_TID) {
+      atomicOr(&R.st->error, BAM_ERR_TID);
+      R.st->bad_tid = tid;
+    } else if (rule == ECB_REC_VALID) {
+      v = 1;
+      if (R.range_min) {
+        const int pos = (int)bam_le32(q + 4);
+        atomicMin(&R.range_min[tid], pos);
+        atomicMax(&R.range_max[tid], pos);
+      }
+    }
   }
   valid[i] = v;
 }
@@ -236,23 +253,32 @@ __global__ void ecb_bam_compact_kernel(BamRules R, const u32* __restrict__ valid
   vrec[rowpos[i]] = R.off[i];
 }
 
+// The valid records of a call in order, as the shared starts and rows kernels read them: record k's trimmed name and
+// refID.  BamRecordAt reads them from the inflated window; SamRecordAt (ecb_sam.cuh) from the parsed lines.
+struct BamRecordAt {
+  const uint8_t* win;
+  const u32* vrec;       // [n_valid] record offsets
+  __device__ __forceinline__ const uint8_t* name(u32 k, u32& len) const {
+    const uint8_t* q = win + vrec[k] + 4;
+    len = bam_trimmed_len(q + 32, (u32)q[8] - 1);
+    return q + 32;
+  }
+  __device__ __forceinline__ int tid(u32 k) const { return (int)bam_le32(win + vrec[k] + 4); }
+};
+
 // starts[k] = 1 iff valid record k's trimmed name differs from the previous valid record's (bamcols.cpp:single_starts)
-__global__ void ecb_bam_starts_kernel(const uint8_t* __restrict__ win, const u32* __restrict__ vrec, u32 n_valid,
-                                      const BamDevState* st, u32* __restrict__ starts) {
+template <class Rec>
+__global__ void ecb_read_starts_kernel(Rec A, u32 n_valid, const ReadCarry* carry, u32* __restrict__ starts) {
   const u32 k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= n_valid) return;
-  const uint8_t* q = win + vrec[k] + 4;
-  const uint8_t* nm = q + 32;
-  const u32 nl = bam_trimmed_len(nm, (u32)q[8] - 1);
+  u32 nl, pl;
+  const uint8_t* nm = A.name(k, nl);
   const uint8_t* pn;
-  u32 pl;
   if (k > 0) {
-    const uint8_t* pq = win + vrec[k - 1] + 4;
-    pn = pq + 32;
-    pl = bam_trimmed_len(pn, (u32)pq[8] - 1);
-  } else if (st->have_name) {
-    pn = (const uint8_t*)st->name;
-    pl = st->name_len;
+    pn = A.name(k - 1, pl);
+  } else if (carry->have_name) {
+    pn = (const uint8_t*)carry->name;
+    pl = carry->name_len;
   } else {
     starts[k] = 1;
     return;
@@ -263,22 +289,24 @@ __global__ void ecb_bam_starts_kernel(const uint8_t* __restrict__ win, const u32
 }
 
 // Rows of the valid records at row0 + k; the open read and the carried name are updated.
-__global__ void ecb_bam_rows_kernel(BamRules R, const u32* __restrict__ vrec, u32 n_valid, const u32* __restrict__ starts,
-                                    const u32* __restrict__ starts_x, long long group0, unsigned long long row0,
-                                    int32_t* __restrict__ rg, int32_t* __restrict__ tg, int32_t* __restrict__ hp) {
+template <class Rec>
+__global__ void ecb_read_rows_kernel(Rec A, u32 n_valid, const u32* __restrict__ starts, const u32* __restrict__ starts_x,
+                                     long long group0, unsigned long long row0, const int32_t* __restrict__ tid_target,
+                                     const int32_t* __restrict__ tid_hap, ReadCarry* carry, int32_t* __restrict__ rg,
+                                     int32_t* __restrict__ tg, int32_t* __restrict__ hp) {
   const u32 k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= n_valid) return;
-  const uint8_t* q = R.win + vrec[k] + 4;
-  const int tid = (int)bam_le32(q);
+  const int tid = A.tid(k);
   const unsigned long long row = row0 + k;
   rg[row] = (int32_t)(group0 + (long long)starts_x[k] + (long long)starts[k]);
-  tg[row] = R.tid_target[tid];
-  hp[row] = R.tid_hap[tid];
-  if (starts[k]) atomicMax(&R.st->open_row, row);
+  tg[row] = tid_target[tid];
+  hp[row] = tid_hap[tid];
+  if (starts[k]) atomicMax(&carry->open_row, row);
   if (k + 1 == n_valid) {
-    const u32 nl = bam_trimmed_len(q + 32, (u32)q[8] - 1);
-    for (u32 j = 0; j < nl; ++j) R.st->name[j] = (char)q[32 + j];
-    R.st->name_len = nl;
-    R.st->have_name = 1;
+    u32 nl;
+    const uint8_t* nm = A.name(k, nl);
+    for (u32 j = 0; j < nl; ++j) carry->name[j] = (char)nm[j];
+    carry->name_len = nl;
+    carry->have_name = 1;
   }
 }

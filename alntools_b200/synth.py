@@ -156,3 +156,45 @@ def columns_to_bam_seq(filename, cols, n_targets, n_haps, read_len=100, level=1,
         for off in range(0, flat.size, per_block):
             fh.write(bam_io.bgzf_block(flat[off:off + per_block].tobytes(), level))
         fh.write(bam_io.BGZF_EOF)
+
+
+def columns_to_sam(filename, cols, n_targets, n_haps, read_len=0, seed=0, chunk=1 << 20):
+    """The alignments of columns_to_bam (read_len=0: CIGAR, SEQ and QUAL '*') or columns_to_bam_seq (read_len > 0: a
+    CIGAR of one read_len-M operation and seeded random bases and qualities) as SAM text, with the same @SQ list, names
+    ('read%09d'), flags (0), POS (11) and mates ('*', 0); written in fixed-width rows with numpy."""
+    tids = cols["target_idx"].astype(np.int64) * n_haps + cols["hap_idx"]
+    ids = np.asarray(cols["read_group"], dtype=np.int64)
+    refs = reference_names(n_targets, n_haps)
+    if read_len == 0:
+        tail = b"*\t*\t0\t0\t*\t*\n"
+    else:
+        tail = b"%dM\t*\t0\t0\t" % read_len
+    head = b"read000000000\t0\tENSMUST00000000000_A\t11\t255\t"
+    width = len(head) + len(tail) + (2 * read_len + 2 if read_len else 0)
+    rng = np.random.default_rng(seed)
+    letters = np.frombuffer(b"ABCDEFGH", dtype=np.uint8)
+    bases = np.frombuffer(b"ACGT", dtype=np.uint8)
+    with open(filename, "wb") as fh:
+        fh.write(b"@HD\tVN:1.0\tSO:queryname\n")
+        fh.write(b"".join(b"@SQ\tSN:%s\tLN:%d\n" % (name.encode(), length) for name, length in refs))
+        for lo in range(0, len(tids), chunk):
+            t, r = tids[lo:lo + chunk], ids[lo:lo + chunk].copy()
+            n = len(t)
+            rows = np.empty((n, width), dtype=np.uint8)
+            rows[:, :len(head)] = np.frombuffer(head, dtype=np.uint8)
+            rows[:, len(head):len(head) + len(tail)] = np.frombuffer(tail, dtype=np.uint8)
+            for d in range(8, -1, -1):                       # read%09d
+                rows[:, 4 + d] = (r % 10 + 48).astype(np.uint8)
+                r //= 10
+            target, hap = t // n_haps, t % n_haps
+            for d in range(10, -1, -1):                      # ENSMUST%011d_<hap>
+                rows[:, 23 + d] = (target % 10 + 48).astype(np.uint8)
+                target //= 10
+            rows[:, 35] = letters[hap]
+            if read_len:
+                at = len(head) + len(tail)
+                rows[:, at:at + read_len] = bases[rng.integers(0, 4, (n, read_len))]
+                rows[:, at + read_len] = ord("\t")
+                rows[:, at + read_len + 1:at + 2 * read_len + 1] = rng.integers(35, 74, (n, read_len), dtype=np.uint8)
+                rows[:, -1] = ord("\n")
+            fh.write(rows.tobytes())

@@ -44,8 +44,9 @@ enum ecb_status {
   ECB_ERR_EMPTY = -5,       /* finalize with zero equivalence classes (the reference raises too:
                                alntools/matrix/Sparse3DMatrix.py:45-46) */
   ECB_ERR_STATE = -6,       /* call sequence error */
-  ECB_ERR_FORMAT = -7       /* malformed BAM input of the device decoder (ecb_bam_decode; since version 2002), or
-                               malformed EC-file arrays (ecb_push_ecs / ecb_sample_append; since version 2007) */
+  ECB_ERR_FORMAT = -7       /* malformed BAM input of the device decoder (ecb_bam_decode; since version 2002),
+                               malformed EC-file arrays (ecb_push_ecs / ecb_sample_append; since version 2007), or
+                               a bad SAM line (ecb_sam_parse; since version 2008) */
 };
 
 /* Longest read (alignments sharing one name) a push accepts by default, and the longest one the grouping kernel
@@ -417,6 +418,46 @@ int ecb_bam_counters(const ecb_bam* d, int64_t* all_alignments, int64_t* n_group
 int ecb_bam_ranges(ecb_bam* d, int32_t* range_min, int32_t* range_max);
 int ecb_bam_get_stats(const ecb_bam* d, ecb_bam_stats* out);
 int ecb_bam_destroy(ecb_bam* d);
+
+/* ---- device parse of single-sample SAM text (since version 2008) -------------------------------------------------
+ * SAM text in, the columns ecb_bam_decode gives for the BAM file that holds the same alignments out, in device memory,
+ * ready for ecb_push(..., on_device = 1): lines found and QNAME, FLAG, RNAME, POS, RNEXT and PNEXT parsed on the GPU,
+ * then the filters, name trimming and the name-change test of the BAM decoder.  A decoder is bound to one context and
+ * uses its device, stream and memory pool; destroy it before the context.  A decoder that has failed refuses further
+ * calls.
+ *
+ * ecb_sam_create: the @SQ names of the header, in order: name t is ref_names[ref_name_off[t], ref_name_off[t + 1])
+ *   (not NUL-terminated; ref_name_off[0] = 0); tid_target / tid_hap[n_references] as for ecb_bam_create (copied).  The
+ *   names go into a device hash table (the first of two equal names wins).  first_line: the line number of the first
+ *   byte the first call gives (the header's line count + 1), for error messages.  track_ranges as for ecb_bam_create.
+ * ecb_sam_parse: one call per run of whole alignment lines (every line ends in '\n', except possibly the last line of
+ *   the `last` call), at most 2 GiB, in input order; the text is copied with one host-to-device copy (pinned host
+ *   memory preferred).  Returns DEVICE pointers to the rows of every read closed by this call (valid until the next
+ *   call); read_group continues from call to call as ecb_bam_decode's does, and reads may span calls.  A bad line fails
+ *   with ECB_ERR_FORMAT and a message "line N: <what>" for the first bad line of the call: a line starting with '@',
+ *   fewer than 11 tab-separated fields, QNAME empty or longer than 254 bytes, FLAG not a decimal in [0, 65535], POS or
+ *   PNEXT not a decimal in [0, 2^31 - 1], RNAME not '*' or an @SQ name, RNEXT not '*', '=' or an @SQ name, or a valid
+ *   alignment whose RNAME is '*'.  MAPQ, CIGAR, TLEN, SEQ, QUAL and tags are not looked at. */
+typedef struct ecb_sam ecb_sam;
+typedef struct ecb_sam_stats {
+  int64_t bytes;           /* text bytes copied host->device                                                  */
+  int64_t lines;           /* alignment lines parsed (= all_alignments)                                       */
+  int64_t calls;
+  double h2d_ms;           /* stream time between CUDA events around each phase, summed over the calls: the   */
+  double lines_ms;         /* lines and fields phases include the host round trips of their count read-backs  */
+  double fields_ms;
+  double rules_ms;
+} ecb_sam_stats;
+int ecb_sam_create(ecb_ctx* ctx, const char* ref_names, const int64_t* ref_name_off, int32_t n_references,
+                   const int32_t* tid_target, const int32_t* tid_hap, int64_t first_line, int track_ranges, ecb_sam** out);
+int ecb_sam_parse(ecb_sam* d, const uint8_t* text, int64_t n_bytes, int last, const int32_t** read_group,
+                  const int32_t** target_idx, const int32_t** hap_idx, int64_t* rows);
+/* alignment lines seen so far (valid or not) and reads started */
+int ecb_sam_counters(const ecb_sam* d, int64_t* all_alignments, int64_t* n_groups);
+/* host int32[n_references] each; min > max where no valid alignment was seen */
+int ecb_sam_ranges(ecb_sam* d, int32_t* range_min, int32_t* range_max);
+int ecb_sam_get_stats(const ecb_sam* d, ecb_sam_stats* out);
+int ecb_sam_destroy(ecb_sam* d);
 
 /* ---- collation of alignments by read name (since version 2003) ----------------------------------------------
  * For files that are not grouped by read name.  A read is the set of valid alignments that share a trimmed name,
