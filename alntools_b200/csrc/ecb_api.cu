@@ -85,13 +85,13 @@ struct ecb_ctx {
   // reads longer than ECB_MAX_READ_ALIGNMENTS (ecb_longread.cuh): the grouping kernel's list, the sorted list with
   // the prefix of the lengths, the run ranks and the per-read sums
   DevBuf lr_list, lr_meta, lr_rank, lr_acc;
-  DevBuf scan_partials;  // u64 block sums + 1 total
+  DevBuf scan_buf;       // single-pass scan state: ticket, one status word per tile, total
   // push bookkeeping
   u64 min_base = ~0ull, max_end = 0;
   int64_t n_alignments = 0;
   u32 push_count = 0;
   // finalize scratch + results (device)
-  DevBuf bitmap, word_rank, first_rel, ecid_of, ec_keep;
+  DevBuf bitmap, word_rank, first_rel, ecid_of, prov_of, ec_keep;
   DevBuf r_a_indptr, r_a_indices, r_a_data, r_n_indptr, r_n_indices, r_n_data, r_cell_order;
   // cells scratch
   CellScratch cells;
@@ -217,31 +217,38 @@ int check_device_error(ecb_ctx* c) {
   return fail(c, ECB_ERR_LIMIT, "device error bits 0x%x", e);
 }
 
+// State of a single-pass scan over n_tiles tiles (ecb_scan.cuh), cleared on the stream: the ticket and the status
+// words; the word after them receives the total.
+int scan_state(ecb_ctx* c, u64 n_tiles, u64** state) {
+  CKR(ensure(c, c->scan_buf, ((size_t)n_tiles + 2) * sizeof(u64)));
+  *state = (u64*)c->scan_buf.p;
+  CK(cudaMemsetAsync(*state, 0, ((size_t)n_tiles + 1) * sizeof(u64), c->stream));
+  return ECB_OK;
+}
+
 // Device address of the total of a device_scan over n items, valid until the next scan: a copy of it enqueued
 // after the scan reads it without a synchronisation of its own.
 const u64* scan_total(const ecb_ctx* c, u64 n) {
-  return (const u64*)c->scan_partials.p + (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
+  return (const u64*)c->scan_buf.p + (n + SCAN_BLOCK - 1) / SCAN_BLOCK + 1;
 }
 
 // Device-wide exclusive scan (in may alias out).  total_out (host) may be NULL.
 template <bool POPC>
 int device_scan(ecb_ctx* c, const u32* in, u32* out, u64 n, u32 base_offset, u64* total_out) {
-  const u32 n_blocks = (u32)((n + SCAN_BLOCK - 1) / SCAN_BLOCK);
-  CKR(ensure(c, c->scan_partials, ((size_t)n_blocks + 2) * sizeof(u64)));
-  u64* partials = (u64*)c->scan_partials.p;
-  u64* d_total = (u64*)scan_total(c, n);
-  if (n_blocks == 0) {
+  const u64 n_tiles = (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
+  if (n_tiles == 0) {
+    CKR(ensure(c, c->scan_buf, 2 * sizeof(u64)));
+    CK(cudaMemsetAsync((u64*)c->scan_buf.p + 1, 0, sizeof(u64), c->stream));   // scan_total() of an empty scan
     if (total_out) *total_out = 0;
     return ECB_OK;
   }
-  scan_block_sums_kernel<POPC><<<n_blocks, SCAN_THREADS, 0, c->stream>>>(in, n, partials);
-  LAUNCH_CHECK("scan_block_sums");
-  scan_partials_kernel<<<1, 1024, 0, c->stream>>>(partials, n_blocks, d_total);
-  LAUNCH_CHECK("scan_partials");
-  scan_apply_kernel<POPC><<<n_blocks, SCAN_THREADS, 0, c->stream>>>(in, n, partials, out, base_offset);
-  LAUNCH_CHECK("scan_apply");
+  if (n_tiles > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "scan of %llu items is too long", (unsigned long long)n);
+  u64* state = nullptr;
+  CKR(scan_state(c, n_tiles, &state));
+  scan_kernel<POPC><<<(unsigned)n_tiles, SCAN_THREADS, 0, c->stream>>>(in, n, out, base_offset, state, (u32)n_tiles);
+  LAUNCH_CHECK("scan");
   if (total_out) {
-    CK(cudaMemcpyAsync(total_out, d_total, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(total_out, state + n_tiles + 1, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     c->stats.d2h_bytes += sizeof(u64);
   }
@@ -380,22 +387,18 @@ void group_geometry(ecb_ctx* c, int64_t n, int* grid, int* chunk_len) {
   *chunk_len = (int)cl;
 }
 
-// Rows of the ECs claimed in this push (ids e0..e1).  No host round trip: the kernels reserve their rows on
-// the device-side arena cursor, the lists of the longer reads are sized on the device, and all four kernels
-// are launched whether their lists turn out empty or not (an empty list costs a few microseconds).
-int harvest_new_rows(ecb_ctx* c, const int32_t* rg, const int32_t* tg, const int32_t* hp, int64_t n, u32 e0,
-                     u32 e1) {
-  if (e1 <= e0) return ECB_OK;
-  // room for one row entry per alignment of this push: the rows of its new ECs come from distinct reads
-  const u64 bound = c->arena_used + (u64)n;
-  if (bound > 0xFFFFFFFFull) return fail(c, ECB_ERR_LIMIT, "row arena exceeds 2^32 entries");
-  CKR(ensure(c, c->arena, (size_t)bound * sizeof(uint2), true));
+// Rows of the ECs claimed since provisional id e0, up to the device's EC counter.  No host round trip: the
+// range ends where the counter stands when the kernels run, the kernels reserve their rows on the device-side
+// arena cursor, the lists of the longer reads are sized on the device, and all four kernels are launched
+// whether their range and lists turn out empty or not (an empty one costs a few microseconds).  The arena has
+// room for the push (push_one sizes it before the grouping kernel).
+int harvest_new_rows(ecb_ctx* c, const int32_t* rg, const int32_t* tg, const int32_t* hp, int64_t n, u32 e0) {
   HarvestParams H{};
   H.rg = rg; H.tg = tg; H.hp = hp; H.n = (int)n;
   H.n_targets = c->n_targets; H.n_haps = c->n_haps;
   H.ec_rep = (const u32*)c->ec_rep.p;
   H.ec_len = (const u32*)c->ec_len.p;
-  H.e0 = e0; H.e1 = e1;
+  H.e0 = e0;
   H.row_len = (u32*)c->row_len.p;
   H.row_off = (u32*)c->row_off.p;
   H.long_list = (u32*)c->long_list.p;
@@ -403,8 +406,7 @@ int harvest_new_rows(ecb_ctx* c, const int32_t* rg, const int32_t* tg, const int
   H.big_list = (u32*)c->big_list.p;
   H.ctr = c->d_ctr;
   H.arena = (uint2*)c->arena.p;
-  const u32 n_new = e1 - e0;
-  ecb_harvest_short_kernel<<<grid_for(n_new, 256, c->sm_count * 16), 256, 0, c->stream>>>(H);
+  ecb_harvest_short_kernel<<<c->sm_count * 16, 256, 0, c->stream>>>(H);
   LAUNCH_CHECK("harvest_short");
   ecb_harvest_warp_kernel<<<c->sm_count * 8, 256, 0, c->stream>>>(H);
   LAUNCH_CHECK("harvest_warp");
@@ -855,6 +857,11 @@ static int push_one(ecb_ctx* c, const int32_t* read_group, const int32_t* target
   CK(cudaMemsetAsync(c->overflow_bits.p, 0, ov_words * 4, c->stream));
   CKR(ensure(c, c->lr_list, ((size_t)n / (ECB_MAX_READ_ALIGNMENTS + 1) + 1) * sizeof(uint2)));
 
+  // room for one row entry per alignment of this push: the rows of its new ECs come from distinct reads
+  const u64 arena_bound = c->arena_used + (u64)n;
+  if (arena_bound > 0xFFFFFFFFull) return fail(c, ECB_ERR_LIMIT, "row arena exceeds 2^32 entries");
+  CKR(ensure(c, c->arena, (size_t)arena_bound * sizeof(uint2), true));
+
   const u32 e_before = c->n_ec;
   CKR(group_prepare_launch(c));
   int grid = 1, chunk_len = 32;
@@ -868,8 +875,19 @@ static int push_one(ecb_ctx* c, const int32_t* read_group, const int32_t* target
   else ecb_group_insert_kernel<false><<<grid, ECB_GTHREADS, sizeof(GroupSmem), c->stream>>>(P);
   LAUNCH_CHECK("group_insert");
   CK(cudaEventRecord(c->ev[2], c->stream));
+  // the rows of the ECs the grouping kernel claimed, before the host has seen the counters: the harvest reads only
+  // ec_rep / ec_len of claimed ECs, which lie inside this push, also when the kernel set a device error
+  CK(cudaEventRecord(c->ev[3], c->stream));
+  CKR(harvest_new_rows(c, rg, tg, hp, n, e_before));
+  CK(cudaEventRecord(c->ev[4], c->stream));
+  CK(cudaEventRecord(c->ev[7], c->stream));   // the end of the push, unless more work follows below
+  // the push's round trip: new-EC count, table overflow, deferred reads, device errors, the arena cursor
   CKR(sync_counters(c));
   CKR(check_device_error(c));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, c->ev[1], c->ev[2])); c->stats.group_ms = ms;
+  CK(cudaEventElapsedTime(&ms, c->ev[3], c->ev[4])); c->stats.harvest_ms = ms;
+  const u32 e_harvested = c->h_ctr->n_ec;   // where the harvest's range ended
   // reads longer than ECB_MAX_READ_ALIGNMENTS: the sort-based pass (only when the grouping kernel deferred some)
   const u32 n_def = c->h_ctr->n_deferred;
   LongParams L{};
@@ -917,15 +935,22 @@ static int push_one(ecb_ctx* c, const int32_t* read_group, const int32_t* target
   if (c->h_ctr->n_triple_overflow) return fail(c, ECB_ERR_LIMIT, "(file, EC, cell) table ran out of probes");
   c->n_ec = c->h_ctr->n_ec;
   c->n_triples = c->h_ctr->n_triples;
-  CK(cudaEventRecord(c->ev[3], c->stream));
-  CKR(harvest_new_rows(c, rg, tg, hp, n, e_before, c->n_ec));
-  CK(cudaEventRecord(c->ev[4], c->stream));
+  // a push without replay, long reads or verification ends here: nothing was enqueued after the round trip above,
+  // so the caller's buffers are free and the counters are current
+  const bool more = c->n_ec > e_harvested || n_def || c->verify_keys;
+  float replay_harvest_ms = 0;
+  if (c->n_ec > e_harvested) {   // ECs claimed by the replay or the deferred long-read pass
+    CK(cudaEventRecord(c->ev[3], c->stream));
+    CKR(harvest_new_rows(c, rg, tg, hp, n, e_harvested));
+    CK(cudaEventRecord(c->ev[4], c->stream));
+  }
   if (n_def) {
     CK(cudaEventRecord(c->ev[5], c->stream));
     CKR(long_rows(c, L));
     CK(cudaEventRecord(c->ev[6], c->stream));
     CK(cudaMemsetAsync(&c->d_ctr->n_deferred, 0, sizeof(u32), c->stream));   // the list is empty for the next push
   }
+  if (more) CK(cudaEventRecord(c->ev[7], c->stream));
   if (c->verify_keys) {
     VerifyParams V{};
     V.rg = rg; V.tg = tg; V.hp = hp; V.n = (int)n; V.drop_last = drop_last_group;
@@ -938,14 +963,16 @@ static int push_one(ecb_ctx* c, const int32_t* read_group, const int32_t* target
     ecb_verify_kernel<<<grid_for((u64)n, 256, c->sm_count * 16), 256, 0, c->stream>>>(V);
     LAUNCH_CHECK("verify");
   }
-  // the push ends with its second (and last) host round trip: the caller's buffers are free again, the
-  // counters (arena cursor, device-side errors of the harvest / verification) are current on the host
-  CKR(sync_counters(c));
-  CKR(check_device_error(c));
-  float ms = 0;
-  CK(cudaEventElapsedTime(&ms, c->ev[1], c->ev[2])); c->stats.group_ms = ms;
-  CK(cudaEventElapsedTime(&ms, c->ev[3], c->ev[4])); c->stats.harvest_ms = ms;
-  CK(cudaEventElapsedTime(&ms, c->ev[0], n_def ? c->ev[6] : c->ev[4])); c->stats.push_ms = ms;
+  if (more) {   // a second round trip: the caller's buffers are free again, the counters (arena cursor, device-side
+                // errors of the replay's harvest, the long-read rows and the verification) are current on the host
+    CKR(sync_counters(c));
+    CKR(check_device_error(c));
+  }
+  if (c->n_ec > e_harvested) {
+    CK(cudaEventElapsedTime(&replay_harvest_ms, c->ev[3], c->ev[4]));
+    c->stats.harvest_ms += replay_harvest_ms;
+  }
+  CK(cudaEventElapsedTime(&ms, c->ev[0], c->ev[7])); c->stats.push_ms = ms;
   if (n_def) {
     CK(cudaEventElapsedTime(&ms, c->ev[5], c->ev[6]));
     c->stats.long_reads += n_def;
@@ -1063,11 +1090,8 @@ static int finalize(ecb_ctx* c, int64_t min_cell_count, bool samples, ecb_result
   F.word_rank = (const u32*)c->word_rank.p;
   F.first_rel = (u64*)c->first_rel.p;
   F.ecid_of = (u32*)c->ecid_of.p;
-  F.wide_count = &c->d_ctr->scratch[2];
-  F.wide_list = (u32*)c->long_list.p;
   CKR(ensure(c, c->count_of, (size_t)n_prov * 4));
   F.count_of = (u32*)c->count_of.p;
-  CK(cudaMemsetAsync(&c->d_ctr->scratch[2], 0, sizeof(u32), c->stream));
 
   CellResult cr{};
   if (c->with_cells) {
@@ -1092,40 +1116,40 @@ static int finalize(ecb_ctx* c, int64_t min_cell_count, bool samples, ecb_result
   if (E + 1 > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "more than 2^31 equivalence classes");
 
   CKR(ensure(c, c->r_a_indptr, (E + 1) * 4));
+  CKR(ensure(c, c->prov_of, E * 4));
   F.a_indptr = (int32_t*)c->r_a_indptr.p;
-  if (!c->with_cells && !samples) {
+  F.prov_of = (u32*)c->prov_of.p;
+  F.n_final = (u32)E;
+  const bool single = !c->with_cells && !samples;
+  if (single) {
     CKR(ensure(c, c->r_n_indptr, 2 * 4));
     CKR(ensure(c, c->r_n_indices, E * 4));
     CKR(ensure(c, c->r_n_data, E * 4));
+    F.n_indptr = (int32_t*)c->r_n_indptr.p;
     F.n_indices = (int32_t*)c->r_n_indices.p;
     F.n_data = (int32_t*)c->r_n_data.p;
   }
-  CK(cudaMemsetAsync((int32_t*)c->r_a_indptr.p + E, 0, 4, c->stream));
-  if (c->with_cells || samples) ecb_fin_rank_kernel<false><<<g_ec, 256, 0, c->stream>>>(F);
-  else ecb_fin_rank_kernel<true><<<g_ec, 256, 0, c->stream>>>(F);
+  ecb_fin_rank_kernel<<<g_ec, 256, 0, c->stream>>>(F);
   LAUNCH_CHECK("fin_rank");
-  // row lengths -> indptr; the rows follow at once: the arena's fill (known on the host since the last push)
+  // rows in id order, indptr scanned in the same pass; the arena's fill (known on the host since the last push)
   // bounds the number of non-zeros, so the result arrays need not wait for the exact figure
-  CKR(device_scan<false>(c, (const u32*)c->r_a_indptr.p, (u32*)c->r_a_indptr.p, E + 1, 0, nullptr));
-  CK(cudaMemcpyAsync(c->h_total, scan_total(c, E + 1), sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
-  c->stats.d2h_bytes += 2 * sizeof(u64);
   const u64 z_bound = std::max<u64>(c->arena_used, 1);
   if (z_bound > 0x7FFFFFFFull) return fail(c, ECB_ERR_LIMIT, "A matrix may have more than 2^31-1 non-zeros");
   CKR(ensure(c, c->r_a_indices, z_bound * 4));
   CKR(ensure(c, c->r_a_data, z_bound * 4));
   F.a_indices = (int32_t*)c->r_a_indices.p;
   F.a_data = (int32_t*)c->r_a_data.p;
-  ecb_fin_rows_kernel<<<grid_for(n_prov, 256, c->sm_count * 16), 256, 0, c->stream>>>(F);
-  LAUNCH_CHECK("fin_rows");
-  ecb_fin_rows_long_kernel<<<c->sm_count * 8, 256, 0, c->stream>>>(F, (const u32*)c->long_list.p, 0xFFFFFFFFu);   // (count on the device)
-  LAUNCH_CHECK("fin_rows_long");
+  F.z_cap = z_bound;
+  F.n_tiles = (u32)((E + FIN_EMIT_TILE - 1) / FIN_EMIT_TILE);
+  CKR(scan_state(c, F.n_tiles, &F.scan_state));
+  if (single) ecb_fin_emit_kernel<true><<<F.n_tiles, FIN_EMIT_THREADS, 0, c->stream>>>(F);
+  else ecb_fin_emit_kernel<false><<<F.n_tiles, FIN_EMIT_THREADS, 0, c->stream>>>(F);
+  LAUNCH_CHECK("fin_emit");
+  CK(cudaMemcpyAsync(c->h_total, F.scan_state + F.n_tiles + 1, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+  c->stats.d2h_bytes += 2 * sizeof(u64);
   CellResult cr2 = cr;
   if (c->with_cells) CKR(cells_emit(c, &cr2, (const u32*)c->ecid_of.p, E));   // N matrix as CSC
   else if (samples) CKR(samples_emit(c, E));
-  else {
-    ecb_set_pair_kernel<<<1, 1, 0, c->stream>>>((int32_t*)c->r_n_indptr.p, 0, (int32_t)E);
-    LAUNCH_CHECK("set_pair");
-  }
   CKR(sync_counters(c));   // the round trip of this call: non-zeros, first-occurrence bits, device-side errors
   CKR(check_device_error(c));
   const u64 Z = *c->h_total;
@@ -2134,7 +2158,7 @@ int ecb_destroy(ecb_ctx* c) {
   DevBuf* bufs[] = {&c->table, &c->ec_slot, &c->ec_rep, &c->ec_len, &c->spill, &c->row_len, &c->row_off, &c->arena, &c->long_list, &c->mid_list, &c->big_list, &c->count_of,
                     &c->ttable, &c->st_rg, &c->st_tg, &c->st_hp, &c->st_cell, &c->st2_rg, &c->st2_tg, &c->st2_hp, &c->st2_cell,
                     &c->overflow_bits, &c->lr_list, &c->lr_meta, &c->lr_rank, &c->lr_acc,
-                    &c->scan_partials, &c->bitmap, &c->word_rank, &c->first_rel, &c->ecid_of, &c->ec_keep,
+                    &c->scan_buf, &c->bitmap, &c->word_rank, &c->first_rel, &c->ecid_of, &c->prov_of, &c->ec_keep,
                     &c->r_a_indptr, &c->r_a_indices, &c->r_a_data, &c->r_n_indptr, &c->r_n_indices,
                     &c->r_n_data, &c->r_cell_order, &c->cx_kept, &c->cx_col_of_cell, &c->cx_col_counts,
                     &c->smp_last, &c->smp_pairs, &c->ecr_acc, &c->ecr_slot, &c->ecr_ec, &c->ecr_dst, &c->ecr_flag,

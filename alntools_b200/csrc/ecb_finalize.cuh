@@ -3,10 +3,17 @@
 // Replaces the id half of alntools/bam_utils.py:693-698 (ec_idx[k] = len(ec_idx): EC id = rank of the
 // key's first occurrence) without a sort: every kept EC sets the bit of its first-occurrence position
 // in a bitmap over the pushed alignment range, a device-wide scan of the word popcounts ranks the
-// bits, and the rank IS the EC id.  Then alntools/bam_utils.py:827-847 + bin_utils.py:208-232:
-// row lengths -> exclusive scan -> a_indptr, rows copied from the arena, counts scattered.
+// bits, and the rank IS the EC id.  Then alntools/bam_utils.py:827-847 + bin_utils.py:208-232 in one
+// pass in EC-id order (ecb_fin_emit_kernel): row lengths -> exclusive scan -> a_indptr, rows copied from
+// the arena, counts.
+//   mark   provisional order: first position and count out of the table, the bitmap bit
+//   rank   provisional order: id = bitmap rank; ecid_of[e] = id and the one scatter prov_of[id] = e
+//   emit   id order, in tiles of FIN_EMIT_TILE ids: the row lengths scanned with the look-back of
+//          ecb_scan.cuh, a_indptr / N written coalesced, the tile's rows copied to their contiguous
+//          output range with coalesced stores
 #pragma once
 #include "ecb_common.cuh"
+#include "ecb_scan.cuh"
 
 struct FinalizeParams {
   const EcbEntry* table;
@@ -21,14 +28,19 @@ struct FinalizeParams {
   const u32* word_rank;
   u64* first_rel;       // [n_ec]
   u32* ecid_of;         // [n_ec] final id or ECB_NONE
-  int32_t* a_indptr;    // [E+1] holds row lengths before the scan
+  u32* prov_of;         // [E] provisional id of every final id
+  u32 n_final;          // E
+  int32_t* a_indptr;    // [E+1]
   int32_t* a_indices;
   int32_t* a_data;
   int32_t* n_indices;   // single-sample N matrix
   int32_t* n_data;
-  u32* wide_count;      // number of rows with more than 8 entries ...
-  u32* wide_list;       // ... and their provisional ids
+  int32_t* n_indptr;    // single-sample N matrix: the pair (0, E)
   u32* count_of;        // [n_ec] reads per EC (copied out of the table by the mark kernel)
+  u64* scan_state;      // look-back state of the emit pass (ecb_scan.cuh); the total of the row lengths lands
+                        // after the status words
+  u32 n_tiles;          // emit tiles
+  u64 z_cap;            // room in a_indices / a_data
 };
 
 __global__ void __launch_bounds__(256) ecb_fin_mark_kernel(const FinalizeParams P) {
@@ -41,23 +53,9 @@ __global__ void __launch_bounds__(256) ecb_fin_mark_kernel(const FinalizeParams 
   }
 }
 
-__device__ __forceinline__ void fin_warp_append(u32* list, u32* counter, bool take, u32 item) {
-  const u32 act = __activemask();
-  const u32 m = __ballot_sync(act, take);
-  if (!m) return;
-  const int lane = threadIdx.x & 31;
-  const int leader = __ffs(m) - 1;
-  u32 base = 0;
-  if (lane == leader) base = atomicAdd(counter, (u32)__popc(m));
-  base = __shfl_sync(act, base, leader);
-  if (take) list[base + (u32)__popc(m & ((1u << lane) - 1u))] = item;
-}
-
-template <bool SINGLE_SAMPLE>
 __global__ void __launch_bounds__(256) ecb_fin_rank_kernel(const FinalizeParams P) {
   for (u32 e = blockIdx.x * blockDim.x + threadIdx.x; e < P.n_ec; e += gridDim.x * blockDim.x) {
     const bool kept = P.ec_keep == nullptr || P.ec_keep[e];
-    if (P.wide_list) fin_warp_append(P.wide_list, P.wide_count, kept && P.row_len[e] > 8, e);
     if (!kept) {
       P.ecid_of[e] = ECB_NONE;
       continue;
@@ -66,59 +64,116 @@ __global__ void __launch_bounds__(256) ecb_fin_rank_kernel(const FinalizeParams 
     const u32 w = (u32)(rel >> 5), b = (u32)(rel & 31);
     const u32 id = P.word_rank[w] + __popc(P.bitmap[w] & ((1u << b) - 1u));
     P.ecid_of[e] = id;
-    const u32 len = P.row_len[e];
-    if (P.a_indptr == nullptr) continue;   // ids only (slice assembly)
-    P.a_indptr[id] = (int32_t)len;
-    if (SINGLE_SAMPLE) {
-      P.n_indices[id] = (int32_t)id;
-      P.n_data[id] = (int32_t)P.count_of[e];
-    }
+    P.prov_of[id] = e;
   }
 }
 
-// Copy rows from the arena to their CSR position.  Rows of up to 8 entries (the bulk): one thread per
-// EC; longer rows: one warp per EC (second launch, only when such rows exist).
-__global__ void __launch_bounds__(256) ecb_fin_rows_kernel(const FinalizeParams P) {
-  for (u32 e = blockIdx.x * blockDim.x + threadIdx.x; e < P.n_ec; e += gridDim.x * blockDim.x) {
-    const u32 id = P.ecid_of[e];
-    if (id == ECB_NONE) continue;
-    const u32 len = P.row_len[e];
-    if (len > 8) continue;
-    const uint2* src = P.arena + P.row_off[e];
-    const size_t dst = (size_t)P.a_indptr[id];
-    for (u32 j = 0; j < len; ++j) {
-      const uint2 v = src[j];
-      P.a_indices[dst + j] = (int32_t)v.x;
-      P.a_data[dst + j] = (int32_t)v.y;
+#define FIN_EMIT_THREADS 256
+#define FIN_EMIT_ITEMS 4                                        // consecutive ids per thread
+#define FIN_EMIT_TILE (FIN_EMIT_THREADS * FIN_EMIT_ITEMS)
+#define FIN_EMIT_WARP_ROWS (32 * FIN_EMIT_ITEMS)
+
+// One tile of FIN_EMIT_TILE final ids per CTA (tiles drawn from the ticket of the look-back state).  Thread t
+// owns ids 4t..4t+3 of the tile, so warp w owns the rows of 128 consecutive ids, which fill one contiguous
+// range of the output.  The warp walks that range 32 entries at a time: entry j belongs to the first row whose
+// end (tile-relative, in shared memory) is beyond j - a search over the warp's 128 row ends - so reads of the
+// arena are one row segment per lane group and the stores are coalesced, for rows of any length.
+template <bool SINGLE_SAMPLE>
+__global__ void __launch_bounds__(FIN_EMIT_THREADS) ecb_fin_emit_kernel(const FinalizeParams P) {
+  __shared__ u32 s_end[FIN_EMIT_TILE];   // tile-relative end of every row
+  __shared__ u32 s_src[FIN_EMIT_TILE];   // its arena offset
+  __shared__ u32 s_scan[9];
+  __shared__ u32 s_tile;
+  __shared__ u64 s_prefix;
+  const u32 tile = scan_take_tile(P.scan_state, &s_tile);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const u32 E = P.n_final;
+  const u32 id0 = tile * FIN_EMIT_TILE + threadIdx.x * FIN_EMIT_ITEMS;
+  const bool full = id0 + FIN_EMIT_ITEMS <= E;
+  u32 e[FIN_EMIT_ITEMS], len[FIN_EMIT_ITEMS], off[FIN_EMIT_ITEMS];
+  if (full) {
+    const uint4 q = *(const uint4*)(P.prov_of + id0);
+    e[0] = q.x; e[1] = q.y; e[2] = q.z; e[3] = q.w;
+  } else {
+#pragma unroll
+    for (int i = 0; i < FIN_EMIT_ITEMS; ++i) e[i] = id0 + i < E ? P.prov_of[id0 + i] : ECB_NONE;
+  }
+  u32 sum = 0;
+#pragma unroll
+  for (int i = 0; i < FIN_EMIT_ITEMS; ++i) {
+    len[i] = 0;
+    off[i] = 0;
+    if (e[i] < P.n_ec) {   // (an id no EC took - only when order_base ranges overlapped, which the host then
+                           // reports - may hold a stale entry: bounded here, and the stores below by z_cap)
+      len[i] = P.row_len[e[i]];
+      off[i] = P.row_off[e[i]];
+    }
+    sum += len[i];
+  }
+  if (SINGLE_SAMPLE) {
+    u32 cnt[FIN_EMIT_ITEMS];
+#pragma unroll
+    for (int i = 0; i < FIN_EMIT_ITEMS; ++i) cnt[i] = e[i] < P.n_ec ? P.count_of[e[i]] : 0u;
+    if (full) {
+      *(int4*)(P.n_indices + id0) = make_int4((int)id0, (int)id0 + 1, (int)id0 + 2, (int)id0 + 3);
+      *(int4*)(P.n_data + id0) = make_int4((int)cnt[0], (int)cnt[1], (int)cnt[2], (int)cnt[3]);
+    } else {
+#pragma unroll
+      for (int i = 0; i < FIN_EMIT_ITEMS; ++i)
+        if (id0 + i < E) {
+          P.n_indices[id0 + i] = (int32_t)(id0 + i);
+          P.n_data[id0 + i] = (int32_t)cnt[i];
+        }
     }
   }
-}
-
-// Rows with more than 8 entries: one warp per row.  With a list (n_wide entries of P.wide_list; 0xFFFFFFFF =
-// as many as *P.wide_count says) only those rows are visited; without one (list == NULL) every EC is looked at.
-__global__ void __launch_bounds__(256) ecb_fin_rows_long_kernel(const FinalizeParams P, const u32* list, u32 n_wide) {
-  const int lane = threadIdx.x & 31;
-  const u32 warp_global = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const u32 n_warps = (gridDim.x * blockDim.x) >> 5;
-  if (n_wide == 0xFFFFFFFFu) n_wide = *P.wide_count;   // the list was counted on the device (same stream, earlier launch)
-  const u32 n_items = list ? n_wide : P.n_ec;
-  for (u32 i = warp_global; i < n_items; i += n_warps) {
-    const u32 e = list ? list[i] : i;
-    const u32 len = P.row_len[e];
-    if (len <= 8) continue;
-    const u32 id = P.ecid_of[e];
-    if (id == ECB_NONE) continue;
-    const size_t src = P.row_off[e];
-    const size_t dst = (size_t)P.a_indptr[id];
-    for (u32 j = lane; j < len; j += 32) {
-      const uint2 v = P.arena[src + j];
-      P.a_indices[dst + j] = (int32_t)v.x;
-      P.a_data[dst + j] = (int32_t)v.y;
+  u32 tile_total;
+  const u32 excl = block_excl_scan_u32(sum, s_scan, tile_total);
+  if (warp == 0) {
+    const u64 p = scan_lookback(P.scan_state, tile, tile_total);
+    if (lane == 0) {
+      s_prefix = p;
+      if (tile == P.n_tiles - 1) {
+        const u64 z = p + tile_total;
+        P.scan_state[P.n_tiles + 1] = z;
+        P.a_indptr[E] = (int32_t)(u32)z;
+        if (SINGLE_SAMPLE) {
+          P.n_indptr[0] = 0;
+          P.n_indptr[1] = (int32_t)E;
+        }
+      }
     }
   }
-}
-
-__global__ void ecb_set_pair_kernel(int32_t* p, int32_t a, int32_t b) {
-  p[0] = a;
-  p[1] = b;
+  __syncthreads();
+  const u64 prefix = s_prefix;
+  u32 run = excl, ptr[FIN_EMIT_ITEMS];
+#pragma unroll
+  for (int i = 0; i < FIN_EMIT_ITEMS; ++i) {
+    ptr[i] = (u32)prefix + run;
+    run += len[i];
+    s_end[threadIdx.x * FIN_EMIT_ITEMS + i] = run;
+    s_src[threadIdx.x * FIN_EMIT_ITEMS + i] = off[i];
+  }
+  if (full) {
+    *(int4*)(P.a_indptr + id0) = make_int4((int)ptr[0], (int)ptr[1], (int)ptr[2], (int)ptr[3]);
+  } else {
+#pragma unroll
+    for (int i = 0; i < FIN_EMIT_ITEMS; ++i)
+      if (id0 + i < E) P.a_indptr[id0 + i] = (int32_t)ptr[i];
+  }
+  __syncwarp();   // the warp reads only the row ends its own lanes wrote
+  const u32 r0 = warp * FIN_EMIT_WARP_ROWS;
+  const u32 w_beg = __shfl_sync(ECB_FULL, excl, 0), w_end = __shfl_sync(ECB_FULL, run, 31);
+  for (u32 j = w_beg + lane; j < w_end; j += 32) {
+    u32 lo = r0, hi = r0 + FIN_EMIT_WARP_ROWS - 1;   // first row whose end is beyond j (one exists: w_end > j)
+    while (lo < hi) {
+      const u32 mid = (lo + hi) >> 1;
+      if (s_end[mid] > j) hi = mid; else lo = mid + 1;
+    }
+    const u32 start = lo == r0 ? w_beg : s_end[lo - 1];
+    const uint2 v = P.arena[(size_t)s_src[lo] + (j - start)];
+    const size_t dst = prefix + j;
+    if (dst >= P.z_cap) break;
+    P.a_indices[dst] = (int32_t)v.x;
+    P.a_data[dst] = (int32_t)v.y;
+  }
 }

@@ -3,8 +3,9 @@
 //
 // Replaces alntools/bam_utils.py:788-825 (EC key -> per-haplotype (ec, target) COO lists) and the
 // canonicalisation scipy performs in alntools/bin_utils.py:208-211 (sum of 2^h * data[h], tocsr()
-// with sorted column indices).  Runs at the end of every push, while the caller's columns are still
-// valid, over the ECs claimed in that push only (E rows, not R reads).  The grouping kernel recorded
+// with sorted column indices).  Runs right after the grouping kernel of every push (and once more after a
+// replay, over the ECs the replay claimed), while the caller's columns are still valid, over the ECs claimed
+// in that push only (E rows, not R reads).  The grouping kernel recorded
 // for every new EC the offset and the length of one read with that key.  A row's place in the arena is
 // reserved when its length is known, with one atomic per warp (short reads) or per row (the rare long
 // ones) on the arena cursor: no scan, no host round trip; the host only provides room for one row entry
@@ -24,7 +25,8 @@ struct HarvestParams {
   int n;
   const u32* ec_rep;
   const u32* ec_len;
-  u32 e0, e1;        // provisional ids claimed in this push
+  u32 e0;            // first provisional id to harvest; the range ends at ctr->n_ec, read on the device, so
+                     // the harvest is launched right after the grouping kernel without a host round trip
   u32* row_len;      // [capacity] out: row length
   u32* row_off;      // [capacity] out: absolute offset inside the arena (reserved here)
   uint2* arena;      // (target, mask) pairs
@@ -75,7 +77,7 @@ __device__ __forceinline__ void warp_append(u32* list, u32* counter, bool take, 
 __global__ void __launch_bounds__(256) ecb_harvest_short_kernel(const HarvestParams P) {
   // whole CTAs walk the id range together (the reservation below is a CTA-wide step)
   __shared__ u32 s_scan[10];
-  const u32 n_new = P.e1 - P.e0;
+  const u32 n_new = P.ctr->n_ec - P.e0;   // (the ECs before e0 are never handed out again)
   const u32 stride = gridDim.x * blockDim.x;
   for (u32 i0 = blockIdx.x * blockDim.x; i0 < n_new; i0 += stride) {
     const u32 i = i0 + threadIdx.x;

@@ -1,6 +1,13 @@
-// ecb_scan.cuh — device-wide exclusive prefix sum over uint32 (three launches: block sums, scan of
-// the block sums by one CTA, block-local scan + offset).  Used for EC ranking (popcounts of the
-// first-occurrence bitmap), CSR row offsets and stream compaction.
+// ecb_scan.cuh — device-wide exclusive prefix sum over uint32 in ONE launch (decoupled look-back).  Used
+// for EC ranking (popcounts of the first-occurrence bitmap), CSR row offsets and stream compaction.
+//
+// Every CTA draws its tile from an atomic ticket (not blockIdx), scans the tile, publishes the tile's
+// aggregate in a status word, and one warp walks back over the status words of the tiles before it until it
+// meets an inclusive prefix.  A tile only ever waits on tiles whose CTAs have already started, so progress
+// does not depend on the order in which CTAs are scheduled.  The state (ticket + one status word per tile)
+// is cleared by a stream-ordered memset before each launch.  Status word: bits 63..62 the flag (0 not yet
+// published, 1 aggregate, 2 inclusive prefix), bits 61..0 the value; a tile's aggregate is the u32 sum of its
+// items (as the sums were before), prefixes are u64.
 #pragma once
 #include "ecb_common.cuh"
 
@@ -46,64 +53,59 @@ __device__ __forceinline__ u32 block_excl_scan_u32(u32 v, u32* smem, u32& total)
   return res;
 }
 
-// in may be a u32 array (POPC=false) or a bitmap whose popcounts are scanned (POPC=true).
-template <bool POPC>
-__global__ void __launch_bounds__(SCAN_THREADS) scan_block_sums_kernel(const u32* __restrict__ in, u64 n,
-                                                                        u64* __restrict__ block_sums) {
-  __shared__ u32 sm[9];
-  const u64 base = (u64)blockIdx.x * SCAN_BLOCK;
-  u32 s = 0;
-#pragma unroll
-  for (int i = 0; i < SCAN_ITEMS; ++i) {
-    u64 idx = base + (u64)i * SCAN_THREADS + threadIdx.x;
-    if (idx < n) {
-      u32 v = in[idx];
-      s += POPC ? (u32)__popc(v) : v;
-    }
-  }
-  u32 total;
-  block_excl_scan_u32(s, sm, total);
-  if (threadIdx.x == 0) block_sums[blockIdx.x] = total;
-}
+#define SCAN_FLAG_AGG (1ull << 62)
+#define SCAN_FLAG_INC (2ull << 62)
+#define SCAN_VALUE_MASK ((1ull << 62) - 1ull)
 
-// One CTA turns block_sums into exclusive offsets in place; total -> *total_out.
-__global__ void __launch_bounds__(1024) scan_partials_kernel(u64* __restrict__ block_sums, u32 n_blocks,
-                                                             u64* __restrict__ total_out) {
-  __shared__ u64 warp_tot[32];
-  __shared__ u64 carry_s;
-  __shared__ u64 chunk_total;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (threadIdx.x == 0) carry_s = 0;
+// Scan state: word 0 the tile ticket, words 1..n_tiles the status words, word n_tiles + 1 the total.
+__device__ __forceinline__ u32 scan_take_tile(u64* state, u32* s_tile) {
+  if (threadIdx.x == 0) *s_tile = atomicAdd((unsigned int*)state, 1u);
   __syncthreads();
-  for (u32 start = 0; start < n_blocks; start += 1024) {
-    u32 idx = start + threadIdx.x;
-    u64 v = idx < n_blocks ? block_sums[idx] : 0ull;
-    u64 inc = warp_incl_scan_u64(v, lane);
-    if (lane == 31) warp_tot[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {
-      u64 w = warp_tot[lane];
-      u64 winc = warp_incl_scan_u64(w, lane);
-      warp_tot[lane] = winc - w;
-      if (lane == 31) chunk_total = winc;
-    }
-    __syncthreads();
-    u64 excl = carry_s + warp_tot[warp] + inc - v;
-    if (idx < n_blocks) block_sums[idx] = excl;
-    __syncthreads();
-    if (threadIdx.x == 0) carry_s += chunk_total;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) *total_out = carry_s;
+  return *s_tile;
 }
 
+// Called by ONE whole warp: publishes the tile's aggregate, looks back for the exclusive prefix of the tile,
+// publishes the inclusive prefix and returns the exclusive one (on every lane).
+__device__ __forceinline__ u64 scan_lookback(u64* state, u32 tile, u64 aggregate) {
+  volatile u64* status = (volatile u64*)(state + 1);
+  const int lane = threadIdx.x & 31;
+  if (tile == 0) {
+    if (lane == 0) status[0] = SCAN_FLAG_INC | aggregate;
+    return 0;
+  }
+  if (lane == 0) status[tile] = SCAN_FLAG_AGG | aggregate;
+  u64 excl = 0;
+  long long top = (long long)tile - 1;   // the 32 tiles top, top-1, ... are looked at together
+  while (true) {
+    const long long idx = top - lane;
+    u64 s;
+    do {
+      s = idx >= 0 ? status[idx] : SCAN_FLAG_INC;
+    } while (__any_sync(ECB_FULL, (s >> 62) == 0ull));
+    const u32 inc = __ballot_sync(ECB_FULL, (s >> 62) == 2ull);
+    const int stop = inc ? __ffs(inc) - 1 : 31;   // the nearest tile with an inclusive prefix ends the walk
+    u64 v = lane <= stop ? (s & SCAN_VALUE_MASK) : 0ull;
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(ECB_FULL, v, d);
+    excl += v;
+    if (inc) break;
+    top -= 32;
+  }
+  if (lane == 0) status[tile] = SCAN_FLAG_INC | ((excl + aggregate) & SCAN_VALUE_MASK);
+  return excl;
+}
+
+// in may be a u32 array (POPC=false) or a bitmap whose popcounts are scanned (POPC=true); in may alias out.
+// The last tile writes the total to state[n_tiles + 1].
 template <bool POPC>
-__global__ void __launch_bounds__(SCAN_THREADS) scan_apply_kernel(const u32* __restrict__ in, u64 n,
-                                                                   const u64* __restrict__ block_offsets,
-                                                                   u32* __restrict__ out, u32 base_offset) {
+__global__ void __launch_bounds__(SCAN_THREADS) scan_kernel(const u32* in, u64 n, u32* out, u32 base_offset,
+                                                            u64* __restrict__ state, u32 n_tiles) {
   __shared__ u32 sm[9];
+  __shared__ u32 s_tile;
+  __shared__ u64 s_prefix;
+  const u32 tile = scan_take_tile(state, &s_tile);
   // blocked arrangement: thread t owns SCAN_ITEMS consecutive elements
-  const u64 base = (u64)blockIdx.x * SCAN_BLOCK + (u64)threadIdx.x * SCAN_ITEMS;
+  const u64 base = (u64)tile * SCAN_BLOCK + (u64)threadIdx.x * SCAN_ITEMS;
   u32 v[SCAN_ITEMS];
   u32 s = 0;
 #pragma unroll
@@ -119,7 +121,15 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_apply_kernel(const u32* __r
   }
   u32 total;
   u32 excl = block_excl_scan_u32(s, sm, total);
-  u32 run = base_offset + (u32)block_offsets[blockIdx.x] + excl;
+  if (threadIdx.x < 32) {
+    const u64 p = scan_lookback(state, tile, total);
+    if (threadIdx.x == 0) {
+      s_prefix = p;
+      if (tile == n_tiles - 1) state[n_tiles + 1] = p + total;
+    }
+  }
+  __syncthreads();
+  u32 run = base_offset + (u32)s_prefix + excl;
 #pragma unroll
   for (int i = 0; i < SCAN_ITEMS; ++i) {
     u64 idx = base + i;
